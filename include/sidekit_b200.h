@@ -174,6 +174,18 @@ int skb_score_gemm_trials_packed(const float* E_dev, int Ne, const skb_packed_t*
                                  double cst, double alpha, int passes, const skb_trial_index_t* trials, float* out_trials_dev,
                                  void* stream);
 
+/* Top-k mode.  Per row i of S (same formula and arguments as skb_score_gemm_trials): the k largest S[i][j], ordered by score
+ * descending, ties by lower j.  values (Ne, k) float32, indices (Ne, k) int64, device.  1 <= k <= min(Nt, 1024).  Each value
+ * equals the skb_score_gemm entry of the same arguments bit for bit.  k <= 32 with D <= 256 selects inside the GEMM epilogue
+ * (the Ne x Nt matrix never reaches memory); larger k or D scores row panels into a bounded scratch matrix and selects per
+ * row.  The order of NaN scores is undefined (finite embeddings do not produce them). */
+int skb_score_gemm_topk(const float* E_dev, const float* T_dev, int Ne, int Nt, int D, const float* rowterm_dev,
+                        const float* colterm_dev, double cst, double alpha, int passes, int k, float* values_dev,
+                        int64_t* indices_dev, void* stream);
+int skb_score_gemm_topk_packed(const float* E_dev, int Ne, const skb_packed_t* T, const float* rowterm_dev,
+                               const float* colterm_dev, double cst, double alpha, int passes, int k, float* values_dev,
+                               int64_t* indices_dev, void* stream);
+
 /* dst[i] = (double)src[i]: the float64 view of a float32 score matrix, produced chunk by chunk on its way to the host
  * (sidekit's PLDA / two-covariance scorers return float64, iv_scoring.py:205, :462). */
 int skb_widen_f32_f64(const float* src_dev, double* dst_dev, int64_t n, void* stream);

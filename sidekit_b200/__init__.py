@@ -13,6 +13,7 @@ from .nnet.xsets import IdMap, IdMapSet
 from .bosaris import Ndx, Scores, Key
 from .statserver import StatServer
 from .iv_scoring import cosine_scoring, PLDA_scoring, fast_PLDA_scoring, full_PLDA_scoring, two_covariance_scoring, mahalanobis_scoring, score_matrix
+from .iv_scoring import score_topk, cosine_topk, PLDA_topk, TopK
 from .score_normalization import asnorm, znorm, tnorm, ztnorm
 from . import detplot
 from .detplot import pavx, rocch, rocch2eer, fast_minDCF, eer

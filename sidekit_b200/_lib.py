@@ -66,6 +66,8 @@ def _declare(lib):
         "skb_trial_index_destroy": (None, [vp]),
         "skb_score_gemm_trials": (i32, [vp, vp, i32, i32, i32, vp, vp, f64, f64, i32, vp, vp, vp]),
         "skb_score_gemm_trials_packed": (i32, [vp, i32, vp, vp, vp, f64, f64, i32, vp, vp, vp]),
+        "skb_score_gemm_topk": (i32, [vp, vp, i32, i32, i32, vp, vp, f64, f64, i32, i32, vp, vp, vp]),
+        "skb_score_gemm_topk_packed": (i32, [vp, i32, vp, vp, vp, f64, f64, i32, i32, vp, vp, vp]),
         "skb_widen_f32_f64": (i32, [vp, vp, i64, vp]),
         "skb_quadratic_prepare": (i32, [vp, vp, vp, vp, i32, i32, vp, vp, vp]),
         "skb_asnorm_stats": (i32, [vp, vp, i32, i32, i32, i32, vp, vp, vp]),

@@ -241,3 +241,43 @@ def asnorm_sharded(enrol_xv, cohort_xv, topk=200, stats_fn=_asnorm_stats_cuda, p
     mean, std = mean[:N].contiguous(), std[:N].contiguous()
     panel = panel_fn(X, lo, hi, mean, std) if hi > lo else torch.zeros((0, N), dtype=torch.float32, device=X.device)
     return lo, hi, panel
+
+
+def _topk_cuda(queries, gallery, k, passes):
+    from .iv_scoring import PackedEmbeddings, score_topk
+    G = gallery if isinstance(gallery, PackedEmbeddings) else PackedEmbeddings(gallery.to(queries.device, torch.float32))
+    return score_topk(queries, G, k, passes=passes)
+
+
+def topk_sharded(queries, gallery, k, passes=3, topk_fn=_topk_cuda):
+    """The ``k`` best gallery rows of every query across ranks: each rank scores ITS query rows (``row_panel``) against the
+    gallery (packed once per call, or passed as a ``PackedEmbeddings``), and ONE ``all_gather_into_tensor`` of values +
+    indices gives every rank the full ``(values (N, k) float32, indices (N, k) int64)``.
+
+    ``passes`` is fixed (1 or 3), not decided from the operands: with ``passes=0`` a rank's pass count and operand scale
+    would follow its own panel's statistics, so the result would depend on the number of ranks.  With a fixed count the
+    rows of rank r equal ``topk_fn`` on that rank's panel.  ``topk_fn(queries, gallery, k, passes) -> (values, indices)`` is
+    ``score_topk`` in production and injectable so the exchange can be tested on CPU."""
+    if passes not in (1, 3):
+        raise ValueError("topk_sharded needs a fixed pass count (1 or 3), got %r" % (passes,))
+    dist, rank, world = _dist()
+    Q = queries.to(torch.float32).contiguous()
+    N = Q.shape[0]
+    lo, hi = row_panel(N, rank, world)
+    if hi > lo:
+        values, indices = topk_fn(Q[lo:hi].contiguous(), gallery, k, passes)
+    else:
+        values = torch.zeros((0, k), dtype=torch.float32, device=Q.device)
+        indices = torch.zeros((0, k), dtype=torch.int64, device=Q.device)
+    if world == 1:
+        return values, indices
+    # one collective: the float32 value bits ride in int64 next to the indices, padded to the panel size
+    per = (N + world - 1) // world
+    dev = _collective_device() or Q.device
+    block = torch.zeros((per, 2 * k), dtype=torch.int64, device=dev)
+    block[: hi - lo, :k] = values.to(dev).contiguous().view(torch.int32).to(torch.int64)
+    block[: hi - lo, k:] = indices.to(dev)
+    gathered = torch.empty((world * per, 2 * k), dtype=torch.int64, device=dev)
+    dist.all_gather_into_tensor(gathered, block)
+    gathered = gathered[:N]
+    return gathered[:, :k].to(torch.int32).view(torch.float32).contiguous(), gathered[:, k:].contiguous()

@@ -209,9 +209,72 @@ struct ScoreParams {
     const uint32_t* word_off;
     int mask_ld;
     int tiles_total, n_ntiles;
+    // top-k mode (out_mode 4): every epilogue warp keeps the best topk_k (score, column) keys of each of its rows among the
+    // columns it visits and leaves them, when it moves off a row panel, in out = uint64 [Ne][topk_segs][topk_k] (see
+    // topk_segment); topk_merge_kernel selects the final k from those partial lists.
+    int topk_k, topk_segs;
 };
 
 struct TrialTables { const uint32_t* words; const uint32_t* offsets; int ld, Ne, Nt; };
+struct TopkLists { unsigned long long* keys; int k, segs; };
+
+// Epilogue modes of score_gemm_body: the (Ne, Nt) matrix (float32 / float64 / float16), the trials of a mask, or the k best
+// columns of every row.
+constexpr int kEpiMatrix = 0, kEpiTrials = 1, kEpiTopk = 2;
+
+// The CTA whose contiguous run of work items (score_gemm_body) contains item t, for `tiles` items over `grid` CTAs: the
+// largest b with floor(tiles * b / grid) <= t.
+__host__ __device__ __forceinline__ int score_cta_of(long long t, int tiles, int grid) {
+    return (int)(((t + 1) * grid + tiles - 1) / tiles) - 1;
+}
+// Top-k mode: the row panel's columns are split over the CTAs whose runs touch the panel and, inside a CTA, over the two
+// epilogue warps of a TMEM lane quadrant (64 columns of every tile each).  Partial list slot of (CTA, part) and the number of
+// slots of a panel -- both pure functions of the partition, so no atomics and a deterministic result.
+__host__ __device__ __forceinline__ int topk_first_cta(int panel, int n_ntiles, int tiles, int grid) {
+    return score_cta_of((long long)panel * n_ntiles, tiles, grid);
+}
+__host__ __device__ __forceinline__ int topk_panel_segs(int panel, int n_ntiles, int tiles, int grid) {
+    return 2 * (score_cta_of((long long)(panel + 1) * n_ntiles - 1, tiles, grid) - topk_first_cta(panel, n_ntiles, tiles, grid) + 1);
+}
+
+// 64-bit total order of the top-k selection: higher score first, lower column first among equal scores.  f2key maps finite
+// floats (and the infinities) order-preservingly onto non-zero 32-bit keys, so key 0 pads a list of fewer than k entries.
+__device__ __forceinline__ unsigned f2key(float f) {   // order-preserving float -> uint
+    const unsigned u = __float_as_uint(f);
+    return (u & 0x80000000u) ? ~u : (u | 0x80000000u);
+}
+__device__ __forceinline__ float key2f(unsigned k) {
+    const unsigned u = (k & 0x80000000u) ? (k & 0x7fffffffu) : ~k;
+    return __uint_as_float(u);
+}
+__device__ __forceinline__ unsigned long long topk_key(float s, int col) {
+    return ((unsigned long long)f2key(s) << 32) | (unsigned)~col;
+}
+// One lane's k best keys as a binary min-heap in a warp's [k][32] shared-memory lists (slot s of lane l at h[32 s + l]: the
+// lanes of a warp touch the same 256 bytes whatever slots they are at).  Replaces the root (the current k-th best) with a
+// larger key and restores the heap; returns the new root.  log2(k) levels instead of a rescan of all k slots.
+__device__ __forceinline__ unsigned long long topk_heap_replace(unsigned long long* h, int lane, int k, unsigned long long key) {
+    int i = 0;
+    for (;;) {
+        int c = 2 * i + 1;
+        if (c >= k) break;
+        unsigned long long kc = h[c * 32 + lane];
+        if (c + 1 < k) {
+            const unsigned long long kr = h[(c + 1) * 32 + lane];
+            if (kr < kc) { kc = kr; ++c; }
+        }
+        if (key <= kc) break;
+        h[i * 32 + lane] = kc;
+        i = c;
+    }
+    h[i * 32 + lane] = key;
+    return h[lane];
+}
+// the float threshold a score has to reach before its key is built and compared (-inf while the list has free slots)
+__device__ __forceinline__ float topk_screen(unsigned long long kth) {
+    const unsigned hi = (unsigned)(kth >> 32);
+    return hi ? key2f(hi) : -INFINITY;
+}
 
 constexpr int kScKChunk = 64;
 
@@ -265,7 +328,13 @@ struct ScoreSmem {
     __host__ __device__ static size_t a_bytes(int Dp) {
         return STREAM_A ? 0 : (kATmem ? (size_t)128 * kAPieceK * 2 : (size_t)MT * kParts * 128 * Dp * 2);
     }
-    static size_t total(int Dp) { return 256 + a_bytes(Dp) + (size_t)kBStages * kRingStageBytes + kEpiWarps * 32 * kStageRowBytes; }
+    // Epilogue region: the warps' [32][36] transpose buffers, or in top-k mode (topk_k > 0, lane = row: no transpose) the
+    // warps' [topk_k][32] lists of 64-bit keys in their place -- 64 KB at k = 32, which the KC 64 ring would not fit next to
+    // the 36 KB of buffers.
+    static size_t epi_bytes(int topk_k) {
+        return topk_k > 0 ? (size_t)kEpiWarps * 32 * topk_k * sizeof(unsigned long long) : (size_t)kEpiWarps * 32 * kStageRowBytes;
+    }
+    static size_t total(int Dp, int topk_k = 0) { return 256 + a_bytes(Dp) + (size_t)kBStages * kRingStageBytes + epi_bytes(topk_k); }
 };
 
 #ifdef SKB_SCORE_TIMING
@@ -280,10 +349,12 @@ __device__ unsigned long long g_score_t[16];
 #define SKB_TIMED_WAIT(i, stmt) stmt
 #endif
 
-template <int PASSES, bool STREAM_A, bool TRIALS, int MT, int KC = 64>
+template <int PASSES, bool STREAM_A, int MODE, int MT, int KC = 64>
 __device__ __forceinline__ void score_gemm_body(const ScoreParams& p) {
     using SM = ScoreSmem<PASSES, STREAM_A, MT, KC>;
     static_assert(MT == 1 || (PASSES == 1 && !STREAM_A), "two row panels per item: single-pass resident-panel variant only");
+    static_assert(MODE != kEpiTopk || (!STREAM_A && MT == 1 && SM::kEpiWarps == 8), "top-k mode: resident-panel variants, one row panel per item, 8 epilogue warps");
+    constexpr bool TRIALS = MODE == kEpiTrials, TOPK = MODE == kEpiTopk;
     extern __shared__ __align__(128) uint8_t smem[];
     uint64_t* a_full = reinterpret_cast<uint64_t*>(smem);
     uint64_t* a_empty = a_full + 1;
@@ -471,7 +542,14 @@ __device__ __forceinline__ void score_gemm_body(const ScoreParams& p) {
         const int part = (warp - 2) >> 2;                  // which NB of the four 32-column blocks
         float* stg = reinterpret_cast<float*>(stage_smem) + (warp - 2) * 32 * 36;   // warp-private [32][36] transpose buffer
         const int esz = p.out_mode == 1 ? 8 : (p.out_mode == 2 ? 2 : 4);
-        const bool out_ok = p.out_mode == 3 ? true
+        // top-k mode: this warp's [k][32] lists (over the transpose buffers, which the mode does not use), and per lane the
+        // k-th best key of its row so far
+        unsigned long long* lst = reinterpret_cast<unsigned long long*>(stage_smem) + (size_t)(warp - 2) * 32 * (TOPK ? p.topk_k : 0);
+        unsigned long long kth = 0ull;
+        float kth_f = -INFINITY;
+        if (TOPK)
+            for (int s = 0; s < p.topk_k; ++s) lst[s * 32 + lane] = 0ull;
+        const bool out_ok = p.out_mode >= 3 ? true
                           : p.out_mode == 2 ? ((p.ld_out * 2) % 8 == 0 && (reinterpret_cast<uintptr_t>(p.out) & 7) == 0)
                                             : ((p.ld_out * esz) % 16 == 0 && (reinterpret_cast<uintptr_t>(p.out) & 15) == 0);
         const bool vec_ok = out_ok && (p.q == nullptr || (reinterpret_cast<uintptr_t>(p.q) & 15) == 0);
@@ -581,6 +659,37 @@ __device__ __forceinline__ void score_gemm_body(const ScoreParams& p) {
                 if (v[0] == 1.2345e-30f) reinterpret_cast<float*>(p.out)[0] = v[1];   // experiment: TMEM loads only
                 continue;
 #endif
+                if (TOPK) {
+                    // lane = row (the accumulator's native layout): the lane screens the 32 scores of its row against its
+                    // k-th best so far; only a score that reaches it builds a key and touches shared memory.  Same roundings
+                    // as the matrix path, so a selected value equals its score_matrix entry bit for bit.
+                    const float mul = ra + a0;
+                    const int jmax = min(32, p.Nt - col0);
+                    // the scaled column term of column col0 + lane: from the prefetched float4s (lane l of the first eight
+                    // holds columns 4l .. 4l + 3), or loaded here at a ragged edge / for an unaligned column term
+                    float ql;
+                    if (p.q != nullptr && vec_ok && jmax == 32) {
+                        const float4 qv = qpre[cbi];
+                        const float x = __shfl_sync(0xffffffffu, qv.x, lane >> 2), y = __shfl_sync(0xffffffffu, qv.y, lane >> 2);
+                        const float z = __shfl_sync(0xffffffffu, qv.z, lane >> 2), w = __shfl_sync(0xffffffffu, qv.w, lane >> 2);
+                        const int c = lane & 3;
+                        ql = __fmul_rn(c == 0 ? x : (c == 1 ? y : (c == 2 ? z : w)), p.rq_scale);
+                    } else {
+                        ql = __fmul_rn((p.q != nullptr && lane < jmax) ? __ldg(p.q + col0 + lane) : 0.f, p.rq_scale);
+                    }
+#pragma unroll
+                    for (int j = 0; j < 32; ++j) {
+                        const float s = __fadd_rn(fmaf(v[j], mul, rr), __shfl_sync(0xffffffffu, ql, j));
+                        if (j < jmax && s >= kth_f) {
+                            const unsigned long long key = topk_key(s, col0 + j);
+                            if (key > kth) {
+                                kth = topk_heap_replace(lst, lane, p.topk_k, key);
+                                kth_f = topk_screen(kth);
+                            }
+                        }
+                    }
+                    continue;
+                }
                 if (TRIALS) {
                     // Only the trials of the mask are written, compacted in row-major order: each lane walks the set bits
                     // of ITS row's word (lane = row, the accumulator's native layout: no transpose).  A block without any
@@ -703,6 +812,18 @@ __device__ __forceinline__ void score_gemm_body(const ScoreParams& p) {
                 }
             }
             }   // panels of the item
+            if (TOPK && (nt + 1 == p.n_ntiles || t + 1 == t_end)) {
+                // leaving the row panel: this warp's lists become the partial lists of its segment, and start over empty
+                const int row = panel * 128 + q * 32 + lane;
+                const int seg = 2 * ((int)blockIdx.x - topk_first_cta(panel, p.n_ntiles, tiles_total, (int)gridDim.x)) + part;
+                unsigned long long* dst = reinterpret_cast<unsigned long long*>(p.out) + ((size_t)row * p.topk_segs + seg) * p.topk_k;
+                for (int s = 0; s < p.topk_k; ++s) {
+                    if (row < p.Ne) dst[s] = lst[s * 32 + lane];
+                    lst[s * 32 + lane] = 0ull;
+                }
+                kth = 0ull;
+                kth_f = -INFINITY;
+            }
             if (++nt == p.n_ntiles) { nt = 0; ++panel; }
         }
         if (warp == 2 && lane == 0) { SKB_TADD(6); }
@@ -714,20 +835,20 @@ __device__ __forceinline__ void score_gemm_body(const ScoreParams& p) {
     }
 }
 
-template <int PASSES, bool STREAM_A, bool TRIALS, int MT, int KC>
+template <int PASSES, bool STREAM_A, int MODE, int MT, int KC>
 __global__ void __launch_bounds__(ScoreSmem<PASSES, STREAM_A, MT, KC>::kThreads, 1) score_gemm_kernel(const ScoreParams p) {
-    score_gemm_body<PASSES, STREAM_A, TRIALS, MT, KC>(p);
+    score_gemm_body<PASSES, STREAM_A, MODE, MT, KC>(p);
 }
 
 // passes decided on the device (passes_req == 0), resident-panel variants: ONE launch that runs the body the statistics
 // select (round 1 launched both instantiations and let one of them return at once: a 3 us no-op per call, 5 % of a
 // 2500-row panel at 8 GPUs).  Shared memory is sized for the larger of the two layouts by launch_score_auto.
 static_assert(ScoreSmem<1, false>::kThreads == ScoreSmem<3, false>::kThreads, "the auto kernel needs one block size");
-template <bool TRIALS, int KC>
+template <int MODE, int KC>
 __global__ void __launch_bounds__(ScoreSmem<1, false>::kThreads, 1) score_gemm_auto_kernel(const ScoreParams p) {
     pdl_wait();
-    if (decide_passes(p.statsE, p.statsT, p.D, p.abs_alpha, 0) == 1) score_gemm_body<1, false, TRIALS, 1, KC>(p);
-    else score_gemm_body<3, false, TRIALS, 1>(p);
+    if (decide_passes(p.statsE, p.statsT, p.D, p.abs_alpha, 0) == 1) score_gemm_body<1, false, MODE, 1, KC>(p);
+    else score_gemm_body<3, false, MODE, 1>(p);
 }
 
 // ----------------------------------------------------------------------------- packed operands, workspace, launch
@@ -842,10 +963,10 @@ static void ws_operand(PackedOp* op, int rows, int D, int slot, size_t offset_ha
     op->exp = reinterpret_cast<int*>(op->stats + 2);
 }
 
-template <int PASSES, bool STREAM_A, bool TRIALS = false, int MT = 1, int KC = 64>
+template <int PASSES, bool STREAM_A, int MODE = kEpiMatrix, int MT = 1, int KC = 64>
 static int launch_score(const ScoreParams& p, int /*grid_unused*/, cudaStream_t st) {
     static PerDeviceOnce configured;
-    const size_t smem = ScoreSmem<PASSES, STREAM_A, MT, KC>::total(p.Dp);
+    const size_t smem = ScoreSmem<PASSES, STREAM_A, MT, KC>::total(p.Dp, p.topk_k);
     const int n_panels = p.Ne_pad / 128;
     const int grid = std::min(((n_panels + MT - 1) / MT) * p.n_ntiles, kNumSMs);
     if (smem > 227 * 1024) {
@@ -853,27 +974,27 @@ static int launch_score(const ScoreParams& p, int /*grid_unused*/, cudaStream_t 
         return SKB_ERR_ARG;
     }
     if (configured.first()) {
-        SKB_CUDA_CHECK(cudaFuncSetAttribute(score_gemm_kernel<PASSES, STREAM_A, TRIALS, MT, KC>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
+        SKB_CUDA_CHECK(cudaFuncSetAttribute(score_gemm_kernel<PASSES, STREAM_A, MODE, MT, KC>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
     }
-    SKB_CUDA_CHECK(launch_pdl(score_gemm_kernel<PASSES, STREAM_A, TRIALS, MT, KC>, dim3(grid), dim3(ScoreSmem<PASSES, STREAM_A, MT, KC>::kThreads), smem, st, p));
+    SKB_CUDA_CHECK(launch_pdl(score_gemm_kernel<PASSES, STREAM_A, MODE, MT, KC>, dim3(grid), dim3(ScoreSmem<PASSES, STREAM_A, MT, KC>::kThreads), smem, st, p));
     g_launches++;
     SKB_CUDA_CHECK(cudaGetLastError());
     return SKB_OK;
 }
 
-template <bool TRIALS, int KC>
+template <int MODE, int KC>
 static int launch_score_auto_kc(const ScoreParams& p, cudaStream_t st) {
     static PerDeviceOnce configured;
-    const size_t smem = std::max(ScoreSmem<1, false, 1, KC>::total(p.Dp), ScoreSmem<3, false>::total(p.Dp));
+    const size_t smem = std::max(ScoreSmem<1, false, 1, KC>::total(p.Dp, p.topk_k), ScoreSmem<3, false>::total(p.Dp, p.topk_k));
     const int grid = std::min((p.Ne_pad / 128) * p.n_ntiles, kNumSMs);
     if (smem > 227 * 1024) {
         set_last_error(__FILE__, __LINE__, "score_gemm: operand panel does not fit in shared memory");
         return SKB_ERR_ARG;
     }
     if (configured.first()) {
-        SKB_CUDA_CHECK(cudaFuncSetAttribute(score_gemm_auto_kernel<TRIALS, KC>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
+        SKB_CUDA_CHECK(cudaFuncSetAttribute(score_gemm_auto_kernel<MODE, KC>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
     }
-    SKB_CUDA_CHECK(launch_pdl(score_gemm_auto_kernel<TRIALS, KC>, dim3(grid), dim3(ScoreSmem<1, false>::kThreads), smem, st, p));
+    SKB_CUDA_CHECK(launch_pdl(score_gemm_auto_kernel<MODE, KC>, dim3(grid), dim3(ScoreSmem<1, false>::kThreads), smem, st, p));
     g_launches++;
     SKB_CUDA_CHECK(cudaGetLastError());
     return SKB_OK;
@@ -887,24 +1008,25 @@ static int stage_width(const ScoreParams& p) {
     if (p.Dp % 128 == 0 && cap >= 128) return 128;
     return 64;
 }
-template <bool TRIALS>
+template <int MODE>
 static int launch_score_auto(const ScoreParams& p, cudaStream_t st) {
     const int kc = stage_width(p);
-    return kc == 256 ? launch_score_auto_kc<TRIALS, 256>(p, st) : (kc == 128 ? launch_score_auto_kc<TRIALS, 128>(p, st) : launch_score_auto_kc<TRIALS, 64>(p, st));
+    return kc == 256 ? launch_score_auto_kc<MODE, 256>(p, st) : (kc == 128 ? launch_score_auto_kc<MODE, 128>(p, st) : launch_score_auto_kc<MODE, 64>(p, st));
 }
-template <bool TRIALS>
+template <int MODE>
 static int launch_score_single_pass(const ScoreParams& p, int grid, cudaStream_t st) {
     const int kc = stage_width(p);
-    return kc == 256 ? launch_score<1, false, TRIALS, 1, 256>(p, grid, st)
-                     : (kc == 128 ? launch_score<1, false, TRIALS, 1, 128>(p, grid, st) : launch_score<1, false, TRIALS, 1, 64>(p, grid, st));
+    return kc == 256 ? launch_score<1, false, MODE, 1, 256>(p, grid, st)
+                     : (kc == 128 ? launch_score<1, false, MODE, 1, 128>(p, grid, st) : launch_score<1, false, MODE, 1, 64>(p, grid, st));
 }
 
 // out = acc * (ra_i + ca_j + a0) + rq_scale * (r_i + q_j) + c0 on two packed operands
 int gemm_packed(const PackedOp& E, const PackedOp& T, const float* ra, const float* ca, float a0, const float* r, const float* q,
                 float c0, float rq_scale, float abs_alpha_for_auto, int passes, int out_mode, void* out, long long ld_out,
-                cudaStream_t st, const TrialTables* trials) {
-    if (E.Dp != T.Dp || !out || (out_mode != 3 && ld_out < T.rows) || (passes != 0 && passes != 1 && passes != 3) || out_mode < 0 ||
-        out_mode > 3 || (out_mode == 3 && (trials == nullptr || trials->Ne != E.rows || trials->Nt != T.rows || ca != nullptr))) {
+                cudaStream_t st, const TrialTables* trials, const TopkLists* topk = nullptr) {
+    if (E.Dp != T.Dp || !out || (out_mode < 3 && ld_out < T.rows) || (passes != 0 && passes != 1 && passes != 3) || out_mode < 0 ||
+        out_mode > 4 || (out_mode == 3 && (trials == nullptr || trials->Ne != E.rows || trials->Nt != T.rows || ca != nullptr)) ||
+        (out_mode == 4 && (topk == nullptr || topk->k < 1 || topk->k > 32 || ca != nullptr))) {
         set_last_error(__FILE__, __LINE__, "gemm_packed: bad arguments");
         return SKB_ERR_ARG;
     }
@@ -921,6 +1043,8 @@ int gemm_packed(const PackedOp& E, const PackedOp& T, const float* ra, const flo
     p.mask_words = trials ? trials->words : nullptr;
     p.word_off = trials ? trials->offsets : nullptr;
     p.mask_ld = trials ? trials->ld : 0;
+    p.topk_k = topk ? topk->k : 0;
+    p.topk_segs = topk ? topk->segs : 0;
     p.n_ntiles = T.rows_pad / 128;
     p.tiles_total = (E.rows_pad / 128) * p.n_ntiles;
     const int grid = std::min(p.tiles_total, kNumSMs);
@@ -933,6 +1057,20 @@ int gemm_packed(const PackedOp& E, const PackedOp& T, const float* ra, const flo
     // L2 bandwidth (profiles/r02_score_epilogue_experiments.txt).  SKB_SCORE_TWO_PANELS=1 enables them.
     static const bool one_panel = getenv("SKB_SCORE_TWO_PANELS") == nullptr;
     const bool stream_a = E.Dp > 256 || force_stream;
+    if (out_mode == 4) {
+        // top-k: resident-panel variants with one row panel per item only (the partial-list slots assume that partition)
+        if (E.Dp > 256) {
+            set_last_error(__FILE__, __LINE__, "top-k epilogue supports embeddings of up to 256 dimensions");
+            return SKB_ERR_ARG;
+        }
+#ifdef SKB_SCORE_EPI16
+        set_last_error(__FILE__, __LINE__, "top-k epilogue is not built with SKB_SCORE_EPI16");
+        return SKB_ERR_ARG;
+#else
+        if (passes == 0) return launch_score_auto<kEpiTopk>(p, st);
+        return passes == 1 ? launch_score_single_pass<kEpiTopk>(p, grid, st) : launch_score<3, false, kEpiTopk>(p, grid, st);
+#endif
+    }
     if (out_mode == 3) {
         if (stream_a) {
             set_last_error(__FILE__, __LINE__, "trial-list mode supports embeddings of up to 256 dimensions");
@@ -940,15 +1078,15 @@ int gemm_packed(const PackedOp& E, const PackedOp& T, const float* ra, const flo
         }
         // two row panels per item when the two resident single-pass panels fit (D <= 256): half the operand stream
         const bool two = p.Dp <= 256 && E.rows_pad >= 256 && !one_panel;
-        if (passes == 0 && !two) return launch_score_auto<true>(p, st);
-        if (passes != 3) rc = two ? launch_score<1, false, true, 2>(p, grid, st) : launch_score_single_pass<true>(p, grid, st);
+        if (passes == 0 && !two) return launch_score_auto<kEpiTrials>(p, st);
+        if (passes != 3) rc = two ? launch_score<1, false, kEpiTrials, 2>(p, grid, st) : launch_score_single_pass<kEpiTrials>(p, grid, st);
         if (rc) return rc;
-        if (passes != 1) rc = launch_score<3, false, true>(p, grid, st);
+        if (passes != 1) rc = launch_score<3, false, kEpiTrials>(p, grid, st);
         return rc;
     }
     const bool two = !stream_a && p.Dp <= 256 && E.rows_pad >= 256 && !one_panel;
-    if (passes == 0 && !stream_a && !two) return launch_score_auto<false>(p, st);
-    if (passes != 3) rc = stream_a ? launch_score<1, true>(p, grid, st) : (two ? launch_score<1, false, false, 2>(p, grid, st) : launch_score_single_pass<false>(p, grid, st));
+    if (passes == 0 && !stream_a && !two) return launch_score_auto<kEpiMatrix>(p, st);
+    if (passes != 3) rc = stream_a ? launch_score<1, true>(p, grid, st) : (two ? launch_score<1, false, kEpiMatrix, 2>(p, grid, st) : launch_score_single_pass<kEpiMatrix>(p, grid, st));
     if (rc) return rc;
     if (passes != 1) rc = stream_a ? launch_score<3, true>(p, grid, st) : launch_score<3, false>(p, grid, st);
     return rc;
@@ -1076,26 +1214,12 @@ __global__ void trial_addbase_kernel(uint32_t* __restrict__ offs, const uint32_t
 }
 
 // ----------------------------------------------------------------------------- as-norm: top-k statistics per row
-__device__ __forceinline__ unsigned f2key(float f) {   // order-preserving float -> uint
-    const unsigned u = __float_as_uint(f);
-    return (u & 0x80000000u) ? ~u : (u | 0x80000000u);
-}
-__device__ __forceinline__ float key2f(unsigned k) {
-    const unsigned u = (k & 0x80000000u) ? (k & 0x7fffffffu) : ~k;
-    return __uint_as_float(u);
-}
-
-// One CTA per row: radix-select the k-th largest score, then mean and unbiased std of the top k
-// (torch.topk + mean + std, sidekit/score_normalization.py:131-133).  Ties at the threshold are
-// counted exactly k - (#greater) times, like a sort would.
-__global__ void __launch_bounds__(256) topk_stats_kernel(const float* __restrict__ S, int C, long long ld, int k,
-                                                         float* __restrict__ mean_out, float* __restrict__ std_out) {
-    extern __shared__ unsigned keys[];
+// Block-wide radix select (blockDim.x == 256, every thread calls it once per launch): the k-th largest of the C keys
+// key_at(0 .. C-1) (.x) and how many of the keys equal to it are among the k largest (.y).  Four 8-bit passes.
+template <class KeyAt>
+__device__ uint2 radix_select_kth(KeyAt key_at, int C, unsigned k) {
     __shared__ unsigned hist[256];
     __shared__ unsigned sel_prefix, sel_remaining;
-    __shared__ double red[2][8];
-    const float* row = S + (size_t)blockIdx.x * ld;
-    for (int i = threadIdx.x; i < C; i += blockDim.x) keys[i] = f2key(row[i]);
     if (threadIdx.x == 0) { sel_prefix = 0; sel_remaining = k; }
     __syncthreads();
     for (int shift = 24; shift >= 0; shift -= 8) {
@@ -1104,7 +1228,7 @@ __global__ void __launch_bounds__(256) topk_stats_kernel(const float* __restrict
         const unsigned prefix = sel_prefix;
         const unsigned mask = shift == 24 ? 0u : (0xffffffffu << (shift + 8));
         for (int i = threadIdx.x; i < C; i += blockDim.x) {
-            const unsigned key = keys[i];
+            const unsigned key = key_at(i);
             if ((key & mask) == (prefix & mask)) atomicAdd(&hist[(key >> shift) & 255], 1u);
         }
         __syncthreads();
@@ -1120,8 +1244,22 @@ __global__ void __launch_bounds__(256) topk_stats_kernel(const float* __restrict
         }
         __syncthreads();
     }
-    const unsigned thr = sel_prefix;
-    const unsigned n_thr = sel_remaining;
+    return make_uint2(sel_prefix, sel_remaining);
+}
+
+// One CTA per row: radix-select the k-th largest score, then mean and unbiased std of the top k
+// (torch.topk + mean + std, sidekit/score_normalization.py:131-133).  Ties at the threshold are
+// counted exactly k - (#greater) times, like a sort would.
+__global__ void __launch_bounds__(256) topk_stats_kernel(const float* __restrict__ S, int C, long long ld, int k,
+                                                         float* __restrict__ mean_out, float* __restrict__ std_out) {
+    extern __shared__ unsigned keys[];
+    __shared__ double red[2][8];
+    const float* row = S + (size_t)blockIdx.x * ld;
+    for (int i = threadIdx.x; i < C; i += blockDim.x) keys[i] = f2key(row[i]);
+    __syncthreads();
+    const uint2 sel = radix_select_kth([&](int i) { return keys[i]; }, C, (unsigned)k);
+    const unsigned thr = sel.x;
+    const unsigned n_thr = sel.y;
     const float thr_f = key2f(thr);
     // pass 1: mean
     double s = 0.0;
@@ -1150,6 +1288,150 @@ __global__ void __launch_bounds__(256) topk_stats_kernel(const float* __restrict
         mean_out[blockIdx.x] = (float)mean;
         std_out[blockIdx.x] = (float)sqrt(vt / (k - 1));
     }
+}
+
+// ----------------------------------------------------------------------------- top-k columns per row
+// Fused path (k <= kTopkFusedMax, D <= 256): the GEMM's top-k epilogue leaves partial lists; one warp per row merges the
+// row's segments (topk_panel_segs of its panel, k keys each, padded with key 0) into the final k, descending.
+constexpr int kTopkFusedMax = 32;
+constexpr int kTopkMax = 1024;
+__global__ void __launch_bounds__(256) topk_merge_kernel(const unsigned long long* __restrict__ lists, int Ne, int k, int segs,
+                                                         int n_ntiles, int tiles, int grid, float* __restrict__ values,
+                                                         int64_t* __restrict__ indices) {
+    pdl_wait();
+    const int row = blockIdx.x * 8 + (threadIdx.x >> 5), lane = threadIdx.x & 31;
+    if (row >= Ne) return;
+    const int n = topk_panel_segs(row >> 7, n_ntiles, tiles, grid) * k;
+    const unsigned long long* __restrict__ L = lists + (size_t)row * segs * k;
+    // k rounds of a warp arg-max below the previous pick (the non-zero keys of a row are distinct: one per column)
+    unsigned long long last = ~0ull;
+    for (int r = 0; r < k; ++r) {
+        unsigned long long best = 0ull;
+        for (int i = lane; i < n; i += 32) {
+            const unsigned long long x = __ldg(L + i);
+            if (x < last && x > best) best = x;
+        }
+#pragma unroll
+        for (int o = 16; o > 0; o >>= 1) best = max(best, __shfl_xor_sync(0xffffffffu, best, o));
+        last = best;
+        if (lane == (r & 31)) {
+            values[(size_t)row * k + r] = key2f((unsigned)(best >> 32));
+            indices[(size_t)row * k + r] = (int64_t)(int)~(unsigned)best;   // padding (key 0) -> -1
+        }
+    }
+}
+
+// Panel path (k > kTopkFusedMax or D > 256): one CTA per row of a float32 score panel.  Radix-select the k-th key, keep every
+// key above it and the lowest-index ties at it (k survivors), sort them in shared memory in the same 64-bit order.
+__global__ void __launch_bounds__(256) topk_select_kernel(const float* __restrict__ S, int C, long long ld, int k,
+                                                          float* __restrict__ values, int64_t* __restrict__ indices) {
+    extern __shared__ unsigned long long cand[];          // [kp], kp = next power of two >= k
+    __shared__ unsigned n_greater, taken, w_cnt[8];
+    const float* __restrict__ row = S + (size_t)blockIdx.x * ld;
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    const uint2 sel = radix_select_kth([&](int i) { return f2key(__ldg(row + i)); }, C, (unsigned)k);
+    const unsigned thr = sel.x, n_thr = sel.y;
+    int kp = 1;
+    while (kp < k) kp <<= 1;
+    for (int i = threadIdx.x; i < kp; i += blockDim.x) cand[i] = 0ull;
+    if (threadIdx.x == 0) { n_greater = 0u; taken = 0u; }
+    __syncthreads();
+    for (int i = threadIdx.x; i < C; i += blockDim.x) {
+        const unsigned key = f2key(__ldg(row + i));
+        if (key > thr) cand[atomicAdd(&n_greater, 1u)] = ((unsigned long long)key << 32) | (unsigned)~i;
+    }
+    __syncthreads();
+    const unsigned g = n_greater;                         // == k - n_thr
+    // the n_thr ties at the threshold with the lowest column indices: a block-wide ordered scan, 256 columns per step
+    for (int base = 0; base < C && taken < n_thr; base += blockDim.x) {
+        const int i = base + threadIdx.x;
+        const bool eq = i < C && f2key(__ldg(row + i)) == thr;
+        const unsigned ball = __ballot_sync(0xffffffffu, eq);
+        if (lane == 0) w_cnt[warp] = __popc(ball);
+        __syncthreads();
+        unsigned pos = taken + __popc(ball & ((1u << lane) - 1u));
+        for (int w = 0; w < warp; ++w) pos += w_cnt[w];
+        if (eq && pos < n_thr) cand[g + pos] = ((unsigned long long)thr << 32) | (unsigned)~i;
+        __syncthreads();
+        if (threadIdx.x == 0)
+            for (int w = 0; w < 8; ++w) taken += w_cnt[w];
+        __syncthreads();
+    }
+    // bitonic sort, descending
+    for (int size = 2; size <= kp; size <<= 1)
+        for (int stride = size >> 1; stride > 0; stride >>= 1) {
+            for (int i = threadIdx.x; i < kp; i += blockDim.x) {
+                const int j = i ^ stride;
+                if (j > i) {
+                    const unsigned long long a = cand[i], b = cand[j];
+                    if ((i & size) == 0 ? a < b : a > b) { cand[i] = b; cand[j] = a; }
+                }
+            }
+            __syncthreads();
+        }
+    for (int r = threadIdx.x; r < k; r += blockDim.x) {
+        const unsigned long long x = cand[r];
+        values[(size_t)blockIdx.x * k + r] = key2f((unsigned)(x >> 32));
+        indices[(size_t)blockIdx.x * k + r] = (int64_t)(int)~(unsigned)x;
+    }
+}
+
+// The k best columns of every row of S = acc * a0 + rq_scale * (r_i + q_j) + c0 for two packed operands.  The operands are
+// packed once for the whole call, so the scale exponents and the pass decision are those of the matching score_matrix call
+// and every selected value is its matrix entry bit for bit.  1 <= k <= min(T.rows, kTopkMax) is checked by the caller.
+static int score_topk_packed(const PackedOp& e, const PackedOp& t, const float* r, const float* q, float a0, float c0, float rq_scale,
+                             float abs_alpha, int passes, int k, float* values, int64_t* indices, cudaStream_t st) {
+    int rc;
+    if (k <= kTopkFusedMax && e.Dp <= 256) {
+        // the partial-list scratch [Ne][segs][k] is sized from the partition score_gemm_body uses (one row panel per item)
+        const int n_panels = e.rows_pad / 128, n_ntiles = t.rows_pad / 128;
+        const int tiles = n_panels * n_ntiles, grid = std::min(tiles, kNumSMs);
+        int segs = 0;
+        for (int P = 0; P < n_panels; ++P) segs = std::max(segs, topk_panel_segs(P, n_ntiles, tiles, grid));
+        if ((rc = ws_ensure(0, (size_t)e.rows * segs * k * sizeof(unsigned long long)))) return rc;
+        TopkLists tl{reinterpret_cast<unsigned long long*>(g_ws.tmp), k, segs};
+        if ((rc = gemm_packed(e, t, nullptr, nullptr, a0, r, q, c0, rq_scale, abs_alpha, passes, 4, tl.keys, 0, st, nullptr, &tl))) return rc;
+        SKB_CUDA_CHECK(launch_pdl(topk_merge_kernel, dim3((unsigned)((e.rows + 7) / 8)), dim3(256), 0, st,
+                                  (const unsigned long long*)tl.keys, e.rows, k, segs, n_ntiles, tiles, grid, values, indices));
+        g_launches++;
+        SKB_CUDA_CHECK(cudaGetLastError());
+        return SKB_OK;
+    }
+    // Row panels of the score matrix through a bounded float32 scratch (<= 1 GB, at least one 128-row tile), each followed by
+    // the per-row select.  A panel is a view of the packed E (whole 128-row tiles): same statistics, same arithmetic.
+    const long long ld = (t.rows + 3) / 4 * 4;
+    constexpr long long kPanelBytes = 1ll << 30;
+    const int rows = (int)std::min<long long>(e.rows_pad, std::max<long long>(128, kPanelBytes / (ld * 4) / 128 * 128));
+    if ((rc = ws_ensure(0, (size_t)rows * ld * sizeof(float)))) return rc;
+    int kp = 1;
+    while (kp < k) kp <<= 1;
+    for (int r0 = 0; r0 < e.rows; r0 += rows) {
+        PackedOp v = e;
+        v.rows = std::min(rows, e.rows - r0);
+        v.rows_pad = (v.rows + 127) / 128 * 128;
+        v.hi = e.hi + (size_t)r0 * e.Dp;
+        v.lo = e.lo + (size_t)r0 * e.Dp;
+        if ((rc = gemm_packed(v, t, nullptr, nullptr, a0, r ? r + r0 : nullptr, q, c0, rq_scale, abs_alpha, passes, 0, g_ws.tmp, ld, st,
+                              nullptr)))
+            return rc;
+        topk_select_kernel<<<v.rows, 256, kp * sizeof(unsigned long long), st>>>(g_ws.tmp, t.rows, ld, k, values + (size_t)r0 * k,
+                                                                                 indices + (size_t)r0 * k);
+        g_launches++;
+    }
+    SKB_CUDA_CHECK(cudaGetLastError());
+    return SKB_OK;
+}
+
+static int topk_check_args(int Ne, int Nt, int k, int passes) {
+    if (Ne < 1 || Nt < 1 || (passes != 0 && passes != 1 && passes != 3)) {
+        set_last_error(__FILE__, __LINE__, "score_gemm_topk: bad arguments");
+        return SKB_ERR_ARG;
+    }
+    if (k < 1 || k > Nt || k > kTopkMax) {
+        set_last_error(__FILE__, __LINE__, "score_gemm_topk: need 1 <= k <= min(Nt, 1024)");
+        return SKB_ERR_ARG;
+    }
+    return SKB_OK;
 }
 
 // ra_i = 0.5 / std_i,  r_i = -0.5 * mean_i / std_i   (the symmetric as-norm as acc*(ra_i+ra_j) + (r_i+r_j))
@@ -1365,6 +1647,50 @@ int skb_score_gemm_trials_packed(const float* E_dev, int Ne, const skb_packed_t*
     TrialTables tt{trials->words, trials->offsets, trials->ld, Ne, T->op.rows};
     return gemm_packed(e, T->op, nullptr, nullptr, (float)alpha, rowterm_dev, colterm_dev, (float)(alpha * cst), (float)alpha,
                        (float)fabs(alpha), passes, 3, out_trials_dev, 0, st, &tt);
+}
+
+int skb_score_gemm_topk(const float* E_dev, const float* T_dev, int Ne, int Nt, int D, const float* rowterm_dev,
+                        const float* colterm_dev, double cst, double alpha, int passes, int k, float* values_dev, int64_t* indices_dev,
+                        void* stream) {
+    if (!E_dev || !T_dev || !values_dev || !indices_dev || D <= 0) {
+        set_last_error(__FILE__, __LINE__, "score_gemm_topk: bad arguments");
+        return SKB_ERR_ARG;
+    }
+    int rc = topk_check_args(Ne, Nt, k, passes);
+    if (rc) return rc;
+    cudaStream_t st = (cudaStream_t)stream;
+    const int Dp = (D + kScKChunk - 1) / kScKChunk * kScKChunk;
+    const size_t eh = (size_t)Dp * ((Ne + 127) / 128 * 128), th = (size_t)Dp * ((Nt + 127) / 128 * 128);
+    if ((rc = ws_ensure(2 * (eh + th) * sizeof(uint16_t), 0))) return rc;
+    PackedOp e, t;
+    ws_operand(&e, Ne, D, 0, 0);
+    ws_operand(&t, Nt, D, 1, 2 * eh);
+    if ((rc = packed_fill(E_dev, &e, T_dev, &t, st))) return rc;
+    return score_topk_packed(e, t, rowterm_dev, colterm_dev, (float)alpha, (float)(alpha * cst), (float)alpha, (float)fabs(alpha), passes,
+                             k, values_dev, indices_dev, st);
+}
+
+int skb_score_gemm_topk_packed(const float* E_dev, int Ne, const skb_packed_t* T, const float* rowterm_dev, const float* colterm_dev,
+                               double cst, double alpha, int passes, int k, float* values_dev, int64_t* indices_dev, void* stream) {
+    if (!E_dev || !T || !values_dev || !indices_dev) {
+        set_last_error(__FILE__, __LINE__, "score_gemm_topk_packed: bad arguments");
+        return SKB_ERR_ARG;
+    }
+    int rc = topk_check_args(Ne, T->op.rows, k, passes);
+    if (rc) return rc;
+    if (T->device != current_device()) {
+        set_last_error(__FILE__, __LINE__, "score_gemm_topk_packed: the packed operand lives on another CUDA device");
+        return SKB_ERR_STATE;
+    }
+    cudaStream_t st = (cudaStream_t)stream;
+    const int D = T->op.D, Dp = T->op.Dp;
+    const size_t eh = (size_t)Dp * ((Ne + 127) / 128 * 128);
+    if ((rc = ws_ensure(2 * eh * sizeof(uint16_t), 0))) return rc;
+    PackedOp e;
+    ws_operand(&e, Ne, D, 0, 0);
+    if ((rc = packed_fill(E_dev, &e, nullptr, nullptr, st))) return rc;
+    return score_topk_packed(e, T->op, rowterm_dev, colterm_dev, (float)alpha, (float)(alpha * cst), (float)alpha, (float)fabs(alpha), passes,
+                             k, values_dev, indices_dev, st);
 }
 
 #ifdef SKB_SCORE_TIMING

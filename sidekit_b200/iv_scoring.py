@@ -7,6 +7,7 @@ enrolled ids, first occurrence wins, every occurrence in the ndx kept) -- and th
 side (CUDA, csrc/scoring.cu): centring, the Psi / Phi folds, the quadratic row / column terms and the
 Ne x Nt score matrix.  The result stays on the device until ``Scores.scoremat`` is read.
 """
+import collections
 import copy
 import ctypes
 import logging
@@ -132,6 +133,35 @@ def score_trials(E, T, trials, rowterm=None, colterm=None, cst=0.0, alpha=1.0, p
             None if colterm is None else colterm.data_ptr(), float(cst), float(alpha), int(passes), trials._ptr, out.data_ptr(),
             _lib.stream_ptr()))
     return out[:trials.n_trials]
+
+
+TOPK_MAX = 1024
+
+
+def score_topk(E, T, k, rowterm=None, colterm=None, cst=0.0, alpha=1.0, passes=0):
+    """The ``k`` largest entries of every row of ``score_matrix(E, T, rowterm, colterm, cst, alpha, passes)`` as CUDA tensors
+    ``(values (Ne, k) float32, indices (Ne, k) int64)``, ordered by score descending and, among equal scores, by lower column
+    -- each value equals its ``score_matrix`` entry bit for bit.  ``T`` may be a ``PackedEmbeddings`` (a gallery packed once
+    and searched by many query batches).  For ``k <= 32`` and ``D <= 256`` the selection runs inside the GEMM epilogue and
+    the (Ne, Nt) matrix never reaches memory; otherwise row panels of it pass through a bounded scratch.  The order of NaN
+    scores is undefined."""
+    Ne, D = E.shape
+    Nt = T.rows if isinstance(T, PackedEmbeddings) else T.shape[0]
+    k = int(k)
+    if not 1 <= k <= min(Nt, TOPK_MAX):
+        raise ValueError("score_topk: need 1 <= k <= min(Nt, %d), got k = %d with Nt = %d" % (TOPK_MAX, k, Nt))
+    values = torch.empty((Ne, k), dtype=torch.float32, device=E.device)
+    indices = torch.empty((Ne, k), dtype=torch.int64, device=E.device)
+    r = None if rowterm is None else rowterm.data_ptr()
+    q = None if colterm is None else colterm.data_ptr()
+    with torch.cuda.device(E.device):
+        if isinstance(T, PackedEmbeddings):
+            _lib.check(_lib.lib().skb_score_gemm_topk_packed(E.data_ptr(), Ne, T._ptr, r, q, float(cst), float(alpha), int(passes), k,
+                                                             values.data_ptr(), indices.data_ptr(), _lib.stream_ptr()))
+        else:
+            _lib.check(_lib.lib().skb_score_gemm_topk(E.data_ptr(), T.data_ptr(), Ne, Nt, D, r, q, float(cst), float(alpha), int(passes),
+                                                      k, values.data_ptr(), indices.data_ptr(), _lib.stream_ptr()))
+    return values, indices
 
 
 def _quadratic_prepare(X, mu, Psi, Phi):
@@ -351,3 +381,67 @@ def two_covariance_scoring(enroll, test, ndx, W, B, check_missing=True):
     Tc, seg_part = _quadratic_prepare(T, None, None, 2.0 * (G - H))
     S = score_matrix(Ep, Tc, model_part, seg_part, passes=0)
     return _finish(clean_ndx, S, numpy.float64)
+
+
+TopK = collections.namedtuple("TopK", ["segset", "models", "scores"])
+TopK.__doc__ = """Best enrolled models per test segment: ``models[i]`` / ``scores[i]`` (both (Nt, k)) are the k best model ids of
+``segset[i]`` and their scores, best first (equal scores: the model listed first in the enrolment wins)."""
+
+
+def _unique_models(enroll):
+    """One row per model id: duplicate ids averaged with ``mean_stat_per_model``, as ``fast_PLDA_scoring`` does (a model
+    must appear once in a ranking).  The caller's object is not modified."""
+    if numpy.unique(enroll.modelset).shape == enroll.modelset.shape:
+        return copy.copy(enroll)
+    logging.warning("Enrollment models are not unique, average i-vectors")
+    return enroll.mean_stat_per_model()
+
+
+def _check_k(k, n_models):
+    k = int(k)
+    if not 1 <= k <= min(n_models, TOPK_MAX):
+        raise ValueError("need 1 <= k <= min(number of models, %d), got k = %d with %d models" % (TOPK_MAX, k, n_models))
+    return k
+
+
+def cosine_topk(enroll, test, k, wccn=None, device=None):
+    """For every test segment (in ``test.segset`` order) the ``k`` enrolled models of highest cosine score -- speaker
+    identification / embedding search over the scores ``cosine_scoring`` computes, without the (models x segments) matrix.
+    The reference has no such function.  Duplicate model ids are averaged first (``mean_stat_per_model``, before the WCCN
+    rotation and length normalisation), so each model appears once.  Returns ``TopK(segset, models, scores)`` with float32
+    scores; the caller's objects are not modified."""
+    assert isinstance(enroll, StatServer), 'First parameter should be a StatServer'
+    assert isinstance(test, StatServer), 'Second parameter should be a StatServer'
+    enroll_copy = _unique_models(enroll)
+    test_copy = copy.copy(test)                # shallow: the StatServer methods below rebind their arrays
+    k = _check_k(k, enroll_copy.modelset.shape[0])
+    if wccn is not None:
+        enroll_copy.rotate_stat1(wccn)
+        test_copy.rotate_stat1(wccn)
+    enroll_copy.norm_stat1()
+    test_copy.norm_stat1()
+    dev = _device(device)
+    Q, M = _dev32(test_copy.stat1, dev), _dev32(enroll_copy.stat1, dev)
+    # queries are the GEMM rows, models the columns; split mode like cosine_scoring
+    values, indices = score_topk(Q, M, k, passes=3)
+    return TopK(numpy.asarray(test.segset).copy(), enroll_copy.modelset[indices.cpu().numpy()], values.cpu().numpy())
+
+
+def PLDA_topk(enroll, test, k, mu, F, Sigma, scaling_factor=1.):
+    """For every test segment (in ``test.segset`` order) the ``k`` enrolled models of highest simplified-PLDA log-likelihood
+    ratio (the scores of ``fast_PLDA_scoring``), without the (models x segments) matrix.  The reference has no such function.
+    Duplicate model ids are averaged first (``mean_stat_per_model``, as ``fast_PLDA_scoring`` does).  The LLR is symmetric in
+    (enrol, test), so Psi is folded into the query side.  Returns ``TopK(segset, models, scores)`` with float64 scores like
+    the PLDA scorers (fp32-class precision); the caller's objects are not modified."""
+    assert isinstance(enroll, StatServer), 'First parameter should be a StatServer'
+    assert isinstance(test, StatServer), 'Second parameter should be a StatServer'
+    assert enroll.stat1.shape[1] == test.stat1.shape[1], 'I-vectors dimension mismatch'
+    enroll_ctr = _unique_models(enroll)
+    k = _check_k(k, enroll_ctr.modelset.shape[0])
+    Phi, Psi, plda_cst = _simplified_plda_terms(F, Sigma, scaling_factor)
+    dev = _device()
+    Q, M = _dev32(test.stat1, dev), _dev32(enroll_ctr.stat1, dev)
+    Qp, seg_part = _quadratic_prepare(Q, mu, Psi.T, Phi)         # (t - mu) Psi' ; e' Psi t = t' Psi' e
+    Mc, model_part = _quadratic_prepare(M, mu, None, Phi)
+    values, indices = score_topk(Qp, Mc, k, seg_part, model_part, cst=plda_cst, alpha=scaling_factor, passes=0)
+    return TopK(numpy.asarray(test.segset).copy(), enroll_ctr.modelset[indices.cpu().numpy()], values.double().cpu().numpy())
