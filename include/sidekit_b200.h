@@ -244,6 +244,30 @@ int skb_plda_em(const double* S1_dev, const double* cls_n_dev, const int* cls_u_
                 const double* cnt_u_dev, int U, const double* mean_dev, const double* sigma_obs_dev, int D, int R, int nb_iter,
                 double sum_n, double* F_dev, double* Sigma_dev, void* stream);
 
+/* ---- embedding conditioning (statserver.py:789-1054, :1279-1333): float64 scatter matrices and row transforms -------
+ * X_dev (N, D) row-major with row stride ld (elements), float32 (x_is_f64 = 0, widened exactly on load) or float64;
+ * 1 <= D <= 1024, N up to 2^31 - 1 rows (row offsets are 64-bit).  No call synchronises the stream.
+ *
+ * skb_gram_f64: G_dev (D, D) = scale * sum_i w_i (x_i - s_k(i)) (x_i - s_k(i))', float64 on mma.sync .f64 (DMMA).
+ * shift_dev (K, D) float64 shift table or NULL (no shift); shift_idx_dev (N) int32 row -> table row or NULL (row 0);
+ * w_dev (N) float64 row weights or NULL (1).  The shift is subtracted on load (no raw-moment shortcut); G is symmetric
+ * bit for bit and bitwise reproducible: rows are split into chunks that depend on (N, D) only, and the chunk partials
+ * (in a stream-ordered workspace of at most ~70 MB) are summed in a fixed order. */
+int skb_gram_f64(const void* X_dev, int x_is_f64, int64_t N, int D, int64_t ld, const double* shift_dev,
+                 const int* shift_idx_dev, const double* w_dev, double scale, double* G_dev, void* stream);
+/* skb_class_stats: mean_dev (D) column mean (row-chunk partials summed in a fixed order); sums_dev (n_cls, D) per-class
+ * sums and counts_dev (n_cls) per-class row counts.  The classes are CSR lists: cls_ptr_dev (n_cls + 1), cls_rows_dev
+ * (N, the rows of class c in input order, which is the order of summation).  Any of the three outputs may be NULL (not
+ * all); the CSR lists are needed only for sums / counts. */
+int skb_class_stats(const void* X_dev, int x_is_f64, int64_t N, int D, int64_t ld, const int* cls_ptr_dev,
+                    const int* cls_rows_dev, int n_cls, double* mean_dev, double* sums_dev, double* counts_dev, void* stream);
+/* skb_affine_rows: y_i = ((x_i - mu) .* d) W, then, with unit_norm, y_i / max(||y_i||, 1e-8) (norm_stat1).  mu_dev (D),
+ * d_dev (D) and W_dev (D, D_out) float64 may each be NULL (no centring / no scaling / identity, then D_out = D).  Y_dev
+ * (N, D_out) float32 (y_is_f64 = 0) or float64, row stride ld_out, must not overlap X.  W runs on DMMA; for D_out <= 256
+ * the length normalisation is fused into the same pass, above that a second row pass scales Y in place. */
+int skb_affine_rows(const void* X_dev, int x_is_f64, int64_t N, int D, int64_t ld, const double* mu_dev, const double* d_dev,
+                    const double* W_dev, int D_out, int unit_norm, void* Y_dev, int y_is_f64, int64_t ld_out, void* stream);
+
 /* ---- feed path: sample-rate conversion (SURVEY.md 8f rank 1) ---------------------------------------------------
  * torchaudio.transforms.Resample(orig_freq, new_freq)(speech) as sidekit/nnet/xsets.py:435, :452 and
  * sidekit/bin/extract_xvectors.py:144 call it (Hann-windowed sinc, lowpass_filter_width 6, rolloff 0.99), on a packed

@@ -20,6 +20,7 @@ from .detplot import pavx, rocch, rocch2eer, fast_minDCF, eer
 from .factor_analyser import FactorAnalyser
 from . import kaldi_io
 from . import bulk
+from . import conditioning
 from .bulk import extract_embeddings
 
 __version__ = "0.1.0"

@@ -80,7 +80,10 @@ def _declare(lib):
         "skb_scoremat_normalise": (i32, [vp, i32, i32, i64, i32, vp, vp, vp, i64, vp]),
         "skb_plda_stats": (i32, [vp, i32, i32, vp, vp, i32, f64, vp, vp, vp, vp]),
         "skb_plda_em": (i32, [vp, vp, vp, i32, vp, vp, i32, vp, vp, i32, i32, i32, f64, vp, vp, vp]),
-        "skb_resample": (i32, [vp, vp, i32, i64, i32, i32, i32, vp, vp, i32, vp, vp]),
+        "skb_gram_f64": (i32, [vp, i32, i64, i32, i64, vp, vp, vp, f64, vp, vp]),
+        "skb_class_stats": (i32, [vp, i32, i64, i32, i64, vp, vp, i32, vp, vp, vp, vp]),
+        "skb_affine_rows": (i32, [vp, i32, i64, i32, i64, vp, vp, vp, i32, i32, vp, i32, i64, vp]),
+        "skb_resample":(i32, [vp, vp, i32, i64, i32, i32, i32, vp, vp, i32, vp, vp]),
     }
     for name, (res, args) in sigs.items():
         fn = getattr(lib, name)       # AttributeError here = header / library mismatch: fail loudly

@@ -13,6 +13,7 @@
 // All matrices are row-major float64; sizes are a few hundred, so the kernels are simple and latency-oriented.
 #include "sidekit_b200.h"
 #include "common.cuh"
+#include "class_sum.cuh"
 
 #include <atomic>
 #include <vector>
@@ -92,17 +93,6 @@ __global__ void dpotrs_kernel(const double* __restrict__ L, int n, double* __res
         for (int k = i + 1; k < n; ++k) s -= l[(size_t)k * n + i] * b[(size_t)k * nrhs + c];
         b[(size_t)i * nrhs + c] = s / l[(size_t)i * n + i];
     }
-}
-
-// per-class sums: S1[c] = sum of the rows of X whose class is c (fixed order: rows are visited in input order by one
-// thread per (class, column) through the CSR lists) ; statserver.py:1335-1355
-__global__ void class_sum_kernel(const double* __restrict__ X, int D, const int* __restrict__ cls_ptr, const int* __restrict__ cls_rows,
-                                 int n_cls, double scale, double* __restrict__ S1) {
-    const int d = blockIdx.x * blockDim.x + threadIdx.x, c = blockIdx.y;
-    if (d >= D || c >= n_cls) return;
-    double s = 0.0;
-    for (int k = cls_ptr[c]; k < cls_ptr[c + 1]; ++k) s += X[(size_t)cls_rows[k] * D + d];
-    S1[(size_t)c * D + d] = s * scale;
 }
 
 __global__ void colmean_kernel(const double* __restrict__ X, int N, int D, double* __restrict__ mean) {
@@ -208,7 +198,7 @@ int skb_plda_stats(const double* X_dev, int n_sess, int D, const int* cls_ptr_de
     center_rows_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(X_dev, nullptr, mean_dev, n, D, xc.p);
     int rc = dgemm(1, 0, D, D, n_sess, 1.0 / n_sess, xc.p, D, xc.p, D, 0.0, sigma_obs_dev, D, st);     // statserver.py:920-928
     if (rc) return rc;
-    class_sum_kernel<<<dim3((D + 127) / 128, n_cls), 128, 0, st>>>(X_dev, D, cls_ptr_dev, cls_rows_dev, n_cls, scaling, S1_dev);
+    class_sum_kernel<double><<<dim3((D + 127) / 128, n_cls), 128, 0, st>>>(X_dev, D, (long long)D, cls_ptr_dev, cls_rows_dev, n_cls, scaling, S1_dev);
     g_launches += 3;
     SKB_CUDA_CHECK(cudaGetLastError());
     SKB_CUDA_CHECK(cudaStreamSynchronize(st));

@@ -25,6 +25,34 @@ def _first_index(have, wanted):
         raise IndexError("id %s not found" % (e,))
 
 
+# D x D algebra of the conditioning functions, shared by the host methods below and by ``conditioning`` (the device path)
+def _inverse_sqrt_factor(sigma):
+    """``V diag(lambda^-1/2)`` of a symmetric matrix, eigenvalues in DESCENDING order (the column order fixes the
+    coordinates of the whitened vectors, so it is part of the contract)."""
+    lam, vec = scipy.linalg.eigh(sigma)
+    order = numpy.argsort(lam.real)[::-1]
+    return vec.real[:, order] / numpy.sqrt(lam.real[order])
+
+
+def _cholesky_whitener(sigma):
+    """Lower Cholesky factor of the precision ``sigma^-1`` (statserver.py:898-918)."""
+    return scipy.linalg.cholesky(scipy.linalg.inv(sigma), lower=True)
+
+
+def _lda_from_scatter(Sb, Sw, rank):
+    """statserver.py:982-1018 from its two scatter matrices (including its ``eigh`` of the non-symmetric discrimination
+    matrix)."""
+    disc = numpy.dot(Sb, scipy.linalg.inv(Sw)).transpose()
+    eigen_values, eigen_vectors = scipy.linalg.eigh(disc)
+    idx = eigen_values.real.argsort()[-rank:][::-1]
+    return eigen_vectors.real[:, idx]
+
+
+def _wccn_from_scatter(class_normalised, n_models):
+    """statserver.py:1030-1054 from the class-normalised within-class scatter."""
+    return scipy.linalg.cholesky(scipy.linalg.inv(class_normalised / n_models)).T
+
+
 class StatServer:
     def __init__(self, statserver_file_name=None):
         if statserver_file_name is not None and not isinstance(statserver_file_name, StatServer):
@@ -184,14 +212,6 @@ class StatServer:
         out.stop = numpy.empty(out.segset.shape, "|O")
         return out, numpy.bincount(inv, minlength=n).astype(STAT_TYPE)
 
-    @staticmethod
-    def _inverse_sqrt_factor(sigma):
-        """``V diag(lambda^-1/2)`` of a symmetric matrix, eigenvalues in DESCENDING order (the column order fixes the
-        coordinates of the whitened vectors, so it is part of the contract)."""
-        lam, vec = scipy.linalg.eigh(sigma)
-        order = numpy.argsort(lam.real)[::-1]
-        return vec.real[:, order] / numpy.sqrt(lam.real[order])
-
     def whiten_stat1(self, mu, sigma, isSqrInvSigma=False):
         """statserver.py:852-896: centre, then whiten with a diagonal (1-D ``sigma``) or full (2-D) covariance; with
         ``isSqrInvSigma`` the 2-D argument already is the whitening matrix."""
@@ -201,7 +221,7 @@ class StatServer:
         if sigma.ndim == 1:
             self.stat1 = self.stat1 / numpy.sqrt(sigma.astype(STAT_TYPE))
         else:
-            self.rotate_stat1(sigma if isSqrInvSigma else self._inverse_sqrt_factor(sigma))
+            self.rotate_stat1(sigma if isSqrInvSigma else _inverse_sqrt_factor(sigma))
 
     def whiten_cholesky_stat1(self, mu, sigma):
         """statserver.py:898-918: as ``whiten_stat1`` with the lower Cholesky factor of the precision as whitening matrix."""
@@ -211,7 +231,7 @@ class StatServer:
         if sigma.ndim == 1:
             self.stat1 = self.stat1 / numpy.sqrt(sigma)
         else:
-            self.stat1 = self.stat1 @ scipy.linalg.cholesky(scipy.linalg.inv(sigma), lower=True)
+            self.stat1 = self.stat1 @ _cholesky_whitener(sigma)
 
     def get_total_covariance_stat1(self):
         """statserver.py:920-928."""
@@ -241,10 +261,7 @@ class StatServer:
         _, means, Sw = self._class_normalised_scatter()
         class_means = means - self.get_mean_stat1()
         Sb = numpy.dot(class_means.transpose(), class_means)
-        disc = numpy.dot(Sb, scipy.linalg.inv(Sw)).transpose()
-        eigen_values, eigen_vectors = scipy.linalg.eigh(disc)
-        idx = eigen_values.real.argsort()[-rank:][::-1]
-        return eigen_vectors.real[:, idx]
+        return _lda_from_scatter(Sb, Sw, rank)
 
     def get_mahalanobis_matrix_stat1(self):
         """statserver.py:1020-1028."""
@@ -253,8 +270,7 @@ class StatServer:
     def get_wccn_choleski_stat1(self):
         """statserver.py:1030-1054."""
         models, _, scatter = self._class_normalised_scatter()
-        WCCN = scatter / models.shape[0]
-        return scipy.linalg.cholesky(scipy.linalg.inv(WCCN)).T
+        return _wccn_from_scatter(scatter, models.shape[0])
 
     def estimate_spectral_norm_stat1(self, it=1, mode='efr'):
         """statserver.py:1279-1314: the (mean, covariance) pairs of ``it`` rounds of "whiten, then length-normalise", each
