@@ -11,9 +11,9 @@ namespace skb {
 int conv_pick_ncta(int cout) { return cout <= 32 ? 32 : (cout <= 64 ? 64 : 128); }
 int conv_tile_m(int n_cta) { return n_cta == 32 ? 512 : 256; }
 
-template <int N_CTA, int MT, bool BF16, bool FUSED>
+template <int N_CTA, int MT, bool BF16, bool FUSED, bool SC = false>
 static int launch_one(const ConvParams& p_in, cudaStream_t st) {
-    using Cfg = ConvCfg<N_CTA, MT>;
+    using Cfg = ConvCfg<N_CTA, MT, SC>;
     static PerDeviceOnce configured;
     ConvParams p = p_in;
     const size_t a_stage = (size_t)p.rows_pad * (kConvKC / 8) * 16;
@@ -26,6 +26,7 @@ static int launch_one(const ConvParams& p_in, cudaStream_t st) {
     p.scale_smem_bytes = 0;
     if (FUSED && N_CTA <= 64 && (size_t)p.n_utt * p.cout * 4 <= 32 * 1024) p.scale_smem_bytes = p.n_utt * p.cout * 4;
     const int scb = p.scale_smem_bytes;
+    if (!SC) p.sc_cin = 0;
     const int n_it = p.n_pairs;
     const int n_split = p.cout / N_CTA;
     int tps = 1, bst = 1;
@@ -40,14 +41,14 @@ static int launch_one(const ConvParams& p_in, cudaStream_t st) {
             }
         }
         b_stage = (size_t)tps * Cfg::kBStageBytes;
-        const size_t left = kConvSmemBudget - Cfg::fixed_bytes(p.cout, p.bias_mma, 0, 0, scb) - 3 * a_stage;
+        const size_t left = kConvSmemBudget - Cfg::fixed_bytes(p.cout, p.bias_mma, 0, 0, scb, p.sc_cin) - 3 * a_stage;
         bst = (int)(left / b_stage);
         if (bst > kConvBStages) bst = kConvBStages;
         if (bst < 2) bst = 2;
     }
     p.tps = tps;
     p.b_stages = bst;
-    const size_t fixed = Cfg::fixed_bytes(p.cout, p.bias_mma, bst, tps, scb);
+    const size_t fixed = Cfg::fixed_bytes(p.cout, p.bias_mma, bst, tps, scb, p.sc_cin);
     int stages = (int)((kConvSmemBudget - fixed) / a_stage);
     if (stages > kConvMaxAStages) stages = kConvMaxAStages;
     if (stages < 2) {
@@ -57,14 +58,14 @@ static int launch_one(const ConvParams& p_in, cudaStream_t st) {
     p.a_stages = stages;
     const size_t smem = fixed + (size_t)stages * a_stage;
     if (configured.first()) {
-        SKB_CUDA_CHECK(cudaFuncSetAttribute(conv_umma_kernel<N_CTA, MT, BF16, FUSED>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+        SKB_CUDA_CHECK(cudaFuncSetAttribute(conv_umma_kernel<N_CTA, MT, BF16, FUSED, SC>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                             227 * 1024));
     }
     const int n_pix = p.p_end - p.G;
     p.n_tiles = (n_pix + Cfg::kTileM - 1) / Cfg::kTileM;
     const int n_items = p.n_tiles * (p.cout / N_CTA);
     const int grid = n_items < kNumSMs ? n_items : kNumSMs;      // persistent: one CTA per SM
-    SKB_CUDA_CHECK(launch_pdl(conv_umma_kernel<N_CTA, MT, BF16, FUSED>, dim3(grid), dim3(kConvThreads), smem, st, p));
+    SKB_CUDA_CHECK(launch_pdl(conv_umma_kernel<N_CTA, MT, BF16, FUSED, SC>, dim3(grid), dim3(kConvThreads), smem, st, p));
     SKB_LAUNCH_CHECK(st);
     return SKB_OK;
 }
@@ -106,7 +107,7 @@ int launch_conv_umma(const ConvParams& p, int n_cta, bool bf16, cudaStream_t st)
     // layers 1 / 2, but the lane-shifted epilogue (64 shuffles + 6 TMEM loads per 32 x 32 block) costs more than the MMAs
     // it saves: 417 / 230 us per launch against 295 / 178 us for conv_umma_kernel (profiles/r01c_fused_taps.txt).
     static const bool fused_taps = [] { const char* e = getenv("SKB_FUSED_TAPS"); return e && e[0] == '1'; }();
-    if (p.w3 != nullptr && fused_taps && p.cout == n_cta && p.taps == 9 && p.cin % kConvKC == 0) {
+    if (p.w3 != nullptr && fused_taps && p.sc_in == nullptr && p.cout == n_cta && p.taps == 9 && p.cin % kConvKC == 0) {
         if (n_cta == 32) return bf16 ? launch_one3<32, 2, true>(p, st) : launch_one3<32, 2, false>(p, st);
         if (n_cta == 64) return bf16 ? launch_one3<64, 1, true>(p, st) : launch_one3<64, 1, false>(p, st);
     }
@@ -115,6 +116,17 @@ int launch_conv_umma(const ConvParams& p, int n_cta, bool bf16, cudaStream_t st)
         return SKB_ERR_ARG;
     }
     const bool fused = p.se_scale != nullptr;
+    if (p.sc_in != nullptr) {
+        // folded shortcut: the narrow layers only (the <128, 2> tiles already use all 512 TMEM columns)
+        if (!fused || p.sc_w == nullptr || p.sc_bias == nullptr || p.sc_cin < kConvKC || p.sc_cin % kConvKC != 0 || p.cout > 256) {
+            set_last_error(__FILE__, __LINE__, "conv_umma: unsupported folded shortcut");
+            return SKB_ERR_ARG;
+        }
+        if (n_cta == 32) return bf16 ? launch_one<32, 4, true, true, true>(p, st) : launch_one<32, 4, false, true, true>(p, st);
+        if (n_cta == 64) return bf16 ? launch_one<64, 2, true, true, true>(p, st) : launch_one<64, 2, false, true, true>(p, st);
+        set_last_error(__FILE__, __LINE__, "conv_umma: folded shortcut needs an N tile of 32 or 64");
+        return SKB_ERR_ARG;
+    }
 #define SKB_CONV_CASE(N, M)                                                                                   \
     case N:                                                                                                   \
         if (fused) return bf16 ? launch_one<N, M, true, true>(p, st) : launch_one<N, M, false, true>(p, st);  \

@@ -70,6 +70,14 @@ struct ConvParams {
     // with cout == 32 support it (32 per-thread 64-bit accumulators, flushed with atomics when the utterance changes).
     unsigned long long* sums;
     unsigned* overflow;     // fp16 range guard: number of threads that stored a saturated (|x| >= 65504) value, or nullptr
+    // Folded 1x1 shortcut (conv2 of a widening / striding block, N_CTA <= 64): the residual is computed here instead of read
+    // from `res`.  Its input (the block input, or phase (0, 0) of a phase-split input: the first sc_cin / 8 planes) arrives
+    // as extra halo-free k-chunks at the end of each item and accumulates into a second TMEM accumulator with the same
+    // bias MMA and k-chunk order as a stand-alone 1x1 launch; the epilogue rounds it to 16 bits as that launch would store it.
+    const uint16_t* sc_in;  // shortcut input planes (plane stride in_plane), or nullptr
+    const uint16_t* sc_w;   // packed 1x1 weights: [n_split][sc_cin / 32] images of [4][N_CTA][8]
+    const float* sc_bias;   // [cout] folded BN bias of the shortcut
+    int sc_cin;
 };
 
 constexpr int kConvKC = 32;            // input channels per A/B stage (two K=16 MMAs)
@@ -79,23 +87,27 @@ constexpr int kConvThreads = 12 * 32;  // warps: 0 A-producer, 1 B-producer, 2-3
 constexpr int kConvCtrlBytes = 1024;
 constexpr int kConvSmemBudget = 225 * 1024;
 
-template <int N_CTA, int MT>
+template <int N_CTA, int MT, bool SC = false>
 struct ConvCfg {
     static constexpr int kAccCols = N_CTA * MT;        // one accumulator set
-    static constexpr int kTmemCols = 2 * kAccCols;     // double-buffered: 256 or 512 columns
+    static constexpr int kTmemCols = (SC ? 4 : 2) * kAccCols;   // double-buffered (+ the shortcut's): 256 or 512 columns
+    static_assert(kTmemCols <= 512, "accumulators exceed tensor memory");
     static constexpr int kBStageBytes = N_CTA * kConvKC * 2;
     static constexpr int kTileM = 128 * MT;
-    // ctrl | bias fp32 [cout] | ones operand (2 planes x 128 rows x 16 B) | bias images (2 planes x cout rows x 16 B) | B | A
+    // ctrl | bias fp32 [cout] | ones operand (2 planes x 128 rows x 16 B) | bias images (2 planes x cout rows x 16 B) |
+    // SE scales | SC: shortcut bias images (as the bias images) + shortcut weights [cout][sc_cin] | B | A
     static constexpr int kOnesBytes = 2 * 128 * 16;
-    static size_t fixed_bytes(int cout, int bias_mma, int b_stages, int tps, int scale_bytes = 0) {
+    __host__ __device__ static size_t sc_bytes(int cout, int sc_cin) { return SC ? (size_t)cout * 32 + (size_t)cout * sc_cin * 2 : 0; }
+    static size_t fixed_bytes(int cout, int bias_mma, int b_stages, int tps, int scale_bytes = 0, int sc_cin = 0) {
         return kConvCtrlBytes + (size_t)cout * 4 + kOnesBytes + (bias_mma ? (size_t)cout * 32 : 0) + scale_bytes +
-               (size_t)b_stages * tps * kBStageBytes;
+               sc_bytes(cout, sc_cin) + (size_t)b_stages * tps * kBStageBytes;
     }
 };
 
-template <int N_CTA, int MT, bool BF16, bool FUSED>
+template <int N_CTA, int MT, bool BF16, bool FUSED, bool SC = false>
 __global__ void __launch_bounds__(kConvThreads, 1) conv_umma_kernel(const ConvParams p) {
-    using Cfg = ConvCfg<N_CTA, MT>;
+    static_assert(!SC || (FUSED && N_CTA <= 64), "the folded shortcut exists for the narrow conv2 epilogue only");
+    using Cfg = ConvCfg<N_CTA, MT, SC>;
     extern __shared__ __align__(128) uint8_t smem[];
     uint64_t* a_full = reinterpret_cast<uint64_t*>(smem);           // [kConvMaxAStages]
     uint64_t* a_empty = a_full + kConvMaxAStages;
@@ -103,12 +115,15 @@ __global__ void __launch_bounds__(kConvThreads, 1) conv_umma_kernel(const ConvPa
     uint64_t* b_empty = b_full + kConvBStages;
     uint64_t* acc_full = b_empty + kConvBStages;                    // [2]
     uint64_t* acc_empty = acc_full + 2;                             // [2]
-    uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(acc_empty + 2);
+    uint64_t* sc_full = acc_empty + 2;                              // SC: shortcut weights resident
+    uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(sc_full + 1);
     float* bias_s = reinterpret_cast<float*>(smem + kConvCtrlBytes);
     uint8_t* ones_smem = smem + kConvCtrlBytes + (size_t)p.cout * 4;
     uint8_t* biasimg_smem = ones_smem + Cfg::kOnesBytes;          // per N split: [2 planes][N_CTA rows][8 halves]
     float* scale_s = reinterpret_cast<float*>(biasimg_smem + (p.bias_mma ? (size_t)p.cout * 32 : 0));   // [n_utt][cout] SE scales
-    uint8_t* b_smem = reinterpret_cast<uint8_t*>(scale_s) + p.scale_smem_bytes;
+    uint8_t* sc_biasimg_smem = reinterpret_cast<uint8_t*>(scale_s) + p.scale_smem_bytes;
+    uint8_t* sc_w_smem = sc_biasimg_smem + (size_t)p.cout * 32;
+    uint8_t* b_smem = reinterpret_cast<uint8_t*>(scale_s) + p.scale_smem_bytes + Cfg::sc_bytes(p.cout, p.sc_cin);
     const uint32_t b_stage_bytes = (uint32_t)p.tps * Cfg::kBStageBytes;
     uint8_t* a_smem = b_smem + (size_t)p.b_stages * b_stage_bytes;
     const uint32_t a_stage_bytes = (uint32_t)p.rows_pad * (kConvKC / 8) * 16;
@@ -129,6 +144,7 @@ __global__ void __launch_bounds__(kConvThreads, 1) conv_umma_kernel(const ConvPa
         for (int i = 0; i < kConvMaxAStages; ++i) { mbar_init(&a_full[i], 1); mbar_init(&a_empty[i], 2); }
         for (int i = 0; i < kConvBStages; ++i) { mbar_init(&b_full[i], 1); mbar_init(&b_empty[i], 2); }   // first b_stages used
         for (int i = 0; i < 2; ++i) { mbar_init(&acc_full[i], 2); mbar_init(&acc_empty[i], 8); }
+        if (SC) mbar_init(sc_full, 1);
         fence_barrier_init();
     }
     for (int i = threadIdx.x; i < p.cout; i += blockDim.x) bias_s[i] = p.bias[i];
@@ -138,16 +154,20 @@ __global__ void __launch_bounds__(kConvThreads, 1) conv_umma_kernel(const ConvPa
         const uint32_t one2 = pack2<BF16>(1.f, 1.f);
         for (int i = threadIdx.x; i < 2 * 128; i += blockDim.x)
             reinterpret_cast<uint4*>(ones_smem)[i] = make_uint4(i < 128 ? one2 : 0u, 0u, 0u, 0u);
-        for (int i = threadIdx.x; i < 2 * p.cout; i += blockDim.x) {
-            const int ns = (i % p.cout) / N_CTA, n = (i % p.cout) % N_CTA, plane = i / p.cout;
-            uint32_t w0 = 0u;
-            if (plane == 0) {
-                const float b = p.bias[ns * N_CTA + n];
-                const float2 hi2 = unpack2<BF16>(pack2<BF16>(b, 0.f));
-                w0 = pack2<BF16>(b, b - hi2.x);
+        auto bias_images = [&](const float* bias, uint8_t* dst) {
+            for (int i = threadIdx.x; i < 2 * p.cout; i += blockDim.x) {
+                const int ns = (i % p.cout) / N_CTA, n = (i % p.cout) % N_CTA, plane = i / p.cout;
+                uint32_t w0 = 0u;
+                if (plane == 0) {
+                    const float b = bias[ns * N_CTA + n];
+                    const float2 hi2 = unpack2<BF16>(pack2<BF16>(b, 0.f));
+                    w0 = pack2<BF16>(b, b - hi2.x);
+                }
+                reinterpret_cast<uint4*>(dst)[(size_t)ns * 2 * N_CTA + plane * N_CTA + n] = make_uint4(w0, 0u, 0u, 0u);
             }
-            reinterpret_cast<uint4*>(biasimg_smem)[(size_t)ns * 2 * N_CTA + plane * N_CTA + n] = make_uint4(w0, 0u, 0u, 0u);
-        }
+        };
+        bias_images(p.bias, biasimg_smem);
+        if (SC) bias_images(p.sc_bias, sc_biasimg_smem);
         asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
     }
     if (warp == 2) tmem_alloc<Cfg::kTmemCols>(tmem_slot);
@@ -182,12 +202,32 @@ __global__ void __launch_bounds__(kConvThreads, 1) conv_umma_kernel(const ConvPa
                     }
                     if (++s == p.a_stages) { s = 0; ph ^= 1; }
                 }
+                if constexpr (SC) {
+                    // shortcut chunks: the tile's own pixels, no halo (same plane stride inside the stage as the slab)
+                    constexpr uint32_t sc_plane_bytes = Cfg::kTileM * 16;
+                    const long long qs = q0 + p.halo;
+                    for (int kc = 0; kc < p.sc_cin / kConvKC; ++kc) {
+                        mbar_wait(&a_empty[s], ph);
+                        mbar_arrive_expect_tx(&a_full[s], (kConvKC / 8) * sc_plane_bytes);
+#pragma unroll
+                        for (int j = 0; j < kConvKC / 8; ++j) {
+                            const uint16_t* src = p.sc_in + ((size_t)(kc * (kConvKC / 8) + j) * p.in_plane + qs) * 8;
+                            bulk_g2s(a_smem + (size_t)s * a_stage_bytes + j * plane_bytes, src, sc_plane_bytes, &a_full[s]);
+                        }
+                        if (++s == p.a_stages) { s = 0; ph ^= 1; }
+                    }
+                }
             }
         }
     } else if (warp == 1) {
         // ---------------------------------------------------------------- B producer: packed weights
         if (lane == 0) {
             const int n_it = p.n_pairs;                // weight images per item
+            if constexpr (SC) {
+                const uint32_t bytes = (uint32_t)p.cout * p.sc_cin * 2;
+                mbar_arrive_expect_tx(sc_full, bytes);
+                bulk_g2s(sc_w_smem, p.sc_w, bytes, sc_full);
+            }
             if (p.b_resident) {
                 // small layers: the whole weight tensor stays in shared memory for the life of the CTA
                 mbar_arrive_expect_tx(&b_full[0], (uint32_t)n_it * Cfg::kBStageBytes);
@@ -232,6 +272,12 @@ __global__ void __launch_bounds__(kConvThreads, 1) conv_umma_kernel(const ConvPa
             mbar_wait(&b_full[0], 0);
             tc_fence_after();
         }
+        if constexpr (SC) {
+            mbar_wait(sc_full, 0);
+            tc_fence_after();
+        }
+        const uint64_t ones_desc = (static_cast<uint64_t>(2048 >> 4) << 16) | (static_cast<uint64_t>(128 >> 4) << 32) |
+                                   (static_cast<uint64_t>(1) << 46) | ((smem_u32(ones_smem) >> 4) & 0x3FFF);
         for (int item = item_begin; item < item_end; ++item, ++n_done) {
             const int buf = (int)(n_done & 1);
             mbar_wait(&acc_empty[buf], ((n_done >> 1) & 1) ^ 1);
@@ -240,8 +286,6 @@ __global__ void __launch_bounds__(kConvThreads, 1) conv_umma_kernel(const ConvPa
             const int ns_item = ns;
             if (++ns == n_split) ns = 0;
             if (p.bias_mma && elect_one()) {
-                const uint64_t ones_desc = (static_cast<uint64_t>(2048 >> 4) << 16) | (static_cast<uint64_t>(128 >> 4) << 32) |
-                                           (static_cast<uint64_t>(1) << 46) | ((smem_u32(ones_smem) >> 4) & 0x3FFF);
                 const uint32_t img = smem_u32(biasimg_smem) + (uint32_t)ns_item * 2 * N_CTA * 16;
                 const uint64_t bias_desc = desc_hi_b | ((img >> 4) & 0x3FFF);
 #pragma unroll
@@ -293,6 +337,38 @@ __global__ void __launch_bounds__(kConvThreads, 1) conv_umma_kernel(const ConvPa
                 if (++as == p.a_stages) { as = 0; a_ph ^= 1; }
                 if (++in_grp == p.kc_per_grp) { in_grp = 0; ++grp; }
             }
+            if constexpr (SC) {
+                // the shortcut's accumulator: bias MMA, then its k-chunks in order -- a stand-alone 1x1 launch's sequence
+                const uint32_t dsc_tmem = tmem_base + (2 + buf) * Cfg::kAccCols;
+                if (elect_one()) {
+                    const uint32_t img = smem_u32(sc_biasimg_smem) + (uint32_t)ns_item * 2 * N_CTA * 16;
+                    const uint64_t bias_desc = desc_hi_b | ((img >> 4) & 0x3FFF);
+#pragma unroll
+                    for (int mt = mtw0; mt < mtw0 + MTW; ++mt) umma_f16(dsc_tmem + mt * N_CTA, ones_desc, bias_desc, idesc, 0u);
+                }
+                __syncwarp();
+                const int sc_kc = p.sc_cin / kConvKC;
+                for (int kc = 0; kc < sc_kc; ++kc) {
+                    mbar_wait(&a_full[as], a_ph);
+                    tc_fence_after();
+                    const uint32_t a_base = smem_u32(a_smem + (size_t)as * a_stage_bytes);
+                    const uint32_t b_img = smem_u32(sc_w_smem) + (uint32_t)(ns_item * sc_kc + kc) * Cfg::kBStageBytes;
+                    if (elect_one()) {
+#pragma unroll
+                        for (int ks = 0; ks < kConvKC / 16; ++ks) {
+                            const uint64_t bdesc = desc_hi_b | (((b_img + ks * 2 * b_lbo) >> 4) & 0x3FFF);
+#pragma unroll
+                            for (int mt = mtw0; mt < mtw0 + MTW; ++mt) {
+                                const uint64_t adesc = desc_hi_a | (((a_base + ks * 2 * a_lbo + mt * 2048) >> 4) & 0x3FFF);
+                                umma_f16(dsc_tmem + mt * N_CTA, adesc, bdesc, idesc, 1u);
+                            }
+                        }
+                        umma_commit(&a_empty[as]);
+                    }
+                    __syncwarp();
+                    if (++as == p.a_stages) { as = 0; a_ph ^= 1; }
+                }
+            }
             if (elect_one()) umma_commit(&acc_full[buf]);
             __syncwarp();
         }
@@ -334,12 +410,13 @@ __global__ void __launch_bounds__(kConvThreads, 1) conv_umma_kernel(const ConvPa
                 }
             }
         };
+        constexpr bool kLoadRes = FUSED && !SC;  // with SC the residual is the shortcut accumulator in TMEM
         uint32_t omax = 0u;                     // fp16 range guard: max |x| of what this thread stored
         int bidx_c[MTH], opix_c[MTH], bidx_n[MTH], opix_n[MTH], bidx_nn[MTH], opix_nn[MTH];
         uint4 rv_c[MTH][NCH], rv_n[MTH][NCH];
         fetch_meta(item_begin, bidx_c, opix_c);
         fetch_meta(item_begin + 1, bidx_n, opix_n);
-        if (FUSED) fetch_res(item_begin, bidx_c, rv_c);
+        if (kLoadRes) fetch_res(item_begin, bidx_c, rv_c);
         uint32_t n_done = 0;
         // fused channel totals (see ConvParams::sums): this thread's pixels stay inside one utterance for hundreds of
         // consecutive tiles, so the totals live in registers and reach memory only when the utterance changes
@@ -363,7 +440,7 @@ __global__ void __launch_bounds__(kConvThreads, 1) conv_umma_kernel(const ConvPa
             const int tile = item / n_split;
             const int n_base = (item - tile * n_split) * N_CTA;
             const int buf = (int)(n_done & 1);
-            if (FUSED) fetch_res(item + 1, bidx_n, rv_n);                  // its metadata arrived during the previous item
+            if (kLoadRes) fetch_res(item + 1, bidx_n, rv_n);               // its metadata arrived during the previous item
             fetch_meta(item + 2, bidx_nn, opix_nn);
             mbar_wait(&acc_full[buf], (n_done >> 1) & 1);
             tc_fence_after();
@@ -389,8 +466,9 @@ __global__ void __launch_bounds__(kConvThreads, 1) conv_umma_kernel(const ConvPa
                             for (int k = 0; k < 4; ++k) sc4[k] = __ldg(sp + k);
                         }
                     }
-                    float v[16];
+                    float v[16], r[16];
                     tmem_ld16(tmem_base + ((uint32_t)(q * 32) << 16) + buf * Cfg::kAccCols + (mt0 + mt) * N_CTA + c0, v);
+                    if (SC) tmem_ld16(tmem_base + ((uint32_t)(q * 32) << 16) + (2 + buf) * Cfg::kAccCols + (mt0 + mt) * N_CTA + c0, r);
                     if (c0 + 16 >= N_CTA && mt == MTH - 1) {
                         // accumulator completely read: hand this TMEM buffer back to the MMA warp
                         tc_fence_before();
@@ -401,7 +479,19 @@ __global__ void __launch_bounds__(kConvThreads, 1) conv_umma_kernel(const ConvPa
 #pragma unroll
                         for (int i = 0; i < 16; ++i) v[i] += bias_s[n_base + c0 + i];
                     }
-                    if (FUSED && valid) {
+                    if (SC && valid) {
+                        // the residual as a stand-alone shortcut launch would have stored it (16-bit, fp16 range guard included)
+                        const float scv[16] = {sc4[0].x, sc4[0].y, sc4[0].z, sc4[0].w, sc4[1].x, sc4[1].y, sc4[1].z, sc4[1].w,
+                                               sc4[2].x, sc4[2].y, sc4[2].z, sc4[2].w, sc4[3].x, sc4[3].y, sc4[3].z, sc4[3].w};
+#pragma unroll
+                        for (int i = 0; i < 8; ++i) {
+                            const uint32_t rw = pack2<BF16>(r[2 * i], r[2 * i + 1]);
+                            if (!BF16) track16(rw, omax);
+                            const float2 r2 = unpack2<BF16>(rw);
+                            v[2 * i] = fmaf(v[2 * i], scv[2 * i], r2.x);
+                            v[2 * i + 1] = fmaf(v[2 * i + 1], scv[2 * i + 1], r2.y);
+                        }
+                    } else if (kLoadRes && valid) {
                         const uint32_t rw[8] = {rv_c[mt][cc].x, rv_c[mt][cc].y, rv_c[mt][cc].z, rv_c[mt][cc].w,
                                                 rv_c[mt][cc + 1].x, rv_c[mt][cc + 1].y, rv_c[mt][cc + 1].z, rv_c[mt][cc + 1].w};
                         const float scv[16] = {sc4[0].x, sc4[0].y, sc4[0].z, sc4[0].w, sc4[1].x, sc4[1].y, sc4[1].z, sc4[1].w,
@@ -447,8 +537,10 @@ __global__ void __launch_bounds__(kConvThreads, 1) conv_umma_kernel(const ConvPa
             for (int mt = 0; mt < MTH; ++mt) {
                 bidx_c[mt] = bidx_n[mt]; opix_c[mt] = opix_n[mt];
                 bidx_n[mt] = bidx_nn[mt]; opix_n[mt] = opix_nn[mt];
+                if (kLoadRes) {
 #pragma unroll
-                for (int k = 0; k < NCH; ++k) rv_c[mt][k] = rv_n[mt][k];
+                    for (int k = 0; k < NCH; ++k) rv_c[mt][k] = rv_n[mt][k];
+                }
             }
         }
         if (kCanSum && do_sums) flush_sums();

@@ -1121,7 +1121,8 @@ static int build_pixmeta(skb_xtractor* h, cudaStream_t st) {
 // phase-split buffer of the next level (`Lnext`).
 static int run_conv(skb_xtractor* h, const ConvW& cw, int kind, const Level& Lg, const uint16_t* in, uint16_t* out, int act,
                     const int* tdnn_shifts, const float* se_scale, const uint16_t* res, const Level* pix_level,
-                    const Level* Lnext, cudaStream_t st, unsigned long long* sums = nullptr) {
+                    const Level* Lnext, cudaStream_t st, unsigned long long* sums = nullptr, const ConvW* sc = nullptr,
+                    const uint16_t* sc_in = nullptr) {
     ConvParams p;
     memset(&p, 0, sizeof(p));
     p.in = in; p.in_plane = Lg.plane; p.w = cw.w; p.bias = cw.bias; p.out = out;
@@ -1171,6 +1172,7 @@ static int run_conv(skb_xtractor* h, const ConvW& cw, int kind, const Level& Lg,
     p.res_plane = Lg.plane;
     p.sums = (sums != nullptr && cw.ncta == 32 && cw.cout == 32 && se_scale == nullptr) ? sums : nullptr;
     p.overflow = (unsigned*)h->ovf.p;
+    if (sc) { p.sc_in = sc_in; p.sc_w = sc->w; p.sc_bias = sc->bias; p.sc_cin = sc->cin; }
     g_launches++;
     return launch_conv_umma(p, cw.ncta, h->m.bf16, st);
 }
@@ -1254,6 +1256,12 @@ static bool no_fused_sums() {
     return v == 1;
 }
 
+// SKB_UNFUSED_SHORTCUT=1: run the 1x1 shortcuts as stand-alone launches through a 16-bit buffer (A/B knob, test reference)
+static bool unfused_shortcut() {
+    static const bool v = [] { const char* e = getenv("SKB_UNFUSED_SHORTCUT"); return e && e[0] == '1'; }();
+    return v;
+}
+
 static int forward_hr34(skb_xtractor* h, const float* wave, int norm_embedding, float* emb_out, float* logits_out,
                         const char* stop, int h_max, float* dbg_out, int64_t* per_utt, cudaStream_t st) {
     const Model& m = h->m;
@@ -1302,12 +1310,15 @@ static int forward_hr34(skb_xtractor* h, const float* wave, int norm_embedding, 
         uint16_t *y1 = buf(level, 2), *scb = buf(level, 4), *nxt = buf(level, cur ^ 1);
         const bool sums_in_conv1 = bw.conv1.ncta == 32 && bw.conv1.cout == 32 && !no_fused_sums();
         const uint16_t* res = x;
+        // narrow layers: conv2 computes the 1x1 shortcut itself, in a second TMEM accumulator (no launch, no round trip
+        // of the shortcut through HBM); the <128, 2> tiles have no tensor memory left for it
+        const bool fold_sc = bw.has_sc && bw.conv2.ncta <= 64 && bw.sc.ncta == bw.conv2.ncta && !unfused_shortcut();
         {
             ProfScope ps(PROF_CONV, st);
             // 32-channel layers: conv1's epilogue also accumulates the per-utterance channel totals of y1 (no plane_sum pass)
             SKB_TRY(run_conv(h, bw.conv1, bw.stride == 2 ? 3 : 1, L, x, y1, 1, nullptr, nullptr, nullptr, nullptr, nullptr, st,
                              sums_in_conv1 ? (unsigned long long*)h->sums.p : nullptr));
-            if (bw.has_sc) {
+            if (bw.has_sc && !fold_sc) {
                 // 1x1 shortcut; with stride 2 it reads phase (0, 0) = the first C_prev/8 planes of the phase-split input
                 SKB_TRY(run_conv(h, bw.sc, 0, L, x, scb, 0, nullptr, nullptr, nullptr, nullptr, nullptr, st));
                 res = scb;
@@ -1335,8 +1346,8 @@ static int forward_hr34(skb_xtractor* h, const float* wave, int norm_embedding, 
             // conv2 with the fused SE tail: out = relu(bn2(conv2(y1)) * scale + residual)
             ProfScope ps(PROF_CONV, st);
             uint16_t* dst = next_strides ? buf(level + 1, 3) : nxt;
-            SKB_TRY(run_conv(h, bw.conv2, 1, L, y1, dst, 1, nullptr, (const float*)h->scale.p, res, nullptr,
-                             next_strides ? &pl.lv[level + 1] : nullptr, st));
+            SKB_TRY(run_conv(h, bw.conv2, 1, L, y1, dst, 1, nullptr, (const float*)h->scale.p, fold_sc ? nullptr : res, nullptr,
+                             next_strides ? &pl.lv[level + 1] : nullptr, st, nullptr, fold_sc ? &bw.sc : nullptr, x));
         }
         x_is_ps = next_strides;
         g_launches += 4;
