@@ -57,21 +57,13 @@ bool sync_check_enabled();
 // (barrier init, TMEM allocation, constant weights), and pdl_wait() -- executed by every such kernel before it reads or
 // writes anything another kernel touches -- blocks until kernel k has completed and its writes are visible.
 // Measured (profiles/r01g_pdl.txt): 8.53 -> 8.45 ms per HalfResNet34 step, e2e +1.5 %.  An EARLY trigger
-// (griddepcontrol.launch_dependents at the top of every kernel, SKB_PDL_EARLY_TRIGGER=1) lets the whole chain park on the
-// SMs while conv1 still runs and is slower (8.7-8.8 ms), so the implicit trigger at CTA exit is what ships.
+// (griddepcontrol.launch_dependents at the top of every kernel) lets the whole chain park on the SMs while conv1 still runs
+// and is slower (8.7-8.8 ms), so the implicit trigger at CTA exit is what the chain uses.
 // SKB_NO_PDL=1 launches everything with plain stream order (A/B knob); pdl_wait() is then a no-op.
 __device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
-#ifndef SKB_PDL_EARLY_TRIGGER
-#define SKB_PDL_EARLY_TRIGGER 0
-#endif
-__device__ __forceinline__ void pdl_trigger() {
-#if SKB_PDL_EARLY_TRIGGER
-    asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
-#endif
-}
-// explicit trigger (whatever SKB_PDL_EARLY_TRIGGER says): the next kernel of the stream may be scheduled once every CTA of
-// this grid has got here -- used by se_border_kernel AFTER its own pdl_wait, so that the channel-total pass that follows
-// (which needs nothing from the border sums) runs beside it instead of behind it
+// explicit trigger: the next kernel of the stream may be scheduled once every CTA of this grid has got here -- used by
+// se_border_kernel AFTER its own pdl_wait, so that the channel-total pass that follows (which needs nothing from the border
+// sums) runs beside it instead of behind it
 __device__ __forceinline__ void pdl_trigger_now() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
 bool pdl_enabled();
 template <typename... KArgs, typename... Args>

@@ -173,7 +173,6 @@ __global__ void __launch_bounds__(kConvThreads, 1) conv_umma_kernel(const ConvPa
     if (warp == 2) tmem_alloc<Cfg::kTmemCols>(tmem_slot);
     // everything above touches only constants (weights, bias) and this CTA's shared / tensor memory: it overlaps the tail of
     // the previous kernel of the stream.  From here on the kernel reads what that kernel wrote.
-    pdl_trigger();
     pdl_wait();
     if (FUSED && p.scale_smem_bytes > 0)
         for (int i = threadIdx.x; i < p.scale_smem_bytes / 4; i += blockDim.x) scale_s[i] = p.se_scale[i];

@@ -1331,16 +1331,12 @@ static int forward_hr34(skb_xtractor* h, const float* wave, int norm_embedding, 
             // Measured and rejected in round 2 (profiles/r02_se_merge.txt): border sums + channel totals in one launch, and the FC
             // layers done by the last-arriving partial-mean CTA -- fewer launches, but both variants were slower.
             // Kept from that experiment's lesson -- separate kernels with their own occupancy -- but OVERLAPPED: the border sums
-            // go first and release the channel-total pass as soon as they have seen conv1 complete (SKB_SE_SERIAL=1: one after
-            // the other, as in round 1)
-            static const bool se_serial = getenv("SKB_SE_SERIAL") != nullptr;
+            // go first and release the channel-total pass as soon as they have seen conv1 complete (faster than one after the
+            // other: profiles/r02u_se_overlap_vs_serial.txt)
             const PlaneSumArgs totals = {L.p_end, pm + L.o_pix_b, pm + L.o_span};
-            if (!sums_in_conv1 && se_serial)
-                SKB_TRY(launch_plane_sum(m.bf16, y1, L.plane, L.G, L.p_end, pm + L.o_pix_b, pm + L.o_span, bw.C,
-                                         (unsigned long long*)h->sums.p, st));
             SKB_TRY(launch_se_scale(m.bf16, (unsigned long long*)h->sums.p, y1, L.plane, L.G, L.Wp, L.W, d32 + L.o_utt_row0,
                                     d32 + L.o_utt_count, B, bw.C, bw.C, bw.w2t, bw.conv2.bias, bw.se_w1, bw.se_w2,
-                                    (float*)h->brd.p, (float*)h->scale.p, st, (!sums_in_conv1 && !se_serial) ? &totals : nullptr));
+                                    (float*)h->brd.p, (float*)h->scale.p, st, sums_in_conv1 ? nullptr : &totals));
         }
         {
             // conv2 with the fused SE tail: out = relu(bn2(conv2(y1)) * scale + residual)

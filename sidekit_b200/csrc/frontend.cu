@@ -436,15 +436,7 @@ size_t frontend_cmvn_scratch_bytes(const FrontendConsts& fc, int B, int t_max) {
 }
 
 // feats: frame-major [sum T][n_out]; api_out optional (B, n_out, t_max).
-// frames per warp of a CTA (experiment knob: SKB_FE_FPW)
-static int fpw_override(int dflt) {
-    static int v = -1;
-    if (v < 0) {
-        const char* e = getenv("SKB_FE_FPW");
-        v = e ? atoi(e) : 0;
-    }
-    return v > 0 ? v : dflt;
-}
+constexpr int kFramesPerWarp = 8;   // frames each warp of a CTA transforms
 
 int frontend_launch(const FrontendConsts& fc, const float* wave, const long long* wave_off, const int* wave_len,
                     const long long* feat_off, const int* n_frames, int B, int t_max, float* feats, float2* cmvn,
@@ -475,7 +467,7 @@ int frontend_launch(const FrontendConsts& fc, const float* wave, const long long
     };
     if (fc.n_fft == 1024) {
         constexpr int NC = 512, WPC = 8;
-        const int frames_per_cta = fpw_override(8) * WPC;
+        const int frames_per_cta = kFramesPerWarp * WPC;
         dim3 grid((t_max + frames_per_cta - 1) / frames_per_cta, B);
         const size_t smem = smem_bytes(NC, WPC, &p.dct_smem_off);
         static PerDeviceOnce configured;
@@ -490,7 +482,7 @@ int frontend_launch(const FrontendConsts& fc, const float* wave, const long long
     } else if (fc.n_fft == 2048) {
         // a frame needs 9.3 KB of shared memory and the tables 52 KB: 16 frame-warps in one CTA per SM
         constexpr int NC = 1024, WPC = 16;
-        const int frames_per_cta = fpw_override(8) * WPC;
+        const int frames_per_cta = kFramesPerWarp * WPC;
         dim3 grid((t_max + frames_per_cta - 1) / frames_per_cta, B);
         const size_t smem = smem_bytes(NC, WPC, &p.dct_smem_off);
         static PerDeviceOnce configured;

@@ -309,17 +309,15 @@ __device__ __forceinline__ void plane_sum_body(const uint16_t* __restrict__ act,
     }
 }
 
-// beside_previous = 1: the previous kernel of the stream is se_border_kernel, which waited for conv1 BEFORE it let this grid
-// start and whose results this kernel does not use -- so the sums start at once, beside the border CTAs, and the wait
-// moves to the end (this grid must not complete before the border grid: the kernel after it waits for this one only).
+// The previous kernel of the stream is se_border_kernel, which waited for conv1 BEFORE it let this grid start and whose
+// results this kernel does not use -- so the sums start at once, beside the border CTAs, and the wait is at the end (this
+// grid must not complete before the border grid: the kernel after it waits for this one only).
 template <bool BF16>
 __global__ void __launch_bounds__(256, 4) plane_sum_kernel(const uint16_t* __restrict__ act, long long plane, int G, int p_end,
                                                         const int* __restrict__ pix_b, const int* __restrict__ span_b, int C,
-                                                        int planes_per_block, unsigned long long* __restrict__ sums, int beside_previous) {
-    pdl_trigger();
-    if (!beside_previous) pdl_wait();
+                                                        int planes_per_block, unsigned long long* __restrict__ sums) {
     plane_sum_body<BF16>(act, plane, G, p_end, pix_b, span_b, C, planes_per_block, sums);
-    if (beside_previous) pdl_wait();
+    pdl_wait();
 }
 
 // span_b table for plane_sum_kernel (built once per batch composition)
@@ -346,17 +344,17 @@ int launch_span_table(const int* pix_b, int n_pix, int* span_b, cudaStream_t st)
     return SKB_OK;
 }
 
-int launch_plane_sum(bool bf16, const uint16_t* act, long long plane, int G, int p_end, const int* pix_b, const int* span_b, int C,
-                     unsigned long long* sums, cudaStream_t st, bool beside_previous) {
+static int launch_plane_sum(bool bf16, const uint16_t* act, long long plane, int G, int p_end, const int* pix_b, const int* span_b,
+                            int C, unsigned long long* sums, cudaStream_t st) {
     const int n = p_end - G;
     const int n_spans = span_table_size(n);
     const int chunks = C / 8;
     const int ppb = chunks >= 16 ? 4 : (chunks >= 8 ? 2 : 1);      // keep >= ~4 waves of CTAs on the small levels
     dim3 grid((n_spans + 7) / 8, chunks / ppb);
     if (bf16)
-        SKB_CUDA_CHECK(launch_pdl(plane_sum_kernel<true>, grid, dim3(256), 0, st, act, plane, G, p_end, pix_b, span_b, C, ppb, sums, beside_previous ? 1 : 0));
+        SKB_CUDA_CHECK(launch_pdl(plane_sum_kernel<true>, grid, dim3(256), 0, st, act, plane, G, p_end, pix_b, span_b, C, ppb, sums));
     else
-        SKB_CUDA_CHECK(launch_pdl(plane_sum_kernel<false>, grid, dim3(256), 0, st, act, plane, G, p_end, pix_b, span_b, C, ppb, sums, beside_previous ? 1 : 0));
+        SKB_CUDA_CHECK(launch_pdl(plane_sum_kernel<false>, grid, dim3(256), 0, st, act, plane, G, p_end, pix_b, span_b, C, ppb, sums));
     SKB_LAUNCH_CHECK(st);
     return SKB_OK;
 }
@@ -449,7 +447,6 @@ __global__ void __launch_bounds__(256) se_mean_partial_kernel(const unsigned lon
 #pragma unroll
         for (int i = 0; i < RPT; ++i) wreg[i] = __ldg(wp + (size_t)i * n_rg * Cout);
     }
-    pdl_trigger();
     pdl_wait();                                    // the weight loads above are constants: they overlap the previous kernel
     const int k0 = blockIdx.x * kSeRows, b0 = blockIdx.y * kSeUtt;
     const int nu = min(kSeUtt, B - b0);
@@ -516,7 +513,6 @@ __global__ void __launch_bounds__(256) se_fc_kernel(unsigned long long* __restri
                                                     const float* __restrict__ fc2 /*[Cout][Cout/16]*/, float* __restrict__ scale) {
     __shared__ float mean[256];
     __shared__ float hid[16];
-    pdl_trigger();
     pdl_wait();
     const int b = blockIdx.x;
     const float inv_n = 1.f / (float)utt_count[b];
@@ -559,7 +555,7 @@ int launch_se_scale(bool bf16, unsigned long long* sums, const uint16_t* y1, lon
     SKB_LAUNCH_CHECK(st);
     // the channel totals (when conv1's epilogue did not produce them) run BESIDE the border sums: see plane_sum_kernel
     if (totals) {
-        int rc = launch_plane_sum(bf16, y1, plane, G, totals->p_end, totals->pix_b, totals->span_b, Cin, sums, st, true);
+        int rc = launch_plane_sum(bf16, y1, plane, G, totals->p_end, totals->pix_b, totals->span_b, Cin, sums, st);
         if (rc) return rc;
     }
     const int n_slices = Cin / kSeCh;

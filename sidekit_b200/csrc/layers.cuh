@@ -26,8 +26,6 @@ int launch_stem7(bool bf16, const float* feats, const long long* feat_off, const
                  const StemConsts& sc, uint16_t* out, long long out_plane, int G, int p_end, int Wp, int W, int F,
                  const int* row_b, const int* row_h, unsigned* overflow, cudaStream_t st);
 int launch_broadcast_rows(const float* bias, int B, int A, float* out, cudaStream_t st);
-int launch_plane_sum(bool bf16, const uint16_t* act, long long plane, int G, int p_end, const int* pix_b, const int* span_b, int C,
-                     unsigned long long* sums, cudaStream_t st, bool beside_previous = false);
 struct PlaneSumArgs { int p_end; const int* pix_b; const int* span_b; };   // launch_se_scale: channel totals beside the border sums
 int span_table_size(int n_pix);
 int launch_span_table(const int* pix_b, int n_pix, int* span_b, cudaStream_t st);

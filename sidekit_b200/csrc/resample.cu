@@ -111,9 +111,7 @@ extern "C" int skb_resample(const float* in_dev, const int64_t* wave_meta_dev, i
     if (max_out == 0) return SKB_OK;
     cudaStream_t st = (cudaStream_t)stream;
     // a CTA takes pcta whole periods; its taps span pcta * orig_r + 2 * width input samples
-    int out_per_cta = kOutPerCta;
-    if (const char* e = getenv("SKB_RESAMPLE_OUT")) out_per_cta = atoi(e) > 0 ? atoi(e) : kOutPerCta;      // tuning knob
-    const int pcta = out_per_cta / new_r > 0 ? out_per_cta / new_r : 1;
+    const int pcta = kOutPerCta / new_r > 0 ? kOutPerCta / new_r : 1;
     const long long win_len = (long long)pcta * orig_r + 2 * width;
     const size_t smem = ((size_t)ntap * new_r + new_r + (size_t)win_len + (new_r > 2 ? (size_t)pcta * (new_r + 1) : 0)) * 4;
     if (smem > 200 * 1024) {

@@ -12,10 +12,11 @@
 // DEVICE from the operands' row norms (no host sync).
 //
 // Kernel: persistent CTAs, each owning a contiguous run of (row panel, column tile) pairs in
-// panel-major order.  The 128-row E panel stays resident in shared memory; 128-column T tiles stream
-// through a ring of 64-deep K chunks (1-D bulk copies); accumulators are double-buffered in TMEM so
-// the epilogue of tile i overlaps the MMAs of tile i+1.  The score matrix is HBM-write-bound
-// (128 FLOP per output byte at D = 256), so the epilogue transposes each 32x32 block through a
+// panel-major order.  For K <= 256 the 128-row E panel stays resident in tensor memory and 128-column
+// T tiles stream through a ring of 64- or 128-wide K stages (1-D bulk copies); for larger K (the dense
+// layers of the extractor) E and T chunks stream through the ring together.  Accumulators are
+// double-buffered in TMEM so the epilogue of tile i overlaps the MMAs of tile i+1.  The score matrix
+// is HBM-write-bound (128 FLOP per output byte at D = 256), so the epilogue transposes each 32x32 block through a
 // warp-private shared buffer and every store instruction writes one full 128-byte row segment.
 #include "sidekit_b200.h"
 #include "common.cuh"
@@ -189,7 +190,7 @@ __global__ void __launch_bounds__(256) pack_split_kernel(const PackArgs a, int D
 // ----------------------------------------------------------------------------- the GEMM
 struct ScoreParams {
     const uint16_t *Ehi, *Elo, *Thi, *Tlo;   // [rows_pad/128][Dp/8][128][8]
-    int Ne, Nt, Ne_pad, Nt_pad, Dp, D;
+    int Ne, Nt, Ne_pad, Dp, D;
     const int *expE, *expT;                   // per-operand scale exponents (on the device)
     const unsigned *statsE, *statsT;          // operand statistics: the pass count is decided from them on the device
     float abs_alpha;
@@ -200,7 +201,6 @@ struct ScoreParams {
     int mul_scaled;                           // 1: ra / ca are also divided by the operand scales
     void* out;
     long long ld_out;
-    int out_f64;                              // == (out_mode == 1); kept for the epilogue's existing tests
     int out_mode;                             // 0 = float32 matrix, 1 = float64 matrix, 2 = float16 matrix, 3 = trial list
     // trial-list mode: only the trials of a mask are written, compacted in row-major order (what the reference selects with
     // scoremat[trialmask], sidekit/nnet/xvector.py:243-245): bit j of mask_words[row][w] = trial (row, 32 w + j),
@@ -208,7 +208,7 @@ struct ScoreParams {
     const uint32_t* mask_words;
     const uint32_t* word_off;
     int mask_ld;
-    int tiles_total, n_ntiles;
+    int n_ntiles;
     // top-k mode (out_mode 4): every epilogue warp keeps the best topk_k (score, column) keys of each of its rows among the
     // columns it visits and leaves them, when it moves off a row panel, in out = uint64 [Ne][topk_segs][topk_k] (see
     // topk_segment); topk_merge_kernel selects the final k from those partial lists.
@@ -278,63 +278,42 @@ __device__ __forceinline__ float topk_screen(unsigned long long kth) {
 
 constexpr int kScKChunk = 64;
 
-// smem: [ctrl 256 B][A hi (+lo)][B ring][8 warps x [32][36] fp32 transpose buffers]
-// MT = row panels per work item (resident-panel single-pass variant only): with MT = 2 a streamed T tile feeds TWO 128-row
-// panels, which halves the L2 -> shared-memory operand traffic per trial (64 KB per 128 x 128 tile at MT = 1: at 20k x 20k
-// that is 1.6 GB per call, as much as the fp32 matrix itself, and what bounds the modes that do not write the matrix).
+// smem: [ctrl 256 B][E staging piece][B ring][8 warps x [32][36] fp32 transpose buffers]
 // KC = K elements per ring stage of the single-pass resident-panel variant (64 or 128).  Every tcgen05.commit costs the
 // tensor pipe a drain of ~140 ns (the MMAs behind it do not start before the ones in front have completed): with 64-wide
 // stages a 128 x 128 x 256 tile is 4 x (4 MMAs + commit) and the pipe idles 60 % of the time; 128-wide stages (8 MMAs per
 // commit, 32 KB bulk copies) take the MMA-only time of a 20k x 20k call from 0.246 to 0.200 ms
 // (profiles/r02x_score_issue_bound.txt).
-#ifndef SKB_KC128_STAGES
-#define SKB_KC128_STAGES 3      // 32 KB stages of the 128-wide variant (4 fit since the E panel is staged through 32 KB, and are slower: profiles/r02x_score_issue_bound.txt)
-#endif
-template <int PASSES, bool STREAM_A, int MT = 1, int KC = 64>
+constexpr int kKc128Stages = 3;   // 32 KB stages of the 128-wide variant (4 fit since the E panel is staged through 32 KB, and are slower: profiles/r02x_score_issue_bound.txt)
+constexpr int kAPieceK = 128;     // E staging piece: 128 K-columns (32 KB) measured faster than 64 and 32 (profiles/r02x_score_issue_bound.txt)
+template <int PASSES, bool STREAM_A, int KC = 64>
 struct ScoreSmem {
     static constexpr int kParts = PASSES == 1 ? 1 : 2;
-    static_assert(KC == 64 || ((KC == 128 || KC == 256) && PASSES == 1 && !STREAM_A && MT == 1), "wide stages: single-pass resident-panel variant only");
+    static_assert(KC == 64 || (KC == 128 && PASSES == 1 && !STREAM_A), "128-wide stages: single-pass resident-panel variant only");
     static constexpr int kChunk = PASSES == 1 ? KC : 32;              // K elements per stage
     static constexpr int kStageBytes = 128 * kChunk * 2;              // one part (hi or lo) of one operand of one stage
     // resident-panel mode: a stage holds a T chunk; streaming mode (large K): an E chunk and a T chunk
     static constexpr int kRingStageBytes = (STREAM_A ? 2 : 1) * kParts * kStageBytes;
-    // Epilogue warps (SKB_SCORE_EPI16 compile-time switch: 16 warps with one 32-column block each for the single-pass /
-    // streaming variants instead of 8 with two; see profiles/r02_score_epilogue_experiments.txt)
-#ifdef SKB_SCORE_EPI16
-    static constexpr int kEpiWarps = (PASSES == 1 || STREAM_A) ? 16 : 8;
-#else
     static constexpr int kEpiWarps = 8;
-#endif
-    static constexpr int kThreads = (2 + kEpiWarps) * 32;  // warps: 0 producer, 1 MMA, 2.. epilogue (kEpiWarps / 4 per TMEM quadrant)
-    static constexpr int kBStages = STREAM_A ? 4 : (PASSES == 1 ? (KC == 256 ? 2 : (KC == 128 ? SKB_KC128_STAGES : (MT == 2 ? 3 : (kEpiWarps == 16 ? 5 : 7)))) : 3);
+    static constexpr int kThreads = (2 + kEpiWarps) * 32;  // warps: 0 producer, 1 MMA, 2.. epilogue (two per TMEM quadrant)
+    static constexpr int kBStages = STREAM_A ? 4 : (PASSES == 3 ? 3 : (KC == 128 ? kKc128Stages : 7));
     // Resident-panel variants keep the E panel in TENSOR memory (copied there once per panel with tcgen05.cp): a tcgen05.mma
     // then reads only the T tile through the shared-memory pipe.  With both operands in shared memory a 128 x 128 x 256 tile
     // moved 128 KB of operand reads + 64 KB of incoming T + 64-128 KB of epilogue staging through a 128 B/clk pipe: 2000-2500
     // cycles against 1024 of math -- every output mode was bound by shared-memory bandwidth (profiles/r02x_score_smem_bound.txt).
-#ifdef SKB_SCORE_A_SMEM
-    static constexpr bool kATmem = false;
-#else
-    static constexpr bool kATmem = !STREAM_A && MT == 1;
-#endif
-    static constexpr int kAccCols = 2 * MT * 128;        // double-buffered accumulators
+    static constexpr bool kATmem = !STREAM_A;
+    static constexpr int kAccCols = 2 * 128;             // double-buffered accumulators
     static constexpr int kTmemCols = kATmem ? 512 : kAccCols;   // + kParts x 128 columns of A (Dp <= 256)
     static constexpr int kStageRowBytes = 36 * 4;        // [32][36] fp32 transpose buffer per epilogue warp (16-byte rows)
-    // E panel in shared memory: the whole panel (MT x kParts x 128 x Dp) when the MMAs read it there; with the panel in tensor
-    // memory only a staging piece (kAPieceK K-columns of one part), through which the panel is passed on piece by piece
-#ifndef SKB_A_PIECE_K
-#define SKB_A_PIECE_K 128    // measured: 128 K-columns (32 KB) beats 64 and 32 (profiles/r02x_score_issue_bound.txt)
-#endif
-    static constexpr int kAPieceK = SKB_A_PIECE_K;
-    __host__ __device__ static size_t a_bytes(int Dp) {
-        return STREAM_A ? 0 : (kATmem ? (size_t)128 * kAPieceK * 2 : (size_t)MT * kParts * 128 * Dp * 2);
-    }
+    // the E panel passes into tensor memory piece by piece through a staging piece of kAPieceK K-columns of one part
+    static constexpr size_t kABytes = kATmem ? (size_t)128 * kAPieceK * 2 : 0;
     // Epilogue region: the warps' [32][36] transpose buffers, or in top-k mode (topk_k > 0, lane = row: no transpose) the
     // warps' [topk_k][32] lists of 64-bit keys in their place -- 64 KB at k = 32, which the KC 64 ring would not fit next to
     // the 36 KB of buffers.
     static size_t epi_bytes(int topk_k) {
         return topk_k > 0 ? (size_t)kEpiWarps * 32 * topk_k * sizeof(unsigned long long) : (size_t)kEpiWarps * 32 * kStageRowBytes;
     }
-    static size_t total(int Dp, int topk_k = 0) { return 256 + a_bytes(Dp) + (size_t)kBStages * kRingStageBytes + epi_bytes(topk_k); }
+    static size_t total(int topk_k) { return 256 + kABytes + (size_t)kBStages * kRingStageBytes + epi_bytes(topk_k); }
 };
 
 #ifdef SKB_SCORE_TIMING
@@ -349,11 +328,10 @@ __device__ unsigned long long g_score_t[16];
 #define SKB_TIMED_WAIT(i, stmt) stmt
 #endif
 
-template <int PASSES, bool STREAM_A, int MODE, int MT, int KC = 64>
+template <int PASSES, bool STREAM_A, int MODE, int KC = 64>
 __device__ __forceinline__ void score_gemm_body(const ScoreParams& p) {
-    using SM = ScoreSmem<PASSES, STREAM_A, MT, KC>;
-    static_assert(MT == 1 || (PASSES == 1 && !STREAM_A), "two row panels per item: single-pass resident-panel variant only");
-    static_assert(MODE != kEpiTopk || (!STREAM_A && MT == 1 && SM::kEpiWarps == 8), "top-k mode: resident-panel variants, one row panel per item, 8 epilogue warps");
+    using SM = ScoreSmem<PASSES, STREAM_A, KC>;
+    static_assert(MODE != kEpiTopk || !STREAM_A, "top-k mode: resident-panel variants only");
     constexpr bool TRIALS = MODE == kEpiTrials, TOPK = MODE == kEpiTopk;
     extern __shared__ __align__(128) uint8_t smem[];
     uint64_t* a_full = reinterpret_cast<uint64_t*>(smem);
@@ -364,19 +342,14 @@ __device__ __forceinline__ void score_gemm_body(const ScoreParams& p) {
     uint64_t* acc_empty = acc_full + 2;             // [2]
     uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(acc_empty + 2);
     uint8_t* a_smem = smem + 256;
-    const uint32_t a_part = 128 * p.Dp * 2;
-    uint8_t* b_smem = a_smem + SM::a_bytes(p.Dp);
+    uint8_t* b_smem = a_smem + SM::kABytes;
     uint8_t* stage_smem = b_smem + SM::kBStages * SM::kRingStageBytes;
 
-    pdl_wait();                                        // the operand statistics / planes come from the kernels before this one
-    // the other instantiation handles this launch when the decision (uniform across the grid) is not ours
-    if (decide_passes(p.statsE, p.statsT, p.D, p.abs_alpha, p.passes_req) != PASSES) return;
-
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    // contiguous run of work items for this CTA (panel-group-major), walked with incremental (group, nt) counters; an item =
-    // MT row panels x one 128-column tile ("panel" below counts panel GROUPS)
+    // contiguous run of work items for this CTA (panel-major), walked with incremental (panel, nt) counters; an item = one
+    // 128-row panel x one 128-column tile
     const int n_panels = p.Ne_pad >> 7;
-    const int tiles_total = ((n_panels + MT - 1) / MT) * p.n_ntiles;
+    const int tiles_total = n_panels * p.n_ntiles;
     const int t_begin = (int)((long long)tiles_total * blockIdx.x / gridDim.x);
     const int t_end = (int)((long long)tiles_total * (blockIdx.x + 1) / gridDim.x);
     const int panel0 = t_begin / p.n_ntiles, nt0 = t_begin % p.n_ntiles;
@@ -406,23 +379,12 @@ __device__ __forceinline__ void score_gemm_body(const ScoreParams& p) {
                 if (SM::kATmem && new_panel) {
                     // piece by piece through the staging buffer (the MMA lane copies each piece on into tensor memory)
                     for (int part = 0; part < SM::kParts; ++part)
-                        for (int k0 = 0; k0 < p.Dp; k0 += SM::kAPieceK) {
+                        for (int k0 = 0; k0 < p.Dp; k0 += kAPieceK) {
                             mbar_wait(a_empty, a_ph);
                             a_ph ^= 1;
-                            const uint32_t bytes = (uint32_t)min(SM::kAPieceK, p.Dp - k0) * 256u;       // 128 rows x 2 bytes per K column
+                            const uint32_t bytes = (uint32_t)min(kAPieceK, p.Dp - k0) * 256u;       // 128 rows x 2 bytes per K column
                             mbar_arrive_expect_tx(a_full, bytes);
                             bulk_g2s(a_smem, (part == 0 ? p.Ehi : p.Elo) + (size_t)panel * p.Dp * 128 + (size_t)k0 * 128, bytes, a_full);
-                        }
-                } else if (!STREAM_A && new_panel) {
-                    mbar_wait(a_empty, a_ph);
-                    a_ph ^= 1;
-                    const int n_pan = min(MT, n_panels - panel * MT);
-                    mbar_arrive_expect_tx(a_full, n_pan * SM::kParts * a_part);
-                    for (int m = 0; m < n_pan; ++m)
-                        for (int part = 0; part < SM::kParts; ++part) {
-                            const uint16_t* src = (part == 0 ? p.Ehi : p.Elo) + (size_t)(panel * MT + m) * p.Dp * 128;
-                            for (uint32_t off = 0; off < a_part; off += 32768)      // whole panel image is contiguous
-                                bulk_g2s(a_smem + (m * SM::kParts + part) * a_part + off, src + off / 2, min(32768u, a_part - off), a_full);
                         }
                 }
                 for (int kc = 0; kc < n_kc; ++kc) {
@@ -431,26 +393,14 @@ __device__ __forceinline__ void score_gemm_body(const ScoreParams& p) {
                     uint8_t* dst = b_smem + (size_t)s * SM::kRingStageBytes;
                     if (STREAM_A) {
                         for (int part = 0; part < SM::kParts; ++part, dst += SM::kStageBytes) {
-                            const uint16_t* src = (part == 0 ? p.Ehi : p.Elo) + ((size_t)panel * p.Dp + (size_t)kc * SM::kChunk) * 128;   // (MT == 1)
+                            const uint16_t* src = (part == 0 ? p.Ehi : p.Elo) + ((size_t)panel * p.Dp + (size_t)kc * SM::kChunk) * 128;
                             bulk_g2s(dst, src, SM::kStageBytes, &b_full[s]);
                         }
                     }
-#ifdef SKB_X_NOCOPY
-                    // experiment: the T tiles are not copied at all (the MMAs run on whatever the ring holds): what does the MMA /
-                    // epilogue pipeline do without the incoming stream?
-                    for (int part = 0; part < SM::kParts; ++part, dst += SM::kStageBytes) {
-                        const uint16_t* src = (part == 0 ? p.Thi : p.Tlo) + ((size_t)(nt & 1) * p.Dp + (size_t)kc * SM::kChunk) * 128;
-                        if (t < t_begin + 2) bulk_g2s(dst, src, SM::kStageBytes, &b_full[s]);
-                        else if (part == 0) {
-                            asm volatile("mbarrier.complete_tx.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(&b_full[s])), "r"((uint32_t)SM::kRingStageBytes) : "memory");
-                        }
-                    }
-#else
                     for (int part = 0; part < SM::kParts; ++part, dst += SM::kStageBytes) {
                         const uint16_t* src = (part == 0 ? p.Thi : p.Tlo) + ((size_t)nt * p.Dp + (size_t)kc * SM::kChunk) * 128;
                         bulk_g2s(dst, src, SM::kStageBytes, &b_full[s]);   // contiguous planes
                     }
-#endif
                     if (++s == SM::kBStages) { s = 0; b_ph ^= 1; }
                 }
                 new_panel = false;
@@ -467,7 +417,7 @@ __device__ __forceinline__ void score_gemm_body(const ScoreParams& p) {
         const uint32_t idesc = umma_idesc_f16(128, 128, false);
         const uint64_t desc_hi = (static_cast<uint64_t>(2048 >> 4) << 16) | (static_cast<uint64_t>(128 >> 4) << 32) |
                                  (static_cast<uint64_t>(1) << 46);
-        int nt = nt0, s = 0, group = panel0;
+        int nt = nt0, s = 0;
         uint32_t b_ph = 0, a_ph = 0, nt_done = 0;
         bool new_panel = true;
         SKB_T0();
@@ -476,36 +426,31 @@ __device__ __forceinline__ void score_gemm_body(const ScoreParams& p) {
                 // the panel moves on into tensor memory piece by piece (behind the MMAs of the previous panel, which execute
                 // first: one in-order pipe); the staging buffer is free again as soon as a piece's copies are done
                 for (int part = 0; part < SM::kParts; ++part)
-                    for (int k0 = 0; k0 < p.Dp; k0 += SM::kAPieceK) {
+                    for (int k0 = 0; k0 < p.Dp; k0 += kAPieceK) {
                         SKB_TIMED_WAIT(3, mbar_wait(a_full, a_ph));
                         a_ph ^= 1;
                         tc_fence_after();
-                        const int n_ks = min(SM::kAPieceK, p.Dp - k0) / 16;
+                        const int n_ks = min(kAPieceK, p.Dp - k0) / 16;
                         for (int ks = 0; ks < n_ks; ++ks)
                             tmem_cp_128x256b(tmem_base + SM::kAccCols + part * 128 + (k0 / 16 + ks) * 8,
                                              desc_hi | (((smem_u32(a_smem) + ks * 2 * 2048) >> 4) & 0x3FFF));
                         umma_commit(a_empty);
                     }
-            } else if (!STREAM_A && new_panel) {
-                SKB_TIMED_WAIT(3, mbar_wait(a_full, a_ph));
-                a_ph ^= 1;
             }
-            const int n_pan = min(MT, n_panels - group * MT);
             const int buf = (int)(nt_done & 1);
             SKB_TIMED_WAIT(2, mbar_wait(&acc_empty[buf], ((nt_done >> 1) & 1) ^ 1));
             tc_fence_after();
-            const uint32_t d_tmem = tmem_base + buf * (MT * 128);
+            const uint32_t d_tmem = tmem_base + buf * 128;
             for (int kc = 0; kc < n_kc; ++kc) {
                 SKB_TIMED_WAIT(1, mbar_wait(&b_full[s], b_ph));
                 tc_fence_after();
+                // streaming mode: the stage holds the E chunk (hi, lo) in front of the T chunk
                 const uint32_t st_base = smem_u32(b_smem + (size_t)s * SM::kRingStageBytes);
                 const uint32_t b_hi = st_base + (STREAM_A ? SM::kParts * SM::kStageBytes : 0);
-                const uint32_t a_hi = STREAM_A ? st_base : smem_u32(a_smem) + kc * (SM::kChunk / 8) * 2048;
-                const uint32_t a_lo_off = STREAM_A ? SM::kStageBytes : a_part;
 #pragma unroll
                 for (int combo = 0; combo < (PASSES == 1 ? 1 : 3); ++combo) {
                     // combo 0: hi*hi, 1: hi*lo, 2: lo*hi
-                    const uint32_t a_b = a_hi + (combo == 2 ? a_lo_off : 0);
+                    const uint32_t a_b = st_base + (combo == 2 ? SM::kStageBytes : 0);
                     const uint32_t b_b = b_hi + (combo == 1 ? SM::kStageBytes : 0);
 #pragma unroll
                     for (int ks = 0; ks < SM::kChunk / 16; ++ks) {
@@ -514,12 +459,8 @@ __device__ __forceinline__ void score_gemm_body(const ScoreParams& p) {
                         if (SM::kATmem) {
                             umma_f16_ts(d_tmem, tmem_base + SM::kAccCols + (combo == 2 ? 128 : 0) + (kc * (SM::kChunk / 16) + ks) * 8, bd, idesc, acc);
                         } else {
-#pragma unroll
-                            for (int m = 0; m < MT; ++m) {
-                                if (m >= n_pan) break;
-                                const uint64_t ad = desc_hi | (((a_b + m * SM::kParts * a_part + ks * 2 * 2048) >> 4) & 0x3FFF);
-                                umma_f16(d_tmem + m * 128, ad, bd, idesc, acc);
-                            }
+                            const uint64_t ad = desc_hi | (((a_b + ks * 2 * 2048) >> 4) & 0x3FFF);
+                            umma_f16(d_tmem, ad, bd, idesc, acc);
                         }
                     }
                 }
@@ -527,17 +468,15 @@ __device__ __forceinline__ void score_gemm_body(const ScoreParams& p) {
                 if (++s == SM::kBStages) { s = 0; b_ph ^= 1; }
             }
             new_panel = false;
-            if (++nt == p.n_ntiles) { nt = 0; new_panel = true; ++group; }
-            const bool last_of_panel = new_panel || (t + 1 == t_end);
+            if (++nt == p.n_ntiles) { nt = 0; new_panel = true; }
             umma_commit(&acc_full[buf]);
-            if (!STREAM_A && !SM::kATmem && last_of_panel) umma_commit(a_empty);
         }
         SKB_TADD(0);
         }
         __syncwarp();
     } else if (warp >= 2) {
-        // ---------------------------------------------------------------- epilogue: kEpiWarps / 4 warps per TMEM lane quadrant
-        constexpr int NB = 16 / SM::kEpiWarps;             // 32-column blocks per warp and tile: 2 (8 warps) or 1 (16 warps)
+        // ---------------------------------------------------------------- epilogue: two warps per TMEM lane quadrant
+        constexpr int NB = 2;                              // 32-column blocks per warp and tile
         const int q = warp & 3;
         const int part = (warp - 2) >> 2;                  // which NB of the four 32-column blocks
         float* stg = reinterpret_cast<float*>(stage_smem) + (warp - 2) * 32 * 36;   // warp-private [32][36] transpose buffer
@@ -562,30 +501,23 @@ __device__ __forceinline__ void score_gemm_body(const ScoreParams& p) {
         // Row terms change only with the panel; column terms are fetched BEFORE waiting for the accumulator, so their
         // L2 latency hides behind the MMAs instead of stalling every 32x32 block (was 52 % of all stall samples).
         int cur_panel = -1;
-        float ra_m[MT], rr_m[MT];
-#pragma unroll
-        for (int m = 0; m < MT; ++m) { ra_m[m] = 0.f; rr_m[m] = 0.f; }
+        float ra = 0.f, rr = 0.f;
         const int c4 = (lane & 7) * 4;
-        uint32_t mwn[MT][NB], mon[MT][NB];                 // trial-list mode: mask words / offsets of the NEXT item
-        auto fetch_mask = [&](int grp, int ntile) {
+        uint32_t mwn[NB], mon[NB];                         // trial-list mode: mask words / offsets of the NEXT item
+        auto fetch_mask = [&](int pnl, int ntile) {
+            const int rown = pnl * 128 + q * 32 + lane;
 #pragma unroll
-            for (int m = 0; m < MT; ++m) {
-                const int rown = (grp * MT + m) * 128 + q * 32 + lane;
-#pragma unroll
-                for (int cbi = 0; cbi < NB; ++cbi) {
-                    const int wcol = ntile * 4 + part * NB + cbi;
-                    mwn[m][cbi] = 0u; mon[m][cbi] = 0u;
-                    if (rown < p.Ne && wcol < p.mask_ld) {
-                        mwn[m][cbi] = __ldg(p.mask_words + (size_t)rown * p.mask_ld + wcol);
-                        mon[m][cbi] = __ldg(p.word_off + (size_t)rown * p.mask_ld + wcol);
-                    }
+            for (int cbi = 0; cbi < NB; ++cbi) {
+                const int wcol = ntile * 4 + part * NB + cbi;
+                mwn[cbi] = 0u; mon[cbi] = 0u;
+                if (rown < p.Ne && wcol < p.mask_ld) {
+                    mwn[cbi] = __ldg(p.mask_words + (size_t)rown * p.mask_ld + wcol);
+                    mon[cbi] = __ldg(p.word_off + (size_t)rown * p.mask_ld + wcol);
                 }
             }
         };
 #pragma unroll
-        for (int m = 0; m < MT; ++m)
-#pragma unroll
-            for (int cbi = 0; cbi < NB; ++cbi) { mwn[m][cbi] = 0u; mon[m][cbi] = 0u; }
+        for (int cbi = 0; cbi < NB; ++cbi) { mwn[cbi] = 0u; mon[cbi] = 0u; }
         if (TRIALS && t_begin < t_end) fetch_mask(panel0, nt0);
         float4 qnext[NB];
         auto fetch_q = [&](int ntile) {
@@ -601,15 +533,11 @@ __device__ __forceinline__ void score_gemm_body(const ScoreParams& p) {
         if (t_begin < t_end) fetch_q(nt0);
         for (int t = t_begin; t < t_end; ++t, ++nt_done) {
             const int buf = (int)(nt_done & 1);
-            const int n_pan = min(MT, n_panels - panel * MT);
             if (panel != cur_panel) {
                 cur_panel = panel;
-#pragma unroll
-                for (int m = 0; m < MT; ++m) {
-                    const int r = (panel * MT + m) * 128 + q * 32 + lane;
-                    ra_m[m] = (p.ra && r < p.Ne) ? p.ra[r] * mscale : 0.f;
-                    rr_m[m] = fmaf((p.r && r < p.Ne) ? p.r[r] : 0.f, p.rq_scale, p.c0);
-                }
+                const int r = panel * 128 + q * 32 + lane;
+                ra = (p.ra && r < p.Ne) ? p.ra[r] * mscale : 0.f;
+                rr = fmaf((p.r && r < p.Ne) ? p.r[r] : 0.f, p.rq_scale, p.c0);
             }
             // column terms: fetched ONE ITEM AHEAD as well (fetched at the top of their own tile they were the first thing the
             // epilogue stalled on whenever the accumulator was already waiting: 15 % of the stall samples)
@@ -624,11 +552,9 @@ __device__ __forceinline__ void score_gemm_body(const ScoreParams& p) {
             // trial-list mode: lane = row (the accumulator's native layout, no transpose): this row's mask words and output
             // offsets, fetched ONE ITEM AHEAD (a mask word comes from L2 / HBM, ~1 us away: loaded at the top of its own tile it
             // was 36 % of the kernel's stall samples and the tensor pipe sat at 4 %)
-            uint32_t mw_m[MT][NB], mo_m[MT][NB];
+            uint32_t mw[NB], mo[NB];
 #pragma unroll
-            for (int m = 0; m < MT; ++m)
-#pragma unroll
-                for (int cbi = 0; cbi < NB; ++cbi) { mw_m[m][cbi] = mwn[m][cbi]; mo_m[m][cbi] = mon[m][cbi]; }
+            for (int cbi = 0; cbi < NB; ++cbi) { mw[cbi] = mwn[cbi]; mo[cbi] = mon[cbi]; }
             if (TRIALS && t + 1 < t_end) {
                 int ntn = nt + 1, pn = panel;
                 if (ntn == p.n_ntiles) { ntn = 0; ++pn; }
@@ -637,28 +563,20 @@ __device__ __forceinline__ void score_gemm_body(const ScoreParams& p) {
             if (warp == 2) { SKB_TIMED_WAIT(5, mbar_wait(&acc_full[buf], (nt_done >> 1) & 1)); }
             else mbar_wait(&acc_full[buf], (nt_done >> 1) & 1);
             tc_fence_after();
-#pragma unroll
-            for (int m = 0; m < MT; ++m) {
-            if (m >= n_pan) break;
-            const int row0 = (panel * MT + m) * 128 + q * 32;
+            const int row0 = panel * 128 + q * 32;
             const int n_rows = min(32, p.Ne - row0);
-            const float ra = ra_m[m], rr = rr_m[m];
 #pragma unroll
             for (int cbi = 0; cbi < NB; ++cbi) {
                 const int cb = part * NB + cbi;
                 const int col0 = nt * 128 + cb * 32;
                 float v[32];
-                tmem_ld32(tmem_base + ((uint32_t)(q * 32) << 16) + buf * (MT * 128) + m * 128 + cb * 32, v);
-                if (cbi == NB - 1 && m == n_pan - 1) {   // this warp's share of the accumulators is read: release the TMEM buffer
+                tmem_ld32(tmem_base + ((uint32_t)(q * 32) << 16) + buf * 128 + cb * 32, v);
+                if (cbi == NB - 1) {   // this warp's share of the accumulators is read: release the TMEM buffer
                     tc_fence_before();
                     __syncwarp();
                     if (lane == 0) mbar_arrive(&acc_empty[buf]);
                 }
                 if (col0 >= p.Nt || n_rows <= 0) continue;
-#ifdef SKB_X_NOEPI
-                if (v[0] == 1.2345e-30f) reinterpret_cast<float*>(p.out)[0] = v[1];   // experiment: TMEM loads only
-                continue;
-#endif
                 if (TOPK) {
                     // lane = row (the accumulator's native layout): the lane screens the 32 scores of its row against its
                     // k-th best so far; only a score that reaches it builds a key and touches shared memory.  Same roundings
@@ -696,7 +614,7 @@ __device__ __forceinline__ void score_gemm_body(const ScoreParams& p) {
                     // trial costs a TMEM load and a vote; otherwise the rows are parked in the warp's staging buffer so that
                     // the set bits can index them.  (Almost) no stores for a sparse mask: the kernel is then bound by the
                     // operand stream / the tensor pipe instead of the HBM write.
-                    uint32_t word = mw_m[m][cbi];
+                    uint32_t word = mw[cbi];
                     if (__any_sync(0xffffffffu, word != 0u)) {
                         __syncwarp();
                         float4* srow = reinterpret_cast<float4*>(stg + lane * 36);
@@ -713,7 +631,7 @@ __device__ __forceinline__ void score_gemm_body(const ScoreParams& p) {
                         }
                         __syncwarp();
                         const float mul = ra + a0;
-                        float* o = reinterpret_cast<float*>(p.out) + mo_m[m][cbi];
+                        float* o = reinterpret_cast<float*>(p.out) + mo[cbi];
                         while (word != 0u) {
                             const int j = __ffs(word) - 1;
                             word &= word - 1u;
@@ -754,7 +672,7 @@ __device__ __forceinline__ void score_gemm_body(const ScoreParams& p) {
                             const __half2 h0 = __floats2half2_rn(__fadd_rn(x.x, qv.x), __fadd_rn(x.y, qv.y)), h1 = __floats2half2_rn(__fadd_rn(x.z, qv.z), __fadd_rn(x.w, qv.w));
                             __stcs(reinterpret_cast<uint2*>(o), make_uint2(*reinterpret_cast<const uint32_t*>(&h0), *reinterpret_cast<const uint32_t*>(&h1)));
                         }
-                    } else if (p.out_f64) {
+                    } else if (p.out_mode == 1) {
                         double* o = reinterpret_cast<double*>(p.out) + (size_t)(row0 + rs) * p.ld_out + col0 + c4;
                         const size_t step = (size_t)4 * p.ld_out;
 #pragma unroll
@@ -806,12 +724,11 @@ __device__ __forceinline__ void score_gemm_body(const ScoreParams& p) {
                     sv = __fadd_rn(sv, qq);
                     if (r < n_rows && col_ok) {
                         if (p.out_mode == 2) oh[(size_t)r * p.ld_out] = __float2half_rn(sv);
-                        else if (p.out_f64) od[(size_t)r * p.ld_out] = (double)sv;
+                        else if (p.out_mode == 1) od[(size_t)r * p.ld_out] = (double)sv;
                         else o[(size_t)r * p.ld_out] = sv;
                     }
                 }
             }
-            }   // panels of the item
             if (TOPK && (nt + 1 == p.n_ntiles || t + 1 == t_end)) {
                 // leaving the row panel: this warp's lists become the partial lists of its segment, and start over empty
                 const int row = panel * 128 + q * 32 + lane;
@@ -835,20 +752,14 @@ __device__ __forceinline__ void score_gemm_body(const ScoreParams& p) {
     }
 }
 
-template <int PASSES, bool STREAM_A, int MODE, int MT, int KC>
-__global__ void __launch_bounds__(ScoreSmem<PASSES, STREAM_A, MT, KC>::kThreads, 1) score_gemm_kernel(const ScoreParams p) {
-    score_gemm_body<PASSES, STREAM_A, MODE, MT, KC>(p);
-}
-
-// passes decided on the device (passes_req == 0), resident-panel variants: ONE launch that runs the body the statistics
-// select (round 1 launched both instantiations and let one of them return at once: a 3 us no-op per call, 5 % of a
-// 2500-row panel at 8 GPUs).  Shared memory is sized for the larger of the two layouts by launch_score_auto.
-static_assert(ScoreSmem<1, false>::kThreads == ScoreSmem<3, false>::kThreads, "the auto kernel needs one block size");
-template <int MODE, int KC>
-__global__ void __launch_bounds__(ScoreSmem<1, false>::kThreads, 1) score_gemm_auto_kernel(const ScoreParams p) {
-    pdl_wait();
-    if (decide_passes(p.statsE, p.statsT, p.D, p.abs_alpha, 0) == 1) score_gemm_body<1, false, MODE, 1, KC>(p);
-    else score_gemm_body<3, false, MODE, 1>(p);
+// ONE launch per call runs the body of the pass count decide_passes returns: forced, or decided from the operand statistics
+// (uniform across the grid).  Round 1 launched both pass variants and let one of them return at once: a 3 us no-op per
+// call, 5 % of a 2500-row panel at 8 GPUs.  Three-pass bodies use 32-wide stages whatever KC.
+template <bool STREAM_A, int MODE, int KC>
+__global__ void __launch_bounds__(ScoreSmem<1, STREAM_A>::kThreads, 1) score_gemm_kernel(const ScoreParams p) {
+    pdl_wait();                                        // the operand statistics / planes come from the kernels before this one
+    if (decide_passes(p.statsE, p.statsT, p.D, p.abs_alpha, p.passes_req) == 1) score_gemm_body<1, STREAM_A, MODE, KC>(p);
+    else score_gemm_body<3, STREAM_A, MODE>(p);
 }
 
 // ----------------------------------------------------------------------------- packed operands, workspace, launch
@@ -963,61 +874,24 @@ static void ws_operand(PackedOp* op, int rows, int D, int slot, size_t offset_ha
     op->exp = reinterpret_cast<int*>(op->stats + 2);
 }
 
-template <int PASSES, bool STREAM_A, int MODE = kEpiMatrix, int MT = 1, int KC = 64>
-static int launch_score(const ScoreParams& p, int /*grid_unused*/, cudaStream_t st) {
+// Shared memory is sized for the forced pass count, or for the larger of the two layouts when the device decides.
+template <bool STREAM_A, int MODE, int KC = 64>
+static int launch_score(const ScoreParams& p, cudaStream_t st) {
     static PerDeviceOnce configured;
-    const size_t smem = ScoreSmem<PASSES, STREAM_A, MT, KC>::total(p.Dp, p.topk_k);
-    const int n_panels = p.Ne_pad / 128;
-    const int grid = std::min(((n_panels + MT - 1) / MT) * p.n_ntiles, kNumSMs);
-    if (smem > 227 * 1024) {
-        set_last_error(__FILE__, __LINE__, "score_gemm: operand panel does not fit in shared memory");
-        return SKB_ERR_ARG;
-    }
-    if (configured.first()) {
-        SKB_CUDA_CHECK(cudaFuncSetAttribute(score_gemm_kernel<PASSES, STREAM_A, MODE, MT, KC>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
-    }
-    SKB_CUDA_CHECK(launch_pdl(score_gemm_kernel<PASSES, STREAM_A, MODE, MT, KC>, dim3(grid), dim3(ScoreSmem<PASSES, STREAM_A, MT, KC>::kThreads), smem, st, p));
-    g_launches++;
-    SKB_CUDA_CHECK(cudaGetLastError());
-    return SKB_OK;
-}
-
-template <int MODE, int KC>
-static int launch_score_auto_kc(const ScoreParams& p, cudaStream_t st) {
-    static PerDeviceOnce configured;
-    const size_t smem = std::max(ScoreSmem<1, false, 1, KC>::total(p.Dp, p.topk_k), ScoreSmem<3, false>::total(p.Dp, p.topk_k));
+    const size_t smem1 = ScoreSmem<1, STREAM_A, KC>::total(p.topk_k), smem3 = ScoreSmem<3, STREAM_A>::total(p.topk_k);
+    const size_t smem = p.passes_req == 1 ? smem1 : (p.passes_req == 3 ? smem3 : std::max(smem1, smem3));
     const int grid = std::min((p.Ne_pad / 128) * p.n_ntiles, kNumSMs);
     if (smem > 227 * 1024) {
-        set_last_error(__FILE__, __LINE__, "score_gemm: operand panel does not fit in shared memory");
+        set_last_error(__FILE__, __LINE__, "score_gemm: the stage ring does not fit in shared memory");
         return SKB_ERR_ARG;
     }
     if (configured.first()) {
-        SKB_CUDA_CHECK(cudaFuncSetAttribute(score_gemm_auto_kernel<MODE, KC>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
+        SKB_CUDA_CHECK(cudaFuncSetAttribute(score_gemm_kernel<STREAM_A, MODE, KC>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
     }
-    SKB_CUDA_CHECK(launch_pdl(score_gemm_auto_kernel<MODE, KC>, dim3(grid), dim3(ScoreSmem<1, false>::kThreads), smem, st, p));
+    SKB_CUDA_CHECK(launch_pdl(score_gemm_kernel<STREAM_A, MODE, KC>, dim3(grid), dim3(ScoreSmem<1, STREAM_A>::kThreads), smem, st, p));
     g_launches++;
     SKB_CUDA_CHECK(cudaGetLastError());
     return SKB_OK;
-}
-
-// The widest ring stage the padded K allows (see ScoreSmem): the whole K = 256 of an x-vector in ONE stage (one commit per
-// tile), else 128- or 64-wide stages.  SKB_SCORE_KC=64|128|256 caps the width (A/B knob).
-static int stage_width(const ScoreParams& p) {
-    static const int cap = getenv("SKB_SCORE_KC") ? atoi(getenv("SKB_SCORE_KC")) : 128;
-    if (p.Dp == 256 && cap >= 256) return 256;
-    if (p.Dp % 128 == 0 && cap >= 128) return 128;
-    return 64;
-}
-template <int MODE>
-static int launch_score_auto(const ScoreParams& p, cudaStream_t st) {
-    const int kc = stage_width(p);
-    return kc == 256 ? launch_score_auto_kc<MODE, 256>(p, st) : (kc == 128 ? launch_score_auto_kc<MODE, 128>(p, st) : launch_score_auto_kc<MODE, 64>(p, st));
-}
-template <int MODE>
-static int launch_score_single_pass(const ScoreParams& p, int grid, cudaStream_t st) {
-    const int kc = stage_width(p);
-    return kc == 256 ? launch_score<1, false, MODE, 1, 256>(p, grid, st)
-                     : (kc == 128 ? launch_score<1, false, MODE, 1, 128>(p, grid, st) : launch_score<1, false, MODE, 1, 64>(p, grid, st));
 }
 
 // out = acc * (ra_i + ca_j + a0) + rq_scale * (r_i + q_j) + c0 on two packed operands
@@ -1034,62 +908,32 @@ int gemm_packed(const PackedOp& E, const PackedOp& T, const float* ra, const flo
     if (rc) return rc;
     ScoreParams p;
     p.Ehi = E.hi; p.Elo = E.lo; p.Thi = T.hi; p.Tlo = T.lo;
-    p.Ne = E.rows; p.Nt = T.rows; p.Ne_pad = E.rows_pad; p.Nt_pad = T.rows_pad; p.Dp = E.Dp; p.D = E.D;
+    p.Ne = E.rows; p.Nt = T.rows; p.Ne_pad = E.rows_pad; p.Dp = E.Dp; p.D = E.D;
     p.expE = E.exp; p.expT = T.exp; p.statsE = E.stats; p.statsT = T.stats;
     p.abs_alpha = abs_alpha_for_auto; p.passes_req = passes;
     p.ra = ra; p.ca = ca; p.r = r; p.q = q; p.a0 = a0; p.c0 = c0; p.rq_scale = rq_scale;
     p.mul_scaled = 1;
-    p.out = out; p.ld_out = ld_out; p.out_f64 = out_mode == 1 ? 1 : 0; p.out_mode = out_mode;
+    p.out = out; p.ld_out = ld_out; p.out_mode = out_mode;
     p.mask_words = trials ? trials->words : nullptr;
     p.word_off = trials ? trials->offsets : nullptr;
     p.mask_ld = trials ? trials->ld : 0;
     p.topk_k = topk ? topk->k : 0;
     p.topk_segs = topk ? topk->segs : 0;
     p.n_ntiles = T.rows_pad / 128;
-    p.tiles_total = (E.rows_pad / 128) * p.n_ntiles;
-    const int grid = std::min(p.tiles_total, kNumSMs);
-    // Large K (dense layers of the pooling / head) streams both operands; K <= 256 keeps the E panel resident.
-    // Both pass variants are launched when the count is decided on the device; exactly one does the work.
-    static const bool force_stream = getenv("SKB_FORCE_STREAM_A") != nullptr;   // experiment knob
-    // Two row panels per work item (MT = 2: a streamed T tile feeds two resident E panels, half the L2 -> SM operand stream)
-    // are built but OFF: measured at 20k x 20k they change the matrix modes by < 2 % and slow the trial-list mode down
-    // (271 -> 318 us) -- the two panels leave a 3-stage T ring, and the stream is bound by ring depth x L2 latency, not by
-    // L2 bandwidth (profiles/r02_score_epilogue_experiments.txt).  SKB_SCORE_TWO_PANELS=1 enables them.
-    static const bool one_panel = getenv("SKB_SCORE_TWO_PANELS") == nullptr;
-    const bool stream_a = E.Dp > 256 || force_stream;
-    if (out_mode == 4) {
-        // top-k: resident-panel variants with one row panel per item only (the partial-list slots assume that partition)
-        if (E.Dp > 256) {
-            set_last_error(__FILE__, __LINE__, "top-k epilogue supports embeddings of up to 256 dimensions");
+    // Large K (dense layers of the pooling / head) streams both operands; K <= 256 keeps the E panel resident, in
+    // 128-wide ring stages whenever the padded K allows (see ScoreSmem)
+    if (E.Dp > 256) {
+        if (out_mode == 3 || out_mode == 4) {
+            set_last_error(__FILE__, __LINE__, out_mode == 3 ? "trial-list mode supports embeddings of up to 256 dimensions"
+                                                             : "top-k epilogue supports embeddings of up to 256 dimensions");
             return SKB_ERR_ARG;
         }
-#ifdef SKB_SCORE_EPI16
-        set_last_error(__FILE__, __LINE__, "top-k epilogue is not built with SKB_SCORE_EPI16");
-        return SKB_ERR_ARG;
-#else
-        if (passes == 0) return launch_score_auto<kEpiTopk>(p, st);
-        return passes == 1 ? launch_score_single_pass<kEpiTopk>(p, grid, st) : launch_score<3, false, kEpiTopk>(p, grid, st);
-#endif
+        return launch_score<true, kEpiMatrix>(p, st);
     }
-    if (out_mode == 3) {
-        if (stream_a) {
-            set_last_error(__FILE__, __LINE__, "trial-list mode supports embeddings of up to 256 dimensions");
-            return SKB_ERR_ARG;
-        }
-        // two row panels per item when the two resident single-pass panels fit (D <= 256): half the operand stream
-        const bool two = p.Dp <= 256 && E.rows_pad >= 256 && !one_panel;
-        if (passes == 0 && !two) return launch_score_auto<kEpiTrials>(p, st);
-        if (passes != 3) rc = two ? launch_score<1, false, kEpiTrials, 2>(p, grid, st) : launch_score_single_pass<kEpiTrials>(p, grid, st);
-        if (rc) return rc;
-        if (passes != 1) rc = launch_score<3, false, kEpiTrials>(p, grid, st);
-        return rc;
-    }
-    const bool two = !stream_a && p.Dp <= 256 && E.rows_pad >= 256 && !one_panel;
-    if (passes == 0 && !stream_a && !two) return launch_score_auto<kEpiMatrix>(p, st);
-    if (passes != 3) rc = stream_a ? launch_score<1, true>(p, grid, st) : (two ? launch_score<1, false, kEpiMatrix, 2>(p, grid, st) : launch_score_single_pass<kEpiMatrix>(p, grid, st));
-    if (rc) return rc;
-    if (passes != 1) rc = stream_a ? launch_score<3, true>(p, grid, st) : launch_score<3, false>(p, grid, st);
-    return rc;
+    const bool wide = E.Dp % 128 == 0;
+    if (out_mode == 3) return wide ? launch_score<false, kEpiTrials, 128>(p, st) : launch_score<false, kEpiTrials, 64>(p, st);
+    if (out_mode == 4) return wide ? launch_score<false, kEpiTopk, 128>(p, st) : launch_score<false, kEpiTopk, 64>(p, st);
+    return wide ? launch_score<false, kEpiMatrix, 128>(p, st) : launch_score<false, kEpiMatrix, 64>(p, st);
 }
 
 // C[m][n] = sum_k A[m][k] * W[n][k] + bias[n] with fp32-class accuracy (split fp16 passes): the dense layers of the
@@ -1125,9 +969,9 @@ int gemm_packed_a(const PackedOp& A, const PackedOp& W, const float* bias, float
 
 // out = acc * (ra_i + ca_j + a0) + rq_scale * (r_i + q_j) + c0 from fp32 row-major operands
 static int score_gemm_general(const float* E, const float* T, int Ne, int Nt, int D, const float* ra, const float* ca, float a0,
-                              const float* r, const float* q, float c0, float rq_scale, float abs_alpha_for_auto, int passes, int out_f64,
+                              const float* r, const float* q, float c0, float rq_scale, float abs_alpha_for_auto, int passes, int out_mode,
                               void* out, long long ld_out, size_t tmp_bytes, cudaStream_t st, const TrialTables* trials = nullptr) {
-    if (!E || !T || !out || Ne <= 0 || Nt <= 0 || D <= 0 || (out_f64 != 3 && ld_out < Nt)) {
+    if (!E || !T || !out || Ne <= 0 || Nt <= 0 || D <= 0 || (out_mode != 3 && ld_out < Nt)) {
         set_last_error(__FILE__, __LINE__, "score_gemm: bad arguments");
         return SKB_ERR_ARG;
     }
@@ -1139,7 +983,7 @@ static int score_gemm_general(const float* E, const float* T, int Ne, int Nt, in
     ws_operand(&e, Ne, D, 0, 0);
     ws_operand(&t, Nt, D, 1, 2 * eh);
     if ((rc = packed_fill(E, &e, T, &t, st))) return rc;
-    return gemm_packed(e, t, ra, ca, a0, r, q, c0, rq_scale, abs_alpha_for_auto, passes, out_f64, out, ld_out, st, trials);
+    return gemm_packed(e, t, ra, ca, a0, r, q, c0, rq_scale, abs_alpha_for_auto, passes, out_mode, out, ld_out, st, trials);
 }
 
 // ----------------------------------------------------------------------------- trial index (trial-list mode)

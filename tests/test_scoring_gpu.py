@@ -289,6 +289,27 @@ def test_packed_test_operand_equals_the_plain_call():
         assert torch.equal(score_matrix(E, Tp, r, q, cst=0.25, alpha=1.5, passes=0), plain)      # same arithmetic, same bits
 
 
+def test_pass_count_decided_on_the_device_is_one_launch_equal_to_the_forced_count():
+    """passes=0 equals the call forced to the pass count the operand statistics pick (one pass on unit-norm rows, three on
+    N(0,1) rows) bit for bit, and costs the same launches whether the E panel is resident (D = 256) or streamed (D = 512)."""
+    from sidekit_b200 import _lib
+    lib = _lib.lib()
+    launches = {}
+    for D in (256, 512):
+        for unit, forced in ((True, 1), (False, 3)):
+            E = torch.from_numpy(synth.synth_embeddings(300, D, seed=91, unit_norm=unit)).float().cuda()
+            T = torch.from_numpy(synth.synth_embeddings(200, D, seed=92, unit_norm=unit)).float().cuda()
+            n0 = lib.skb_kernel_launches()
+            want = sk.score_matrix(E, T, passes=forced)
+            n1 = lib.skb_kernel_launches()
+            got = sk.score_matrix(E, T, passes=0)
+            launches[D, unit] = lib.skb_kernel_launches() - n1
+            assert torch.equal(got, want), (D, unit)
+            assert launches[D, unit] == n1 - n0, (D, unit)
+    for unit in (True, False):
+        assert launches[512, unit] == launches[256, unit]
+
+
 def test_large_matrix_reaches_the_host_through_the_pinned_path_widened():
     """Scores.scoremat of the PLDA family: float32 on the device, float64 on the host (widened on the way out)."""
     from sidekit_b200.bosaris import _device_to_numpy

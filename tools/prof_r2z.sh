@@ -9,5 +9,6 @@ python bench.py --steps 20 --warmup 3 > $O/r02z_bench_n1.json 2> $O/r02z_bench_n
 python tools/ab_print.py $O/r02z_bench_n1.json
 ncu --metrics gpu__time_duration.sum --clock-control none --csv --log-file $O/r02z_launches_hr34.csv python tools/step_for_ncu.py hr34 1 > /dev/null 2>&1
 python tools/step_summary.py $O/r02z_launches_hr34.csv > $O/r02z_launches_hr34_step_summary.txt 2>&1; head -3 $O/r02z_launches_hr34_step_summary.txt
-ncu --set full --clock-control none --import-source on -k regex:score_gemm_auto_kernel --launch-skip 3 --launch-count 3 -o /tmp/sg -f python tools/score_modes_probe.py > /dev/null 2>&1
+# (the r02z_ncu_score_mode*.txt outputs were taken when the kernel was named score_gemm_auto_kernel)
+ncu --set full --clock-control none --import-source on -k regex:score_gemm_kernel --launch-skip 3 --launch-count 3 -o /tmp/sg -f python tools/score_modes_probe.py > /dev/null 2>&1
 for i in 0 1 2; do python tools/ncu_summary.py /tmp/sg.ncu-rep $i > $O/r02z_ncu_score_mode$i.txt 2>&1; head -2 $O/r02z_ncu_score_mode$i.txt | cut -c1-130; done
