@@ -174,6 +174,20 @@ int skb_score_gemm_trials_packed(const float* E_dev, int Ne, const skb_packed_t*
                                  double cst, double alpha, int passes, const skb_trial_index_t* trials, float* out_trials_dev,
                                  void* stream);
 
+/* Pair-list mode: replaces the dense trial matrix of sidekit/iv_scoring.py:108-109, :451-462 and the N x N as-norm matrix of
+ * sidekit/score_normalization.py:135-138 for lists given as (enrolment row, test row) pairs, such as VoxCeleb1-E / -H.  For
+ * p < n_pairs, i = rows_dev[p], j = cols_dev[p] (int32, device):
+ *   s = alpha * (rowterm[i] + colterm[j] + cst) + alpha * sum_k E[i][k] * T[j][k]    (float32 FMAs over the float32 rows)
+ * and out_dev[p] = s, or, when the four statistic vectors are given (all four or none),
+ *   out_dev[p] = 0.5 * (s - mean_e[i]) / std_e[i] + 0.5 * (s - mean_t[j]) / std_t[j].
+ * rowterm / colterm may be NULL (0).  The bits of out_dev[p] depend on D and the two rows only (fixed reduction order), not
+ * on p or n_pairs.  An index outside [0, Ne) / [0, Nt) is not dereferenced: that trial gets NaN.  Any D >= 1 (16-byte loads
+ * when D % 4 == 0 and both bases are 16-byte aligned).  n_pairs == 0 is a no-op. */
+int skb_score_pairs(const float* E_dev, const float* T_dev, int Ne, int Nt, int D, const int32_t* rows_dev, const int32_t* cols_dev,
+                    int64_t n_pairs, const float* rowterm_dev, const float* colterm_dev, float cst, float alpha,
+                    const float* mean_e_dev, const float* std_e_dev, const float* mean_t_dev, const float* std_t_dev,
+                    float* out_dev, void* stream);
+
 /* Top-k mode.  Per row i of S (same formula and arguments as skb_score_gemm_trials): the k largest S[i][j], ordered by score
  * descending, ties by lower j.  values (Ne, k) float32, indices (Ne, k) int64, device.  1 <= k <= min(Nt, 1024).  Each value
  * equals the skb_score_gemm entry of the same arguments bit for bit.  k <= 32 with D <= 256 selects inside the GEMM epilogue

@@ -10,11 +10,12 @@ from . import _lib
 from .nnet import Xtractor, MeanStdPooling, AttentivePooling, PreHalfResNet34, MfccFrontEnd, MelSpecFrontEnd
 from .nnet.xsets import IdMap, IdMapSet
 
-from .bosaris import Ndx, Scores, Key
+from .bosaris import Ndx, Scores, Key, TrialList, TrialScores
 from .statserver import StatServer
 from .iv_scoring import cosine_scoring, PLDA_scoring, fast_PLDA_scoring, full_PLDA_scoring, two_covariance_scoring, mahalanobis_scoring, score_matrix
 from .iv_scoring import score_topk, cosine_topk, PLDA_topk, TopK
-from .score_normalization import asnorm, znorm, tnorm, ztnorm
+from .iv_scoring import score_pairs, cosine_scoring_trials, PLDA_scoring_trials
+from .score_normalization import asnorm, znorm, tnorm, ztnorm, asnorm_trials
 from . import detplot
 from .detplot import pavx, rocch, rocch2eer, fast_minDCF, eer
 from .factor_analyser import FactorAnalyser

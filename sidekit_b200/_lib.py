@@ -66,6 +66,7 @@ def _declare(lib):
         "skb_trial_index_destroy": (None, [vp]),
         "skb_score_gemm_trials": (i32, [vp, vp, i32, i32, i32, vp, vp, f64, f64, i32, vp, vp, vp]),
         "skb_score_gemm_trials_packed": (i32, [vp, i32, vp, vp, vp, f64, f64, i32, vp, vp, vp]),
+        "skb_score_pairs": (i32, [vp, vp, i32, i32, i32, vp, vp, i64, vp, vp, f32, f32, vp, vp, vp, vp, vp, vp]),
         "skb_score_gemm_topk": (i32, [vp, vp, i32, i32, i32, vp, vp, f64, f64, i32, i32, vp, vp, vp]),
         "skb_score_gemm_topk_packed": (i32, [vp, i32, vp, vp, vp, f64, f64, i32, i32, vp, vp, vp]),
         "skb_widen_f32_f64": (i32, [vp, vp, i64, vp]),

@@ -259,6 +259,117 @@ class Ndx:
         return bool(ok)
 
 
+class TrialList:
+    """A trial list as three aligned 1-D arrays, one entry per trial in list order: ``enrolset`` / ``testset`` (ids) and
+    ``labels`` (bool, True = target; None for an unlabelled list).  Unlike ``Key`` / ``Ndx`` it is never a (models x
+    segments) matrix, so lists of VoxCeleb1-E / -H size (about 145 000 utterances, 580 000 trials) stay O(trials)."""
+
+    def __init__(self, enrolset=(), testset=(), labels=None):
+        self.enrolset = numpy.asarray(enrolset)
+        self.testset = numpy.asarray(testset)
+        self.labels = None if labels is None else numpy.asarray(labels, dtype=bool)
+        if self.enrolset.ndim != 1 or self.testset.shape != self.enrolset.shape or \
+                (self.labels is not None and self.labels.shape != self.enrolset.shape):
+            raise ValueError("TrialList: enrolset, testset and labels must be aligned 1-D arrays")
+
+    def __len__(self):
+        return self.enrolset.shape[0]
+
+    @classmethod
+    def read_txt(cls, path):
+        """The ``Key`` text format, ``model segment target|nontarget`` per line (what ``Key.write_txt`` writes), in file
+        order.  A line with any other label is an error."""
+        rows = _read_columns(path, 3)
+        label = numpy.array([r[2] for r in rows], dtype="U")
+        bad = (label != "target") & (label != "nontarget")
+        if bad.any():
+            raise ValueError("%s: label %r is neither 'target' nor 'nontarget'" % (path, label[bad][0]))
+        return cls(numpy.array([r[0] for r in rows], dtype="U"), numpy.array([r[1] for r in rows], dtype="U"), label == "target")
+
+    def write_txt(self, path):
+        """One ``model segment target|nontarget`` line per trial, in list order (``Key.read_txt`` reads it)."""
+        if self.labels is None:
+            raise ValueError("TrialList.write_txt: the list has no labels")
+        _makedirs_for(path)
+        with open(path, "w") as fid:
+            fid.writelines("{} {} {}\n".format(m, s, "target" if t else "nontarget")
+                           for m, s, t in zip(self.enrolset.tolist(), self.testset.tolist(), self.labels.tolist()))
+
+    @classmethod
+    def read_voxceleb(cls, path):
+        """The VoxCeleb list format, ``1|0 enrolment_path test_path`` per line (1 = target)."""
+        rows = _read_columns(path, 3)
+        label = numpy.array([r[0] for r in rows], dtype="U")
+        bad = (label != "1") & (label != "0")
+        if bad.any():
+            raise ValueError("%s: label %r is neither 1 nor 0" % (path, label[bad][0]))
+        return cls(numpy.array([r[1] for r in rows], dtype="U"), numpy.array([r[2] for r in rows], dtype="U"), label == "1")
+
+    @classmethod
+    def _from_mask(cls, modelset, segset, mask, tar=None):
+        idx = numpy.flatnonzero(mask)            # row-major: the order of scoremat[trialmask] and score_trials
+        n_seg = mask.shape[1]
+        return cls(numpy.asarray(modelset)[idx // n_seg], numpy.asarray(segset)[idx % n_seg],
+                   None if tar is None else tar.reshape(-1)[idx])
+
+    @classmethod
+    def from_key(cls, key):
+        """The trials of a ``Key`` (targets and non-targets) in row-major ``tar | non`` order."""
+        return cls._from_mask(key.modelset, key.segset, key.tar | key.non, key.tar)
+
+    @classmethod
+    def from_ndx(cls, ndx):
+        """The trials of an ``Ndx`` in row-major ``trialmask`` order, unlabelled."""
+        return cls._from_mask(ndx.modelset, ndx.segset, ndx.trialmask)
+
+    def subset(self, keep):
+        """The trials selected by a bool mask or an index array, in list order."""
+        return TrialList(self.enrolset[keep], self.testset[keep], None if self.labels is None else self.labels[keep])
+
+    def index(self, enrol_ids, test_ids):
+        """``(rows, cols, keep)``: for the trials whose enrolment id is in ``enrol_ids`` and whose test id is in ``test_ids``
+        (``keep``, a bool mask over the list), the int32 position of the FIRST occurrence of each id.  Other trials are
+        dropped, as ``Ndx.filter`` drops unknown models / segments, and logged at INFO."""
+        if max(len(enrol_ids), len(test_ids)) > numpy.iinfo(numpy.int32).max:
+            raise ValueError("TrialList.index: more than 2^31 - 1 rows")
+        etab = _first_index(enrol_ids)
+        ttab = etab if test_ids is enrol_ids else _first_index(test_ids)
+        n = len(self)
+        rows = numpy.fromiter((etab.get(v, -1) for v in self.enrolset.tolist()), dtype=numpy.int64, count=n)
+        cols = numpy.fromiter((ttab.get(v, -1) for v in self.testset.tolist()), dtype=numpy.int64, count=n)
+        keep = (rows >= 0) & (cols >= 0)
+        n_keep = int(keep.sum())
+        if n_keep < n:
+            logging.info('trials reduced from %d to %d (%d unknown enrolment ids, %d unknown test ids)', n, n_keep,
+                         int((rows < 0).sum()), int((cols < 0).sum()))
+            rows, cols = rows[keep], cols[keep]
+        return rows.astype(numpy.int32), cols.astype(numpy.int32), keep
+
+
+class TrialScores:
+    """Scores of a ``TrialList``, one per trial in list order: ``trials`` (the trials scored), ``scores`` (host numpy,
+    copied from ``scores_device`` when first read, like ``Scores.scoremat``)."""
+
+    def __init__(self, trials, scores_device, np_dtype=None):
+        self.trials = trials
+        self.scores_device = scores_device
+        self.scores_dtype = np_dtype         # numpy dtype of ``scores`` when it differs from the device tensor's
+        self._scores = None
+
+    @property
+    def scores(self):
+        if self._scores is None:
+            self._scores = _device_to_numpy(self.scores_device, self.scores_dtype)
+        return self._scores
+
+    def get_tar_non(self):
+        """Target and non-target score vectors, each in list order (``Scores.get_tar_non`` for a labelled list)."""
+        if self.trials.labels is None:
+            raise ValueError("TrialScores.get_tar_non: the trial list has no labels")
+        s = self.scores
+        return s[self.trials.labels], s[~self.trials.labels]
+
+
 class Scores:
     """Score matrix container (scores.py:52-81).  ``scoremat`` is materialised lazily: the CUDA result stays on
     the device (``scoremat_device``, a torch tensor) until the numpy array is first read."""

@@ -1314,6 +1314,74 @@ __global__ void widen_kernel(const float* __restrict__ src, double* __restrict__
     }
 }
 
+// ----------------------------------------------------------------------------- pair-list scoring
+// One score per (rows[p], cols[p]) trial: a gather of two rows and a D-term dot product, about 8 bytes read per 2 FLOP, so
+// the kernel is bound by the row loads and the tensor core has nothing to add.  kPairLanes lanes own one trial: lane l sums
+// the products of columns l, l + kPairLanes, ... (float4 units when VEC) in ascending order with float32 FMAs, then a fixed
+// xor butterfly over the group adds the partials.  So the bits of a score depend on D and the two rows only, not on the
+// trial's position, the list length or the grid.  Any D works (the loop has no tile); VEC needs D % 4 == 0 and 16-byte
+// aligned bases.  An index outside [0, Ne) / [0, Nt) is never dereferenced: its trial gets NaN.
+constexpr int kPairLanes = 8;
+constexpr int kPairThreads = 256;
+constexpr int kPairsPerCta = kPairThreads / kPairLanes;
+struct PairArgs {
+    const float* E; const float* T; int Ne, Nt, D;
+    const int32_t* rows; const int32_t* cols; long long n;
+    const float* rowterm; const float* colterm; float cst, alpha;
+    const float* mean_e; const float* std_e; const float* mean_t; const float* std_t;    // all NULL: no as-norm
+    float* out;
+};
+
+template <bool VEC>
+__global__ void __launch_bounds__(kPairThreads) score_pairs_kernel(const PairArgs a) {
+    pdl_wait();
+    const int sub = threadIdx.x & (kPairLanes - 1);
+    const long long p = (long long)blockIdx.x * kPairsPerCta + threadIdx.x / kPairLanes;
+    int i = -1, j = -1;
+    if (p < a.n) { i = __ldg(a.rows + p); j = __ldg(a.cols + p); }
+    const bool ok = p < a.n && (unsigned)i < (unsigned)a.Ne && (unsigned)j < (unsigned)a.Nt;
+    float acc = 0.f;
+    if (ok) {
+        const float* __restrict__ e = a.E + (size_t)i * a.D;
+        const float* __restrict__ t = a.T + (size_t)j * a.D;
+        if (VEC) {
+            const float4* __restrict__ e4 = reinterpret_cast<const float4*>(e);
+            const float4* __restrict__ t4 = reinterpret_cast<const float4*>(t);
+            const int n4 = a.D >> 2;
+            int k = sub;
+            for (; k + 3 * kPairLanes < n4; k += 4 * kPairLanes) {          // four float4 of each row in flight per lane
+                float4 x[4], y[4];
+#pragma unroll
+                for (int u = 0; u < 4; ++u) { x[u] = __ldg(e4 + k + u * kPairLanes); y[u] = __ldg(t4 + k + u * kPairLanes); }
+#pragma unroll
+                for (int u = 0; u < 4; ++u) {
+                    acc = fmaf(x[u].x, y[u].x, acc); acc = fmaf(x[u].y, y[u].y, acc);
+                    acc = fmaf(x[u].z, y[u].z, acc); acc = fmaf(x[u].w, y[u].w, acc);
+                }
+            }
+            for (; k < n4; k += kPairLanes) {
+                const float4 x = __ldg(e4 + k), y = __ldg(t4 + k);
+                acc = fmaf(x.x, y.x, acc); acc = fmaf(x.y, y.y, acc); acc = fmaf(x.z, y.z, acc); acc = fmaf(x.w, y.w, acc);
+            }
+        } else {
+            for (int k = sub; k < a.D; k += kPairLanes) acc = fmaf(__ldg(e + k), __ldg(t + k), acc);
+        }
+    }
+#pragma unroll
+    for (int o = kPairLanes / 2; o > 0; o >>= 1) acc += __shfl_xor_sync(0xffffffffu, acc, o);
+    if (p >= a.n || sub != 0) return;
+    if (!ok) {
+        a.out[p] = __int_as_float(0x7fc00000);
+        return;
+    }
+    // the score_matrix convention: alpha * (rowterm_i + colterm_j + cst) + alpha * dot
+    const float terms = (a.rowterm ? __ldg(a.rowterm + i) : 0.f) + (a.colterm ? __ldg(a.colterm + j) : 0.f) + a.cst;
+    float s = fmaf(a.alpha, acc, a.alpha * terms);
+    if (a.mean_e)      // symmetric as-norm, sidekit/score_normalization.py:135-138
+        s = 0.5f * (s - __ldg(a.mean_e + i)) / __ldg(a.std_e + i) + 0.5f * (s - __ldg(a.mean_t + j)) / __ldg(a.std_t + j);
+    a.out[p] = s;
+}
+
 }  // namespace skb
 
 using namespace skb;
@@ -1623,6 +1691,36 @@ int skb_asnorm_apply_panel(const float* X_dev, int N, int D, int row0, int n_row
     g_launches++;
     return score_gemm_general(X_dev + (size_t)row0 * D, X_dev, n_rows, N, D, ra + row0, ra, 0.f, r + row0, r, 0.f, 1.f, 30.f, 3, 0,
                               out_dev, ld_out, tmp_bytes, st);
+}
+
+int skb_score_pairs(const float* E_dev, const float* T_dev, int Ne, int Nt, int D, const int32_t* rows_dev, const int32_t* cols_dev,
+                    int64_t n_pairs, const float* rowterm_dev, const float* colterm_dev, float cst, float alpha, const float* mean_e_dev,
+                    const float* std_e_dev, const float* mean_t_dev, const float* std_t_dev, float* out_dev, void* stream) {
+    const int n_stats = (mean_e_dev != nullptr) + (std_e_dev != nullptr) + (mean_t_dev != nullptr) + (std_t_dev != nullptr);
+    if (Ne < 0 || Nt < 0 || D < 0 || n_pairs < 0 || (n_stats != 0 && n_stats != 4)) {
+        set_last_error(__FILE__, __LINE__, "score_pairs: bad arguments (negative size, or some but not all four as-norm vectors)");
+        return SKB_ERR_ARG;
+    }
+    if (n_pairs == 0) return SKB_OK;
+    if (!E_dev || !T_dev || !rows_dev || !cols_dev || !out_dev || D == 0) {
+        set_last_error(__FILE__, __LINE__, "score_pairs: null operand or D = 0");
+        return SKB_ERR_ARG;
+    }
+    const long long ctas = (n_pairs + kPairsPerCta - 1) / kPairsPerCta;
+    if (ctas > 0x7fffffffLL) {
+        set_last_error(__FILE__, __LINE__, "score_pairs: too many trials for one launch");
+        return SKB_ERR_ARG;
+    }
+    const PairArgs a{E_dev, T_dev, Ne, Nt, D, rows_dev, cols_dev, (long long)n_pairs, rowterm_dev, colterm_dev, cst, alpha,
+                     mean_e_dev, std_e_dev, mean_t_dev, std_t_dev, out_dev};
+    const bool vec = (D & 3) == 0 && (reinterpret_cast<uintptr_t>(E_dev) & 15) == 0 && (reinterpret_cast<uintptr_t>(T_dev) & 15) == 0;
+    cudaStream_t st = (cudaStream_t)stream;
+    if (vec)
+        SKB_CUDA_CHECK(launch_pdl(score_pairs_kernel<true>, dim3((unsigned)ctas), dim3(kPairThreads), 0, st, a));
+    else
+        SKB_CUDA_CHECK(launch_pdl(score_pairs_kernel<false>, dim3((unsigned)ctas), dim3(kPairThreads), 0, st, a));
+    g_launches++;
+    return SKB_OK;
 }
 
 }  // extern "C"

@@ -16,7 +16,7 @@ import numpy
 import torch
 
 from . import _lib
-from .bosaris import Ndx, Scores
+from .bosaris import Ndx, Scores, TrialScores
 from .statserver import StatServer
 
 
@@ -133,6 +133,112 @@ def score_trials(E, T, trials, rowterm=None, colterm=None, cst=0.0, alpha=1.0, p
             None if colterm is None else colterm.data_ptr(), float(cst), float(alpha), int(passes), trials._ptr, out.data_ptr(),
             _lib.stream_ptr()))
     return out[:trials.n_trials]
+
+
+def score_pairs(E, T, rows, cols, rowterm=None, colterm=None, cst=0.0, alpha=1.0):
+    """The scores of the trials ``(rows[p], cols[p])`` as a 1-D float32 CUDA tensor: entry p is
+    ``alpha * (rowterm[i] + colterm[j] + cst) + alpha * E[i] . T[j]`` with ``i = rows[p]``, ``j = cols[p]`` -- the
+    ``score_matrix`` entry (i, j) -- at O(trials) cost, for lists too large for an (Ne, Nt) mask (VoxCeleb1-E / -H).
+    ``E`` (Ne, D), ``T`` (Nt, D), ``rowterm`` (Ne,), ``colterm`` (Nt,): CUDA float32; ``rows`` / ``cols``: integer arrays
+    (numpy or torch).  The dot products are float32 FMAs over the float32 rows in a fixed order, so a trial's score has the
+    same bits wherever it sits in whichever list.  An index out of range gives NaN."""
+    return _score_pairs(E, T, rows, cols, rowterm, colterm, cst, alpha)
+
+
+def _score_pairs(E, T, rows, cols, rowterm=None, colterm=None, cst=0.0, alpha=1.0, asnorm_stats=None):
+    """``score_pairs``; ``asnorm_stats = (mean_e, std_e, mean_t, std_t)`` (float32 CUDA, indexed like ``E`` / ``T``)
+    normalises every score with the symmetric as-norm formula in the same kernel."""
+    dev = E.device
+    if dev.type != "cuda":
+        raise ValueError("score_pairs: E and T must be CUDA tensors")
+    rows = torch.as_tensor(rows).to(dev, torch.int32).contiguous()
+    cols = torch.as_tensor(cols).to(dev, torch.int32).contiguous()
+    if rows.dim() != 1 or rows.shape != cols.shape:
+        raise ValueError("score_pairs: rows and cols must be 1-D arrays of one length")
+    if E.dim() != 2 or T.dim() != 2 or E.shape[1] != T.shape[1]:
+        raise ValueError("score_pairs: E and T must be (Ne, D) and (Nt, D)")
+    vectors = [(rowterm, E.shape[0]), (colterm, T.shape[0])]
+    if asnorm_stats is not None:
+        vectors += [(asnorm_stats[0], E.shape[0]), (asnorm_stats[1], E.shape[0]), (asnorm_stats[2], T.shape[0]), (asnorm_stats[3], T.shape[0])]
+    for t, n in [(E, None), (T, None)] + vectors:
+        if t is not None and (t.dtype != torch.float32 or t.device != dev or (n is not None and tuple(t.shape) != (n,))):
+            raise ValueError("score_pairs: operands and per-row vectors must be float32 on %s, one value per row" % dev)
+    E, T = E.contiguous(), T.contiguous()
+    ptr = lambda t: None if t is None else t.contiguous().data_ptr()
+    me, se, mt, st = asnorm_stats if asnorm_stats is not None else (None,) * 4
+    out = torch.empty((rows.shape[0],), dtype=torch.float32, device=dev)
+    with torch.cuda.device(dev):
+        _lib.check(_lib.lib().skb_score_pairs(E.data_ptr(), T.data_ptr(), E.shape[0], T.shape[0], E.shape[1], rows.data_ptr(),
+                                              cols.data_ptr(), rows.shape[0], ptr(rowterm), ptr(colterm), float(cst), float(alpha),
+                                              ptr(me), ptr(se), ptr(mt), ptr(st), out.data_ptr(), _lib.stream_ptr()))
+    return out
+
+
+def _referenced(rows, cols, shared):
+    """The rows a trial list references and the trials' positions among them: ``(ref_e, ref_t, r, c)`` with ``ref_e`` /
+    ``ref_t`` sorted row numbers and ``r`` / ``c`` int32 indices into them.  ``shared``: enrolment and test rows index one
+    matrix, so one set serves both sides (one upload, one preparation)."""
+    if shared:
+        ref, inv = numpy.unique(numpy.concatenate([rows, cols]), return_inverse=True)
+        inv = inv.astype(numpy.int32)
+        return ref, ref, inv[:rows.shape[0]], inv[rows.shape[0]:]
+    ref_e, r = numpy.unique(rows, return_inverse=True)
+    ref_t, c = numpy.unique(cols, return_inverse=True)
+    return ref_e, ref_t, r.astype(numpy.int32), c.astype(numpy.int32)
+
+
+def _trial_rows(server, ref):
+    """A StatServer holding rows ``ref`` of ``server.stat1`` only (for the StatServer methods, which rebind ``stat1``)."""
+    out = StatServer()
+    out.stat1 = server.stat1[ref]
+    return out
+
+
+def cosine_scoring_trials(enroll, test, trials, wccn=None):
+    """Cosine similarities of the trials of a ``TrialList`` -- ``cosine_scoring`` at O(trials) cost.  Trials whose ids are
+    not in ``enroll.modelset`` / ``test.segset`` are dropped (the first occurrence of an id wins, as in
+    ``cosine_scoring``).  Rows are WCCN-rotated and length-normalised like ``cosine_scoring``; when ``enroll`` and
+    ``test`` share their embeddings (one StatServer for both, the VoxCeleb1-E / -H case) they are prepared once.
+    Returns ``TrialScores`` with float32 scores; the caller's objects are not modified."""
+    assert isinstance(enroll, StatServer), 'First parameter should be a StatServer'
+    assert isinstance(test, StatServer), 'Second parameter should be a StatServer'
+    rows, cols, keep = trials.index(enroll.modelset, test.segset)
+    shared = enroll.stat1 is test.stat1
+    ref_e, ref_t, r, c = _referenced(rows, cols, shared)
+    dev = _device()
+    sides = []
+    for server, ref in ((enroll, ref_e), (test, ref_t))[:1 if shared else 2]:
+        part = _trial_rows(server, ref)
+        if wccn is not None:
+            part.rotate_stat1(wccn)
+        part.norm_stat1()
+        sides.append(_dev32(part.stat1, dev))
+    E, T = sides[0], sides[-1]
+    return TrialScores(trials.subset(keep), _score_pairs(E, T, r, c))
+
+
+def PLDA_scoring_trials(enroll, test, trials, mu, F, Sigma, scaling_factor=1.):
+    """Simplified PLDA log-likelihood ratios of the trials of a ``TrialList`` -- ``fast_PLDA_scoring`` at O(trials) cost:
+    duplicate enrolment ids are averaged first (``mean_stat_per_model``), trials with unknown ids are dropped, and the
+    row / column terms come from the same device preparation (``_quadratic_prepare``).  Returns ``TrialScores`` with
+    float64 scores like the PLDA scorers (float32-class precision); the caller's objects are not modified."""
+    assert isinstance(enroll, StatServer), 'First parameter should be a StatServer'
+    assert isinstance(test, StatServer), 'Second parameter should be a StatServer'
+    assert enroll.stat1.shape[1] == test.stat1.shape[1], 'I-vectors dimension mismatch'
+    enroll_ctr = _unique_models(enroll)
+    rows, cols, keep = trials.index(enroll_ctr.modelset, test.segset)
+    kept = trials.subset(keep)
+    dev = _device()
+    if not keep.any():
+        return TrialScores(kept, torch.empty((0,), dtype=torch.float32, device=dev), numpy.float64)
+    shared = enroll_ctr.stat1 is test.stat1
+    ref_e, ref_t, r, c = _referenced(rows, cols, shared)
+    Phi, Psi, plda_cst = _simplified_plda_terms(F, Sigma, scaling_factor)
+    E = _dev32(enroll_ctr.stat1[ref_e], dev)
+    T = E if shared else _dev32(test.stat1[ref_t], dev)
+    Ep, model_part = _quadratic_prepare(E, mu, Psi, Phi)
+    Tc, seg_part = _quadratic_prepare(T, mu, None, Phi)
+    return TrialScores(kept, _score_pairs(Ep, Tc, r, c, model_part, seg_part, cst=plda_cst, alpha=scaling_factor), numpy.float64)
 
 
 TOPK_MAX = 1024

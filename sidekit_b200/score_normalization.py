@@ -90,3 +90,48 @@ def asnorm(enrol_xv, cohort_xv, ndx=None, topk=200, return_device=False):
         return out
     from .bosaris import _device_to_numpy
     return _device_to_numpy(out)                     # pinned, PCIe-speed path for large matrices
+
+
+def _ids_and_rows(side, ids_attr):
+    """``(ids, embeddings)`` of an ``asnorm_trials`` operand: a StatServer (``ids_attr``, ``stat1``) or an ``(ids, X)`` pair."""
+    from .statserver import StatServer
+    if isinstance(side, StatServer):
+        return getattr(side, ids_attr), side.stat1
+    ids, X = side
+    return ids, X
+
+
+def _rows_on_device(X, ref, dev):
+    """Rows ``ref`` (sorted) of ``X`` (numpy or torch, any device) as a contiguous float32 tensor on ``dev``; the whole
+    matrix as it is when every row is referenced."""
+    if ref.shape[0] != X.shape[0]:
+        X = X[ref] if not torch.is_tensor(X) else X[torch.from_numpy(ref).to(X.device)]
+    return torch.as_tensor(X).to(dev, torch.float32).contiguous()
+
+
+def asnorm_trials(enroll, test, trials, cohort_xv, topk=200):
+    """Symmetric adaptive s-norm of the cosine scores of the trials of a ``TrialList``: per trial (e, t),
+    ``0.5 (s - mu_e) / sigma_e + 0.5 (s - mu_t) / sigma_t`` with ``s = e . t``, the entry of ``asnorm``'s N x N matrix
+    without the matrix (VoxCeleb1-E / -H: 145 000 utterances, 84 GB as a float32 matrix).  ``asnorm``'s conventions: rows
+    are taken as given (unit-norm embeddings expected, no normalisation here), the cohort is L2-normalised, mu / sigma are
+    the mean and unbiased std of a row's ``topk`` best cohort scores, which needs ``topk <= C <= 51 200`` cohort rows.
+
+    ``enroll`` / ``test``: StatServers (ids ``enroll.modelset`` / ``test.segset``, rows ``stat1``) or ``(ids, X)`` pairs
+    with X an (N, D) numpy array or torch tensor.  The statistics are computed for the rows the kept trials reference, once
+    when both sides are the same object or share their embeddings.  Trials with unknown ids are dropped.  Returns
+    ``TrialScores`` with float32 scores."""
+    from . import bulk
+    from .bosaris import TrialScores
+    from .iv_scoring import _device, _referenced, _score_pairs
+    ids_e, Xe = _ids_and_rows(enroll, "modelset")
+    ids_t, Xt = _ids_and_rows(test, "segset")
+    rows, cols, keep = trials.index(ids_e, ids_t)
+    shared = enroll is test or Xe is Xt
+    dev = Xe.device if torch.is_tensor(Xe) and Xe.is_cuda else _device()
+    ref_e, ref_t, r, c = _referenced(rows, cols, shared)
+    E = _rows_on_device(Xe, ref_e, dev)
+    T = E if shared else _rows_on_device(Xt, ref_t, dev)
+    coh = torch.nn.functional.normalize(torch.as_tensor(cohort_xv).to(dev, torch.float32), dim=1).contiguous()
+    mean_e, std_e = bulk._asnorm_stats_cuda(E, coh, topk)
+    mean_t, std_t = (mean_e, std_e) if shared else bulk._asnorm_stats_cuda(T, coh, topk)
+    return TrialScores(trials.subset(keep), _score_pairs(E, T, r, c, asnorm_stats=(mean_e, std_e, mean_t, std_t)))
