@@ -7,6 +7,7 @@
 #include <cuda_bf16.h>
 #include <stdint.h>
 #include <stdio.h>
+#include <atomic>
 
 namespace skb {
 
@@ -41,15 +42,6 @@ struct PerDeviceOnce {
 
 void set_last_error(const char* file, int line, const char* msg);
 
-// Launch check.  With SKB_SYNC_CHECK=1 in the environment every launch is followed by a stream synchronisation, so an
-// execution fault is reported at the kernel that caused it (compute-sanitizer is not always available).
-bool sync_check_enabled();
-#define SKB_LAUNCH_CHECK(stream)                                                              \
-    do {                                                                                      \
-        SKB_CUDA_CHECK(cudaGetLastError());                                                   \
-        if (skb::sync_check_enabled()) SKB_CUDA_CHECK(cudaStreamSynchronize(stream));         \
-    } while (0)
-
 // ----------------------------------------------------------------------------- programmatic dependent launch (PDL)
 // The kernels of the per-block chain (conv1 -> channel sums -> border sums -> SE partial means -> SE FC -> conv2) depend on
 // each other one after the other.  Launched with the programmatic-stream-serialization attribute, kernel k+1 is scheduled
@@ -66,19 +58,33 @@ __device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;"
 // sums) runs beside it instead of behind it
 __device__ __forceinline__ void pdl_trigger_now() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
 bool pdl_enabled();
+
+// ----------------------------------------------------------------------------- kernel launch
+// Every kernel of the library is launched here, so that skb_kernel_launches() counts each one and SKB_SYNC_CHECK=1
+// synchronises the stream after each one: an execution fault is then reported at the SKB_CUDA_CHECK of the launch that
+// caused it (compute-sanitizer is not always available).  pdl = true launches with the programmatic-stream-serialization
+// attribute (see above; SKB_NO_PDL=1 turns it off), pdl = false in plain stream order.
+extern std::atomic<long long> g_launches;
+bool sync_check_enabled();
 template <typename... KArgs, typename... Args>
-inline cudaError_t launch_pdl(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t st, Args&&... args) {
+inline cudaError_t launch_kernel(bool pdl, void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t st,
+                                 Args&&... args) {
     cudaLaunchConfig_t cfg = {};
     cfg.gridDim = grid;
     cfg.blockDim = block;
     cfg.dynamicSmemBytes = smem;
     cfg.stream = st;
     cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[0].val.programmaticStreamSerializationAllowed = pdl_enabled() ? 1 : 0;
-    cfg.attrs = attr;
-    cfg.numAttrs = 1;
-    return cudaLaunchKernelEx(&cfg, kernel, KArgs(args)...);
+    if (pdl) {
+        attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+        attr[0].val.programmaticStreamSerializationAllowed = pdl_enabled() ? 1 : 0;
+        cfg.attrs = attr;
+        cfg.numAttrs = 1;
+    }
+    const cudaError_t e = cudaLaunchKernelEx(&cfg, kernel, KArgs(args)...);
+    if (e != cudaSuccess) return e;
+    ++g_launches;
+    return sync_check_enabled() ? cudaStreamSynchronize(st) : cudaSuccess;
 }
 
 // ----------------------------------------------------------------------------- shared-memory address

@@ -18,10 +18,8 @@
 #include "class_sum.cuh"
 
 #include <algorithm>
-#include <atomic>
 
 namespace skb {
-extern std::atomic<long long> g_launches;
 
 namespace {
 
@@ -379,12 +377,10 @@ int gram_launch(const T* X, long long N, int D, long long ld, const double* shif
     const GramPlan p = gram_plan(N, D);
     Workspace ws(st);
     SKB_CUDA_CHECK(ws.alloc((size_t)p.chunks * p.tiles * kGT * kGT));
-    gram_f64_kernel<T><<<dim3(p.tiles, (unsigned)p.chunks), kGThreads, 0, st>>>(X, N, D, ld, shift, shift_idx, w, p.chunk_rows, ws.p);
-    SKB_LAUNCH_CHECK(st);
+    SKB_CUDA_CHECK(launch_kernel(false, gram_f64_kernel<T>, dim3(p.tiles, (unsigned)p.chunks), kGThreads, 0, st, X, N, D, ld, shift, shift_idx, w,
+                                 p.chunk_rows, ws.p));
     const long long n = (long long)D * D;
-    gram_reduce_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(ws.p, p.chunks, p.tiles, D, scale, G);
-    SKB_LAUNCH_CHECK(st);
-    g_launches += 2;
+    SKB_CUDA_CHECK(launch_kernel(false, gram_reduce_kernel, (unsigned)((n + 255) / 256), 256, 0, st, ws.p, p.chunks, p.tiles, D, scale, G));
     return SKB_OK;
 }
 
@@ -395,22 +391,13 @@ int class_stats_launch(const T* X, long long N, int D, long long ld, const int* 
         const long long chunks = (N + kMeanRows - 1) / kMeanRows;
         Workspace ws(st);
         SKB_CUDA_CHECK(ws.alloc((size_t)chunks * D));
-        colsum_partial_kernel<T><<<dim3((unsigned)chunks, (D + 127) / 128), 128, 0, st>>>(X, N, D, ld, ws.p);
-        SKB_LAUNCH_CHECK(st);
-        colsum_final_kernel<<<(D + 127) / 128, 128, 0, st>>>(ws.p, chunks, D, 1.0 / (double)N, mean);
-        SKB_LAUNCH_CHECK(st);
-        g_launches += 2;
+        SKB_CUDA_CHECK(launch_kernel(false, colsum_partial_kernel<T>, dim3((unsigned)chunks, (D + 127) / 128), 128, 0, st, X, N, D, ld, ws.p));
+        SKB_CUDA_CHECK(launch_kernel(false, colsum_final_kernel, (D + 127) / 128, 128, 0, st, ws.p, chunks, D, 1.0 / (double)N, mean));
     }
-    if (sums) {
-        class_sum_kernel<T><<<dim3((D + 127) / 128, n_cls), 128, 0, st>>>(X, D, ld, cls_ptr, cls_rows, n_cls, 1.0, sums);
-        SKB_LAUNCH_CHECK(st);
-        g_launches++;
-    }
-    if (counts) {
-        class_count_kernel<<<(n_cls + 255) / 256, 256, 0, st>>>(cls_ptr, n_cls, counts);
-        SKB_LAUNCH_CHECK(st);
-        g_launches++;
-    }
+    if (sums)
+        SKB_CUDA_CHECK(launch_kernel(false, class_sum_kernel<T>, dim3((D + 127) / 128, n_cls), 128, 0, st, X, D, ld, cls_ptr, cls_rows, n_cls, 1.0,
+                                     sums));
+    if (counts) SKB_CUDA_CHECK(launch_kernel(false, class_count_kernel, (n_cls + 255) / 256, 256, 0, st, cls_ptr, n_cls, counts));
     return SKB_OK;
 }
 
@@ -419,9 +406,8 @@ int affine_launch(const T* X, long long N, int D, long long ld, const double* mu
                   int unit_norm, U* Y, long long ld_out, cudaStream_t st) {
     if (!W) {
         const long long threads = N * 32;
-        affine_diag_rows_kernel<T, U><<<(unsigned)((threads + 255) / 256), 256, 0, st>>>(X, N, D, ld, mu, dsc, unit_norm, Y, ld_out);
-        SKB_LAUNCH_CHECK(st);
-        g_launches++;
+        SKB_CUDA_CHECK(launch_kernel(false, affine_diag_rows_kernel<T, U>, (unsigned)((threads + 255) / 256), 256, 0, st, X, N, D, ld, mu, dsc,
+                                     unit_norm, Y, ld_out));
         return SKB_OK;
     }
     static PerDeviceOnce once;
@@ -429,14 +415,11 @@ int affine_launch(const T* X, long long N, int D, long long ld, const double* mu
         SKB_CUDA_CHECK(cudaFuncSetAttribute(affine_dmma_kernel<T, U>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kAffineSmem));
     const bool fused = D_out <= kAN;
     dim3 grid((unsigned)((N + kAM - 1) / kAM), (D_out + kAN - 1) / kAN);
-    affine_dmma_kernel<T, U><<<grid, kAThreads, kAffineSmem, st>>>(X, N, D, ld, mu, dsc, W, D_out, unit_norm && fused, Y, ld_out);
-    SKB_LAUNCH_CHECK(st);
-    g_launches++;
+    SKB_CUDA_CHECK(launch_kernel(false, affine_dmma_kernel<T, U>, grid, kAThreads, kAffineSmem, st, X, N, D, ld, mu, dsc, W, D_out,
+                                 unit_norm && fused, Y, ld_out));
     if (unit_norm && !fused) {
         const long long threads = N * 32;
-        unit_norm_rows_kernel<U><<<(unsigned)((threads + 255) / 256), 256, 0, st>>>(Y, N, D_out, ld_out);
-        SKB_LAUNCH_CHECK(st);
-        g_launches++;
+        SKB_CUDA_CHECK(launch_kernel(false, unit_norm_rows_kernel<U>, (unsigned)((threads + 255) / 256), 256, 0, st, Y, N, D_out, ld_out));
     }
     return SKB_OK;
 }

@@ -65,8 +65,7 @@ static int launch_one(const ConvParams& p_in, cudaStream_t st) {
     p.n_tiles = (n_pix + Cfg::kTileM - 1) / Cfg::kTileM;
     const int n_items = p.n_tiles * (p.cout / N_CTA);
     const int grid = n_items < kNumSMs ? n_items : kNumSMs;      // persistent: one CTA per SM
-    SKB_CUDA_CHECK(launch_pdl(conv_umma_kernel<N_CTA, MT, BF16, FUSED, SC>, dim3(grid), dim3(kConvThreads), smem, st, p));
-    SKB_LAUNCH_CHECK(st);
+    SKB_CUDA_CHECK(launch_kernel(true, conv_umma_kernel<N_CTA, MT, BF16, FUSED, SC>, dim3(grid), dim3(kConvThreads), smem, st, p));
     return SKB_OK;
 }
 
@@ -97,8 +96,7 @@ static int launch_one3(const ConvParams& p_in, cudaStream_t st) {
     const int n_pix = p.p_end - p.G;
     p.n_tiles = (n_pix + Cfg::kTileOut - 1) / Cfg::kTileOut;
     const int grid = p.n_tiles < kNumSMs ? p.n_tiles : kNumSMs;
-    conv3_umma_kernel<N_CTA, MT, BF16><<<grid, kConvThreads, smem, st>>>(p);
-    SKB_LAUNCH_CHECK(st);
+    SKB_CUDA_CHECK(launch_kernel(false, conv3_umma_kernel<N_CTA, MT, BF16>, grid, kConvThreads, smem, st, p));
     return SKB_OK;
 }
 

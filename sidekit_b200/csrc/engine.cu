@@ -1006,8 +1006,7 @@ static int activate_plan(skb_xtractor* h, cudaStream_t st) {
         a.n_sums = B * Cmax;
         a.sums_first_block = blocks;
         blocks += (a.n_sums + 255) / 256;
-        plan_activate_kernel<<<blocks, 256, 0, st>>>(a);
-        SKB_CUDA_CHECK(cudaGetLastError());
+        SKB_CUDA_CHECK(launch_kernel(false, plan_activate_kernel, blocks, 256, 0, st, a));
     }
     if ((rc = h->feats.ensure((size_t)pl.total_frames * m.fe.n_out * sizeof(float)))) return rc;
     if ((rc = h->cmvn.ensure((size_t)B * m.fe.n_out * sizeof(float2)))) return rc;
@@ -1110,8 +1109,7 @@ static int build_pixmeta(skb_xtractor* h, cudaStream_t st) {
         M.phase_stride = Lo ? (long long)(L.C / 8) * Lo->plane : 0;
         blocks += (span_table_size(M.n) + 7) / 8;
     }
-    if (blocks > 0) planmeta_kernel<<<blocks, 256, 0, st>>>(a);
-    SKB_CUDA_CHECK(cudaGetLastError());
+    if (blocks > 0) SKB_CUDA_CHECK(launch_kernel(false, planmeta_kernel, blocks, 256, 0, st, a));
     return SKB_OK;
 }
 
@@ -1173,7 +1171,6 @@ static int run_conv(skb_xtractor* h, const ConvW& cw, int kind, const Level& Lg,
     p.sums = (sums != nullptr && cw.ncta == 32 && cw.cout == 32 && se_scale == nullptr) ? sums : nullptr;
     p.overflow = (unsigned*)h->ovf.p;
     if (sc) { p.sc_in = sc_in; p.sc_w = sc->w; p.sc_bias = sc->bias; p.sc_cin = sc->cin; }
-    g_launches++;
     return launch_conv_umma(p, cw.ncta, h->m.bf16, st);
 }
 
@@ -1217,11 +1214,8 @@ static int export_stage(skb_xtractor* h, const uint16_t* act, const Level& L, in
     const long long total = (long long)h->plan.B * L.C * h_max * L.W;
     *per_utt = (int64_t)L.C * h_max * L.W;
     const int blocks = (int)((total + 255) / 256);
-    if (h->m.bf16)
-        unpack_planes_kernel<true><<<blocks, 256, 0, st>>>(act, L.plane, L.C, L.W, L.Wp, L.G, h->d32 + L.o_utt_row0, h->d32 + L.o_utt_count, h_max, out, total);
-    else
-        unpack_planes_kernel<false><<<blocks, 256, 0, st>>>(act, L.plane, L.C, L.W, L.Wp, L.G, h->d32 + L.o_utt_row0, h->d32 + L.o_utt_count, h_max, out, total);
-    SKB_CUDA_CHECK(cudaGetLastError());
+    SKB_CUDA_CHECK(launch_kernel(false, h->m.bf16 ? unpack_planes_kernel<true> : unpack_planes_kernel<false>, blocks, 256, 0, st, act, L.plane,
+                                 L.C, L.W, L.Wp, L.G, h->d32 + L.o_utt_row0, h->d32 + L.o_utt_count, h_max, out, total));
     return SKB_OK;
 }
 
@@ -1236,12 +1230,10 @@ static int head_and_logits(skb_xtractor* h, int norm_embedding, float* emb_out, 
     SKB_TRY(launch_skinny_gemm((const float*)h->pooled.p, B, 2 * D, m.lin_w, m.emb, m.lin_b, 1.f, (float*)h->lin.p, m.emb,
                                (float*)h->skinny_ws.p, st));
     SKB_TRY(launch_head_norm((const float*)h->lin.p, m.be_s, m.be_t, B, m.emb, norm_embedding, (float*)h->emb_pre.p, emb_out, st));
-    g_launches += 2;
     if (logits_out && m.n_spk > 0) {   // ArcMarginProduct(target=None): s * cos (loss.py:299-310); 'aps': Linear(x) (loss.py:356-359)
         SKB_TRY(launch_skinny_gemm(m.head_linear ? (const float*)h->emb_pre.p : emb_out, B, m.emb, m.spk_wn, m.n_spk,
                                    m.head_linear ? m.spk_b : nullptr, m.head_linear ? 1.f : m.margin_s, logits_out, m.n_spk,
                                    (float*)h->skinny_ws.p, st));
-        g_launches++;
     }
     return SKB_OK;
 }
@@ -1276,7 +1268,6 @@ static int forward_hr34(skb_xtractor* h, const float* wave, int norm_embedding, 
         SKB_TRY(frontend_launch(m.fe, wave, d64 + pl.o_wave_off, d32 + pl.o_wave_len, d64 + pl.o_feat_off, d32 + pl.o_nframes, B,
                                 pl.t_max, feats, (float2*)h->cmvn.p, h->cmvn_part.p, false, nullptr, st));
     }
-    g_launches += 3;
     auto buf = [&](int level, int k) { return (uint16_t*)h->act[level * 5 + k].p; };
     const Level& L1 = pl.lv[0];
     {
@@ -1288,7 +1279,6 @@ static int forward_hr34(skb_xtractor* h, const float* wave, int norm_embedding, 
             SKB_TRY(launch_stem(m.bf16, m.stem_c, feats, d64 + pl.o_feat_off, d32 + pl.o_nframes, (const float2*)h->cmvn.p, m.stem, buf(0, 0),
                                 L1.plane, L1.G, L1.p_end, L1.Wp, L1.W, d32 + L1.o_row_b, d32 + L1.o_row_h, (unsigned*)h->ovf.p, st));
     }
-    g_launches++;
     int level = 0, cur = 0;   // current activation = buf(level, cur), cur in {0, 1}
     if (stop && !strcmp(stop, "stem")) return export_stage(h, buf(0, 0), L1, h_max, dbg_out, per_utt, st);
     bool x_is_ps = false;     // the current activation lives phase-split in buf(level + 1, 3) instead of buf(level, cur)
@@ -1346,7 +1336,6 @@ static int forward_hr34(skb_xtractor* h, const float* wave, int norm_embedding, 
                              next_strides ? &pl.lv[level + 1] : nullptr, st, nullptr, fold_sc ? &bw.sc : nullptr, x));
         }
         x_is_ps = next_strides;
-        g_launches += 4;
         cur ^= 1;
         if (stop && !strcmp(stop, name)) return export_stage(h, buf(level, cur), L, h_max, dbg_out, per_utt, st);
     }
@@ -1381,7 +1370,6 @@ static int forward_hr34(skb_xtractor* h, const float* wave, int norm_embedding, 
     SKB_TRY(launch_att_act(Hh, (const float*)h->hb.p, d32 + pl.o_frame_utt, m.att_bn_s, m.att_bn_t, F, A, st));
     SKB_TRY(gemm_nt_split(Hh, F, A, m.p_w2, m.att_b2, 1.f, Lg, D, st));
     SKB_TRY(launch_softmax_pool(m.bf16, X, Lg, d64 + pl.o_pool_off, d32 + pl.o_pool_nfr, B, D, (float*)h->pooled.p, st));
-    g_launches += 7;
     if (stop && !strcmp(stop, "pooled")) {
         *per_utt = 2 * D;
         SKB_CUDA_CHECK(cudaMemcpyAsync(dbg_out, h->pooled.p, (size_t)B * 2 * D * sizeof(float), cudaMemcpyDeviceToDevice, st));
@@ -1411,7 +1399,6 @@ static int forward_tdnn(skb_xtractor* h, const float* wave, int norm_embedding, 
     const Level& L0 = pl.lv[0];
     SKB_TRY(launch_pack_frames(m.bf16, feats, m.fe.n_out, L0.C, (int)pl.total_frames, d32 + pl.o_row_src, d32 + L0.o_row_b,
                                (const float2*)h->cmvn.p, (uint16_t*)h->act[0].p, L0.plane, L0.G, st));
-    g_launches += 4;
     for (int i = 0; i < 5; ++i) {
         int shifts[10];
         for (int k = 0; k < m.tdnn_k[i]; ++k) shifts[k] = k * m.tdnn_d[i];
@@ -1434,7 +1421,6 @@ static int forward_tdnn(skb_xtractor* h, const float* wave, int norm_embedding, 
     // a frame; the first T - 14 rows of an utterance are its valid output frames)
     SKB_TRY(launch_meanstd_planes(m.bf16, (const uint16_t*)h->act[5].p, L5.plane, L5.G, d32 + L5.o_utt_row0, d32 + pl.o_pool_nfr, B, D,
                                   m.pool_s, m.pool_t, (float*)h->pooled.p, st));
-    g_launches += 1;
     if (stop && !strcmp(stop, "pooled")) {
         *per_utt = 2 * D;
         SKB_CUDA_CHECK(cudaMemcpyAsync(dbg_out, h->pooled.p, (size_t)B * 2 * D * sizeof(float), cudaMemcpyDeviceToDevice, st));
@@ -1683,7 +1669,6 @@ int skb_xtractor_frontend(skb_xtractor_t* h, const float* wave_dev, const int64_
         return SKB_ERR_ARG;
     }
     SKB_CUDA_CHECK(cudaMemsetAsync(feats_dev, 0, (size_t)n_utt * h->m.fe.n_out * t_max * sizeof(float), st));
-    g_launches += 4;
     return frontend_launch(h->m.fe, wave_dev, h->d64 + pl.o_wave_off, h->d32 + pl.o_wave_len, h->d64 + pl.o_feat_off,
                            h->d32 + pl.o_nframes, n_utt, t_max, (float*)h->feats.p, (float2*)h->cmvn.p, h->cmvn_part.p, true,
                            feats_dev, st);

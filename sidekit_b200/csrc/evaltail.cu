@@ -11,14 +11,12 @@
 #include "common.cuh"
 
 #include <algorithm>
-#include <atomic>
 #include <cmath>
 #include <cstring>
 #include <numeric>
 #include <vector>
 
 namespace skb {
-extern std::atomic<long long> g_launches;
 
 // ----------------------------------------------------------------------------- PAV
 // detplot.py:289-347.  Returns the number of bins.  `ghat` reproduces the reference's output INCLUDING its quirk: the
@@ -271,20 +269,19 @@ int skb_scoremat_stats(const void* S_dev, int M, int N, int64_t ld, int is_f64, 
         return SKB_ERR_ARG;
     }
     cudaStream_t st = (cudaStream_t)stream;
+    const double* S64 = (const double*)S_dev;
+    const float* S32 = (const float*)S_dev;
     if (axis == 1) {
-        if (is_f64) stats_rows_kernel<double><<<(M + 7) / 8, 256, 0, st>>>((const double*)S_dev, M, N, ld, sym, mean_dev, std_dev);
-        else stats_rows_kernel<float><<<(M + 7) / 8, 256, 0, st>>>((const float*)S_dev, M, N, ld, sym, mean_dev, std_dev);
+        if (is_f64) SKB_CUDA_CHECK(launch_kernel(false, stats_rows_kernel<double>, (M + 7) / 8, 256, 0, st, S64, M, N, ld, sym, mean_dev, std_dev));
+        else SKB_CUDA_CHECK(launch_kernel(false, stats_rows_kernel<float>, (M + 7) / 8, 256, 0, st, S32, M, N, ld, sym, mean_dev, std_dev));
         if (sym) {
-            if (is_f64) sym_var_kernel<double><<<(M + 7) / 8, 256, 0, st>>>((const double*)S_dev, M, N, ld, mean_dev, std_dev);
-            else sym_var_kernel<float><<<(M + 7) / 8, 256, 0, st>>>((const float*)S_dev, M, N, ld, mean_dev, std_dev);
-            g_launches++;
+            if (is_f64) SKB_CUDA_CHECK(launch_kernel(false, sym_var_kernel<double>, (M + 7) / 8, 256, 0, st, S64, M, N, ld, mean_dev, std_dev));
+            else SKB_CUDA_CHECK(launch_kernel(false, sym_var_kernel<float>, (M + 7) / 8, 256, 0, st, S32, M, N, ld, mean_dev, std_dev));
         }
     } else {
-        if (is_f64) stats_cols_kernel<double><<<(N + 127) / 128, 128, 0, st>>>((const double*)S_dev, M, N, ld, mean_dev, std_dev);
-        else stats_cols_kernel<float><<<(N + 127) / 128, 128, 0, st>>>((const float*)S_dev, M, N, ld, mean_dev, std_dev);
+        if (is_f64) SKB_CUDA_CHECK(launch_kernel(false, stats_cols_kernel<double>, (N + 127) / 128, 128, 0, st, S64, M, N, ld, mean_dev, std_dev));
+        else SKB_CUDA_CHECK(launch_kernel(false, stats_cols_kernel<float>, (N + 127) / 128, 128, 0, st, S32, M, N, ld, mean_dev, std_dev));
     }
-    g_launches++;
-    SKB_LAUNCH_CHECK(st);
     return SKB_OK;
 }
 
@@ -297,10 +294,12 @@ int skb_scoremat_normalise(const void* S_dev, int M, int N, int64_t ld, int is_f
     cudaStream_t st = (cudaStream_t)stream;
     const long long total = (long long)M * N;
     const unsigned blocks = (unsigned)((total + 255) / 256);
-    if (is_f64) normalise_kernel<double><<<blocks, 256, 0, st>>>((const double*)S_dev, M, N, ld, sub_dev, div_dev, (double*)out_dev, ld_out);
-    else normalise_kernel<float><<<blocks, 256, 0, st>>>((const float*)S_dev, M, N, ld, sub_dev, div_dev, (float*)out_dev, ld_out);
-    g_launches++;
-    SKB_LAUNCH_CHECK(st);
+    if (is_f64)
+        SKB_CUDA_CHECK(launch_kernel(false, normalise_kernel<double>, blocks, 256, 0, st, (const double*)S_dev, M, N, ld, sub_dev, div_dev,
+                                     (double*)out_dev, ld_out));
+    else
+        SKB_CUDA_CHECK(launch_kernel(false, normalise_kernel<float>, blocks, 256, 0, st, (const float*)S_dev, M, N, ld, sub_dev, div_dev,
+                                     (float*)out_dev, ld_out));
     return SKB_OK;
 }
 

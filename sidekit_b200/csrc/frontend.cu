@@ -478,7 +478,7 @@ int frontend_launch(const FrontendConsts& fc, const float* wave, const long long
             set_last_error(__FILE__, __LINE__, "front-end: tables do not fit in shared memory");
             return SKB_ERR_ARG;
         }
-        frontend_kernel<NC, WPC><<<grid, WPC * 32, smem, stream>>>(p, frames_per_cta);
+        SKB_CUDA_CHECK(launch_kernel(false, frontend_kernel<NC, WPC>, grid, WPC * 32, smem, stream, p, frames_per_cta));
     } else if (fc.n_fft == 2048) {
         // a frame needs 9.3 KB of shared memory and the tables 52 KB: 16 frame-warps in one CTA per SM
         constexpr int NC = 1024, WPC = 16;
@@ -493,21 +493,20 @@ int frontend_launch(const FrontendConsts& fc, const float* wave, const long long
             set_last_error(__FILE__, __LINE__, "front-end: tables do not fit in shared memory");
             return SKB_ERR_ARG;
         }
-        frontend_kernel<NC, WPC><<<grid, WPC * 32, smem, stream>>>(p, frames_per_cta);
+        SKB_CUDA_CHECK(launch_kernel(false, frontend_kernel<NC, WPC>, grid, WPC * 32, smem, stream, p, frames_per_cta));
     } else {
         set_last_error(__FILE__, __LINE__, "unsupported n_fft (1024 or 2048)");
         return SKB_ERR_ARG;
     }
-    SKB_LAUNCH_CHECK(stream);
     const int max_chunks = (t_max + kCmvnChunk - 1) / kCmvnChunk;
-    cmvn_partial_kernel<<<dim3(max_chunks, B), 128, 0, stream>>>(feats, feat_off, n_frames, fc.n_out, max_chunks, (double2*)cmvn_part);
-    cmvn_final_kernel<<<B, 128, 0, stream>>>((const double2*)cmvn_part, n_frames, fc.n_out, max_chunks, cmvn);
+    SKB_CUDA_CHECK(launch_kernel(false, cmvn_partial_kernel, dim3(max_chunks, B), 128, 0, stream, feats, feat_off, n_frames, fc.n_out, max_chunks,
+                                 (double2*)cmvn_part));
+    SKB_CUDA_CHECK(launch_kernel(false, cmvn_final_kernel, B, 128, 0, stream, (const double2*)cmvn_part, n_frames, fc.n_out, max_chunks, cmvn));
     if (normalise) {
         const long long per_utt = (long long)t_max * fc.n_out;
-        cmvn_apply_kernel<<<dim3((unsigned)((per_utt + 255) / 256), B), 256, 0, stream>>>(feats, feat_off, n_frames, fc.n_out, cmvn,
-                                                                                        api_out, t_max);
+        SKB_CUDA_CHECK(launch_kernel(false, cmvn_apply_kernel, dim3((unsigned)((per_utt + 255) / 256), B), 256, 0, stream, feats, feat_off, n_frames,
+                                     fc.n_out, cmvn, api_out, t_max));
     }
-    SKB_LAUNCH_CHECK(stream);
     return SKB_OK;
 }
 

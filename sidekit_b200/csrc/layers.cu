@@ -94,15 +94,14 @@ int launch_stem(bool bf16, int cout, const float* feats, const long long* feat_o
     const int n = p_end - G;
     const int threads = 128;
     const int blocks = (n + threads * kStemPix - 1) / (threads * kStemPix);
-#define SKB_STEM(BF, C) stem_kernel<BF, C><<<blocks, threads, 0, st>>>(sc, feats, feat_off, n_frames, cmvn, out, out_plane, G, p_end, Wp, W, row_b, row_h, overflow)
-    if (cout == 32) { if (bf16) SKB_STEM(true, 32); else SKB_STEM(false, 32); }
-    else if (cout == 128) { if (bf16) SKB_STEM(true, 128); else SKB_STEM(false, 128); }
-    else {
+    if (cout != 32 && cout != 128) {
         set_last_error(__FILE__, __LINE__, "stem: 32 or 128 output channels");
         return SKB_ERR_ARG;
     }
-#undef SKB_STEM
-    SKB_LAUNCH_CHECK(st);
+    const auto kernel = cout == 32 ? (bf16 ? stem_kernel<true, 32> : stem_kernel<false, 32>)
+                                   : (bf16 ? stem_kernel<true, 128> : stem_kernel<false, 128>);
+    SKB_CUDA_CHECK(launch_kernel(false, kernel, blocks, threads, 0, st, sc, feats, feat_off, n_frames, cmvn, out, out_plane, G, p_end, Wp, W, row_b,
+                                 row_h, overflow));
     return SKB_OK;
 }
 
@@ -168,11 +167,8 @@ int launch_stem7(bool bf16, const float* feats, const long long* feat_off, const
     const int n = p_end - G;
     const int threads = 128;
     const int blocks = (n + threads - 1) / threads;
-    if (bf16)
-        stem7_kernel<true><<<blocks, threads, 0, st>>>(sc, feats, feat_off, n_frames, cmvn, out, out_plane, G, p_end, Wp, W, F, row_b, row_h, overflow);
-    else
-        stem7_kernel<false><<<blocks, threads, 0, st>>>(sc, feats, feat_off, n_frames, cmvn, out, out_plane, G, p_end, Wp, W, F, row_b, row_h, overflow);
-    SKB_LAUNCH_CHECK(st);
+    SKB_CUDA_CHECK(launch_kernel(false, bf16 ? stem7_kernel<true> : stem7_kernel<false>, blocks, threads, 0, st, sc, feats, feat_off, n_frames, cmvn,
+                                 out, out_plane, G, p_end, Wp, W, F, row_b, row_h, overflow));
     return SKB_OK;
 }
 
@@ -183,8 +179,7 @@ __global__ void broadcast_rows_kernel(const float* __restrict__ bias, int B, int
 }
 
 int launch_broadcast_rows(const float* bias, int B, int A, float* out, cudaStream_t st) {
-    broadcast_rows_kernel<<<(B * A + 255) / 256, 256, 0, st>>>(bias, B, A, out);
-    SKB_LAUNCH_CHECK(st);
+    SKB_CUDA_CHECK(launch_kernel(false, broadcast_rows_kernel, (B * A + 255) / 256, 256, 0, st, bias, B, A, out));
     return SKB_OK;
 }
 
@@ -339,8 +334,7 @@ int span_table_size(int n_pix) { return (n_pix + kSpanPix - 1) / kSpanPix; }
 
 int launch_span_table(const int* pix_b, int n_pix, int* span_b, cudaStream_t st) {
     const int n_spans = span_table_size(n_pix);
-    span_table_kernel<<<(n_spans + 7) / 8, 256, 0, st>>>(pix_b, n_pix, n_spans, span_b);
-    SKB_LAUNCH_CHECK(st);
+    SKB_CUDA_CHECK(launch_kernel(false, span_table_kernel, (n_spans + 7) / 8, 256, 0, st, pix_b, n_pix, n_spans, span_b));
     return SKB_OK;
 }
 
@@ -351,11 +345,8 @@ static int launch_plane_sum(bool bf16, const uint16_t* act, long long plane, int
     const int chunks = C / 8;
     const int ppb = chunks >= 16 ? 4 : (chunks >= 8 ? 2 : 1);      // keep >= ~4 waves of CTAs on the small levels
     dim3 grid((n_spans + 7) / 8, chunks / ppb);
-    if (bf16)
-        SKB_CUDA_CHECK(launch_pdl(plane_sum_kernel<true>, grid, dim3(256), 0, st, act, plane, G, p_end, pix_b, span_b, C, ppb, sums));
-    else
-        SKB_CUDA_CHECK(launch_pdl(plane_sum_kernel<false>, grid, dim3(256), 0, st, act, plane, G, p_end, pix_b, span_b, C, ppb, sums));
-    SKB_LAUNCH_CHECK(st);
+    SKB_CUDA_CHECK(launch_kernel(true, bf16 ? plane_sum_kernel<true> : plane_sum_kernel<false>, grid, dim3(256), 0, st, act, plane, G, p_end, pix_b,
+                                 span_b, C, ppb, sums));
     return SKB_OK;
 }
 
@@ -548,11 +539,8 @@ int launch_se_scale(bool bf16, unsigned long long* sums, const uint16_t* y1, lon
         return SKB_ERR_ARG;
     }
     dim3 grid(B, Cin / 8);
-    if (bf16)
-        SKB_CUDA_CHECK(launch_pdl(se_border_kernel<true>, grid, dim3(256), 0, st, y1, plane, G, Wp, W, utt_row0, utt_count, Cin, brd_ws));
-    else
-        SKB_CUDA_CHECK(launch_pdl(se_border_kernel<false>, grid, dim3(256), 0, st, y1, plane, G, Wp, W, utt_row0, utt_count, Cin, brd_ws));
-    SKB_LAUNCH_CHECK(st);
+    SKB_CUDA_CHECK(launch_kernel(true, bf16 ? se_border_kernel<true> : se_border_kernel<false>, grid, dim3(256), 0, st, y1, plane, G, Wp, W, utt_row0,
+                                 utt_count, Cin, brd_ws));
     // the channel totals (when conv1's epilogue did not produce them) run BESIDE the border sums: see plane_sum_kernel
     if (totals) {
         int rc = launch_plane_sum(bf16, y1, plane, G, totals->p_end, totals->pix_b, totals->span_b, Cin, sums, st);
@@ -561,17 +549,14 @@ int launch_se_scale(bool bf16, unsigned long long* sums, const uint16_t* y1, lon
     const int n_slices = Cin / kSeCh;
     float* partial = brd_ws + (size_t)B * 8 * Cin;
     dim3 g2(n_slices, (B + kSeUtt - 1) / kSeUtt);
-    if (Cout == 32) SKB_CUDA_CHECK(launch_pdl(se_mean_partial_kernel<32>, g2, dim3(256), 0, st, sums, brd_ws, B, Cin, w2t, partial));
-    else if (Cout == 64) SKB_CUDA_CHECK(launch_pdl(se_mean_partial_kernel<64>, g2, dim3(256), 0, st, sums, brd_ws, B, Cin, w2t, partial));
-    else if (Cout == 128) SKB_CUDA_CHECK(launch_pdl(se_mean_partial_kernel<128>, g2, dim3(256), 0, st, sums, brd_ws, B, Cin, w2t, partial));
-    else if (Cout == 256) SKB_CUDA_CHECK(launch_pdl(se_mean_partial_kernel<256>, g2, dim3(256), 0, st, sums, brd_ws, B, Cin, w2t, partial));
-    else {
+    const auto mean_partial = Cout == 32 ? se_mean_partial_kernel<32> : Cout == 64 ? se_mean_partial_kernel<64>
+                            : Cout == 128 ? se_mean_partial_kernel<128> : Cout == 256 ? se_mean_partial_kernel<256> : nullptr;
+    if (!mean_partial) {
         set_last_error(__FILE__, __LINE__, "squeeze-excitation: unsupported channel count");
         return SKB_ERR_ARG;
     }
-    SKB_LAUNCH_CHECK(st);
-    SKB_CUDA_CHECK(launch_pdl(se_fc_kernel, dim3(B), dim3(256), 0, st, sums, partial, n_slices, utt_count, B, Cin, Cout, b2, fc1, fc2, scale));
-    SKB_LAUNCH_CHECK(st);
+    SKB_CUDA_CHECK(launch_kernel(true, mean_partial, g2, dim3(256), 0, st, sums, brd_ws, B, Cin, w2t, partial));
+    SKB_CUDA_CHECK(launch_kernel(true, se_fc_kernel, dim3(B), dim3(256), 0, st, sums, partial, n_slices, utt_count, B, Cin, Cout, b2, fc1, fc2, scale));
     return SKB_OK;
 }
 
@@ -624,8 +609,8 @@ int launch_gather_pack(const uint16_t* act, long long plane, int C, int W, int W
                        uint16_t* hi, cudaStream_t st) {
     const long long total = (long long)n_frames * W * (C / 8);
     if (total == 0) return SKB_OK;
-    gather_pack_kernel<<<(unsigned)((total + 255) / 256), 256, 0, st>>>(act, plane, C, W, Wp, G, frame_row, n_frames, hi);
-    SKB_LAUNCH_CHECK(st);
+    SKB_CUDA_CHECK(launch_kernel(false, gather_pack_kernel, (unsigned)((total + 255) / 256), 256, 0, st, act, plane, C, W, Wp, G, frame_row, n_frames,
+                                 hi));
     return SKB_OK;
 }
 
@@ -635,11 +620,8 @@ int launch_gather_frames(bool bf16, const uint16_t* act, long long plane, int C,
     const int threads = 256;
     const int blocks = (int)((total + threads - 1) / threads);
     if (blocks == 0) return SKB_OK;
-    if (bf16)
-        gather_frames_kernel<true><<<blocks, threads, 0, st>>>(act, plane, C, W, Wp, G, frame_row, n_frames, X);
-    else
-        gather_frames_kernel<false><<<blocks, threads, 0, st>>>(act, plane, C, W, Wp, G, frame_row, n_frames, X);
-    SKB_LAUNCH_CHECK(st);
+    SKB_CUDA_CHECK(launch_kernel(false, bf16 ? gather_frames_kernel<true> : gather_frames_kernel<false>, blocks, threads, 0, st, act, plane, C, W, Wp,
+                                 G, frame_row, n_frames, X));
     return SKB_OK;
 }
 
@@ -754,9 +736,8 @@ __global__ void __launch_bounds__(256) meanstd_planes_kernel(const uint16_t* __r
 int launch_meanstd_planes(bool bf16, const uint16_t* act, long long plane, int G, const int* utt_row0, const int* n_fr, int B, int D,
                           const float* aff_s, const float* aff_t, float* out, cudaStream_t st) {
     dim3 grid((D / 8 + 7) / 8, B);
-    if (bf16) meanstd_planes_kernel<true><<<grid, 256, 0, st>>>(act, plane, G, utt_row0, n_fr, D, aff_s, aff_t, out);
-    else meanstd_planes_kernel<false><<<grid, 256, 0, st>>>(act, plane, G, utt_row0, n_fr, D, aff_s, aff_t, out);
-    SKB_LAUNCH_CHECK(st);
+    SKB_CUDA_CHECK(launch_kernel(false, bf16 ? meanstd_planes_kernel<true> : meanstd_planes_kernel<false>, grid, 256, 0, st, act, plane, G, utt_row0,
+                                 n_fr, D, aff_s, aff_t, out));
     return SKB_OK;
 }
 
@@ -767,9 +748,8 @@ int launch_meanstd(bool bf16, const uint16_t* X, const long long* frame_off, con
         return SKB_ERR_ARG;
     }
     dim3 grid((D + 63) / 64, B);
-    if (bf16) meanstd_kernel<true><<<grid, dim3(32, 8), 0, st>>>(X, frame_off, n_fr, D, aff_s, aff_t, out);
-    else meanstd_kernel<false><<<grid, dim3(32, 8), 0, st>>>(X, frame_off, n_fr, D, aff_s, aff_t, out);
-    SKB_LAUNCH_CHECK(st);
+    SKB_CUDA_CHECK(launch_kernel(false, bf16 ? meanstd_kernel<true> : meanstd_kernel<false>, grid, dim3(32, 8), 0, st, X, frame_off, n_fr, D, aff_s,
+                                 aff_t, out));
     return SKB_OK;
 }
 
@@ -792,8 +772,7 @@ int launch_att_act(float* h, const float* hb, const int* frame_utt, const float*
                    int A, cudaStream_t st) {
     const long long total = (long long)n_frames * A;
     if (total == 0) return SKB_OK;
-    att_act_kernel<<<(int)((total + 255) / 256), 256, 0, st>>>(h, hb, frame_utt, bn_s, bn_t, n_frames, A);
-    SKB_LAUNCH_CHECK(st);
+    SKB_CUDA_CHECK(launch_kernel(false, att_act_kernel, (int)((total + 255) / 256), 256, 0, st, h, hb, frame_utt, bn_s, bn_t, n_frames, A));
     return SKB_OK;
 }
 
@@ -876,9 +855,8 @@ int launch_softmax_pool(bool bf16, const uint16_t* X, const float* logit, const 
         return SKB_ERR_ARG;
     }
     dim3 grid((D + 63) / 64, B);
-    if (bf16) softmax_pool_kernel<true><<<grid, dim3(32, 8), 0, st>>>(X, logit, frame_off, n_fr, D, out);
-    else softmax_pool_kernel<false><<<grid, dim3(32, 8), 0, st>>>(X, logit, frame_off, n_fr, D, out);
-    SKB_LAUNCH_CHECK(st);
+    SKB_CUDA_CHECK(launch_kernel(false, bf16 ? softmax_pool_kernel<true> : softmax_pool_kernel<false>, grid, dim3(32, 8), 0, st, X, logit, frame_off,
+                                 n_fr, D, out));
     return SKB_OK;
 }
 
@@ -921,8 +899,7 @@ __global__ void head_norm_kernel(const float* __restrict__ x, const float* __res
 
 int launch_head_norm(const float* x, const float* aff_s, const float* aff_t, int B, int E, int norm_embedding,
                      float* emb_pre, float* emb, cudaStream_t st) {
-    head_norm_kernel<<<B, 256, E * sizeof(float), st>>>(x, aff_s, aff_t, E, norm_embedding, emb_pre, emb);
-    SKB_LAUNCH_CHECK(st);
+    SKB_CUDA_CHECK(launch_kernel(false, head_norm_kernel, B, 256, E * sizeof(float), st, x, aff_s, aff_t, E, norm_embedding, emb_pre, emb));
     return SKB_OK;
 }
 
@@ -994,8 +971,7 @@ int launch_sgemm_nt(const float* A, const float* B, float* C, const float* bias,
                     int ldc, float alpha, cudaStream_t st) {
     if (M == 0 || N == 0) return SKB_OK;
     dim3 grid((N + 63) / 64, (M + 63) / 64);
-    sgemm_nt_kernel<<<grid, 256, 0, st>>>(A, B, C, bias, M, N, K, lda, ldb, ldc, alpha, K);
-    SKB_LAUNCH_CHECK(st);
+    SKB_CUDA_CHECK(launch_kernel(false, sgemm_nt_kernel, grid, 256, 0, st, A, B, C, bias, M, N, K, lda, ldb, ldc, alpha, K));
     return SKB_OK;
 }
 
@@ -1031,12 +1007,11 @@ int launch_skinny_gemm(const float* A, int M, int K, const float* W, int N, cons
     const int zz = (K + k_slice - 1) / k_slice;
     dim3 grid((N + 63) / 64, (M + 63) / 64, zz);
     if (zz == 1) {
-        sgemm_nt_kernel<<<grid, 256, 0, st>>>(A, W, C, bias, M, N, K, K, K, ldc, alpha, K);
+        SKB_CUDA_CHECK(launch_kernel(false, sgemm_nt_kernel, grid, 256, 0, st, A, W, C, bias, M, N, K, K, K, ldc, alpha, K));
     } else {
-        sgemm_nt_kernel<<<grid, 256, 0, st>>>(A, W, ws, nullptr, M, N, K, K, K, N, 1.f, k_slice);
-        splitk_reduce_kernel<<<(M * N + 255) / 256, 256, 0, st>>>(ws, zz, M, N, bias, alpha, C, ldc);
+        SKB_CUDA_CHECK(launch_kernel(false, sgemm_nt_kernel, grid, 256, 0, st, A, W, ws, nullptr, M, N, K, K, K, N, 1.f, k_slice));
+        SKB_CUDA_CHECK(launch_kernel(false, splitk_reduce_kernel, (M * N + 255) / 256, 256, 0, st, ws, zz, M, N, bias, alpha, C, ldc));
     }
-    SKB_LAUNCH_CHECK(st);
     return SKB_OK;
 }
 
@@ -1072,11 +1047,8 @@ int launch_pack_frames(bool bf16, const float* X, int C_src, int C_dst, int n_ro
     const long long total = (long long)n_rows * (C_dst / 8);
     if (total == 0) return SKB_OK;
     const int blocks = (int)((total + 255) / 256);
-    if (bf16)
-        pack_frames_kernel<true><<<blocks, 256, 0, st>>>(X, C_src, C_dst, n_rows, row_src, row_b, cmvn, out, plane, G);
-    else
-        pack_frames_kernel<false><<<blocks, 256, 0, st>>>(X, C_src, C_dst, n_rows, row_src, row_b, cmvn, out, plane, G);
-    SKB_LAUNCH_CHECK(st);
+    SKB_CUDA_CHECK(launch_kernel(false, bf16 ? pack_frames_kernel<true> : pack_frames_kernel<false>, blocks, 256, 0, st, X, C_src, C_dst, n_rows,
+                                 row_src, row_b, cmvn, out, plane, G));
     return SKB_OK;
 }
 

@@ -244,34 +244,27 @@ int skb_conv2d_bn_act(const float* x_dev, int B, int Cin, int H, int W, const fl
         const unsigned blocks = (unsigned)((total + 255) / 256);
         const int* ps = stride == 2 ? pm + L0.o_pix_sub : nullptr;
         const long long plane = stride == 2 ? Lg.plane : L0.plane;
-        if (bf16)
-            pack_dense_kernel<true><<<blocks, 256, 0, st>>>(x_dev, B, Cin, H, W, pre_scale_dev, pre_shift_dev, pre_slope, (uint16_t*)h->act[0].p,
-                                                            plane, L0.G, L0.Wp, h->d32 + L0.o_utt_row0, ps, cin_pad / 8, (unsigned*)h->ovf.p);
-        else
-            pack_dense_kernel<false><<<blocks, 256, 0, st>>>(x_dev, B, Cin, H, W, pre_scale_dev, pre_shift_dev, pre_slope, (uint16_t*)h->act[0].p,
-                                                             plane, L0.G, L0.Wp, h->d32 + L0.o_utt_row0, ps, cin_pad / 8, (unsigned*)h->ovf.p);
+        SKB_CUDA_CHECK(launch_kernel(false, bf16 ? pack_dense_kernel<true> : pack_dense_kernel<false>, blocks, 256, 0, st, x_dev, B, Cin, H, W,
+                                     pre_scale_dev, pre_shift_dev, pre_slope, (uint16_t*)h->act[0].p, plane, L0.G, L0.Wp,
+                                     h->d32 + L0.o_utt_row0, ps, cin_pad / 8, (unsigned*)h->ovf.p));
     }
     const float* scale = nullptr;
     if (fused) {
         if (residual_dev != nullptr) {
             const long long total = (long long)B * Ho * Wo * (cout_pad / 8);
             const unsigned blocks = (unsigned)((total + 255) / 256);
-            if (bf16)
-                pack_dense_kernel<true><<<blocks, 256, 0, st>>>(residual_dev, B, Cout, Ho, Wo, nullptr, nullptr, 1.f, (uint16_t*)h->act[2].p, Lg.plane,
-                                                                Lg.G, Lg.Wp, h->d32 + Lg.o_utt_row0, nullptr, cout_pad / 8, nullptr);
-            else
-                pack_dense_kernel<false><<<blocks, 256, 0, st>>>(residual_dev, B, Cout, Ho, Wo, nullptr, nullptr, 1.f, (uint16_t*)h->act[2].p, Lg.plane,
-                                                                 Lg.G, Lg.Wp, h->d32 + Lg.o_utt_row0, nullptr, cout_pad / 8, nullptr);
+            SKB_CUDA_CHECK(launch_kernel(false, bf16 ? pack_dense_kernel<true> : pack_dense_kernel<false>, blocks, 256, 0, st, residual_dev, B,
+                                         Cout, Ho, Wo, nullptr, nullptr, 1.f, (uint16_t*)h->act[2].p, Lg.plane, Lg.G, Lg.Wp,
+                                         h->d32 + Lg.o_utt_row0, nullptr, cout_pad / 8, nullptr));
         }
         SKB_TRY(h->scale.ensure((size_t)B * cout_pad * sizeof(float)));
         const long long n = (long long)B * cout_pad;
-        fill_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>((float*)h->scale.p, n, 1.f);
+        SKB_CUDA_CHECK(launch_kernel(false, fill_kernel, (unsigned)((n + 255) / 256), 256, 0, st, (float*)h->scale.p, n, 1.f));
         if (se_scale_dev != nullptr)
             SKB_CUDA_CHECK(cudaMemcpy2DAsync(h->scale.p, (size_t)cout_pad * sizeof(float), se_scale_dev, (size_t)Cout * sizeof(float),
                                              (size_t)Cout * sizeof(float), B, cudaMemcpyDeviceToDevice, st));
         scale = (const float*)h->scale.p;
     }
-    SKB_CUDA_CHECK(cudaGetLastError());
     // ---- weights: zero-padded to (cout_pad, cin_pad), packed for the tcgen05 kernel
     std::vector<double> wf((size_t)cout_pad * cin_pad * taps, 0.0), bias((size_t)cout_pad, 0.0);
     for (int co = 0; co < Cout; ++co) {
@@ -300,9 +293,12 @@ int skb_conv2d_bn_act(const float* x_dev, int B, int Cin, int H, int W, const fl
         int64_t per = 0;
         rc = export_stage(h, (const uint16_t*)h->act[1].p, Lx, Ho, y_dev, &per, st);
     }
-    if (!rc && cudaStreamSynchronize(st) != cudaSuccess) rc = SKB_ERR_CUDA;      // the packed weights are freed below
+    // a failed launch in run_conv / export_stage has recorded its own file:line; the packed weights are freed below
+    if (!rc) {
+        const cudaError_t e = cudaStreamSynchronize(st);
+        if (e != cudaSuccess) { set_last_error(__FILE__, __LINE__, cudaGetErrorString(e)); rc = SKB_ERR_CUDA; }
+    }
     free_conv(&cw);
-    if (rc == SKB_ERR_CUDA) set_last_error(__FILE__, __LINE__, cudaGetErrorString(cudaGetLastError()));
     return rc;
 }
 
@@ -320,9 +316,7 @@ int skb_channel_mean(const float* x_dev, int B, int C, int64_t hw, float* out_de
         set_last_error(__FILE__, __LINE__, "channel_mean: bad arguments");
         return SKB_ERR_ARG;
     }
-    channel_mean_kernel<<<B * C, 256, 0, (cudaStream_t)stream>>>(x_dev, (long long)hw, out_dev);
-    g_launches++;
-    SKB_CUDA_CHECK(cudaGetLastError());
+    SKB_CUDA_CHECK(launch_kernel(false, channel_mean_kernel, B * C, 256, 0, (cudaStream_t)stream, x_dev, (long long)hw, out_dev));
     return SKB_OK;
 }
 
@@ -331,9 +325,8 @@ int skb_se_gate(const float* mean_dev, const float* fc1_dev, const float* fc2_de
         set_last_error(__FILE__, __LINE__, "se_gate: bad arguments");
         return SKB_ERR_ARG;
     }
-    se_gate_kernel<<<B, 256, (size_t)(C + R) * sizeof(float), (cudaStream_t)stream>>>(mean_dev, fc1_dev, fc2_dev, C, R, scale_dev);
-    g_launches++;
-    SKB_CUDA_CHECK(cudaGetLastError());
+    SKB_CUDA_CHECK(launch_kernel(false, se_gate_kernel, B, 256, (size_t)(C + R) * sizeof(float), (cudaStream_t)stream, mean_dev, fc1_dev,
+                                 fc2_dev, C, R, scale_dev));
     return SKB_OK;
 }
 
@@ -344,10 +337,8 @@ int skb_scale_residual_act(const float* y_dev, const float* scale_dev, const flo
         return SKB_ERR_ARG;
     }
     const long long total = (long long)B * C * hw;
-    scale_residual_act_kernel<<<(unsigned)((total + 255) / 256), 256, 0, (cudaStream_t)stream>>>(y_dev, scale_dev, res_dev, (long long)hw, total,
-                                                                                              slope, out_dev);
-    g_launches++;
-    SKB_CUDA_CHECK(cudaGetLastError());
+    SKB_CUDA_CHECK(launch_kernel(false, scale_residual_act_kernel, (unsigned)((total + 255) / 256), 256, 0, (cudaStream_t)stream, y_dev,
+                                 scale_dev, res_dev, (long long)hw, total, slope, out_dev));
     return SKB_OK;
 }
 
@@ -356,9 +347,7 @@ int skb_l2_normalize(const float* x_dev, int N, int D, float eps, float* out_dev
         set_last_error(__FILE__, __LINE__, "l2_normalize: bad arguments");
         return SKB_ERR_ARG;
     }
-    l2_normalize_kernel<<<(N + 7) / 8, 256, 0, (cudaStream_t)stream>>>(x_dev, N, D, eps, out_dev);
-    g_launches++;
-    SKB_CUDA_CHECK(cudaGetLastError());
+    SKB_CUDA_CHECK(launch_kernel(false, l2_normalize_kernel, (N + 7) / 8, 256, 0, (cudaStream_t)stream, x_dev, N, D, eps, out_dev));
     return SKB_OK;
 }
 
@@ -379,7 +368,8 @@ int skb_attentive_pool(const float* x_dev, int B, int D, int T, const float* w1_
     do {
         if ((rc = X.ensure(F * D * sizeof(float))) || (rc = Hh.ensure(F * A * sizeof(float))) || (rc = Lg.ensure(F * D * sizeof(float))) ||
             (rc = hb.ensure((size_t)B * A * sizeof(float))) || (rc = w1x.ensure((size_t)A * D * sizeof(float)))) break;
-        bdt_to_frames_kernel<<<dim3((T + 31) / 32, (D + 31) / 32, B), dim3(32, 8), 0, st>>>(x_dev, D, T, (float*)X.p);
+        if (launch_kernel(false, bdt_to_frames_kernel, dim3((T + 31) / 32, (D + 31) / 32, B), dim3(32, 8), 0, st, x_dev, D, T, (float*)X.p) !=
+            cudaSuccess) { rc = SKB_ERR_CUDA; break; }
         // split the first Conv1d's weight (A, in_factor * D) into the part that multiplies x and the time-constant part
         if (cudaMemcpy2DAsync(w1x.p, (size_t)D * sizeof(float), w1_dev, (size_t)in_factor * D * sizeof(float), (size_t)D * sizeof(float), A,
                               cudaMemcpyDeviceToDevice, st) != cudaSuccess) { rc = SKB_ERR_CUDA; break; }
@@ -394,14 +384,12 @@ int skb_attentive_pool(const float* x_dev, int B, int D, int T, const float* w1_
         if ((rc = packed_create((const float*)w1x.p, A, D, &p1, st))) break;
         if ((rc = packed_create(w2_dev, D, A, &p2, st))) break;
         if ((rc = gemm_nt_split((const float*)X.p, (int)F, D, p1, nullptr, 1.f, (float*)Hh.p, A, st))) break;
-        {
-            const long long total = (long long)F * A;
-            att_act_dense_kernel<<<(unsigned)((total + 255) / 256), 256, 0, st>>>((float*)Hh.p, (const float*)hb.p, bn_s_dev, bn_t_dev, total, A, T);
-        }
+        const long long total = (long long)F * A;
+        if (launch_kernel(false, att_act_dense_kernel, (unsigned)((total + 255) / 256), 256, 0, st, (float*)Hh.p, (const float*)hb.p, bn_s_dev,
+                          bn_t_dev, total, A, T) != cudaSuccess) { rc = SKB_ERR_CUDA; break; }
         if ((rc = gemm_nt_split((const float*)Hh.p, (int)F, A, p2, b2_dev, 1.f, (float*)Lg.p, D, st))) break;
-        softmax_pool_dense_kernel<<<dim3((D + 127) / 128, B), 128, 0, st>>>((const float*)X.p, (const float*)Lg.p, D, T, out_dev);
-        g_launches += 4;
-        if (cudaGetLastError() != cudaSuccess || cudaStreamSynchronize(st) != cudaSuccess) rc = SKB_ERR_CUDA;
+        if (launch_kernel(false, softmax_pool_dense_kernel, dim3((D + 127) / 128, B), 128, 0, st, (const float*)X.p, (const float*)Lg.p, D, T,
+                          out_dev) != cudaSuccess || cudaStreamSynchronize(st) != cudaSuccess) rc = SKB_ERR_CUDA;
     } while (false);
     if (rc == SKB_ERR_CUDA) set_last_error(__FILE__, __LINE__, cudaGetErrorString(cudaGetLastError()));
     cudaStreamSynchronize(st);

@@ -3,10 +3,7 @@
 #include "common.cuh"
 #include "layers.cuh"
 
-#include <atomic>
-
 namespace skb {
-extern std::atomic<long long> g_launches;
 
 // MeanStdPooling on the reference's (B, D, T) layout: one warp per (b, d) row, two-pass statistics.
 __global__ void meanstd_bdt_kernel(const float* __restrict__ x, int D, int T, float* __restrict__ out, long long rows) {
@@ -40,8 +37,7 @@ extern "C" int skb_meanstd_pool(const float* x_dev, int n_utt, int D, int T, flo
     }
     const long long rows = (long long)n_utt * D;
     const int warps = 8;
-    meanstd_bdt_kernel<<<(unsigned)((rows + warps - 1) / warps), warps * 32, 0, (cudaStream_t)stream>>>(x_dev, D, T, out_dev, rows);
-    g_launches++;
-    SKB_CUDA_CHECK(cudaGetLastError());
+    SKB_CUDA_CHECK(launch_kernel(false, meanstd_bdt_kernel, (unsigned)((rows + warps - 1) / warps), warps * 32, 0, (cudaStream_t)stream, x_dev,
+                                 D, T, out_dev, rows));
     return SKB_OK;
 }

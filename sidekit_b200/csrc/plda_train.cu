@@ -15,11 +15,9 @@
 #include "common.cuh"
 #include "class_sum.cuh"
 
-#include <atomic>
 #include <vector>
 
 namespace skb {
-extern std::atomic<long long> g_launches;
 
 // C[M][N] = alpha * op(A) op(B) + beta * C, op = identity or transpose; 16 x 16 tiles through shared memory
 __global__ void __launch_bounds__(256) dgemm_kernel(int ta, int tb, int M, int N, int K, double alpha, const double* __restrict__ A, int lda,
@@ -43,9 +41,8 @@ __global__ void __launch_bounds__(256) dgemm_kernel(int ta, int tb, int M, int N
 
 static int dgemm(int ta, int tb, int M, int N, int K, double alpha, const double* A, int lda, const double* B, int ldb, double beta,
                  double* C, int ldc, cudaStream_t st) {
-    dgemm_kernel<<<dim3((N + 15) / 16, (M + 15) / 16), 256, 0, st>>>(ta, tb, M, N, K, alpha, A, lda, B, ldb, beta, C, ldc);
-    g_launches++;
-    SKB_CUDA_CHECK(cudaGetLastError());
+    SKB_CUDA_CHECK(launch_kernel(false, dgemm_kernel, dim3((N + 15) / 16, (M + 15) / 16), 256, 0, st, ta, tb, M, N, K, alpha, A, lda, B, ldb,
+                                 beta, C, ldc));
     return SKB_OK;
 }
 
@@ -193,14 +190,13 @@ int skb_plda_stats(const double* X_dev, int n_sess, int D, const int* cls_ptr_de
     cudaStream_t st = (cudaStream_t)stream;
     DBuf xc;
     if (xc.alloc((size_t)n_sess * D)) { set_last_error(__FILE__, __LINE__, "plda_stats: out of memory"); return SKB_ERR_CUDA; }
-    colmean_kernel<<<(D + 127) / 128, 128, 0, st>>>(X_dev, n_sess, D, mean_dev);
+    SKB_CUDA_CHECK(launch_kernel(false, colmean_kernel, (D + 127) / 128, 128, 0, st, X_dev, n_sess, D, mean_dev));
     const long long n = (long long)n_sess * D;
-    center_rows_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(X_dev, nullptr, mean_dev, n, D, xc.p);
+    SKB_CUDA_CHECK(launch_kernel(false, center_rows_kernel, (unsigned)((n + 255) / 256), 256, 0, st, X_dev, nullptr, mean_dev, n, D, xc.p));
     int rc = dgemm(1, 0, D, D, n_sess, 1.0 / n_sess, xc.p, D, xc.p, D, 0.0, sigma_obs_dev, D, st);     // statserver.py:920-928
     if (rc) return rc;
-    class_sum_kernel<double><<<dim3((D + 127) / 128, n_cls), 128, 0, st>>>(X_dev, D, (long long)D, cls_ptr_dev, cls_rows_dev, n_cls, scaling, S1_dev);
-    g_launches += 3;
-    SKB_CUDA_CHECK(cudaGetLastError());
+    SKB_CUDA_CHECK(launch_kernel(false, class_sum_kernel<double>, dim3((D + 127) / 128, n_cls), 128, 0, st, X_dev, D, (long long)D, cls_ptr_dev,
+                                 cls_rows_dev, n_cls, scaling, S1_dev));
     SKB_CUDA_CHECK(cudaStreamSynchronize(st));
     return SKB_OK;
 }
@@ -228,48 +224,55 @@ int skb_plda_em(const double* S1_dev, const double* cls_n_dev, const int* cls_u_
         return SKB_ERR_CUDA;
     }
     cudaMemsetAsync(flag, 0, sizeof(int), st);
-    int rc = SKB_OK;
     const long long nx = (long long)n_cls * D;
     const long long nl = (long long)U * R * R;
-    // the centred class statistics S - n mu' never change (the mean is not re-estimated, factor_analyser.py:857)
-    center_rows_kernel<<<(unsigned)((nx + 255) / 256), 256, 0, st>>>(S1_dev, cls_n_dev, mean_dev, nx, D, Xc.p);
-    for (int it = 0; it < nb_iter && !rc; ++it) {
-        // P = Sigma^-1 F  (Cholesky of Sigma; the strictly upper triangle of the copy is never read)
-        cudaMemcpyAsync(Ls.p, Sigma_dev, (size_t)D * D * sizeof(double), cudaMemcpyDeviceToDevice, st);
-        cudaMemcpyAsync(P.p, F_dev, (size_t)D * R * sizeof(double), cudaMemcpyDeviceToDevice, st);
-        dpotrf_kernel<<<1, 1024, 0, st>>>(Ls.p, D, flag);
-        dpotrs_kernel<<<dim3((R + 63) / 64, 1), 64, 0, st>>>(Ls.p, D, P.p, R, 0, 0);
-        // A0 = F' Sigma^-1 F ;  Linv_u = (n_u A0 + I)^-1 for every distinct session count (fa_model_loop :183-186)
-        if ((rc = dgemm(1, 0, R, R, D, 1.0, F_dev, R, P.p, R, 0.0, A0.p, R, st))) break;
-        lambda_kernel<<<(unsigned)((nl + 255) / 256), 256, 0, st>>>(A0.p, uniq_n_dev, R, U, Lam.p);
-        identity_kernel<<<(unsigned)((nl + 255) / 256), 256, 0, st>>>(Linv.p, R, U);
-        dpotrf_kernel<<<U, 1024, 0, st>>>(Lam.p, R, flag);
-        dpotrs_kernel<<<dim3((R + 63) / 64, U), 64, 0, st>>>(Lam.p, R, Linv.p, R, (long long)R * R, (long long)R * R);
-        // aux = (S - n mu') Sigma^-1 F ;  E[h_i] = aux_i Linv_{n_i}  (:188-190)
-        if ((rc = dgemm(0, 0, n_cls, R, D, 1.0, Xc.p, D, P.p, R, 0.0, aux.p, R, st))) break;
-        posterior_mean_kernel<<<n_cls, 128, (size_t)R * sizeof(double), st>>>(aux.p, Linv.p, cls_u_dev, cls_n_dev, R, eh.p, ehn.p);
-        // accumulators (:907-912): R = sum E[hh'] / C,  A = sum n_i E[hh'],  C = E[h]' (S - n mu')
-        if ((rc = dgemm(1, 0, R, R, n_cls, 1.0, eh.p, R, eh.p, R, 0.0, Rm.p, R, st))) break;
-        if ((rc = dgemm(1, 0, R, R, n_cls, 1.0, ehn.p, R, eh.p, R, 0.0, Am.p, R, st))) break;
-        accumulators_kernel<<<(R * R + 255) / 256, 256, 0, st>>>(Linv.p, cnt_u_dev, uniq_n_dev, U, R, 1.0 / n_cls, Rm.p, Am.p);
-        if ((rc = dgemm(1, 0, R, D, n_cls, 1.0, eh.p, R, Xc.p, D, 0.0, Cm.p, D, st))) break;
-        // M-step (:915): F = solve(A, C)'  -- A is symmetric positive definite
-        cudaMemcpyAsync(Xs.p, Cm.p, (size_t)R * D * sizeof(double), cudaMemcpyDeviceToDevice, st);
-        dpotrf_kernel<<<1, 1024, 0, st>>>(Am.p, R, flag);
-        dpotrs_kernel<<<dim3((D + 63) / 64, 1), 64, 0, st>>>(Am.p, R, Xs.p, D, 0, 0);
-        const long long nf = (long long)R * D;
-        transpose_kernel<<<(unsigned)((nf + 255) / 256), 256, 0, st>>>(Xs.p, R, D, Ft.p);            // F_new (D, R)
-        // residual covariance (:918): Sigma = sigma_obs - F_new C / sum n
-        cudaMemcpyAsync(Sigma_dev, sigma_obs_dev, (size_t)D * D * sizeof(double), cudaMemcpyDeviceToDevice, st);
-        if ((rc = dgemm(0, 0, D, D, R, -1.0 / sum_n, Ft.p, R, Cm.p, D, 1.0, Sigma_dev, D, st))) break;
-        // minimum divergence (:921): F = F_new chol(R), scipy's upper factor U = L'
-        dpotrf_kernel<<<1, 1024, 0, st>>>(Rm.p, R, flag);
-        tril_kernel<<<(R * R + 255) / 256, 256, 0, st>>>(Rm.p, R);
-        if ((rc = dgemm(0, 1, D, R, R, 1.0, Ft.p, R, Rm.p, R, 0.0, F_dev, R, st))) break;
-        g_launches += 14;
-    }
+    // a failed launch leaves the EM loop with its error code, for the clean-up below
+    int rc = [&]() -> int {
+        // the centred class statistics S - n mu' never change (the mean is not re-estimated, factor_analyser.py:857)
+        SKB_CUDA_CHECK(launch_kernel(false, center_rows_kernel, (unsigned)((nx + 255) / 256), 256, 0, st, S1_dev, cls_n_dev, mean_dev, nx, D,
+                                     Xc.p));
+        for (int it = 0; it < nb_iter; ++it) {
+            // P = Sigma^-1 F  (Cholesky of Sigma; the strictly upper triangle of the copy is never read)
+            cudaMemcpyAsync(Ls.p, Sigma_dev, (size_t)D * D * sizeof(double), cudaMemcpyDeviceToDevice, st);
+            cudaMemcpyAsync(P.p, F_dev, (size_t)D * R * sizeof(double), cudaMemcpyDeviceToDevice, st);
+            SKB_CUDA_CHECK(launch_kernel(false, dpotrf_kernel, 1, 1024, 0, st, Ls.p, D, flag));
+            SKB_CUDA_CHECK(launch_kernel(false, dpotrs_kernel, dim3((R + 63) / 64, 1), 64, 0, st, Ls.p, D, P.p, R, 0, 0));
+            // A0 = F' Sigma^-1 F ;  Linv_u = (n_u A0 + I)^-1 for every distinct session count (fa_model_loop :183-186)
+            if (int e = dgemm(1, 0, R, R, D, 1.0, F_dev, R, P.p, R, 0.0, A0.p, R, st)) return e;
+            SKB_CUDA_CHECK(launch_kernel(false, lambda_kernel, (unsigned)((nl + 255) / 256), 256, 0, st, A0.p, uniq_n_dev, R, U, Lam.p));
+            SKB_CUDA_CHECK(launch_kernel(false, identity_kernel, (unsigned)((nl + 255) / 256), 256, 0, st, Linv.p, R, U));
+            SKB_CUDA_CHECK(launch_kernel(false, dpotrf_kernel, U, 1024, 0, st, Lam.p, R, flag));
+            SKB_CUDA_CHECK(launch_kernel(false, dpotrs_kernel, dim3((R + 63) / 64, U), 64, 0, st, Lam.p, R, Linv.p, R, (long long)R * R,
+                                         (long long)R * R));
+            // aux = (S - n mu') Sigma^-1 F ;  E[h_i] = aux_i Linv_{n_i}  (:188-190)
+            if (int e = dgemm(0, 0, n_cls, R, D, 1.0, Xc.p, D, P.p, R, 0.0, aux.p, R, st)) return e;
+            SKB_CUDA_CHECK(launch_kernel(false, posterior_mean_kernel, n_cls, 128, (size_t)R * sizeof(double), st, aux.p, Linv.p, cls_u_dev,
+                                         cls_n_dev, R, eh.p, ehn.p));
+            // accumulators (:907-912): R = sum E[hh'] / C,  A = sum n_i E[hh'],  C = E[h]' (S - n mu')
+            if (int e = dgemm(1, 0, R, R, n_cls, 1.0, eh.p, R, eh.p, R, 0.0, Rm.p, R, st)) return e;
+            if (int e = dgemm(1, 0, R, R, n_cls, 1.0, ehn.p, R, eh.p, R, 0.0, Am.p, R, st)) return e;
+            SKB_CUDA_CHECK(launch_kernel(false, accumulators_kernel, (R * R + 255) / 256, 256, 0, st, Linv.p, cnt_u_dev, uniq_n_dev, U, R,
+                                         1.0 / n_cls, Rm.p, Am.p));
+            if (int e = dgemm(1, 0, R, D, n_cls, 1.0, eh.p, R, Xc.p, D, 0.0, Cm.p, D, st)) return e;
+            // M-step (:915): F = solve(A, C)'  -- A is symmetric positive definite
+            cudaMemcpyAsync(Xs.p, Cm.p, (size_t)R * D * sizeof(double), cudaMemcpyDeviceToDevice, st);
+            SKB_CUDA_CHECK(launch_kernel(false, dpotrf_kernel, 1, 1024, 0, st, Am.p, R, flag));
+            SKB_CUDA_CHECK(launch_kernel(false, dpotrs_kernel, dim3((D + 63) / 64, 1), 64, 0, st, Am.p, R, Xs.p, D, 0, 0));
+            const long long nf = (long long)R * D;
+            SKB_CUDA_CHECK(launch_kernel(false, transpose_kernel, (unsigned)((nf + 255) / 256), 256, 0, st, Xs.p, R, D, Ft.p));   // F_new (D, R)
+            // residual covariance (:918): Sigma = sigma_obs - F_new C / sum n
+            cudaMemcpyAsync(Sigma_dev, sigma_obs_dev, (size_t)D * D * sizeof(double), cudaMemcpyDeviceToDevice, st);
+            if (int e = dgemm(0, 0, D, D, R, -1.0 / sum_n, Ft.p, R, Cm.p, D, 1.0, Sigma_dev, D, st)) return e;
+            // minimum divergence (:921): F = F_new chol(R), scipy's upper factor U = L'
+            SKB_CUDA_CHECK(launch_kernel(false, dpotrf_kernel, 1, 1024, 0, st, Rm.p, R, flag));
+            SKB_CUDA_CHECK(launch_kernel(false, tril_kernel, (R * R + 255) / 256, 256, 0, st, Rm.p, R));
+            if (int e = dgemm(0, 1, D, R, R, 1.0, Ft.p, R, Rm.p, R, 0.0, F_dev, R, st)) return e;
+        }
+        return SKB_OK;
+    }();
     int bad = 0;
     if (!rc) {
+        // cudaGetLastError: the unchecked device-to-device copies of the loop
         if (cudaGetLastError() != cudaSuccess || cudaMemcpyAsync(&bad, flag, sizeof(int), cudaMemcpyDeviceToHost, st) != cudaSuccess ||
             cudaStreamSynchronize(st) != cudaSuccess) {
             set_last_error(__FILE__, __LINE__, cudaGetErrorString(cudaGetLastError()));

@@ -23,11 +23,9 @@
 #include "sidekit_b200.h"
 #include "common.cuh"
 
-#include <atomic>
 #include <stdlib.h>
 
 namespace skb {
-extern std::atomic<long long> g_launches;
 
 constexpr int kOutPerCta = 2048;       // target outputs per CTA (rounded down to whole periods); sweep in profiles/r01g_resample.txt
 constexpr int kResThreads = 256;
@@ -122,9 +120,8 @@ extern "C" int skb_resample(const float* in_dev, const int64_t* wave_meta_dev, i
     SKB_CUDA_CHECK(cudaFuncSetAttribute(resample_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     const long long per_cta = (long long)pcta * new_r;
     dim3 grid((unsigned)((max_out + per_cta - 1) / per_cta), (unsigned)n_wav);
-    resample_kernel<<<grid, kResThreads, smem, st>>>(in_dev, out_dev, reinterpret_cast<const ResampleWave*>(wave_meta_dev), orig_r,
-                                                     new_r, width, ntap, bank_dev, start_dev, pcta, (int)win_len);
-    g_launches++;
-    SKB_LAUNCH_CHECK(st);
+    SKB_CUDA_CHECK(launch_kernel(false, resample_kernel, grid, kResThreads, smem, st, in_dev, out_dev,
+                                 reinterpret_cast<const ResampleWave*>(wave_meta_dev), orig_r, new_r, width, ntap, bank_dev, start_dev, pcta,
+                                 (int)win_len));
     return SKB_OK;
 }

@@ -22,13 +22,11 @@
 #include "common.cuh"
 #include "layers.cuh"
 
-#include <atomic>
 #include <cmath>
 #include <cstdlib>
 #include <vector>
 
 namespace skb {
-extern std::atomic<long long> g_launches;
 
 // ----------------------------------------------------------------------------- operand preparation
 // stats[0] = max |x| (as float bits), stats[1] = max row sum of squares (float bits).  blockIdx.y selects the operand, so
@@ -44,7 +42,7 @@ __global__ void __launch_bounds__(kAbsmaxWarps * 32) absmax_kernel(const AbsmaxA
     // depend on the launch shape), eight loads in flight per lane
     __shared__ float smx[kAbsmaxWarps], sss[kAbsmaxWarps];
     __shared__ bool s_last;
-    pdl_wait();                                        // launched with launch_pdl (common.cuh): the scratch list may still be read
+    pdl_wait();                                        // launched with PDL (common.cuh): the scratch list may still be read
     const float* __restrict__ X = a.X[blockIdx.y];
     const int rows = a.rows[blockIdx.y];
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -843,11 +841,10 @@ static int packed_fill(const float* X0, PackedOp* op0, const float* X1, PackedOp
             max_tiles = std::max(max_tiles, o->rows_pad / 128);
         }
     }
-    SKB_CUDA_CHECK(launch_pdl(absmax_kernel, dim3(std::max(1, std::min((max_rows + kAbsmaxWarps - 1) / kAbsmaxWarps, kAbsmaxMaxCtas)), n_ops),
-                              dim3(kAbsmaxWarps * 32), 0, st, aa, op0->D));
-    SKB_CUDA_CHECK(launch_pdl(pack_split_kernel, dim3((unsigned)std::max(1, max_tiles), op0->Dp / 64, n_ops), dim3(256), 0, st, pa, op0->D, op0->Dp));
-    g_launches += 2;
-    SKB_CUDA_CHECK(cudaGetLastError());
+    SKB_CUDA_CHECK(launch_kernel(true, absmax_kernel, dim3(std::max(1, std::min((max_rows + kAbsmaxWarps - 1) / kAbsmaxWarps, kAbsmaxMaxCtas)), n_ops),
+                                 dim3(kAbsmaxWarps * 32), 0, st, aa, op0->D));
+    SKB_CUDA_CHECK(launch_kernel(true, pack_split_kernel, dim3((unsigned)std::max(1, max_tiles), op0->Dp / 64, n_ops), dim3(256), 0, st, pa, op0->D,
+                                 op0->Dp));
     return SKB_OK;
 }
 
@@ -888,9 +885,7 @@ static int launch_score(const ScoreParams& p, cudaStream_t st) {
     if (configured.first()) {
         SKB_CUDA_CHECK(cudaFuncSetAttribute(score_gemm_kernel<STREAM_A, MODE, KC>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
     }
-    SKB_CUDA_CHECK(launch_pdl(score_gemm_kernel<STREAM_A, MODE, KC>, dim3(grid), dim3(ScoreSmem<1, STREAM_A>::kThreads), smem, st, p));
-    g_launches++;
-    SKB_CUDA_CHECK(cudaGetLastError());
+    SKB_CUDA_CHECK(launch_kernel(true, score_gemm_kernel<STREAM_A, MODE, KC>, dim3(grid), dim3(ScoreSmem<1, STREAM_A>::kThreads), smem, st, p));
     return SKB_OK;
 }
 
@@ -1235,10 +1230,8 @@ static int score_topk_packed(const PackedOp& e, const PackedOp& t, const float* 
         if ((rc = ws_ensure(0, (size_t)e.rows * segs * k * sizeof(unsigned long long)))) return rc;
         TopkLists tl{reinterpret_cast<unsigned long long*>(g_ws.tmp), k, segs};
         if ((rc = gemm_packed(e, t, nullptr, nullptr, a0, r, q, c0, rq_scale, abs_alpha, passes, 4, tl.keys, 0, st, nullptr, &tl))) return rc;
-        SKB_CUDA_CHECK(launch_pdl(topk_merge_kernel, dim3((unsigned)((e.rows + 7) / 8)), dim3(256), 0, st,
-                                  (const unsigned long long*)tl.keys, e.rows, k, segs, n_ntiles, tiles, grid, values, indices));
-        g_launches++;
-        SKB_CUDA_CHECK(cudaGetLastError());
+        SKB_CUDA_CHECK(launch_kernel(true, topk_merge_kernel, dim3((unsigned)((e.rows + 7) / 8)), dim3(256), 0, st,
+                                     (const unsigned long long*)tl.keys, e.rows, k, segs, n_ntiles, tiles, grid, values, indices));
         return SKB_OK;
     }
     // Row panels of the score matrix through a bounded float32 scratch (<= 1 GB, at least one 128-row tile), each followed by
@@ -1258,11 +1251,9 @@ static int score_topk_packed(const PackedOp& e, const PackedOp& t, const float* 
         if ((rc = gemm_packed(v, t, nullptr, nullptr, a0, r ? r + r0 : nullptr, q, c0, rq_scale, abs_alpha, passes, 0, g_ws.tmp, ld, st,
                               nullptr)))
             return rc;
-        topk_select_kernel<<<v.rows, 256, kp * sizeof(unsigned long long), st>>>(g_ws.tmp, t.rows, ld, k, values + (size_t)r0 * k,
-                                                                                 indices + (size_t)r0 * k);
-        g_launches++;
+        SKB_CUDA_CHECK(launch_kernel(false, topk_select_kernel, dim3(v.rows), dim3(256), kp * sizeof(unsigned long long), st, g_ws.tmp, t.rows,
+                                     ld, k, values + (size_t)r0 * k, indices + (size_t)r0 * k));
     }
-    SKB_CUDA_CHECK(cudaGetLastError());
     return SKB_OK;
 }
 
@@ -1400,12 +1391,12 @@ int skb_quadratic_prepare(const float* X_dev, const float* mu_dev, const float* 
     if (rc) return rc;
     float* xc = g_ws.tmp;
     float* tmp = g_ws.tmp + nd;
-    center_kernel<<<(unsigned)((nd + 255) / 256), 256, 0, st>>>(X_dev, mu_dev, N, D, xc);
+    SKB_CUDA_CHECK(launch_kernel(false, center_kernel, dim3((unsigned)((nd + 255) / 256)), dim3(256), 0, st, X_dev, mu_dev, N, D, xc));
     // tmp = xc . Phi  (Phi symmetric, so rows of Phi serve as the K-major "T" operand)
     rc = score_gemm_general(xc, Phi_dev, N, D, D, nullptr, nullptr, 1.f, nullptr, nullptr, 0.f, 1.f, 1.f, 3, 0, tmp, D,
                             2 * nd * sizeof(float), st);
     if (rc) return rc;
-    half_rowdot_kernel<<<(N + 7) / 8, 256, 0, st>>>(tmp, xc, N, D, rowterm_dev);
+    SKB_CUDA_CHECK(launch_kernel(false, half_rowdot_kernel, dim3((N + 7) / 8), dim3(256), 0, st, tmp, xc, N, D, rowterm_dev));
     if (PsiT_dev) {
         rc = score_gemm_general(xc, PsiT_dev, N, D, D, nullptr, nullptr, 1.f, nullptr, nullptr, 0.f, 1.f, 1.f, 3, 0, Xout_dev, D,
                                 2 * nd * sizeof(float), st);
@@ -1413,8 +1404,6 @@ int skb_quadratic_prepare(const float* X_dev, const float* mu_dev, const float* 
     } else {
         SKB_CUDA_CHECK(cudaMemcpyAsync(Xout_dev, xc, nd * sizeof(float), cudaMemcpyDeviceToDevice, st));
     }
-    g_launches += 2;
-    SKB_CUDA_CHECK(cudaGetLastError());
     return SKB_OK;
 }
 
@@ -1501,12 +1490,16 @@ int skb_trial_index_create(const uint8_t* mask_dev, int Ne, int Nt, int64_t ld_m
         skb_trial_index_destroy(t);
         return SKB_ERR_CUDA;
     }
-    trial_words_kernel<<<(Ne + 7) / 8, 256, 0, st>>>(mask_dev, Ne, Nt, (long long)ld_mask, t->words, t->offsets, t->ld, t->row_total);
-    trial_rowscan_kernel<<<1, 1024, 0, st>>>(t->row_total, Ne, t->row_base, t->n_dev);
-    trial_addbase_kernel<<<(unsigned)((nw + 255) / 256), 256, 0, st>>>(t->offsets, t->row_base, (long long)nw, t->ld);
-    g_launches += 3;
-    if (cudaMemcpyAsync(&total, t->n_dev, 8, cudaMemcpyDeviceToHost, st) != cudaSuccess || cudaStreamSynchronize(st) != cudaSuccess) {
-        set_last_error(__FILE__, __LINE__, cudaGetErrorString(cudaGetLastError()));
+    cudaError_t e = launch_kernel(false, trial_words_kernel, dim3((Ne + 7) / 8), dim3(256), 0, st, mask_dev, Ne, Nt, (long long)ld_mask,
+                                  t->words, t->offsets, t->ld, t->row_total);
+    if (e == cudaSuccess) e = launch_kernel(false, trial_rowscan_kernel, dim3(1), dim3(1024), 0, st, t->row_total, Ne, t->row_base, t->n_dev);
+    if (e == cudaSuccess)
+        e = launch_kernel(false, trial_addbase_kernel, dim3((unsigned)((nw + 255) / 256)), dim3(256), 0, st, t->offsets, t->row_base,
+                          (long long)nw, t->ld);
+    if (e == cudaSuccess) e = cudaMemcpyAsync(&total, t->n_dev, 8, cudaMemcpyDeviceToHost, st);
+    if (e == cudaSuccess) e = cudaStreamSynchronize(st);
+    if (e != cudaSuccess) {
+        set_last_error(__FILE__, __LINE__, cudaGetErrorString(e));
         skb_trial_index_destroy(t);
         return SKB_ERR_CUDA;
     }
@@ -1621,9 +1614,8 @@ int skb_widen_f32_f64(const float* src_dev, double* dst_dev, int64_t n, void* st
         return SKB_ERR_ARG;
     }
     if (n == 0) return SKB_OK;
-    widen_kernel<<<(unsigned)((n + 1023) / 1024), 256, 0, (cudaStream_t)stream>>>(src_dev, dst_dev, (long long)n);
-    g_launches++;
-    SKB_CUDA_CHECK(cudaGetLastError());
+    SKB_CUDA_CHECK(launch_kernel(false, widen_kernel, dim3((unsigned)((n + 1023) / 1024)), dim3(256), 0, (cudaStream_t)stream, src_dev, dst_dev,
+                                 (long long)n));
     return SKB_OK;
 }
 
@@ -1652,10 +1644,9 @@ int skb_asnorm_stats(const float* X_dev, const float* cohort_dev, int N, int C, 
         rc = score_gemm_general(X_dev + (size_t)r0 * D, cohort_dev, rows, C, D, nullptr, nullptr, 1.f, nullptr, nullptr, 0.f, 1.f, 1.f, 3, 0,
                                 g_ws.tmp, ld, tmp_bytes, st);
         if (rc) return rc;
-        topk_stats_kernel<<<rows, 256, C * sizeof(unsigned), st>>>(g_ws.tmp, C, ld, top_k, mean_dev + r0, std_dev + r0);
-        g_launches++;
+        SKB_CUDA_CHECK(launch_kernel(false, topk_stats_kernel, dim3(rows), dim3(256), C * sizeof(unsigned), st, g_ws.tmp, C, ld, top_k,
+                                     mean_dev + r0, std_dev + r0));
     }
-    SKB_CUDA_CHECK(cudaGetLastError());
     return SKB_OK;
 }
 
@@ -1667,8 +1658,7 @@ int skb_asnorm_apply(const float* X_dev, int N, int D, const float* mean_dev, co
     if (rc) return rc;
     float* ra = g_ws.tmp;
     float* r = ra + N;
-    asnorm_terms_kernel<<<(N + 255) / 256, 256, 0, st>>>(mean_dev, std_dev, N, ra, r);
-    g_launches++;
+    SKB_CUDA_CHECK(launch_kernel(false, asnorm_terms_kernel, dim3((N + 255) / 256), dim3(256), 0, st, mean_dev, std_dev, N, ra, r));
     return score_gemm_general(X_dev, X_dev, N, N, D, ra, ra, 0.f, r, r, 0.f, 1.f, 30.f, 3, 0, out_dev, N, tmp_bytes, st);
 }
 
@@ -1687,8 +1677,7 @@ int skb_asnorm_apply_panel(const float* X_dev, int N, int D, int row0, int n_row
     if (rc) return rc;
     float* ra = g_ws.tmp;
     float* r = ra + N;
-    asnorm_terms_kernel<<<(N + 255) / 256, 256, 0, st>>>(mean_dev, std_dev, N, ra, r);
-    g_launches++;
+    SKB_CUDA_CHECK(launch_kernel(false, asnorm_terms_kernel, dim3((N + 255) / 256), dim3(256), 0, st, mean_dev, std_dev, N, ra, r));
     return score_gemm_general(X_dev + (size_t)row0 * D, X_dev, n_rows, N, D, ra + row0, ra, 0.f, r + row0, r, 0.f, 1.f, 30.f, 3, 0,
                               out_dev, ld_out, tmp_bytes, st);
 }
@@ -1715,11 +1704,8 @@ int skb_score_pairs(const float* E_dev, const float* T_dev, int Ne, int Nt, int 
                      mean_e_dev, std_e_dev, mean_t_dev, std_t_dev, out_dev};
     const bool vec = (D & 3) == 0 && (reinterpret_cast<uintptr_t>(E_dev) & 15) == 0 && (reinterpret_cast<uintptr_t>(T_dev) & 15) == 0;
     cudaStream_t st = (cudaStream_t)stream;
-    if (vec)
-        SKB_CUDA_CHECK(launch_pdl(score_pairs_kernel<true>, dim3((unsigned)ctas), dim3(kPairThreads), 0, st, a));
-    else
-        SKB_CUDA_CHECK(launch_pdl(score_pairs_kernel<false>, dim3((unsigned)ctas), dim3(kPairThreads), 0, st, a));
-    g_launches++;
+    SKB_CUDA_CHECK(launch_kernel(true, vec ? score_pairs_kernel<true> : score_pairs_kernel<false>, dim3((unsigned)ctas), dim3(kPairThreads), 0,
+                                 st, a));
     return SKB_OK;
 }
 
