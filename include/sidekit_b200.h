@@ -293,6 +293,24 @@ int skb_affine_rows(const void* X_dev, int x_is_f64, int64_t N, int D, int64_t l
 int skb_resample(const float* in_dev, const int64_t* wave_meta_dev, int n_wav, int64_t max_out, int orig_r, int new_r,
                  int width, const float* bank_dev, const int32_t* start_dev, int ntap, float* out_dev, void* stream);
 
+/* ---- feed path: FLAC decoding (RFC 9639, up to 24 bits per sample) -----------------------------------------------
+ * Replaces torchaudio.load(path) of sidekit/nnet/xsets.py:419-464 (IdMapSet with file_extension="flac") and
+ * soundfile.read of sidekit/bin/extract_xvectors.py:37-72 for .flac files: channel 0 of every file of a batch, as float32
+ * int / 2^(bps - 1), back to back in out_dev.  bytes_dev: the files' frame bytes back to back (n_bytes); files_dev: n_files
+ * rows of nine int64 {first frame byte, end of the file's bytes, output offset, total samples, first frame slot, frame
+ * slots, sample rate, channels, bits per sample} (device), ordered by byte range and by slot; the last five come from
+ * STREAMINFO, which the host parses (sidekit_b200/flac.py).  n_slots = sum of the slot counts (an upper bound on each
+ * file's frame count).  work_dev: at least skb_flac_workspace_bytes(n_bytes, n_files, n_slots) bytes, 16-byte aligned.
+ * status_dev (n_files, int32) receives SKB_FLAC_OK or the reason the file is corrupt; a corrupt file's output range is
+ * left unwritten.  Three launches whatever n_files; no synchronisation; never reads outside bytes_dev. */
+#define SKB_FLAC_OK 0
+#define SKB_FLAC_BAD_FRAME 1      /* no valid frame (header CRC-8, subframes, CRC-16) where the chain needs one */
+#define SKB_FLAC_BAD_NUMBER 2     /* frame / sample number or blocking strategy out of sequence */
+#define SKB_FLAC_BAD_LENGTH 3     /* block sizes overrun STREAMINFO's total samples, or more frames than slots */
+int64_t skb_flac_workspace_bytes(int64_t n_bytes, int n_files, int64_t n_slots);
+int skb_flac_decode(const uint8_t* bytes_dev, int64_t n_bytes, const int64_t* files_dev, int n_files, int64_t n_slots,
+                    void* work_dev, int64_t work_bytes, float* out_dev, int32_t* status_dev, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

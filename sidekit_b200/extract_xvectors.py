@@ -8,6 +8,8 @@ is embedded in length-bucketed packed batches (``bulk.make_batches`` + ``Xtracto
 device where a file's rate differs from the model's (``preprocessor.Resample``); only the batch being embedded is on
 the device, and the ark is written window by window.  The packed engine is exact per utterance, so the vectors are
 those of the one-by-one loop.
+``.flac`` paths and pipe entries whose output is a FLAC stream (``cat x.flac |``) are decoded on the device
+(``sidekit_b200.flac``), all FLAC entries of a window in one batched call.
 ``--vad`` needs the silero model that the reference fetches with ``torch.hub`` at run time (no network here): it raises.
 Tables are written with ``sidekit_b200.kaldi_io`` in the layout ``kaldiio.WriteHelper('ark,scp:...')`` produces.
 """
@@ -19,7 +21,7 @@ import wave as _wave
 import numpy
 import torch
 
-from . import bulk, kaldi_io
+from . import bulk, flac, kaldi_io
 from .nnet.preprocessor import Resample
 from .nnet.xsets import load_checkpoint, read_wav
 
@@ -45,18 +47,34 @@ def _wav_bytes_to_tensor(raw):
     return torch.from_numpy(a.astype(numpy.float32) / numpy.float32(32768.0 if width == 2 else 2147483648.0)), rate
 
 
-def prepare(wav):
-    """A ``wav.scp`` entry (a path, or a shell command ending in ``|`` whose standard output is a wav file) ->
-    ``(float32 tensor (n,), sample_rate)`` scaled like ``soundfile.read`` / ``torchaudio.load`` (:37-72)."""
+def _read_entry(wav):
+    """A ``wav.scp`` entry -> ``(signal, sample_rate, flac_bytes)``: a FLAC file or pipe output comes back undecoded
+    (``signal`` None, ``flac_bytes`` its bytes), anything else decoded as wav (``flac_bytes`` None)."""
     wav = " ".join(wav) if not isinstance(wav, str) else wav
     if wav.strip().endswith("|"):
         try:
             with open(os.devnull, "w") as devnull:
                 out = subprocess.Popen(wav.strip()[:-1], stdout=subprocess.PIPE, shell=True, stderr=devnull).communicate()[0]
-            return _wav_bytes_to_tensor(out)
+            if flac.is_flac(out):
+                return None, flac.parse(out, wav).sample_rate, out
+            return _wav_bytes_to_tensor(out) + (None,)
         except Exception as e:
             raise IOError("Error processing wav file: {}\n{}".format(wav, e))
-    return read_wav(wav)
+    if wav.endswith(".flac"):
+        with open(wav, "rb") as f:
+            data = f.read()
+        return None, flac.parse(data, wav).sample_rate, data
+    return read_wav(wav) + (None,)
+
+
+def prepare(wav):
+    """A ``wav.scp`` entry (a path, or a shell command ending in ``|`` whose standard output is a wav or FLAC file) ->
+    ``(float32 tensor (n,), sample_rate)`` scaled like ``soundfile.read`` / ``torchaudio.load`` (:37-72)."""
+    signal, sr, data = _read_entry(wav)
+    if data is not None:
+        out, _, _ = flac.decode([data])
+        signal = out.cpu()
+    return signal, sr
 
 
 def load_model(model_path, device):
@@ -85,6 +103,11 @@ def main(xtractor, kaldi_wav_scp, out_file, device, vad=False, num_samples_per_w
         order.  Only the batch being embedded lives on the device."""
         if not window:
             return
+        coded = [i for i, (_, sig, _) in enumerate(window) if isinstance(sig, bytes)]
+        if coded:                                          # every FLAC entry of the window in one decode call
+            out, n, _ = flac.decode([window[i][1] for i in coded], device)
+            for i, x in zip(coded, torch.split(out, n.tolist())):
+                window[i] = (window[i][0], x, window[i][2])
         lengths = numpy.array([-(-int(sig.shape[0]) * model_sample_rate // sr) for _, sig, sr in window], dtype=numpy.int64)
         order = numpy.argsort(lengths, kind="stable")
         emb = torch.empty((len(window), xtractor.embedding_size), dtype=torch.float32)
@@ -109,9 +132,13 @@ def main(xtractor, kaldi_wav_scp, out_file, device, vad=False, num_samples_per_w
     with kaldi_io.ArkScpWriter(out_ark, os.path.realpath(out_file)) as writer:
         window, window_s = [], 0.0
         for key, wav in utt2wav.items():
-            signal, sr = prepare(wav)
-            window.append((key, signal, sr))
-            window_s += float(signal.shape[0]) / sr
+            signal, sr, data = _read_entry(wav)
+            if data is not None:                           # decoded at flush time, with the window's other FLAC entries
+                window.append((key, data, sr))
+                window_s += float(flac.parse(data, key).total_samples) / sr
+            else:
+                window.append((key, signal, sr))
+                window_s += float(signal.shape[0]) / sr
             if window_s >= window_audio_seconds:
                 flush(window, writer)
                 window, window_s = [], 0.0

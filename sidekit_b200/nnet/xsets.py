@@ -8,8 +8,10 @@ ALL segments / sliding windows of the id map are cut on the host, length-buckete
 ``Xtractor.extract_varlen`` as packed batches (``bulk.make_batches``): the engine's packed layout makes a batch of
 different lengths exact, so the embeddings are the same as the one-by-one loop, bit for bit.  Augmentation
 (``transform_pipeline``) and HDF5 IO are out of scope and raise; files at another sample rate are resampled on the
-device (``preprocessor.Resample``); ``IdMap`` reads / writes the reference's text format.
+device (``preprocessor.Resample``); ``IdMap`` reads / writes the reference's text format.  ``file_extension="flac"``
+reads FLAC files, decoded on the device (``sidekit_b200.flac``); ``extract_embeddings`` decodes them in batched calls.
 """
+import os
 import wave as _wave
 
 import numpy
@@ -170,6 +172,11 @@ class IdMapSet:
         self.window_len = int(window_len * self.sample_rate)
         self.window_shift = int(window_shift * self.sample_rate)
         self._resamplers = {}
+        if file_extension == "flac":
+            from ..flac import read_flac
+            self._read = read_flac
+        else:
+            self._read = read_wav
 
     def __len__(self):
         return self.len
@@ -187,7 +194,7 @@ class IdMapSet:
         start = 0 if self.idmap.start[index] is None else int(self.idmap.start[index] * 0.01 * self.sample_rate)
         if self.idmap.stop[index] is None:
             # whole file (xsets.py:430-435; note: the file is NOT cut at `start` in this branch, only `duration` is)
-            speech, fs = read_wav(self._path(index))
+            speech, fs = self._read(self._path(index))
             if fs != self.sample_rate:
                 # torchaudio.transforms.Resample(nfo.sample_rate, self.sample_rate) of :434-435, on the device
                 speech = self._resampler(fs)(speech.cuda(non_blocking=True))
@@ -198,12 +205,34 @@ class IdMapSet:
                 middle = start + duration // 2
                 start = int(max(0, int(middle - (self.min_duration * self.sample_rate / 2))))
                 duration = int(self.min_duration * self.sample_rate)
-            speech, fs = read_wav(self._path(index), frame_offset=start, num_frames=duration)
+            speech, fs = self._read(self._path(index), frame_offset=start, num_frames=duration)
             assert fs == self.sample_rate
         stop = start + duration
         if self.sliding_window:
             speech = speech.unfold(0, self.window_len, self.window_shift)
         return speech, self.idmap.leftids[index], self.idmap.rightids[index], start, stop
+
+
+def _predecode_flac(dataset, device, max_bytes=1 << 28):
+    """Decode every FLAC file of ``dataset`` on ``device`` in batched calls of at most ~``max_bytes`` compressed bytes,
+    and make the dataset read from the decoded waveforms (device tensors) instead of decoding file by file."""
+    from .. import flac
+    paths = list(dict.fromkeys(dataset._path(i) for i in range(len(dataset))))
+    decoded = {}
+    chunk, size = [], 0
+    for k, path in enumerate(paths):
+        chunk.append(path)
+        size += os.path.getsize(path)
+        if size >= max_bytes or k == len(paths) - 1:
+            out, lengths, rates = flac.decode(chunk, device)
+            for p, x, fs in zip(chunk, torch.split(out, lengths.tolist()), rates.tolist()):
+                decoded[p] = (x, int(fs))
+            chunk, size = [], 0
+
+    def read(path, frame_offset=0, num_frames=-1):
+        x, fs = decoded[path]
+        return flac.slice_samples(x, frame_offset, num_frames), fs
+    dataset._read = read
 
 
 def load_checkpoint(model_path, device, embedding_size=None):
@@ -242,6 +271,8 @@ def extract_embeddings(idmap_name, model_filename, data_root_name, device, batch
                        sample_rate, min_duration=win_duration)
     model.eval()
     model.to(device)
+    if file_extension == "flac":
+        _predecode_flac(dataset, device)
     waves, modelset, segset, starts, stops = [], [], [], [], []
     last_chunks = 1
     for idx in range(len(dataset)):
