@@ -140,7 +140,9 @@ int skb_meanstd_pool(const float* x_dev, int n_utt, int D, int T, float* out_dev
  * S[i][j] = alpha * (rowterm[i] + colterm[j] + cst) + alpha * sum_k E[i][k] * T[j][k]
  * E_dev (Ne, D), T_dev (Nt, D) fp32 row-major; rowterm/colterm may be NULL (treated as 0).
  * passes: 1 = single 16-bit pass, 3 = split (hi*hi + hi*lo + lo*hi) for fp32-class accuracy,
- * 0 = choose from the operand magnitudes so that the absolute error stays below 2.5e-4.
+ * 0 = choose from the operand magnitudes: 1 when an estimate of the absolute error for operands whose fp16 rounding
+ * errors are uncorrelated stays below 2.5e-4 (on S, alpha included), else 3.  Coherent rounding errors (e.g. rows of one repeated value)
+ * can exceed 2.5e-4 with 1 pass; passes = 3 is the bound for them.
  * out_dtype: 0 = float32, 1 = float64, 2 = float16 (halves the HBM-bound write; 11-bit mantissa: meant for cosine-range
  * scores).  out_dev is (Ne, Nt) row-major with leading dimension ld_out. */
 int skb_score_gemm(const float* E_dev, const float* T_dev, int Ne, int Nt, int D, const float* rowterm_dev,

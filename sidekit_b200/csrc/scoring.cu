@@ -107,11 +107,15 @@ __device__ __forceinline__ int scale_exponent(const unsigned* stats) {
     return e;
 }
 
-// 1 or 3 passes.  Single-pass error estimate: fp16 rounding 2^-11 per operand, random-sign accumulation over D terms.
+// 1 or 3 passes.  Single-pass error estimate: fp16 rounding 2^-11 per operand, random-sign accumulation over D terms, and a
+// factor 7 for the tail of the largest matrices: on 20 000 x 20 000 unit-norm Gaussian rows the worst entry is the diagonal of
+// E = T (a squared norm, whose two roundings per term coincide), about 6 x 2^-11 / sqrt(D); with the factor, unit rows of D < 187
+// take three passes and D = 256 / 512 one.  The estimate holds for operands whose fp16 rounding errors are uncorrelated: rows
+// whose errors add coherently (one repeated value) can exceed it with one pass, and passes = 3 is the bound for them.
 __device__ __forceinline__ int decide_passes(const unsigned* statsE, const unsigned* statsT, int D, float abs_alpha, int passes_req) {
     if (passes_req != 0) return passes_req;
     const float nE = sqrtf(__uint_as_float(statsE[1])), nT = sqrtf(__uint_as_float(statsT[1]));
-    const float est = abs_alpha * 4.8828125e-4f * nE * nT * 4.f * rsqrtf((float)D);
+    const float est = abs_alpha * 4.8828125e-4f * nE * nT * 7.f * rsqrtf((float)D);
     return est < 2.5e-4f ? 1 : 3;
 }
 

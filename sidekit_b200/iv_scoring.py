@@ -40,13 +40,51 @@ def _dev32(a, device):
     return torch.as_tensor(numpy.ascontiguousarray(a, dtype=numpy.float32)).to(device, non_blocking=True)
 
 
+def _operands(name, E, T, vectors=()):
+    """The checks every score GEMM wrapper makes before a library call, which reads its operands through bare pointers:
+    ``E`` (Ne, D) and ``T`` (Nt, D) 2-D float32 tensors on one CUDA device (``T`` may be a ``PackedEmbeddings`` of width
+    D there), and every ``(vector, length)`` of ``vectors`` None or float32 of shape (length,) on that device.  Raises
+    ``ValueError``; returns ``E``, ``T`` and the vectors made contiguous."""
+    packed = isinstance(T, PackedEmbeddings)
+    for X in (E,) if packed else (E, T):
+        if not torch.is_tensor(X) or X.dim() != 2 or X.dtype != torch.float32 or X.device.type != "cuda":
+            raise ValueError("%s: E and T must be 2-D float32 CUDA tensors" % name)
+    dev = E.device
+    if T.device != dev:
+        raise ValueError("%s: E is on %s, T on %s" % (name, dev, T.device))
+    D_t = T.D if packed else T.shape[1]
+    if E.shape[1] != D_t:
+        raise ValueError("%s: E and T must be (Ne, D) and (Nt, D), got D = %d and %d" % (name, E.shape[1], D_t))
+    for t, n in vectors:
+        if t is not None and (not torch.is_tensor(t) or t.dtype != torch.float32 or t.device != dev or tuple(t.shape) != (n,)):
+            raise ValueError("%s: per-row vectors must be float32 on %s, one value per row" % (name, dev))
+    return (E.contiguous(), T if packed else T.contiguous()) + tuple(None if t is None else t.contiguous() for t, _ in vectors)
+
+
+def _rows(T):
+    return T.rows if isinstance(T, PackedEmbeddings) else T.shape[0]
+
+
 def score_matrix(E, T, rowterm=None, colterm=None, cst=0.0, alpha=1.0, passes=0, out_dtype=torch.float32, out=None):
     """S = alpha*(rowterm_i + colterm_j + cst) + alpha * E T^T on the device (all arguments torch CUDA fp32; ``T`` may be a
-    ``PackedEmbeddings``).  ``out_dtype`` float32, float64 or float16 (half the HBM-bound write; 11-bit mantissa)."""
+    ``PackedEmbeddings``).  ``out_dtype`` float32, float64 or float16 (half the HBM-bound write; 11-bit mantissa); ``out``
+    an (Ne, Nt) tensor of one of those types with unit column stride (a view into a wider matrix is fine).
+
+    ``passes``: 3 multiplies split fp16 operands (hi*hi + hi*lo + lo*hi) for float32-class accuracy; 1 multiplies fp16
+    operands once; 0 picks 1 when an error estimate for operands whose fp16 rounding errors are uncorrelated stays below
+    2.5e-4 (on S, alpha included), else 3.  Operands whose rounding errors add coherently (e.g. rows of one repeated value) can exceed
+    that with 1 pass; ``passes=3`` is the bound for them."""
+    E, T, rowterm, colterm = _operands("score_matrix", E, T, [(rowterm, E.shape[0]), (colterm, _rows(T))])
     Ne, D = E.shape
-    Nt = T.rows if isinstance(T, PackedEmbeddings) else T.shape[0]
+    Nt = _rows(T)
     if out is None:
+        if out_dtype not in _OUT_DTYPE:
+            raise ValueError("score_matrix: out_dtype must be float32, float64 or float16")
         out = torch.empty((Ne, Nt), dtype=out_dtype, device=E.device)
+    elif (not torch.is_tensor(out) or out.dtype not in _OUT_DTYPE or out.device != E.device or tuple(out.shape) != (Ne, Nt) or
+          out.stride(1) != 1):
+        raise ValueError("score_matrix: out must be an (Ne, Nt) = (%d, %d) float32 / float64 / float16 tensor on %s with unit "
+                         "column stride" % (Ne, Nt, E.device))
     if isinstance(T, PackedEmbeddings):
         with torch.cuda.device(E.device):
             _lib.check(_lib.lib().skb_score_gemm_packed(
@@ -116,6 +154,7 @@ def score_trials(E, T, trials, rowterm=None, colterm=None, cst=0.0, alpha=1.0, p
     """The scores of the trials of a mask only, as a 1-D float32 CUDA tensor in row-major mask order -- what the reference
     selects with ``scoremat[trialmask]`` (xvector.py:243-245) -- without the Ne x Nt matrix ever reaching HBM.
     ``trials``: a ``TrialIndex`` or an (Ne, Nt) bool mask; ``T`` may be a ``PackedEmbeddings``."""
+    E, T, rowterm, colterm = _operands("score_trials", E, T, [(rowterm, E.shape[0]), (colterm, _rows(T))])
     if not isinstance(trials, TrialIndex):
         trials = TrialIndex(trials, E.device)
     Ne, D = E.shape
@@ -148,24 +187,19 @@ def score_pairs(E, T, rows, cols, rowterm=None, colterm=None, cst=0.0, alpha=1.0
 def _score_pairs(E, T, rows, cols, rowterm=None, colterm=None, cst=0.0, alpha=1.0, asnorm_stats=None):
     """``score_pairs``; ``asnorm_stats = (mean_e, std_e, mean_t, std_t)`` (float32 CUDA, indexed like ``E`` / ``T``)
     normalises every score with the symmetric as-norm formula in the same kernel."""
-    dev = E.device
-    if dev.type != "cuda":
-        raise ValueError("score_pairs: E and T must be CUDA tensors")
-    rows = torch.as_tensor(rows).to(dev, torch.int32).contiguous()
-    cols = torch.as_tensor(cols).to(dev, torch.int32).contiguous()
-    if rows.dim() != 1 or rows.shape != cols.shape:
-        raise ValueError("score_pairs: rows and cols must be 1-D arrays of one length")
-    if E.dim() != 2 or T.dim() != 2 or E.shape[1] != T.shape[1]:
+    if not torch.is_tensor(E) or not torch.is_tensor(T) or E.dim() != 2 or T.dim() != 2:
         raise ValueError("score_pairs: E and T must be (Ne, D) and (Nt, D)")
     vectors = [(rowterm, E.shape[0]), (colterm, T.shape[0])]
     if asnorm_stats is not None:
         vectors += [(asnorm_stats[0], E.shape[0]), (asnorm_stats[1], E.shape[0]), (asnorm_stats[2], T.shape[0]), (asnorm_stats[3], T.shape[0])]
-    for t, n in [(E, None), (T, None)] + vectors:
-        if t is not None and (t.dtype != torch.float32 or t.device != dev or (n is not None and tuple(t.shape) != (n,))):
-            raise ValueError("score_pairs: operands and per-row vectors must be float32 on %s, one value per row" % dev)
-    E, T = E.contiguous(), T.contiguous()
-    ptr = lambda t: None if t is None else t.contiguous().data_ptr()
-    me, se, mt, st = asnorm_stats if asnorm_stats is not None else (None,) * 4
+    E, T, rowterm, colterm, *stats = _operands("score_pairs", E, T, vectors)
+    dev = E.device
+    rows = torch.as_tensor(rows).to(dev, torch.int32).contiguous()
+    cols = torch.as_tensor(cols).to(dev, torch.int32).contiguous()
+    if rows.dim() != 1 or rows.shape != cols.shape:
+        raise ValueError("score_pairs: rows and cols must be 1-D arrays of one length")
+    ptr = lambda t: None if t is None else t.data_ptr()
+    me, se, mt, st = stats if asnorm_stats is not None else (None,) * 4
     out = torch.empty((rows.shape[0],), dtype=torch.float32, device=dev)
     with torch.cuda.device(dev):
         _lib.check(_lib.lib().skb_score_pairs(E.data_ptr(), T.data_ptr(), E.shape[0], T.shape[0], E.shape[1], rows.data_ptr(),
@@ -251,8 +285,9 @@ def score_topk(E, T, k, rowterm=None, colterm=None, cst=0.0, alpha=1.0, passes=0
     and searched by many query batches).  For ``k <= 32`` and ``D <= 256`` the selection runs inside the GEMM epilogue and
     the (Ne, Nt) matrix never reaches memory; otherwise row panels of it pass through a bounded scratch.  The order of NaN
     scores is undefined."""
+    E, T, rowterm, colterm = _operands("score_topk", E, T, [(rowterm, E.shape[0]), (colterm, _rows(T))])
     Ne, D = E.shape
-    Nt = T.rows if isinstance(T, PackedEmbeddings) else T.shape[0]
+    Nt = _rows(T)
     k = int(k)
     if not 1 <= k <= min(Nt, TOPK_MAX):
         raise ValueError("score_topk: need 1 <= k <= min(Nt, %d), got k = %d with Nt = %d" % (TOPK_MAX, k, Nt))
