@@ -313,6 +313,25 @@ int64_t skb_flac_workspace_bytes(int64_t n_bytes, int n_files, int64_t n_slots);
 int skb_flac_decode(const uint8_t* bytes_dev, int64_t n_bytes, const int64_t* files_dev, int n_files, int64_t n_slots,
                     void* work_dev, int64_t work_bytes, float* out_dev, int32_t* status_dev, void* stream);
 
+/* ---- feed path: uncompressed audio (WAV and NIST SPHERE, every PCM encoding) ------------------------------------------
+ * Replaces torchaudio.load(path) of sidekit/nnet/xsets.py:419-464 and soundfile.read of sidekit/bin/extract_xvectors.py:37-72
+ * for .wav / .sph files: channel 0 of every file of a batch as float32, at the file's output offset in out_dev, scaled as
+ * those readers do -- signed integers x / 2^(8 bytes - 1) (32-bit: rounded to float32 first), unsigned 8-bit
+ * (x - 128) / 128, float32 copied, float64 rounded to float32, G.711 mu-law / A-law expanded to 16 bits (Sun g711.c) / 2^15.
+ * bytes_dev: the files' sample bytes (interleaved frames); files_dev: n_files rows of eight int64 {byte offset of the
+ * file's first frame in bytes_dev, frames, channels, SKB_PCM_* encoding, bytes per sample (1-4 for integers, 1 for
+ * G.711, 4 or 8 for float), big-endian flag, output offset, first tile}, ordered by first tile; a file owns
+ * ceil(frames / 256) tiles, numbered file after file, and n_tiles is their total.  The host parses the containers
+ * (sidekit_b200/pcm.py).  Reads stay inside [offset, offset + frames * channels * bytes) of each file.  One launch
+ * whatever n_files (also when n_tiles is 0, when bytes_dev and out_dev may be NULL); no synchronisation. */
+#define SKB_PCM_INT 0             /* signed integer, any byte count 1-4 */
+#define SKB_PCM_U8 1              /* unsigned 8-bit (WAV) */
+#define SKB_PCM_FLOAT 2           /* IEEE float, 4 or 8 bytes */
+#define SKB_PCM_ULAW 3            /* G.711 mu-law, 1 byte */
+#define SKB_PCM_ALAW 4            /* G.711 A-law, 1 byte */
+int skb_pcm_decode(const uint8_t* bytes_dev, const int64_t* files_dev, int n_files, int64_t n_tiles, float* out_dev,
+                   void* stream);
+
 #ifdef __cplusplus
 }
 #endif

@@ -87,6 +87,7 @@ def _declare(lib):
         "skb_resample":(i32, [vp, vp, i32, i64, i32, i32, i32, vp, vp, i32, vp, vp]),
         "skb_flac_workspace_bytes": (i64, [i64, i32, i64]),
         "skb_flac_decode": (i32, [vp, i64, vp, i32, i64, vp, i64, vp, vp, vp]),
+        "skb_pcm_decode": (i32, [vp, vp, i32, i64, vp, vp]),
     }
     for name, (res, args) in sigs.items():
         fn = getattr(lib, name)       # AttributeError here = header / library mismatch: fail loudly

@@ -8,22 +8,20 @@ is embedded in length-bucketed packed batches (``bulk.make_batches`` + ``Xtracto
 device where a file's rate differs from the model's (``preprocessor.Resample``); only the batch being embedded is on
 the device, and the ark is written window by window.  The packed engine is exact per utterance, so the vectors are
 those of the one-by-one loop.
-``.flac`` paths and pipe entries whose output is a FLAC stream (``cat x.flac |``) are decoded on the device
-(``sidekit_b200.flac``), all FLAC entries of a window in one batched call.
+Paths and pipe entries (``cat x.sph |``, ``sph2pipe -f wav x.sph |``) may hold FLAC, WAV or NIST SPHERE in every PCM
+encoding; the entries of a window are read as bytes and decoded on the device in one batched call (``sidekit_b200.audio``).
 ``--vad`` needs the silero model that the reference fetches with ``torch.hub`` at run time (no network here): it raises.
 Tables are written with ``sidekit_b200.kaldi_io`` in the layout ``kaldiio.WriteHelper('ark,scp:...')`` produces.
 """
-import io
 import os
 import subprocess
-import wave as _wave
 
 import numpy
 import torch
 
-from . import bulk, flac, kaldi_io
+from . import audio, bulk, kaldi_io
 from .nnet.preprocessor import Resample
-from .nnet.xsets import load_checkpoint, read_wav
+from .nnet.xsets import load_checkpoint
 
 
 def read_wav_scp(wav_scp):
@@ -37,44 +35,30 @@ def read_wav_scp(wav_scp):
     return utt2wav
 
 
-def _wav_bytes_to_tensor(raw):
-    with _wave.open(io.BytesIO(raw), "rb") as f:
-        rate, width, chans = f.getframerate(), f.getsampwidth(), f.getnchannels()
-        if width not in (2, 4):
-            raise NotImplementedError("only 16- and 32-bit PCM is supported")
-        data = f.readframes(f.getnframes())
-    a = numpy.frombuffer(data, dtype=numpy.int16 if width == 2 else numpy.int32).reshape(-1, chans)[:, 0]
-    return torch.from_numpy(a.astype(numpy.float32) / numpy.float32(32768.0 if width == 2 else 2147483648.0)), rate
-
-
 def _read_entry(wav):
-    """A ``wav.scp`` entry -> ``(signal, sample_rate, flac_bytes)``: a FLAC file or pipe output comes back undecoded
-    (``signal`` None, ``flac_bytes`` its bytes), anything else decoded as wav (``flac_bytes`` None)."""
+    """A ``wav.scp`` entry -> ``(name, file bytes, sample_rate, frames)``, undecoded.  A pipe entry's output is checked to be
+    a readable FLAC, WAV or NIST SPHERE stream here, so that a failing command raises ``IOError`` naming it."""
     wav = " ".join(wav) if not isinstance(wav, str) else wav
     if wav.strip().endswith("|"):
         try:
             with open(os.devnull, "w") as devnull:
                 out = subprocess.Popen(wav.strip()[:-1], stdout=subprocess.PIPE, shell=True, stderr=devnull).communicate()[0]
-            if flac.is_flac(out):
-                return None, flac.parse(out, wav).sample_rate, out
-            return _wav_bytes_to_tensor(out) + (None,)
+            frames, sr = audio.length(*audio.parse(out, wav))
+            return wav, out, sr, frames
         except Exception as e:
             raise IOError("Error processing wav file: {}\n{}".format(wav, e))
-    if wav.endswith(".flac"):
-        with open(wav, "rb") as f:
-            data = f.read()
-        return None, flac.parse(data, wav).sample_rate, data
-    return read_wav(wav) + (None,)
+    with open(wav, "rb") as f:
+        data = f.read()
+    frames, sr = audio.length(*audio.parse(data, wav))
+    return wav, data, sr, frames
 
 
 def prepare(wav):
-    """A ``wav.scp`` entry (a path, or a shell command ending in ``|`` whose standard output is a wav or FLAC file) ->
-    ``(float32 tensor (n,), sample_rate)`` scaled like ``soundfile.read`` / ``torchaudio.load`` (:37-72)."""
-    signal, sr, data = _read_entry(wav)
-    if data is not None:
-        out, _, _ = flac.decode([data])
-        signal = out.cpu()
-    return signal, sr
+    """A ``wav.scp`` entry (a path, or a shell command ending in ``|`` whose standard output is an audio file) ->
+    ``(float32 tensor (n,), sample_rate)`` scaled like ``soundfile.read`` / ``torchaudio.load`` (:37-72).  FLAC, WAV and
+    NIST SPHERE in every PCM encoding (``sidekit_b200.audio.read``)."""
+    name, data, _, _ = _read_entry(wav)
+    return audio.read(data, name=name)
 
 
 def load_model(model_path, device):
@@ -99,15 +83,12 @@ def main(xtractor, kaldi_wav_scp, out_file, device, vad=False, num_samples_per_w
     all_emb = []
 
     def flush(window, writer):
-        """Embed one window of utterances (host tensors) in length-bucketed packed batches and write its entries in file
-        order.  Only the batch being embedded lives on the device."""
+        """Decode one window of entries (file bytes) in one call, embed it in length-bucketed packed batches and write its
+        entries in file order.  Only the window's waveforms and the batch being embedded live on the device."""
         if not window:
             return
-        coded = [i for i, (_, sig, _) in enumerate(window) if isinstance(sig, bytes)]
-        if coded:                                          # every FLAC entry of the window in one decode call
-            out, n, _ = flac.decode([window[i][1] for i in coded], device)
-            for i, x in zip(coded, torch.split(out, n.tolist())):
-                window[i] = (window[i][0], x, window[i][2])
+        out, n, _ = audio.decode([data for _, _, data, _ in window], device, names=[name for _, name, _, _ in window])
+        window = [(key, x, sr) for (key, _, _, sr), x in zip(window, torch.split(out, n.tolist()))]
         lengths = numpy.array([-(-int(sig.shape[0]) * model_sample_rate // sr) for _, sig, sr in window], dtype=numpy.int64)
         order = numpy.argsort(lengths, kind="stable")
         emb = torch.empty((len(window), xtractor.embedding_size), dtype=torch.float32)
@@ -132,13 +113,9 @@ def main(xtractor, kaldi_wav_scp, out_file, device, vad=False, num_samples_per_w
     with kaldi_io.ArkScpWriter(out_ark, os.path.realpath(out_file)) as writer:
         window, window_s = [], 0.0
         for key, wav in utt2wav.items():
-            signal, sr, data = _read_entry(wav)
-            if data is not None:                           # decoded at flush time, with the window's other FLAC entries
-                window.append((key, data, sr))
-                window_s += float(flac.parse(data, key).total_samples) / sr
-            else:
-                window.append((key, signal, sr))
-                window_s += float(signal.shape[0]) / sr
+            name, data, sr, frames = _read_entry(wav)
+            window.append((key, name, data, sr))           # decoded at flush time, with the window's other entries
+            window_s += float(frames) / sr
             if window_s >= window_audio_seconds:
                 flush(window, writer)
                 window, window_s = [], 0.0

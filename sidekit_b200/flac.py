@@ -95,6 +95,50 @@ def _workspace(device, nbytes):
     return w
 
 
+def device_of(device):
+    """``device`` (None: the current CUDA device) as a ``torch.device`` with an index; raises without CUDA."""
+    if not torch.cuda.is_available():
+        raise RuntimeError("sidekit_b200 needs a CUDA device (B200, sm_100a); there is no CPU fallback")
+    device = torch.device("cuda", torch.cuda.current_device()) if device is None else torch.device(device)
+    if device.index is None:
+        device = torch.device("cuda", torch.cuda.current_device())
+    return device
+
+
+def table(infos, byte_begin, out_begin):
+    """Rows of ``skb_flac_decode``'s file table (int64, (n, 9)) for files whose frame bytes start at ``byte_begin`` of the
+    byte buffer and whose samples go to ``out_begin`` of the output, and the frame-slot total."""
+    nbytes = numpy.array([i.frames_end - i.frames_begin for i in infos], dtype=numpy.int64)
+    totals = numpy.array([i.total_samples for i in infos], dtype=numpy.int64)
+    # frame slots per file: an upper bound on its frame count (every frame but the last holds at least STREAMINFO's minimum
+    # block size, and no frame is shorter than 10 bytes); a stream that needs more is corrupt
+    min_bs = numpy.array([max(i.min_blocksize, 1) for i in infos], dtype=numpy.int64)
+    caps = numpy.minimum(-(-totals // min_bs) + 1, nbytes // 10 + 1)
+    t = numpy.zeros((len(infos), 9), dtype=numpy.int64)
+    t[:, 0], t[:, 1] = byte_begin, numpy.asarray(byte_begin) + nbytes
+    t[:, 2], t[:, 3] = out_begin, totals
+    t[:, 4], t[:, 5] = numpy.cumsum(caps) - caps, caps
+    t[:, 6] = [i.sample_rate for i in infos]
+    t[:, 7] = [i.channels for i in infos]
+    t[:, 8] = [i.bits_per_sample for i in infos]
+    return t, int(caps.sum())
+
+
+def launch(device, bytes_ptr, n_bytes, table_ptr, n_files, n_slots, out_ptr):
+    """One ``skb_flac_decode`` call on the current stream of ``device``; returns the per-file status (device int32)."""
+    lib = _lib.lib()
+    status = torch.empty(n_files, dtype=torch.int32, device=device)
+    work = _workspace(device, int(lib.skb_flac_workspace_bytes(n_bytes, n_files, n_slots)))
+    _lib.check(lib.skb_flac_decode(bytes_ptr, n_bytes, table_ptr, n_files, n_slots, work.data_ptr(), work.numel(), out_ptr,
+                                   status.data_ptr(), _lib.stream_ptr()))
+    return status
+
+
+def status_errors(names, status):
+    """``["name: reason", ...]`` for the files whose status (host int array) is not OK."""
+    return ["%s: %s" % (names[i], _STATUS.get(int(status[i]), "status %d" % status[i])) for i in numpy.nonzero(status)[0]]
+
+
 def decode(files, device=None):
     """Decode a batch of FLAC files (paths or bytes) on ``device`` (default: the current CUDA device) in one native call.
 
@@ -102,11 +146,7 @@ def decode(files, device=None):
     back, ``lengths`` (int64 numpy) the files' sample counts and ``sample_rates`` (int64 numpy) their rates.  The
     compressed bytes go to the device in one copy; a corrupt or truncated file raises ``ValueError`` naming every bad
     file of the call."""
-    if not torch.cuda.is_available():
-        raise RuntimeError("sidekit_b200 needs a CUDA device (B200, sm_100a); there is no CPU fallback")
-    device = torch.device("cuda", torch.cuda.current_device()) if device is None else torch.device(device)
-    if device.index is None:
-        device = torch.device("cuda", torch.cuda.current_device())
+    device = device_of(device)
     files = list(files)
     if not files:
         return torch.empty(0, dtype=torch.float32, device=device), numpy.zeros(0, numpy.int64), numpy.zeros(0, numpy.int64)
@@ -116,44 +156,27 @@ def decode(files, device=None):
     nf = len(files)
     nbytes = numpy.array([i.frames_end - i.frames_begin for i in infos], dtype=numpy.int64)
     totals = numpy.array([i.total_samples for i in infos], dtype=numpy.int64)
-    # frame slots per file: an upper bound on its frame count (every frame but the last holds at least STREAMINFO's minimum
-    # block size, and no frame is shorter than 10 bytes); a stream that needs more is corrupt
-    min_bs = numpy.array([max(i.min_blocksize, 1) for i in infos], dtype=numpy.int64)
-    caps = numpy.minimum(-(-totals // min_bs) + 1, nbytes // 10 + 1)
-    begin = numpy.cumsum(nbytes) - nbytes
-    table = numpy.zeros((nf, 9), dtype=numpy.int64)
-    table[:, 0], table[:, 1] = begin, begin + nbytes
-    table[:, 2], table[:, 3] = numpy.cumsum(totals) - totals, totals
-    table[:, 4], table[:, 5] = numpy.cumsum(caps) - caps, caps
-    table[:, 6] = [i.sample_rate for i in infos]
-    table[:, 7] = [i.channels for i in infos]
-    table[:, 8] = [i.bits_per_sample for i in infos]
-    n_bytes, n_slots = int(nbytes.sum()), int(caps.sum())
+    table_, n_slots = table(infos, numpy.cumsum(nbytes) - nbytes, numpy.cumsum(totals) - totals)
+    n_bytes = int(nbytes.sum())
     if n_bytes == 0:
         raise ValueError("corrupt FLAC: " + "; ".join("%s: no frames" % nm for nm in names))
     # one pinned staging buffer, one host-to-device copy: the file table, then the frame bytes
-    head = table.nbytes
+    head = table_.nbytes
     host = torch.empty(head + n_bytes, dtype=torch.uint8, pin_memory=True)
     hv = host.numpy()
-    hv[:head] = table.view(numpy.uint8).reshape(-1)
+    hv[:head] = table_.view(numpy.uint8).reshape(-1)
     o = head
     for d, info in zip(datas, infos):
         hv[o:o + info.frames_end - info.frames_begin] = numpy.frombuffer(d, dtype=numpy.uint8, offset=info.frames_begin)
         o += info.frames_end - info.frames_begin
-    lib = _lib.lib()
     with torch.cuda.device(device):
         staged = host.to(device, non_blocking=True)
         out = torch.empty(int(totals.sum()), dtype=torch.float32, device=device)
-        status = torch.empty(nf, dtype=torch.int32, device=device)
-        need = int(lib.skb_flac_workspace_bytes(n_bytes, nf, n_slots))
-        work = _workspace(device, need)
-        _lib.check(lib.skb_flac_decode(staged.data_ptr() + head, n_bytes, staged.data_ptr(), nf, n_slots, work.data_ptr(),
-                                       work.numel(), out.data_ptr(), status.data_ptr(), _lib.stream_ptr()))
-        st = status.cpu().numpy()
-    bad = numpy.nonzero(st)[0]
-    if bad.size:
-        raise ValueError("corrupt FLAC: " + "; ".join("%s: %s" % (names[i], _STATUS.get(int(st[i]), "status %d" % st[i])) for i in bad))
-    return out, totals, table[:, 6].copy()
+        st = launch(device, staged.data_ptr() + head, n_bytes, staged.data_ptr(), nf, n_slots, out.data_ptr()).cpu().numpy()
+    bad = status_errors(names, st)
+    if bad:
+        raise ValueError("corrupt FLAC: " + "; ".join(bad))
+    return out, totals, table_[:, 6].copy()
 
 
 def read_flac(path, frame_offset=0, num_frames=-1):

@@ -2,14 +2,15 @@
 reference's signatures (sidekit/bosaris/idmap.py:43-73, sidekit/nnet/xsets.py:368-480,
 sidekit/nnet/xvector.py:1796-1916).
 
-What changes against the reference: wav files are read with the standard library (``torchaudio.load`` needs
-torchcodec), and instead of one ``forward`` per file -- a few hundred small launches and a device-to-host sync each --
-ALL segments / sliding windows of the id map are cut on the host, length-bucketed and pushed through
+What changes against the reference: a single 16- or 32-bit PCM wav file is read with the standard library
+(``torchaudio.load`` needs torchcodec), other audio is decoded on the device; and instead of one ``forward`` per file --
+a few hundred small launches and a device-to-host sync each -- ALL segments / sliding windows of the id map are cut on the host, length-bucketed and pushed through
 ``Xtractor.extract_varlen`` as packed batches (``bulk.make_batches``): the engine's packed layout makes a batch of
 different lengths exact, so the embeddings are the same as the one-by-one loop, bit for bit.  Augmentation
 (``transform_pipeline``) and HDF5 IO are out of scope and raise; files at another sample rate are resampled on the
-device (``preprocessor.Resample``); ``IdMap`` reads / writes the reference's text format.  ``file_extension="flac"``
-reads FLAC files, decoded on the device (``sidekit_b200.flac``); ``extract_embeddings`` decodes them in batched calls.
+device (``preprocessor.Resample``); ``IdMap`` reads / writes the reference's text format.  Files are recognised by their
+content, whatever ``file_extension`` says: FLAC, WAV and NIST SPHERE in every PCM encoding (``sidekit_b200.audio``);
+``extract_embeddings`` decodes every file of the dataset on the device in batched calls.
 """
 import os
 import wave as _wave
@@ -172,11 +173,8 @@ class IdMapSet:
         self.window_len = int(window_len * self.sample_rate)
         self.window_shift = int(window_shift * self.sample_rate)
         self._resamplers = {}
-        if file_extension == "flac":
-            from ..flac import read_flac
-            self._read = read_flac
-        else:
-            self._read = read_wav
+        from ..audio import read
+        self._read = read
 
     def __len__(self):
         return self.len
@@ -213,10 +211,12 @@ class IdMapSet:
         return speech, self.idmap.leftids[index], self.idmap.rightids[index], start, stop
 
 
-def _predecode_flac(dataset, device, max_bytes=1 << 28):
-    """Decode every FLAC file of ``dataset`` on ``device`` in batched calls of at most ~``max_bytes`` compressed bytes,
-    and make the dataset read from the decoded waveforms (device tensors) instead of decoding file by file."""
-    from .. import flac
+def _predecode(dataset, device, max_bytes=1 << 28):
+    """Decode every file of ``dataset`` on ``device`` in batched calls of at most ~``max_bytes`` file bytes, and make the
+    dataset read from the decoded waveforms (device tensors) instead of reading file by file.  The float32 waveforms of
+    the whole dataset stay on the device until extraction ends: 4 bytes per sample, about 230 GB per 1000 hours at
+    16 kHz, so an id map larger than device memory allows is to be split (``IdMap.split``) and extracted part by part."""
+    from .. import audio, flac
     paths = list(dict.fromkeys(dataset._path(i) for i in range(len(dataset))))
     decoded = {}
     chunk, size = [], 0
@@ -224,7 +224,7 @@ def _predecode_flac(dataset, device, max_bytes=1 << 28):
         chunk.append(path)
         size += os.path.getsize(path)
         if size >= max_bytes or k == len(paths) - 1:
-            out, lengths, rates = flac.decode(chunk, device)
+            out, lengths, rates = audio.decode(chunk, device)
             for p, x, fs in zip(chunk, torch.split(out, lengths.tolist()), rates.tolist()):
                 decoded[p] = (x, int(fs))
             chunk, size = [], 0
@@ -260,7 +260,8 @@ def extract_embeddings(idmap_name, model_filename, data_root_name, device, batch
     ``model_filename`` is an ``Xtractor`` or the path of a checkpoint written by the reference's training loop
     (``speaker_number`` / ``model_archi`` / ``model_state_dict``, xvector.py:1834-1843); ``batch_size``, ``num_thread`` and
     ``mixed_precision`` are accepted and ignored: batches are formed by total audio (``max_audio_seconds``) and the
-    kernels pick their own precision.  ``start`` / ``stop`` follow the reference, including its sliding-window
+    kernels pick their own precision.  Every file is decoded on the device first, and the waveforms of the whole id map
+    stay there until the embeddings are done (4 bytes per sample): split a very large id map (``IdMap.split``).  ``start`` / ``stop`` follow the reference, including its sliding-window
     ``stop = start + <number of 100-window chunks of the last file>`` (xvector.py:1897, :1911).
     """
     from .. import bulk
@@ -271,8 +272,7 @@ def extract_embeddings(idmap_name, model_filename, data_root_name, device, batch
                        sample_rate, min_duration=win_duration)
     model.eval()
     model.to(device)
-    if file_extension == "flac":
-        _predecode_flac(dataset, device)
+    _predecode(dataset, device)
     waves, modelset, segset, starts, stops = [], [], [], [], []
     last_chunks = 1
     for idx in range(len(dataset)):
