@@ -285,6 +285,12 @@ __device__ __forceinline__ float2 unpack2(uint32_t u) {
     }
 }
 
+__device__ __forceinline__ long long shfl_xor_ll(long long v, int off) {
+    const int lo = __shfl_xor_sync(0xffffffffu, (int)(v & 0xffffffffll), off);
+    const int hi = __shfl_xor_sync(0xffffffffu, (int)(v >> 32), off);
+    return ((long long)hi << 32) | (unsigned int)lo;
+}
+
 __device__ __forceinline__ float warp_sum(float v) {
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);

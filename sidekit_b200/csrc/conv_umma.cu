@@ -10,8 +10,10 @@ namespace skb {
 
 int conv_pick_ncta(int cout) { return cout <= 32 ? 32 : (cout <= 64 ? 64 : 128); }
 int conv_tile_m(int n_cta) { return n_cta == 32 ? 512 : 256; }
+// N tiles whose plain epilogue can accumulate ConvParams::sums: one N split below 128 channels, at most two (ConvTotals) at 128
+bool conv_sums_supported(int n_cta, int cout) { return n_cta == 128 ? (cout == 128 || cout == 256) : cout == n_cta; }
 
-template <int N_CTA, int MT, bool BF16, bool FUSED, bool SC = false>
+template <int N_CTA, int MT, bool BF16, bool FUSED, bool SC = false, bool TOT = false>
 static int launch_one(const ConvParams& p_in, cudaStream_t st) {
     using Cfg = ConvCfg<N_CTA, MT, SC>;
     static PerDeviceOnce configured;
@@ -41,14 +43,14 @@ static int launch_one(const ConvParams& p_in, cudaStream_t st) {
             }
         }
         b_stage = (size_t)tps * Cfg::kBStageBytes;
-        const size_t left = kConvSmemBudget - Cfg::fixed_bytes(p.cout, p.bias_mma, 0, 0, scb, p.sc_cin) - 3 * a_stage;
+        const size_t left = kConvSmemBudget - Cfg::fixed_bytes(p.cout, p.bias_mma, 0, 0, scb, p.sc_cin, TOT) - 3 * a_stage;
         bst = (int)(left / b_stage);
         if (bst > kConvBStages) bst = kConvBStages;
         if (bst < 2) bst = 2;
     }
     p.tps = tps;
     p.b_stages = bst;
-    const size_t fixed = Cfg::fixed_bytes(p.cout, p.bias_mma, bst, tps, scb, p.sc_cin);
+    const size_t fixed = Cfg::fixed_bytes(p.cout, p.bias_mma, bst, tps, scb, p.sc_cin, TOT);
     int stages = (int)((kConvSmemBudget - fixed) / a_stage);
     if (stages > kConvMaxAStages) stages = kConvMaxAStages;
     if (stages < 2) {
@@ -58,14 +60,14 @@ static int launch_one(const ConvParams& p_in, cudaStream_t st) {
     p.a_stages = stages;
     const size_t smem = fixed + (size_t)stages * a_stage;
     if (configured.first()) {
-        SKB_CUDA_CHECK(cudaFuncSetAttribute(conv_umma_kernel<N_CTA, MT, BF16, FUSED, SC>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+        SKB_CUDA_CHECK(cudaFuncSetAttribute(conv_umma_kernel<N_CTA, MT, BF16, FUSED, SC, TOT>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                             227 * 1024));
     }
     const int n_pix = p.p_end - p.G;
     p.n_tiles = (n_pix + Cfg::kTileM - 1) / Cfg::kTileM;
     const int n_items = p.n_tiles * (p.cout / N_CTA);
     const int grid = n_items < kNumSMs ? n_items : kNumSMs;      // persistent: one CTA per SM
-    SKB_CUDA_CHECK(launch_kernel(true, conv_umma_kernel<N_CTA, MT, BF16, FUSED, SC>, dim3(grid), dim3(kConvThreads), smem, st, p));
+    SKB_CUDA_CHECK(launch_kernel(true, conv_umma_kernel<N_CTA, MT, BF16, FUSED, SC, TOT>, dim3(grid), dim3(kConvThreads), smem, st, p));
     return SKB_OK;
 }
 
@@ -105,7 +107,8 @@ int launch_conv_umma(const ConvParams& p, int n_cta, bool bf16, cudaStream_t st)
     // layers 1 / 2, but the lane-shifted epilogue (64 shuffles + 6 TMEM loads per 32 x 32 block) costs more than the MMAs
     // it saves: 417 / 230 us per launch against 295 / 178 us for conv_umma_kernel (profiles/r01c_fused_taps.txt).
     static const bool fused_taps = [] { const char* e = getenv("SKB_FUSED_TAPS"); return e && e[0] == '1'; }();
-    if (p.w3 != nullptr && fused_taps && p.sc_in == nullptr && p.cout == n_cta && p.taps == 9 && p.cin % kConvKC == 0) {
+    // (the fused-tap kernel has no channel totals in its epilogue)
+    if (p.w3 != nullptr && fused_taps && p.sc_in == nullptr && p.sums == nullptr && p.cout == n_cta && p.taps == 9 && p.cin % kConvKC == 0) {
         if (n_cta == 32) return bf16 ? launch_one3<32, 2, true>(p, st) : launch_one3<32, 2, false>(p, st);
         if (n_cta == 64) return bf16 ? launch_one3<64, 1, true>(p, st) : launch_one3<64, 1, false>(p, st);
     }
@@ -114,6 +117,10 @@ int launch_conv_umma(const ConvParams& p, int n_cta, bool bf16, cudaStream_t st)
         return SKB_ERR_ARG;
     }
     const bool fused = p.se_scale != nullptr;
+    if (p.sums != nullptr && (fused || p.sc_in != nullptr || p.pix_sub != nullptr || !conv_sums_supported(n_cta, p.cout))) {
+        set_last_error(__FILE__, __LINE__, "conv_umma: channel totals unsupported for this shape");
+        return SKB_ERR_ARG;
+    }
     if (p.sc_in != nullptr) {
         // folded shortcut: the narrow layers only (the <128, 2> tiles already use all 512 TMEM columns)
         if (!fused || p.sc_w == nullptr || p.sc_bias == nullptr || p.sc_cin < kConvKC || p.sc_cin % kConvKC != 0 || p.cout > 256) {
@@ -129,6 +136,10 @@ int launch_conv_umma(const ConvParams& p, int n_cta, bool bf16, cudaStream_t st)
     case N:                                                                                                   \
         if (fused) return bf16 ? launch_one<N, M, true, true>(p, st) : launch_one<N, M, false, true>(p, st);  \
         return bf16 ? launch_one<N, M, true, false>(p, st) : launch_one<N, M, false, false>(p, st);
+    if (p.sums != nullptr && n_cta == 64)
+        return bf16 ? launch_one<64, 2, true, false, false, true>(p, st) : launch_one<64, 2, false, false, false, true>(p, st);
+    if (p.sums != nullptr && n_cta == 128)
+        return bf16 ? launch_one<128, 2, true, false, false, true>(p, st) : launch_one<128, 2, false, false, false, true>(p, st);
     switch (n_cta) {
         SKB_CONV_CASE(32, 4)
         SKB_CONV_CASE(64, 2)

@@ -66,8 +66,9 @@ struct ConvParams {
     const uint16_t* res;           // residual planes in the INPUT pixel geometry (block input or shortcut conv), or nullptr
     long long res_plane;
     // Per-(utterance, channel) totals of the STORED 16-bit outputs in 2^-15 fixed point (what plane_sum_kernel computes with
-    // one more pass over the tensor), accumulated by the epilogue: [n_utt][cout] or nullptr.  Only the N_CTA == 32 kernels
-    // with cout == 32 support it (32 per-thread 64-bit accumulators, flushed with atomics when the utterance changes).
+    // one more pass over the tensor), accumulated by the epilogue of an unfused, stride-1-output conv: [n_utt][cout] or
+    // nullptr.  N_CTA == 32 with cout == 32: 32 per-thread 64-bit accumulators; N_CTA == 64 with cout == 64 and N_CTA == 128
+    // with cout <= 256: the transposed ownership of ConvTotals.  Flushed with atomics when the utterance changes.
     unsigned long long* sums;
     unsigned* overflow;     // fp16 range guard: number of threads that stored a saturated (|x| >= 65504) value, or nullptr
     // Folded 1x1 shortcut (conv2 of a widening / striding block, N_CTA <= 64): the residual is computed here instead of read
@@ -95,18 +96,155 @@ struct ConvCfg {
     static constexpr int kBStageBytes = N_CTA * kConvKC * 2;
     static constexpr int kTileM = 128 * MT;
     // ctrl | bias fp32 [cout] | ones operand (2 planes x 128 rows x 16 B) | bias images (2 planes x cout rows x 16 B) |
-    // SE scales | SC: shortcut bias images (as the bias images) + shortcut weights [cout][sc_cin] | B | A
+    // SE scales | SC: shortcut bias images (as the bias images) + shortcut weights [cout][sc_cin] | totals tiles | B | A
     static constexpr int kOnesBytes = 2 * 128 * 16;
+    // channel totals with transposed ownership (ConvTotals, the TOT kernels): 32-row x 16-channel tiles per epilogue warp,
+    // two (alternating chunks, one warp barrier per chunk) on the latency-bound 64-column epilogue
+    static constexpr int kTotalsTileBytes = 32 * 16 * 2;
+    static constexpr int kTotalsTiles = N_CTA == 64 ? 2 : 1;
     __host__ __device__ static size_t sc_bytes(int cout, int sc_cin) { return SC ? (size_t)cout * 32 + (size_t)cout * sc_cin * 2 : 0; }
-    static size_t fixed_bytes(int cout, int bias_mma, int b_stages, int tps, int scale_bytes = 0, int sc_cin = 0) {
+    __host__ __device__ static constexpr size_t totals_bytes(bool tot) { return tot ? (size_t)8 * kTotalsTiles * kTotalsTileBytes : 0; }
+    static size_t fixed_bytes(int cout, int bias_mma, int b_stages, int tps, int scale_bytes = 0, int sc_cin = 0, bool tot = false) {
         return kConvCtrlBytes + (size_t)cout * 4 + kOnesBytes + (bias_mma ? (size_t)cout * 32 : 0) + scale_bytes +
-               sc_bytes(cout, sc_cin) + (size_t)b_stages * tps * kBStageBytes;
+               sc_bytes(cout, sc_cin) + totals_bytes(tot) + (size_t)b_stages * tps * kBStageBytes;
     }
 };
 
-template <int N_CTA, int MT, bool BF16, bool FUSED, bool SC = false>
+// Per-(utterance, channel) totals of the stored outputs on the 64- to 256-channel layers (ConvParams::sums): the integers
+// plane_sum_kernel adds (2^-15 fixed point), so the result is bit-identical to that pass whatever the tile order, grid, N
+// split or packing.  One accumulator per channel and thread, as on the 32-channel layers, would take 64-256 int64 registers
+// here (168 registers and spills at 64 channels: profiles/r01g_rejected_experiments.txt), so ownership is transposed per
+// epilogue warp: after storing a 16-channel chunk of its 32-row block, the warp also writes the packed words to a 1 KB
+// shared-memory tile and reads it back column-wise.  Lane l owns channel pair p = l & 7 of the chunk and rows 4i + (l >> 3),
+// i < 8 (conflict-free with the half swap below), and adds them to int64 registers that persist across items: acc[sel][k]
+// holds channels (sel * KC + k) * 16 + 2p, + 1.  They reach memory only when the utterance changes and at the end of the
+// CTA's range: two 64-bit shuffle-adds over the four row groups, one atomic per channel.  A block whose valid rows belong to
+// more than one utterance (a few per utterance and level) adds each utterance's rows with atomics directly.
+// The conversion is plane_sum's __float2int_rn(x * 2^15) computed as bits(fma(x, 2^15, 1.5 * 2^23)) - bits(1.5 * 2^23): the
+// FMA rounds x * 2^15 + 1.5 * 2^23 once, to nearest even, and while the result stays in [2^23, 2^24) (|x| < 128) its
+// significand is that integer exactly.  A lane sums its eight rows in 32 bits (< 2^25) and widens once; a lane with any value
+// outside that binade (|x| >= 128, inf, NaN) takes F2I and 64-bit adds for the chunk instead.  NBUF = 2: chunks alternate
+// between two tiles, so the tile of chunk c is rewritten only after the barrier of chunk c + 1, which every lane reaches after
+// its reads of chunk c.
+template <bool BF16, int NSEL, int KC, int NBUF>
+struct ConvTotals {
+    static_assert(NBUF == 1 || NBUF == 2, "one or two tiles per warp");
+    static constexpr float kMagic = 12582912.f;            // 1.5 * 2^23
+    static constexpr uint32_t kMagicBits = 0x4B400000u;
+    long long acc[NSEL][KC][2];
+    int b;               // utterance acc belongs to (warp-uniform), -1 = none yet
+    int row_b;           // utterance of this lane's row of the current block
+    unsigned valid;      // rows of the current block that hold an output
+    bool mixed;          // the current block straddles utterances
+
+    __device__ __forceinline__ void init() {
+        b = -1;
+        mixed = false;
+#pragma unroll
+        for (int s = 0; s < NSEL; ++s)
+#pragma unroll
+            for (int k = 0; k < KC; ++k) acc[s][k][0] = acc[s][k][1] = 0ll;
+    }
+    __device__ __forceinline__ static void fix_add2(uint32_t w, long long& t0, long long& t1) {   // plane_sum_kernel's arithmetic
+        float2 f = unpack2<BF16>(w);
+        if (BF16) { f.x = fminf(fmaxf(f.x, -65504.f), 65504.f); f.y = fminf(fmaxf(f.y, -65504.f), 65504.f); }
+        t0 += (long long)__float2int_rn(f.x * 32768.f);
+        t1 += (long long)__float2int_rn(f.y * 32768.f);
+    }
+    __device__ __forceinline__ void flush(unsigned long long* sums, int cout, int lane) {
+        if (b < 0) return;
+#pragma unroll
+        for (int s = 0; s < NSEL; ++s)
+#pragma unroll
+            for (int k = 0; k < KC; ++k)
+#pragma unroll
+                for (int e = 0; e < 2; ++e) {
+                    long long v = acc[s][k][e];
+                    v += shfl_xor_ll(v, 8);
+                    v += shfl_xor_ll(v, 16);
+                    if (lane < 8 && v != 0ll)
+                        atomicAdd(sums + (size_t)b * cout + (s * KC + k) * 16 + 2 * lane + e, (unsigned long long)v);
+                    acc[s][k][e] = 0ll;
+                }
+    }
+    // once per 32-row block, by the whole warp, before its chunks: the fast path needs every valid row in utterance b
+    __device__ __forceinline__ void begin_block(int bidx, unsigned long long* sums, int cout, int lane) {
+        row_b = bidx;
+        valid = __ballot_sync(0xffffffffu, bidx >= 0);
+        mixed = false;
+        const unsigned other = __ballot_sync(0xffffffffu, bidx >= 0 && bidx != b);
+        if (other != 0u) {
+            const int nb = __shfl_sync(0xffffffffu, bidx, __ffs(other) - 1);
+            if (__ballot_sync(0xffffffffu, bidx >= 0 && bidx != nb) != 0u) {
+                mixed = true;
+            } else {
+                flush(sums, cout, lane);
+                b = nb;
+            }
+        }
+    }
+    // this lane's row (= lane) of the chunk, 16 channels as two packed uint4 (j = 0, 1), zeros for rows without output;
+    // the 16-byte halves of every other group of four rows are swapped so that the column reads hit 32 distinct banks
+    __device__ __forceinline__ static void put(uint4* tile, int lane, int j, const uint4& o) {
+        tile[lane * 2 + (j ^ ((lane >> 2) & 1))] = o;
+    }
+    // after both put()s of a chunk, by the whole warp; sel is warp-uniform, k a compile-time constant after unrolling
+    __device__ __forceinline__ void add_chunk(const uint4* tile, int sel, int k, unsigned long long* sums, int cout, int lane) {
+        __syncwarp();
+        const uint32_t* t = reinterpret_cast<const uint32_t*>(tile);
+        const int p = lane & 7, rg = lane >> 3;
+        uint32_t w[8];
+#pragma unroll
+        for (int i = 0; i < 8; ++i) w[i] = t[(4 * i + rg) * 8 + ((((p >> 2) ^ (i & 1))) << 2) + (p & 3)];
+        if (NBUF == 1) __syncwarp();         // the tile is free for the next chunk
+        if (!mixed) {
+            uint32_t all = 0xffffffffu, any = 0u, s0 = 0u, s1 = 0u;     // the sums wrap; their difference below does not
+#pragma unroll
+            for (int i = 0; i < 8; ++i) {
+                const float2 f = unpack2<BF16>(w[i]);
+                const uint32_t r0 = __float_as_uint(fmaf(f.x, 32768.f, kMagic)), r1 = __float_as_uint(fmaf(f.y, 32768.f, kMagic));
+                all &= r0 & r1;
+                any |= r0 | r1;
+                s0 += r0;
+                s1 += r1;
+            }
+            long long t0, t1;
+            if ((all & 0xFF800000u) == 0x4B000000u && (any & 0xFF800000u) == 0x4B000000u) {   // every result in [2^23, 2^24)
+                t0 = (long long)(int)(s0 - 8u * kMagicBits);
+                t1 = (long long)(int)(s1 - 8u * kMagicBits);
+            } else {
+                t0 = t1 = 0ll;
+#pragma unroll
+                for (int i = 0; i < 8; ++i) fix_add2(w[i], t0, t1);
+            }
+#pragma unroll
+            for (int s = 0; s < NSEL; ++s)
+                if (s == sel) { acc[s][k][0] += t0; acc[s][k][1] += t1; }
+            return;
+        }
+        unsigned left = valid;
+        while (left != 0u) {
+            const int u = __shfl_sync(0xffffffffu, row_b, __ffs(left) - 1);
+            const unsigned m = __ballot_sync(0xffffffffu, row_b == u);
+            left &= ~m;
+            long long t0 = 0ll, t1 = 0ll;
+#pragma unroll
+            for (int i = 0; i < 8; ++i)
+                if ((m >> (4 * i + rg)) & 1u) fix_add2(w[i], t0, t1);
+            t0 += shfl_xor_ll(t0, 8); t0 += shfl_xor_ll(t0, 16);
+            t1 += shfl_xor_ll(t1, 8); t1 += shfl_xor_ll(t1, 16);
+            unsigned long long* dst = sums + (size_t)u * cout + (sel * KC + k) * 16 + 2 * p;
+            if (lane < 8 && t0 != 0ll) atomicAdd(dst, (unsigned long long)t0);
+            if (lane < 8 && t1 != 0ll) atomicAdd(dst + 1, (unsigned long long)t1);
+        }
+    }
+};
+
+// TOT: this instantiation accumulates ConvParams::sums (non-null) with ConvTotals; the others carry none of its code
+template <int N_CTA, int MT, bool BF16, bool FUSED, bool SC = false, bool TOT = false>
 __global__ void __launch_bounds__(kConvThreads, 1) conv_umma_kernel(const ConvParams p) {
     static_assert(!SC || (FUSED && N_CTA <= 64), "the folded shortcut exists for the narrow conv2 epilogue only");
+    static_assert(!TOT || (!FUSED && N_CTA >= 64), "ConvTotals: the unfused 64- and 128-column epilogues");
     using Cfg = ConvCfg<N_CTA, MT, SC>;
     extern __shared__ __align__(128) uint8_t smem[];
     uint64_t* a_full = reinterpret_cast<uint64_t*>(smem);           // [kConvMaxAStages]
@@ -123,7 +261,8 @@ __global__ void __launch_bounds__(kConvThreads, 1) conv_umma_kernel(const ConvPa
     float* scale_s = reinterpret_cast<float*>(biasimg_smem + (p.bias_mma ? (size_t)p.cout * 32 : 0));   // [n_utt][cout] SE scales
     uint8_t* sc_biasimg_smem = reinterpret_cast<uint8_t*>(scale_s) + p.scale_smem_bytes;
     uint8_t* sc_w_smem = sc_biasimg_smem + (size_t)p.cout * 32;
-    uint8_t* b_smem = reinterpret_cast<uint8_t*>(scale_s) + p.scale_smem_bytes + Cfg::sc_bytes(p.cout, p.sc_cin);
+    uint8_t* totals_smem = reinterpret_cast<uint8_t*>(scale_s) + p.scale_smem_bytes + Cfg::sc_bytes(p.cout, p.sc_cin);   // ConvTotals tiles
+    uint8_t* b_smem = totals_smem + Cfg::totals_bytes(TOT);
     const uint32_t b_stage_bytes = (uint32_t)p.tps * Cfg::kBStageBytes;
     uint8_t* a_smem = b_smem + (size_t)p.b_stages * b_stage_bytes;
     const uint32_t a_stage_bytes = (uint32_t)p.rows_pad * (kConvKC / 8) * 16;
@@ -435,12 +574,20 @@ __global__ void __launch_bounds__(kConvThreads, 1) conv_umma_kernel(const ConvPa
                 }
             }
         };
+        // 64 channels: transposed ownership (ConvTotals), one 32-row block per warp and item
+        constexpr bool kTSum = TOT;
+        static_assert(!kTSum || MTH == 1, "ConvTotals takes one 32-row block per warp and item");
+        static_assert(!kTSum || (NCH / 2) % Cfg::kTotalsTiles == 0, "chunks per item: a multiple of the tiles (parity across items)");
+        ConvTotals<BF16, 1, N_CTA / 16, Cfg::kTotalsTiles> tot;
+        uint4* tot_tile = reinterpret_cast<uint4*>(totals_smem + (warp - 4) * Cfg::kTotalsTiles * Cfg::kTotalsTileBytes);
+        if constexpr (kTSum) tot.init();
         for (int item = item_begin; item < item_end; ++item, ++n_done) {
             const int tile = item / n_split;
             const int n_base = (item - tile * n_split) * N_CTA;
             const int buf = (int)(n_done & 1);
             if (kLoadRes) fetch_res(item + 1, bidx_n, rv_n);               // its metadata arrived during the previous item
             fetch_meta(item + 2, bidx_nn, opix_nn);
+            if constexpr (kTSum) tot.begin_block(bidx_c[0], p.sums, p.cout, lane);   // a flush overlaps the MMAs
             mbar_wait(&acc_full[buf], (n_done >> 1) & 1);
             tc_fence_after();
 #pragma unroll
@@ -504,15 +651,19 @@ __global__ void __launch_bounds__(kConvThreads, 1) conv_umma_kernel(const ConvPa
                     }
 #pragma unroll
                     for (int i = 0; i < 16; ++i) v[i] = fmaxf(v[i], v[i] * slope);
+                    auto pack_out = [&](int j) {
+                        uint4 o;
+                        o.x = valid ? pack2<BF16>(v[j * 8 + 0], v[j * 8 + 1]) : 0u;
+                        o.y = valid ? pack2<BF16>(v[j * 8 + 2], v[j * 8 + 3]) : 0u;
+                        o.z = valid ? pack2<BF16>(v[j * 8 + 4], v[j * 8 + 5]) : 0u;
+                        o.w = valid ? pack2<BF16>(v[j * 8 + 6], v[j * 8 + 7]) : 0u;
+                        return o;
+                    };
                     if (opix_c[mt] >= 0) {
                         uint16_t* dst = p.out + (size_t)opix_c[mt] * 8 + (size_t)((n_base + c0) >> 3) * plane8;
 #pragma unroll
                         for (int j = 0; j < 2; ++j) {
-                            uint4 o;
-                            o.x = valid ? pack2<BF16>(v[j * 8 + 0], v[j * 8 + 1]) : 0u;
-                            o.y = valid ? pack2<BF16>(v[j * 8 + 2], v[j * 8 + 3]) : 0u;
-                            o.z = valid ? pack2<BF16>(v[j * 8 + 4], v[j * 8 + 5]) : 0u;
-                            o.w = valid ? pack2<BF16>(v[j * 8 + 6], v[j * 8 + 7]) : 0u;
+                            const uint4 o = pack_out(j);
                             *reinterpret_cast<uint4*>(dst + j * plane8) = o;
                             if (!BF16) track16(o, omax);
                             if constexpr (kCanSum) {
@@ -530,6 +681,13 @@ __global__ void __launch_bounds__(kConvThreads, 1) conv_umma_kernel(const ConvPa
                             }
                         }
                     }
+                    if constexpr (kTSum) {
+                        // without pix_sub every valid row is a stored row; the others put zeros in the tile
+                        uint4* tile = tot_tile + ((cc / 2) % Cfg::kTotalsTiles) * (Cfg::kTotalsTileBytes / 16);
+                        tot.put(tile, lane, 0, pack_out(0));
+                        tot.put(tile, lane, 1, pack_out(1));
+                        tot.add_chunk(tile, 0, cc / 2, p.sums, p.cout, lane);
+                    }
                 }
             }
 #pragma unroll
@@ -543,6 +701,7 @@ __global__ void __launch_bounds__(kConvThreads, 1) conv_umma_kernel(const ConvPa
             }
         }
         if (kCanSum && do_sums) flush_sums();
+        if constexpr (kTSum) tot.flush(p.sums, p.cout, lane);
         if (!BF16 && p.overflow != nullptr && saturated16(omax)) atomicAdd(p.overflow, 1u);
         } else {
         // ---------------------------------------------------------------- epilogue warps (4..11)
@@ -552,6 +711,16 @@ __global__ void __launch_bounds__(kConvThreads, 1) conv_umma_kernel(const ConvPa
         const int mt0 = ((warp - 4) >> 2) * MTH;
         uint32_t n_done = 0;
         uint32_t omax = 0u;                     // fp16 range guard: max |x| of what this thread stored
+        constexpr int NCH = N_CTA / 8;          // 8-channel chunks per pixel in this N slice
+        constexpr int RCH = NCH > 8 ? 8 : NCH;  // chunks per residual prefetch group
+        constexpr int NG = NCH / RCH;           // prefetch groups
+        // channel totals (transposed ownership, ConvTotals): up to two N splits (cout <= 256), acc[ns * NG + g][cc / 2]
+        constexpr bool kTSum = TOT;
+        static_assert(!kTSum || MTH == 1, "ConvTotals takes one 32-row block per warp and item");
+        static_assert(Cfg::kTotalsTiles == 1, "one tile per warp on the 128-column epilogue");
+        ConvTotals<BF16, 2 * NG, RCH / 2, 1> tot;
+        uint4* tot_tile = reinterpret_cast<uint4*>(totals_smem + (warp - 4) * Cfg::kTotalsTileBytes);
+        if constexpr (kTSum) tot.init();
         int tile_next = item_begin / n_split, ns_next = item_begin % n_split;
         for (int item = item_begin; item < item_end; ++item, ++n_done) {
             const int tile = tile_next, ns = ns_next;
@@ -577,10 +746,8 @@ __global__ void __launch_bounds__(kConvThreads, 1) conv_umma_kernel(const ConvPa
             const size_t rplane8 = (size_t)p.res_plane * 8;
             const float slope = p.act_slope;
             constexpr bool fused = FUSED;
-            // Fused SE tail: the residual comes from HBM/L2 (~1 us away).  Fetch it in groups of up to 8 channel chunks per
+            // Fused SE tail: the residual comes from HBM/L2 (~1 us away).  Fetch it in groups of RCH channel chunks per
             // pixel, the first group BEFORE waiting for the accumulator so its latency hides behind the MMAs.
-            constexpr int NCH = N_CTA / 8;                 // 8-channel chunks per pixel in this N slice
-            constexpr int RCH = NCH > 8 ? 8 : NCH;         // chunks per prefetch group
             uint4 rv[MTH][RCH];
             auto fetch_res = [&](int g) {
 #pragma unroll
@@ -594,10 +761,11 @@ __global__ void __launch_bounds__(kConvThreads, 1) conv_umma_kernel(const ConvPa
                     }
             };
             fetch_res(0);
+            if constexpr (kTSum) tot.begin_block(bidx[0], p.sums, p.cout, lane);   // a flush overlaps the MMAs
             mbar_wait(&acc_full[buf], (n_done >> 1) & 1);
             tc_fence_after();
 #pragma unroll 1
-            for (int g = 0; g < NCH / RCH; ++g) {
+            for (int g = 0; g < NG; ++g) {
                 if (g > 0) fetch_res(g);
 #pragma unroll
                 for (int cc = 0; cc < RCH; cc += 2) {
@@ -637,23 +805,34 @@ __global__ void __launch_bounds__(kConvThreads, 1) conv_umma_kernel(const ConvPa
                         }
 #pragma unroll
                         for (int i = 0; i < 16; ++i) v[i] = fmaxf(v[i], v[i] * slope);
+                        auto pack_out = [&](int j) {
+                            uint4 o;
+                            o.x = valid ? pack2<BF16>(v[j * 8 + 0], v[j * 8 + 1]) : 0u;
+                            o.y = valid ? pack2<BF16>(v[j * 8 + 2], v[j * 8 + 3]) : 0u;
+                            o.z = valid ? pack2<BF16>(v[j * 8 + 4], v[j * 8 + 5]) : 0u;
+                            o.w = valid ? pack2<BF16>(v[j * 8 + 6], v[j * 8 + 7]) : 0u;
+                            return o;
+                        };
                         if (optr[mt] != nullptr) {
                             uint16_t* dst = optr[mt] + (size_t)((n_base + c0) >> 3) * plane8;
 #pragma unroll
                             for (int j = 0; j < 2; ++j) {
-                                uint4 o;
-                                o.x = valid ? pack2<BF16>(v[j * 8 + 0], v[j * 8 + 1]) : 0u;
-                                o.y = valid ? pack2<BF16>(v[j * 8 + 2], v[j * 8 + 3]) : 0u;
-                                o.z = valid ? pack2<BF16>(v[j * 8 + 4], v[j * 8 + 5]) : 0u;
-                                o.w = valid ? pack2<BF16>(v[j * 8 + 6], v[j * 8 + 7]) : 0u;
+                                const uint4 o = pack_out(j);
                                 *reinterpret_cast<uint4*>(dst + j * plane8) = o;
                                 if (!BF16) track16(o, omax);
                             }
+                        }
+                        if constexpr (kTSum) {
+                            // without pix_sub every valid row is a stored row; the others put zeros in the tile
+                            tot.put(tot_tile, lane, 0, pack_out(0));
+                            tot.put(tot_tile, lane, 1, pack_out(1));
+                            tot.add_chunk(tot_tile, ns * NG + g, cc / 2, p.sums, p.cout, lane);
                         }
                     }
                 }
             }
         }
+        if constexpr (kTSum) tot.flush(p.sums, p.cout, lane);
         if (!BF16 && p.overflow != nullptr && saturated16(omax)) atomicAdd(p.overflow, 1u);
         }
         tc_fence_before();

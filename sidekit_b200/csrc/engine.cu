@@ -1168,7 +1168,7 @@ static int run_conv(skb_xtractor* h, const ConvW& cw, int kind, const Level& Lg,
     p.se_scale = se_scale;
     p.res = res;
     p.res_plane = Lg.plane;
-    p.sums = (sums != nullptr && cw.ncta == 32 && cw.cout == 32 && se_scale == nullptr) ? sums : nullptr;
+    p.sums = sums;
     p.overflow = (unsigned*)h->ovf.p;
     if (sc) { p.sc_in = sc_in; p.sc_w = sc->w; p.sc_bias = sc->bias; p.sc_cin = sc->cin; }
     return launch_conv_umma(p, cw.ncta, h->m.bf16, st);
@@ -1238,7 +1238,7 @@ static int head_and_logits(skb_xtractor* h, int norm_embedding, float* emb_out, 
     return SKB_OK;
 }
 
-// SKB_NO_FUSED_SUMS=1: keep the separate plane_sum pass on the 32-channel layers (A/B knob)
+// SKB_NO_FUSED_SUMS=1: keep the separate plane_sum pass on every level (A/B knob, test reference)
 static bool no_fused_sums() {
     static int v = -1;
     if (v < 0) {
@@ -1298,14 +1298,15 @@ static int forward_hr34(skb_xtractor* h, const float* wave, int norm_embedding, 
             return SKB_ERR_STATE;
         }
         uint16_t *y1 = buf(level, 2), *scb = buf(level, 4), *nxt = buf(level, cur ^ 1);
-        const bool sums_in_conv1 = bw.conv1.ncta == 32 && bw.conv1.cout == 32 && !no_fused_sums();
+        const bool sums_in_conv1 = conv_sums_supported(bw.conv1.ncta, bw.conv1.cout) && !no_fused_sums();
         const uint16_t* res = x;
         // narrow layers: conv2 computes the 1x1 shortcut itself, in a second TMEM accumulator (no launch, no round trip
         // of the shortcut through HBM); the <128, 2> tiles have no tensor memory left for it
         const bool fold_sc = bw.has_sc && bw.conv2.ncta <= 64 && bw.sc.ncta == bw.conv2.ncta && !unfused_shortcut();
         {
             ProfScope ps(PROF_CONV, st);
-            // 32-channel layers: conv1's epilogue also accumulates the per-utterance channel totals of y1 (no plane_sum pass)
+            // conv1's epilogue also accumulates the per-utterance channel totals of y1 (no plane_sum pass); they are complete
+            // when conv1 is, which every kernel of the SE chain waits for (pdl_wait), and se_fc re-zeroes them for the next block
             SKB_TRY(run_conv(h, bw.conv1, bw.stride == 2 ? 3 : 1, L, x, y1, 1, nullptr, nullptr, nullptr, nullptr, nullptr, st,
                              sums_in_conv1 ? (unsigned long long*)h->sums.p : nullptr));
             if (bw.has_sc && !fold_sc) {
@@ -1321,8 +1322,8 @@ static int forward_hr34(skb_xtractor* h, const float* wave, int norm_embedding, 
             // Measured and rejected in round 2 (profiles/r02_se_merge.txt): border sums + channel totals in one launch, and the FC
             // layers done by the last-arriving partial-mean CTA -- fewer launches, but both variants were slower.
             // Kept from that experiment's lesson -- separate kernels with their own occupancy -- but OVERLAPPED: the border sums
-            // go first and release the channel-total pass as soon as they have seen conv1 complete (faster than one after the
-            // other: profiles/r02u_se_overlap_vs_serial.txt)
+            // go first and release the channel-total pass (when conv1 did not produce the totals) as soon as they have seen
+            // conv1 complete (faster than one after the other: profiles/r02u_se_overlap_vs_serial.txt)
             const PlaneSumArgs totals = {L.p_end, pm + L.o_pix_b, pm + L.o_span};
             SKB_TRY(launch_se_scale(m.bf16, (unsigned long long*)h->sums.p, y1, L.plane, L.G, L.Wp, L.W, d32 + L.o_utt_row0,
                                     d32 + L.o_utt_count, B, bw.C, bw.C, bw.w2t, bw.conv2.bias, bw.se_w1, bw.se_w2,

@@ -220,11 +220,6 @@ __device__ __forceinline__ void fix_add8(const uint4& a, long long (&t)[8]) {
 // 64-bit shuffles in all.  Lane l ends up with the total of value e = 4*b4 + 2*b3 + b2 (bits of l); the result is
 // returned by the lanes with b1 = b0 = 0, i.e. lane 4*e' ... see `sum8_slot`.  __reduce_add_sync (REDUX) measured
 // ~20 cycles per instruction per SM here and made this kernel REDUX-bound on the small levels.
-__device__ __forceinline__ long long shfl_xor_ll(long long v, int off) {
-    const int lo = __shfl_xor_sync(0xffffffffu, (int)(v & 0xffffffffll), off);
-    const int hi = __shfl_xor_sync(0xffffffffu, (int)(v >> 32), off);
-    return ((long long)hi << 32) | (unsigned int)lo;
-}
 __device__ __forceinline__ int sum8_slot(int lane) { return ((lane >> 4) & 1) * 4 + ((lane >> 3) & 1) * 2 + ((lane >> 2) & 1); }
 __device__ __forceinline__ long long warp_sum8_i64(const long long (&t)[8], int lane) {
     long long v[8];

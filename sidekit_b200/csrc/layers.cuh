@@ -77,6 +77,7 @@ int gemm_packed_a(const PackedOp& A, const PackedOp& W, const float* bias, float
 int launch_conv_umma(const ConvParams& p, int n_cta, bool bf16, cudaStream_t st);
 int conv_tile_m(int n_cta);          // output pixels per CTA for a given N_CTA configuration
 int conv_pick_ncta(int cout);        // 32 / 64 / 128
+bool conv_sums_supported(int n_cta, int cout);   // can an unfused conv's epilogue accumulate the SE channel totals (ConvParams::sums)
 
 // frontend.cu
 int frontend_consts_create(FrontendConsts* fc, int n_fft, int win, int hop, int n_mels, int n_out, const float* window,
