@@ -48,6 +48,69 @@ def _align16(x):
     return (x + 15) & ~15
 
 
+def no_frames(kind, info):
+    """True for a FLAC stream whose metadata ends the file: ``decode`` names it ``"<name>: no frames"``."""
+    return kind == "flac" and info.frames_end <= info.frames_begin
+
+
+class Staging:
+    """Host side of one decode call: the native calls' file tables and the files' frame / sample bytes in one pinned
+    buffer, laid out as ``head`` (int64 rows of the caller's own device tables), FLAC table, PCM table, FLAC frame bytes,
+    then each PCM file's sample bytes at a 16-byte boundary.  Files whose ``kind`` is None are left out."""
+
+    def __init__(self, datas, kinds, infos, out_offsets, head=None):
+        head = numpy.zeros((0,), numpy.int64) if head is None else numpy.ascontiguousarray(head, dtype=numpy.int64)
+        self.fl = [i for i, k in enumerate(kinds) if k == "flac"]
+        self.pc = [i for i, k in enumerate(kinds) if k == "pcm"]
+        out_offsets = numpy.asarray(out_offsets, dtype=numpy.int64)
+        fl_bytes = numpy.array([infos[i].frames_end - infos[i].frames_begin for i in self.fl], numpy.int64)
+        pc_bytes = numpy.array([pcm.data_bytes(infos[i]) for i in self.pc], numpy.int64)
+        self.fl_bytes = int(fl_bytes.sum())
+        pc_begin = numpy.zeros(len(self.pc), numpy.int64)
+        o = 0
+        for k, nb in enumerate(pc_bytes.tolist()):
+            pc_begin[k] = o
+            o = _align16(o + nb)
+        fl_table, self.n_slots = flac.table([infos[i] for i in self.fl], numpy.cumsum(fl_bytes) - fl_bytes, out_offsets[self.fl])
+        pc_table, self.n_tiles = pcm.table([infos[i] for i in self.pc], pc_begin, out_offsets[self.pc])
+        self.fl_table_at = head.nbytes
+        self.pc_table_at = self.fl_table_at + fl_table.nbytes
+        self.fl_at = self.pc_table_at + pc_table.nbytes
+        self.pc_at = _align16(self.fl_at + self.fl_bytes)
+        self.host = torch.empty(max(self.pc_at + o, 1), dtype=torch.uint8, pin_memory=True)
+        hv = self.host.numpy()
+        hv[:self.fl_table_at] = head.view(numpy.uint8)
+        hv[self.fl_table_at:self.pc_table_at] = fl_table.view(numpy.uint8).reshape(-1)
+        hv[self.pc_table_at:self.fl_at] = pc_table.view(numpy.uint8).reshape(-1)
+        p = self.fl_at
+        for i, nb in zip(self.fl, fl_bytes.tolist()):
+            hv[p:p + nb] = numpy.frombuffer(datas[i], dtype=numpy.uint8, count=nb, offset=infos[i].frames_begin)
+            p += nb
+        for i, b0, nb in zip(self.pc, pc_begin.tolist(), pc_bytes.tolist()):
+            hv[self.pc_at + b0:self.pc_at + b0 + nb] = numpy.frombuffer(datas[i], dtype=numpy.uint8, count=nb, offset=infos[i].data_begin)
+
+    def launch(self, out, device):
+        """The device side, on the current stream of ``device``: ONE host-to-device copy of the buffer, at most one FLAC and
+        one PCM native call writing ``out`` (float32 CUDA tensor) at the offsets given to the constructor.  Returns
+        ``(staged, status)``: the device copy (its first bytes are ``head``) and the FLAC calls' per-file status (device
+        int32, None without FLAC files), to be read with ``flac_errors`` once the stream has run."""
+        with torch.cuda.device(device):
+            staged = self.host.to(device, non_blocking=True)
+            base = staged.data_ptr()
+            status = None
+            if self.fl:
+                status = flac.launch(device, base + self.fl_at, self.fl_bytes, base + self.fl_table_at, len(self.fl), self.n_slots,
+                                     out.data_ptr())
+            if self.pc:
+                pcm.launch(base + self.pc_at, base + self.pc_table_at, len(self.pc), self.n_tiles, out.data_ptr())
+        return staged, status
+
+    def flac_errors(self, status, names):
+        """``{file index: ValueError}`` for the FLAC files whose status (host int array) is not OK."""
+        return {self.fl[k]: ValueError("corrupt FLAC: " + flac.status_errors([names[self.fl[k]]], status[k:k + 1])[0])
+                for k in numpy.nonzero(status)[0]}
+
+
 def decode(files, device=None, names=None):
     """Decode a batch of audio files (paths or bytes; FLAC, WAV or NIST SPHERE, mixed freely) on ``device`` (default: the
     current CUDA device).  ``names`` (optional) name the files in error messages instead of their paths.
@@ -77,48 +140,15 @@ def decode(files, device=None, names=None):
     for i, (kind, info) in enumerate(zip(kinds, infos)):
         if kind is not None:
             lengths[i], rates[i] = length(kind, info)
-    out_off = numpy.cumsum(lengths) - lengths
-    fl = [i for i, k in enumerate(kinds) if k == "flac" and infos[i].frames_end > infos[i].frames_begin]
-    for i, k in enumerate(kinds):
-        if k == "flac" and i not in fl:
+        if no_frames(kind, info):
             errors[i] = ValueError("%s: no frames" % names[i])
-    pc = [i for i, k in enumerate(kinds) if k == "pcm"]
-    # staging layout: FLAC table, PCM table, FLAC frame bytes, then each PCM file's sample bytes at a 16-byte boundary
-    fl_bytes = numpy.array([infos[i].frames_end - infos[i].frames_begin for i in fl], numpy.int64)
-    pc_bytes = numpy.array([pcm.data_bytes(infos[i]) for i in pc], numpy.int64)
-    fl_table, n_slots = flac.table([infos[i] for i in fl], numpy.cumsum(fl_bytes) - fl_bytes, out_off[fl])
-    pc_begin = numpy.zeros(len(pc), numpy.int64)
-    o = 0
-    for k, nb in enumerate(pc_bytes.tolist()):
-        pc_begin[k] = o
-        o = _align16(o + nb)
-    pc_table, n_tiles = pcm.table([infos[i] for i in pc], pc_begin, out_off[pc])
-    fl_at = fl_table.nbytes + pc_table.nbytes
-    pc_at = _align16(fl_at + int(fl_bytes.sum()))
-    host = torch.empty(max(pc_at + o, 1), dtype=torch.uint8, pin_memory=True)
-    hv = host.numpy()
-    hv[:fl_table.nbytes] = fl_table.view(numpy.uint8).reshape(-1)
-    hv[fl_table.nbytes:fl_at] = pc_table.view(numpy.uint8).reshape(-1)
-    p = fl_at
-    for i in fl:
-        nb = infos[i].frames_end - infos[i].frames_begin
-        hv[p:p + nb] = numpy.frombuffer(datas[i], dtype=numpy.uint8, count=nb, offset=infos[i].frames_begin)
-        p += nb
-    for i, b0, nb in zip(pc, pc_begin.tolist(), pc_bytes.tolist()):
-        hv[pc_at + b0:pc_at + b0 + nb] = numpy.frombuffer(datas[i], dtype=numpy.uint8, count=nb, offset=infos[i].data_begin)
+            kinds[i] = None
+    staging = Staging(datas, kinds, infos, numpy.cumsum(lengths) - lengths)
     with torch.cuda.device(device):
-        staged = host.to(device, non_blocking=True)
-        base = staged.data_ptr()
         out = torch.empty(int(lengths.sum()), dtype=torch.float32, device=device)
-        status = None
-        if fl:
-            status = flac.launch(device, base + fl_at, int(fl_bytes.sum()), base, len(fl), n_slots, out.data_ptr())
-        if pc:
-            pcm.launch(base + pc_at, base + fl_table.nbytes, len(pc), n_tiles, out.data_ptr())
-        if status is not None:
-            st = status.cpu().numpy()
-            for k in numpy.nonzero(st)[0]:
-                errors[fl[k]] = ValueError("corrupt FLAC: " + flac.status_errors([names[fl[k]]], st[k:k + 1])[0])
+    _, status = staging.launch(out, device)
+    if status is not None:
+        errors.update(staging.flac_errors(status.cpu().numpy(), names))
     if errors:
         kinds_of = {type(e) for e in errors.values()}
         raise (NotImplementedError if kinds_of == {NotImplementedError} else ValueError)(

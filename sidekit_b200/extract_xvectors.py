@@ -3,24 +3,27 @@ means) out, with the reference's function names and arguments (``read_wav_scp`` 
 ``load_model`` :74-91, ``main`` :93-173, the argparse block :175-203).
 
 What changes against the reference: the utterances are not pushed through the model one by one (a few hundred small
-launches and a device-to-host copy each) but streamed in windows of ~80 minutes of audio (host memory), and each window
-is embedded in length-bucketed packed batches (``bulk.make_batches`` + ``Xtractor.extract_varlen``), resampled on the
-device where a file's rate differs from the model's (``preprocessor.Resample``); only the batch being embedded is on
-the device, and the ark is written window by window.  The packed engine is exact per utterance, so the vectors are
-those of the one-by-one loop.
+launches and a device-to-host copy each) but streamed in windows of ~80 minutes of audio (host memory) through the
+window pipeline of ``sidekit_b200.corpus``: a background thread reads and parses the next window while the current one
+is on the device; a window's files go to the device in one copy, are decoded (one FLAC and one PCM call) straight into
+their slots of the length-bucketed packed batches (``bulk.make_batches``), files at another rate through one resampling
+call per rate (``preprocessor.Resample``), and are embedded by ``Xtractor.extract_packed`` without a synchronisation
+until the window's rows come back; the ark is written window by window.  The packed engine is exact per utterance, so
+the vectors are those of the one-by-one loop.  Under ``torchrun --nproc-per-node N`` the entries are sharded over the N
+GPUs in contiguous blocks and rank 0 writes the same tables as one process.
 Paths and pipe entries (``cat x.sph |``, ``sph2pipe -f wav x.sph |``) may hold FLAC, WAV or NIST SPHERE in every PCM
-encoding; the entries of a window are read as bytes and decoded on the device in one batched call (``sidekit_b200.audio``).
+encoding (``sidekit_b200.audio``).
 ``--vad`` needs the silero model that the reference fetches with ``torch.hub`` at run time (no network here): it raises.
 Tables are written with ``sidekit_b200.kaldi_io`` in the layout ``kaldiio.WriteHelper('ark,scp:...')`` produces.
 """
+import contextlib
 import os
 import subprocess
 
 import numpy
 import torch
 
-from . import audio, bulk, kaldi_io
-from .nnet.preprocessor import Resample
+from . import audio, bulk, corpus, flac, kaldi_io
 from .nnet.xsets import load_checkpoint
 
 
@@ -35,22 +38,51 @@ def read_wav_scp(wav_scp):
     return utt2wav
 
 
-def _read_entry(wav):
-    """A ``wav.scp`` entry -> ``(name, file bytes, sample_rate, frames)``, undecoded.  A pipe entry's output is checked to be
-    a readable FLAC, WAV or NIST SPHERE stream here, so that a failing command raises ``IOError`` naming it."""
-    wav = " ".join(wav) if not isinstance(wav, str) else wav
-    if wav.strip().endswith("|"):
+def _source(wav):
+    return " ".join(wav) if not isinstance(wav, str) else wav
+
+
+def _is_pipe(wav):
+    return wav.strip().endswith("|")
+
+
+def _read_source(wav):
+    """A ``wav.scp`` entry -> ``(name, bytes)``: the file's bytes, or the standard output of a pipe command (``IOError``
+    naming the entry when the command fails)."""
+    wav = _source(wav)
+    if _is_pipe(wav):
         try:
             with open(os.devnull, "w") as devnull:
-                out = subprocess.Popen(wav.strip()[:-1], stdout=subprocess.PIPE, shell=True, stderr=devnull).communicate()[0]
-            frames, sr = audio.length(*audio.parse(out, wav))
-            return wav, out, sr, frames
+                proc = subprocess.Popen(wav.strip()[:-1], stdout=subprocess.PIPE, shell=True, stderr=devnull)
+                out = proc.communicate()[0]
+            return wav, out
         except Exception as e:
             raise IOError("Error processing wav file: {}\n{}".format(wav, e))
     with open(wav, "rb") as f:
-        data = f.read()
-    frames, sr = audio.length(*audio.parse(data, wav))
-    return wav, data, sr, frames
+        return wav, f.read()
+
+
+def _parse_source(name, data):
+    """``(kind, info)`` of an entry's bytes; a pipe's output that is not a readable FLAC, WAV or NIST SPHERE stream raises
+    ``IOError`` naming the command.  A FLAC stream without frames raises ``ValueError("<name>: no frames")``, as
+    ``audio.decode`` does, whether it came from a path or a pipe."""
+    if _is_pipe(name):
+        try:
+            kind, info = audio.parse(data, name)
+        except Exception as e:
+            raise IOError("Error processing wav file: {}\n{}".format(name, e))
+    else:
+        kind, info = audio.parse(data, name)
+    if audio.no_frames(kind, info):
+        raise ValueError("%s: no frames" % name)
+    return kind, info
+
+
+def _read_entry(wav):
+    """A ``wav.scp`` entry -> ``(name, file bytes, sample_rate, frames)``, undecoded."""
+    name, data = _read_source(wav)
+    frames, sr = audio.length(*_parse_source(name, data))
+    return name, data, sr, frames
 
 
 def prepare(wav):
@@ -69,59 +101,69 @@ def load_model(model_path, device):
 
 @torch.no_grad()
 def main(xtractor, kaldi_wav_scp, out_file, device, vad=False, num_samples_per_window=2000, min_silence_samples=1500,
-         model_sample_rate=16000, out_file_spk="", spk2utt_file="", max_audio_seconds=1200.0, window_audio_seconds=4800.0):
+         model_sample_rate=16000, out_file_spk="", spk2utt_file="", max_audio_seconds=1200.0, window_audio_seconds=4800.0,
+         stats=None):
     """Embed every utterance of ``kaldi_wav_scp`` and write ``<out_file stem>.ark`` + ``out_file`` (scp); with
-    ``out_file_spk`` also the L2-normalised mean x-vector of every speaker of ``spk2utt_file`` (:93-173)."""
+    ``out_file_spk`` also the L2-normalised mean x-vector of every speaker of ``spk2utt_file`` (:93-173).  Returns the
+    (n, E) float32 host tensor of the embeddings in ``wav.scp`` order.
+
+    Under an initialised ``torch.distributed`` process group (one rank per GPU, ``device`` this rank's), the entries are
+    cut into one contiguous block per rank, balanced by file size (``corpus.plan_blocks``); each rank embeds its block,
+    one all-gather brings the rows together, rank 0 writes the tables -- the same bytes a one-process run writes -- and
+    every rank returns the full tensor.  A bad entry on any rank makes every rank raise, naming it.
+    ``stats`` (optional list) receives this rank's per-window timings (``corpus.run_windows``)."""
     if vad:
         raise NotImplementedError("--vad loads snakers4/silero-vad through torch.hub (network); run VAD upstream")
-    device = torch.device(device)
+    device = flac.device_of(device)
     utt2wav = read_wav_scp(kaldi_wav_scp)
+    keys, entries = list(utt2wav.keys()), [_source(w) for w in utt2wav.values()]
     xtractor.eval()
     xtractor.to(device)
-    resamplers = {}
+    E = xtractor.embedding_size
     out_ark = os.path.realpath(os.path.join(os.path.dirname(out_file), os.path.splitext(os.path.basename(out_file))[0])) + ".ark"
-    all_emb = []
 
-    def flush(window, writer):
-        """Decode one window of entries (file bytes) in one call, embed it in length-bucketed packed batches and write its
-        entries in file order.  Only the window's waveforms and the batch being embedded live on the device."""
-        if not window:
-            return
-        out, n, _ = audio.decode([data for _, _, data, _ in window], device, names=[name for _, name, _, _ in window])
-        window = [(key, x, sr) for (key, _, _, sr), x in zip(window, torch.split(out, n.tolist()))]
-        lengths = numpy.array([-(-int(sig.shape[0]) * model_sample_rate // sr) for _, sig, sr in window], dtype=numpy.int64)
+    def prepare(win):
+        """Reading thread: the window's length-sorted packing (largest batch first) and its decode straight into it."""
+        lengths = corpus.model_lengths(win.frames, win.rates, model_sample_rate)
         order = numpy.argsort(lengths, kind="stable")
-        emb = torch.empty((len(window), xtractor.embedding_size), dtype=torch.float32)
-        for batch in reversed(bulk.make_batches(order.tolist(), lengths, max_audio_seconds, sample_rate=model_sample_rate)):
-            waves = []
-            for i in batch:
-                _, sig, sr = window[i]
-                sig = sig.to(device, non_blocking=True)
-                if sr != model_sample_rate:
-                    if sr not in resamplers:
-                        resamplers[sr] = Resample(orig_freq=sr, new_freq=model_sample_rate)
-                    sig = resamplers[sr](sig)
-                waves.append(sig)
-            emb[torch.as_tensor(batch)] = xtractor.extract_varlen(waves).cpu()
-        for (key, _, _), vec in zip(window, emb.numpy()):
-            writer(key, vec[None, :])                      # the reference writes the (1, E) output of the model
-        all_emb.append(emb)
+        batches = list(reversed(bulk.make_batches(order.tolist(), lengths, max_audio_seconds, sample_rate=model_sample_rate)))
+        packed = numpy.array([i for b in batches for i in b], dtype=numpy.int64)
+        slots = numpy.empty_like(lengths)
+        slots[packed] = numpy.cumsum(lengths[packed]) - lengths[packed]
+        with torch.cuda.device(device):
+            win.prepared = (corpus.WindowDecode(win, model_sample_rate, slots, int(lengths.sum())), lengths, batches, packed)
 
-    # The wav.scp is STREAMED in windows of `window_audio_seconds` of audio (host memory; a pipe entry has no length until
-    # it has been read): a corpus of hundreds of hours never sits in memory, and the ark grows window by window in file
-    # order, like the reference's one-file-at-a-time loop.
-    with kaldi_io.ArkScpWriter(out_ark, os.path.realpath(out_file)) as writer:
-        window, window_s = [], 0.0
-        for key, wav in utt2wav.items():
-            name, data, sr, frames = _read_entry(wav)
-            window.append((key, name, data, sr))           # decoded at flush time, with the window's other entries
-            window_s += float(frames) / sr
-            if window_s >= window_audio_seconds:
-                flush(window, writer)
-                window, window_s = [], 0.0
-        flush(window, writer)
-    emb = torch.cat(all_emb) if all_emb else torch.empty((0, xtractor.embedding_size), dtype=torch.float32)
-    if out_file_spk:
+    def embed(win):
+        dec, lengths, batches, packed = win.prepared
+        wave, _, status = dec.launch(device)
+        emb = torch.empty((len(win), E), dtype=torch.float32, device=device)
+        corpus.extract_batches(xtractor, wave, lengths, batches, emb)
+
+        def finish():
+            corpus.check_window(xtractor, dec, status, win.names)
+            rows = torch.empty((len(win), E), dtype=torch.float32)
+            rows[torch.from_numpy(packed)] = emb.cpu()
+            return rows
+        return finish
+
+    _, rank, _ = bulk._dist()
+    # The wav.scp is STREAMED in windows of `window_audio_seconds` of audio (host memory): a corpus of hundreds of hours
+    # never sits in memory, and rank 0 writes the ark window by window in file order, like the reference's
+    # one-file-at-a-time loop; the rows of the other ranks' blocks follow after the gather.
+    with contextlib.ExitStack() as stack:
+        writer = stack.enter_context(kaldi_io.ArkScpWriter(out_ark, os.path.realpath(out_file))) if rank == 0 else None
+
+        def emit(index, rows):
+            if writer is not None:
+                for i, vec in zip(index, rows.numpy()):
+                    writer(keys[i], vec[None, :])               # the reference writes the (1, E) output of the model
+        with torch.cuda.device(device):
+            emb, blocks = corpus.extract_sharded(entries, corpus.entry_weights([None if _is_pipe(e) else e for e in entries]),
+                                                 _read_source, embed, E, window_audio_seconds, prepare, emit, _parse_source, device,
+                                                 stats)
+        if writer is not None:
+            emit(range(blocks[0][1], len(keys)), emb[blocks[0][1]:])
+    if out_file_spk and rank == 0:
         spk2utt = {}
         with open(spk2utt_file) as f:
             for line in f:
@@ -152,6 +194,14 @@ if __name__ == "__main__":
     if args.out_spk_scp:
         assert os.path.isdir(os.path.dirname(args.out_spk_scp)), "NO SUCH DIRECTORY: %s" % args.out_spk_scp
         assert os.path.isfile(args.spk2utt_file), "NO SUCH FILE: %s" % args.spk2utt_file
-    model, _ = load_model(args.model, args.device.strip().lower())
-    main(model, args.wav_scp, args.out_scp, args.device, args.vad, args.vad_num_samples_per_window, args.vad_min_silence_samples,
+    device = args.device.strip().lower()
+    if "LOCAL_RANK" in os.environ:           # under torchrun: one rank per GPU, NCCL from the environment
+        import torch.distributed as dist
+        device = "cuda:%d" % int(os.environ["LOCAL_RANK"])
+        torch.cuda.set_device(device)
+        dist.init_process_group("nccl", device_id=torch.device(device))
+    model, _ = load_model(args.model, device)
+    main(model, args.wav_scp, args.out_scp, device, args.vad, args.vad_num_samples_per_window, args.vad_min_silence_samples,
          args.sample_rate, args.out_spk_scp, args.spk2utt_file)
+    if "LOCAL_RANK" in os.environ:
+        dist.destroy_process_group()

@@ -209,13 +209,20 @@ class Resample(torch.nn.Module):
         if out.numel() == 0:
             return out
         meta = numpy.stack([numpy.cumsum(n_in) - n_in, n_in, numpy.cumsum(n_out) - n_out, n_out], axis=1)
-        bank, start = self._device_bank(wave.device)
         with torch.cuda.device(wave.device):
             meta_dev = torch.from_numpy(meta).pin_memory().to(wave.device, non_blocking=True)
-            _lib.check(_lib.lib().skb_resample(wave.data_ptr(), meta_dev.data_ptr(), len(n_in), int(n_out.max()), orig_r, new_r,
-                                               width, bank.data_ptr(), start.data_ptr(), bank.shape[0], out.data_ptr(),
-                                               _lib.stream_ptr()))
+            self.launch(wave, meta_dev, out, int(n_out.max()))
         return out
+
+    def launch(self, src, meta_dev, dst, max_out):
+        """One ``skb_resample`` call on the current stream: row ``i`` of ``meta_dev`` (int64 CUDA tensor (n, 4), n <= 65535)
+        resamples ``src[in_off : in_off + in_len]`` into ``dst[out_off : out_off + out_len]`` (``in_off, in_len, out_off,
+        out_len``).  ``src`` and ``dst`` may be the same tensor when the rows' input and output ranges do not overlap."""
+        from .. import _lib
+        orig_r, new_r, width = self._bank[:3]
+        bank, start = self._device_bank(dst.device)
+        _lib.check(_lib.lib().skb_resample(src.data_ptr(), meta_dev.data_ptr(), int(meta_dev.shape[0]), int(max_out), orig_r, new_r,
+                                           width, bank.data_ptr(), start.data_ptr(), bank.shape[0], dst.data_ptr(), _lib.stream_ptr()))
 
     def forward(self, waveform):
         if self._bank is None:

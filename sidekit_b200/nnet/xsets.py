@@ -4,13 +4,13 @@ sidekit/nnet/xvector.py:1796-1916).
 
 What changes against the reference: a single 16- or 32-bit PCM wav file is read with the standard library
 (``torchaudio.load`` needs torchcodec), other audio is decoded on the device; and instead of one ``forward`` per file --
-a few hundred small launches and a device-to-host sync each -- ALL segments / sliding windows of the id map are cut on the host, length-bucketed and pushed through
-``Xtractor.extract_varlen`` as packed batches (``bulk.make_batches``): the engine's packed layout makes a batch of
+a few hundred small launches and a device-to-host sync each -- the segments / sliding windows are cut on the device, length-bucketed and pushed through
+``Xtractor.extract_packed`` as packed batches (``bulk.make_batches``): the engine's packed layout makes a batch of
 different lengths exact, so the embeddings are the same as the one-by-one loop, bit for bit.  Augmentation
 (``transform_pipeline``) and HDF5 IO are out of scope and raise; files at another sample rate are resampled on the
 device (``preprocessor.Resample``); ``IdMap`` reads / writes the reference's text format.  Files are recognised by their
 content, whatever ``file_extension`` says: FLAC, WAV and NIST SPHERE in every PCM encoding (``sidekit_b200.audio``);
-``extract_embeddings`` decodes every file of the dataset on the device in batched calls.
+``extract_embeddings`` streams the dataset's files through the window pipeline of ``sidekit_b200.corpus``.
 """
 import os
 import wave as _wave
@@ -211,30 +211,6 @@ class IdMapSet:
         return speech, self.idmap.leftids[index], self.idmap.rightids[index], start, stop
 
 
-def _predecode(dataset, device, max_bytes=1 << 28):
-    """Decode every file of ``dataset`` on ``device`` in batched calls of at most ~``max_bytes`` file bytes, and make the
-    dataset read from the decoded waveforms (device tensors) instead of reading file by file.  The float32 waveforms of
-    the whole dataset stay on the device until extraction ends: 4 bytes per sample, about 230 GB per 1000 hours at
-    16 kHz, so an id map larger than device memory allows is to be split (``IdMap.split``) and extracted part by part."""
-    from .. import audio, flac
-    paths = list(dict.fromkeys(dataset._path(i) for i in range(len(dataset))))
-    decoded = {}
-    chunk, size = [], 0
-    for k, path in enumerate(paths):
-        chunk.append(path)
-        size += os.path.getsize(path)
-        if size >= max_bytes or k == len(paths) - 1:
-            out, lengths, rates = audio.decode(chunk, device)
-            for p, x, fs in zip(chunk, torch.split(out, lengths.tolist()), rates.tolist()):
-                decoded[p] = (x, int(fs))
-            chunk, size = [], 0
-
-    def read(path, frame_offset=0, num_frames=-1):
-        x, fs = decoded[path]
-        return flac.slice_samples(x, frame_offset, num_frames), fs
-    dataset._read = read
-
-
 def load_checkpoint(model_path, device, embedding_size=None):
     """Checkpoint file -> ``Xtractor`` in eval mode on ``device``, as ``extract_embeddings`` (xvector.py:1834-1843) and
     ``extract_xvectors.py:load_model`` (:74-91) do it: ``torch.load`` of a dict holding ``speaker_number``,
@@ -252,60 +228,190 @@ def load_checkpoint(model_path, device, embedding_size=None):
     return model.to(device)
 
 
+def _segment(dataset, index, file_len):
+    """``IdMapSet.__getitem__``'s cut of item ``index`` from its file (``file_len`` samples at the model rate):
+    ``(offset, length, start, stop)`` of the segment within the file, ``start`` / ``stop`` as the item returns them."""
+    sr = dataset.sample_rate
+    start = 0 if dataset.idmap.start[index] is None else int(dataset.idmap.start[index] * 0.01 * sr)
+    if dataset.idmap.stop[index] is None:
+        return 0, file_len, start, file_len                       # whole file: NOT cut at `start` (xsets.py:430-435)
+    duration = int(dataset.idmap.stop[index] * 0.01 * sr) - start
+    if duration <= dataset.min_duration * sr:
+        middle = start + duration // 2
+        start = int(max(0, int(middle - (dataset.min_duration * sr / 2))))
+        duration = int(dataset.min_duration * sr)
+    off = min(max(0, start), file_len)                            # read_wav's clamping
+    return off, min(duration, file_len - off), start, start + duration
+
+
+def _windows_of(dataset, seg_len):
+    """(number of sliding windows, window length, shift) of a segment of ``seg_len`` samples (``Tensor.unfold``)."""
+    wl, ws = dataset.window_len, dataset.window_shift
+    if seg_len < wl:
+        raise RuntimeError("maximum size for tensor at dimension 0 is %d but size is %d" % (seg_len, wl))
+    return (seg_len - wl) // ws + 1, wl, ws
+
+
 def extract_embeddings(idmap_name, model_filename, data_root_name, device, batch_size=1, file_extension="wav",
                        transform_pipeline={}, sliding_window=False, win_duration=3., win_shift=1.5, num_thread=1,
-                       sample_rate=16000, mixed_precision=False, norm_embeddings=True, max_audio_seconds=1200.0):
+                       sample_rate=16000, mixed_precision=False, norm_embeddings=True, max_audio_seconds=1200.0,
+                       window_audio_seconds=4800.0):
     """xvector.py:1796-1916: a ``StatServer`` with one embedding per segment (or per sliding window).
 
     ``model_filename`` is an ``Xtractor`` or the path of a checkpoint written by the reference's training loop
     (``speaker_number`` / ``model_archi`` / ``model_state_dict``, xvector.py:1834-1843); ``batch_size``, ``num_thread`` and
     ``mixed_precision`` are accepted and ignored: batches are formed by total audio (``max_audio_seconds``) and the
-    kernels pick their own precision.  Every file is decoded on the device first, and the waveforms of the whole id map
-    stay there until the embeddings are done (4 bytes per sample): split a very large id map (``IdMap.split``).  ``start`` / ``stop`` follow the reference, including its sliding-window
-    ``stop = start + <number of 100-window chunks of the last file>`` (xvector.py:1897, :1911).
+    kernels pick their own precision.  ``start`` / ``stop`` follow the reference, including its sliding-window
+    ``stop = start + <number of 100-window chunks of the last segment>`` (xvector.py:1897, :1911).
+
+    The id map's files are streamed through the window pipeline of ``sidekit_b200.corpus`` in windows of
+    ``window_audio_seconds`` of audio: only one window's waveforms are on the device at a time (plus the next window in
+    host memory), so an id map of any size is extracted in one call.  A window's files are decoded on the device in one
+    batched call, resampled to ``sample_rate`` where needed, and its segments / sliding windows are cut from them by one
+    device gather per length-bucketed packed batch.  Under an initialised ``torch.distributed`` process group the
+    files are sharded over the ranks in contiguous blocks balanced by size, each segment goes with its file, and every
+    rank returns the same ``StatServer`` as one process.
     """
-    from .. import bulk
+    from .. import bulk, corpus, flac
     model = model_filename
     if isinstance(model, str):
         model = load_checkpoint(model, device, embedding_size=256)          # xvector.py:1838: the size is forced to 256
     dataset = IdMapSet(idmap_name, data_root_name, file_extension, transform_pipeline, 0, sliding_window, win_duration, win_shift,
                        sample_rate, min_duration=win_duration)
     model.eval()
+    device = flac.device_of(device)
     model.to(device)
-    _predecode(dataset, device)
-    waves, modelset, segset, starts, stops = [], [], [], [], []
+    E = model.embedding_size
+    n_seg = len(dataset)
+    paths = [dataset._path(i) for i in range(n_seg)]
+    files = list(dict.fromkeys(paths))
+    file_of = {p: k for k, p in enumerate(files)}
+    segs_of = [[] for _ in files]
+    for i, p in enumerate(paths):
+        segs_of[file_of[p]].append(i)
+    dist, rank, world = bulk._dist()
+    blocks = corpus.plan_blocks(corpus.entry_weights(files), world)
+    lo, hi = blocks[rank]
+    seg_len = {}                                   # this rank's segments -> length at the model rate
+
+    def prepare(win):
+        """Reading thread: files at the model rate back to back in window order, then the segments / sliding windows
+        (in id-map order) cut from them into length-sorted packed batches."""
+        flen = corpus.model_lengths(win.frames, win.rates, sample_rate)
+        foff = numpy.cumsum(flen) - flen
+        segs, src, lens = [], [], []
+        for i, k in sorted((i, k) for k, f in enumerate(win.index) for i in segs_of[lo + f]):
+            off, n, _, _ = _segment(dataset, i, int(flen[k]))
+            if dataset.idmap.stop[i] is not None:
+                assert win.rates[k] == sample_rate
+            rows = [(off, n)]
+            if sliding_window:
+                m, wl, ws = _windows_of(dataset, n)
+                rows = [(off + j * ws, wl) for j in range(m)]
+            segs.append((i, n, len(rows)))
+            src.extend(int(foff[k]) + o for o, _ in rows)
+            lens.extend(l for _, l in rows)
+        lens = numpy.array(lens, dtype=numpy.int64)
+        order = numpy.argsort(lens, kind="stable")
+        batches = list(reversed(bulk.make_batches(order.tolist(), lens, max_audio_seconds, sample_rate=sample_rate)))
+        packed = numpy.array([i for b in batches for i in b], dtype=numpy.int64)
+        table = numpy.stack([numpy.array(src, dtype=numpy.int64)[packed], lens[packed]]) if len(packed) else numpy.zeros((2, 0), numpy.int64)
+        with torch.cuda.device(device):
+            dec = corpus.WindowDecode(win, sample_rate, foff, int(flen.sum()), extra=table)
+        win.prepared, win.segs = (dec, lens, batches, packed), segs
+
+    def embed(win):
+        dec, lens, batches, packed = win.prepared
+        buf, table, status = dec.launch(device)
+        emb = torch.empty((len(lens), E), dtype=torch.float32, device=device)
+        if len(lens):
+            with torch.cuda.device(device):
+                src, n = table.view(2, -1)                 # per wave, in packed order: offset in buf, length
+                row = 0
+                for b in batches:
+                    # the batch's waves cut from buf by one gather: its sample t is buf[src of its wave + (t - first sample
+                    # of its wave)]; built batch by batch, the index never outgrows one batch (max_audio_seconds)
+                    k, total = len(b), int(lens[b].sum())
+                    s, m = src[row:row + k], n[row:row + k]
+                    idx = torch.repeat_interleave(s - (torch.cumsum(m, 0) - m), m, output_size=total)
+                    idx += torch.arange(total, device=device)
+                    model.extract_packed(buf[idx], lens[b], norm_embedding=norm_embeddings, out=emb[row:row + k])
+                    row += k
+
+        def finish():
+            corpus.check_window(model, dec, status, win.names)
+            rows = torch.empty((len(lens), E), dtype=torch.float32)
+            rows[torch.from_numpy(packed)] = emb.cpu()
+            return rows
+        return finish
+
+    parts = []
+
+    def emit(win, rows):
+        parts.append((win.segs, rows))
+        for i, n, _ in win.segs:
+            seg_len[i] = n
+
+    error = None
+    with torch.no_grad(), torch.cuda.device(device):
+        try:
+            corpus.run_windows(files[lo:hi], corpus.read_file, window_audio_seconds, embed, emit, prepare)
+        except Exception as e:
+            if dist is None:
+                raise
+            error = e
+        owner = numpy.searchsorted(numpy.array([b for _, b in blocks]), [file_of[p] for p in paths], side="right")
+        return _assemble(dataset, parts, seg_len, error, owner, E, win_shift, device)
+
+
+def _assemble(dataset, parts, seg_len, error, owner, embedding_size, win_shift, device=None):
+    """The ``StatServer`` of ``extract_embeddings`` on every rank from this rank's ``parts`` (``(segments, rows)`` per
+    window: ``(index, length, rows)`` of its segments in id-map order and their rows), ``seg_len`` (its segments' lengths
+    at the model rate) and ``error`` (None, or what stopped its windows); ``owner``: the rank of every segment.
+
+    One small exchange shares the errors and every segment's length, from which every rank knows every segment's row
+    count (sliding windows depend on it) and so where each rank's rows go; then one gather of the rows."""
+    from .. import bulk, corpus
+    dist, rank, world = bulk._dist()
+    n_seg, sliding = len(dataset), dataset.sliding_window
+    lengths = {}
+    for part in corpus.exchange(error, seg_len):
+        lengths.update(part)
+    n_rows = numpy.array([_windows_of(dataset, lengths[i])[0] if sliding else 1 for i in range(n_seg)], dtype=numpy.int64)
+    row0 = numpy.cumsum(n_rows) - n_rows
+    # local rows come window by window; the gather takes this rank's segments in id-map order
+    pieces = {}
+    for segs, rows in parts:
+        r = 0
+        for i, _, m in segs:
+            pieces[i] = rows[r:r + m]
+            r += m
+    local = torch.cat([pieces[i] for i in sorted(pieces)]) if pieces else None
+    if dist is None:
+        emb = local if local is not None else torch.zeros((0, embedding_size), dtype=torch.float32)
+    else:
+        shards = [numpy.concatenate([numpy.arange(row0[i], row0[i] + n_rows[i]) for i in range(n_seg) if owner[i] == r] or
+                                    [numpy.zeros(0, numpy.int64)]).astype(numpy.int64) for r in range(world)]
+        emb = bulk.gather_embeddings(local, shards, embedding_size, device).cpu()
+    sample_rate = dataset.sample_rate
+    modelset, segset, starts, stops = [], [], [], []
     last_chunks = 1
-    for idx in range(len(dataset)):
-        data, mod, seg, start, stop = dataset[idx]
-        if data.dim() == 1:
-            data = data.unsqueeze(0)
-        n = data.shape[0]
-        waves.extend(data[i] for i in range(n))
-        modelset.extend([mod] * n)
-        segset.extend([seg] * n)
-        if sliding_window:
+    for i in range(n_seg):
+        _, _, start, _ = _segment(dataset, i, lengths[i])
+        n = int(n_rows[i])
+        modelset.extend([dataset.idmap.leftids[i]] * n)
+        segset.extend([dataset.idmap.rightids[i]] * n)
+        if sliding:
             starts.extend((numpy.arange(0, n * win_shift, win_shift) * sample_rate + start).tolist())
             last_chunks = len(range(0, n, max(1, n // max(1, n // 100))))          # len(torch.split(...)) of :1885
         else:
             starts.append(start)
-            stops.append(int(data.shape[1]))
-    lengths = numpy.array([int(w.shape[0]) for w in waves], dtype=numpy.int64)
-    order = numpy.argsort(lengths, kind="stable")
-    emb = torch.empty((len(waves), model.embedding_size), dtype=torch.float32)
-    with torch.no_grad():
-        # largest batch first: the engine sizes its work buffers once instead of growing them batch after batch; the
-        # embeddings stay on the device until the end, so the host plans and enqueues batch k+1 while batch k runs
-        outs, index = [], []
-        for batch in reversed(bulk.make_batches(order.tolist(), lengths, max_audio_seconds, sample_rate=sample_rate)):
-            outs.append(model.extract_varlen([waves[i].to(device, non_blocking=True) for i in batch], norm_embedding=norm_embeddings))
-            index.extend(batch)
-        if outs:
-            emb[torch.as_tensor(index)] = torch.cat(outs).cpu()
+            stops.append(lengths[i])
     embeddings = StatServer()
     embeddings.stat1 = emb.numpy().astype(numpy.float32)
     embeddings.modelset = numpy.array(modelset).astype('>U')
     embeddings.segset = numpy.array(segset).astype('>U')
     embeddings.start = numpy.array(starts).squeeze()
-    embeddings.stop = embeddings.start + (last_chunks if sliding_window else numpy.array(stops).squeeze())
+    embeddings.stop = embeddings.start + (last_chunks if sliding else numpy.array(stops).squeeze())
     embeddings.stat0 = numpy.ones((embeddings.modelset.shape[0], 1))
     return embeddings

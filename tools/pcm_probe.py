@@ -4,10 +4,9 @@
 (a) device time of skb_pcm_decode on the staged batch (CUDA events over repeated calls, after warm-up; min / median / max
     over windows), and the kernel's row in torch.profiler (a separate pass);
 (b) bytes copied to the device per batch: the sample bytes against the float32 samples of a host decode;
-(c) wall time of extract_embeddings over the 16-bit WAV files (HalfResNet34): the host path (read_wav per file, forced by
-    turning the device predecode off) against the device predecode, alternated, median of several calls per round;
-    embeddings compared bit for bit.  Then a breakdown of one device-path call: reading the files, the decode call, and
-    the rest (Python and extraction).
+(c) wall time of extract_embeddings over the 16-bit WAV files (HalfResNet34), median of several calls per round, with
+    the embeddings compared bit for bit against read_wav + extract_varlen.  Then a breakdown of one call: reading the
+    files, a batched decode call over them, and the rest (Python and extraction).
 Prints the card's name and power limit first.  Usage: python tools/pcm_probe.py [--out FILE]."""
 import argparse
 import os
@@ -107,9 +106,8 @@ for label, datas in batches.items():
     emit("(b) host-to-device bytes per batch: samples %.2f MB (+ table %.1f kB) against %.2f MB as float32 (ratio %.3f)"
          % (blob.nbytes / 1e6, tab.nbytes / 1e3, n.sum() * 4 / 1e6, blob.nbytes / (n.sum() * 4)))
 
-# (c) extract_embeddings from 16-bit WAV: host read_wav per file against the device predecode
+# (c) extract_embeddings from 16-bit WAV (the streamed window pipeline), checked against read_wav + extract_varlen
 m = make_xtractor("halfresnet34", 32, 256).cuda()
-predecode = xsets._predecode
 with tempfile.TemporaryDirectory() as d:
     for i, data in enumerate(batches["16 kHz 16-bit WAV"]):
         with open(os.path.join(d, "u%d.wav" % i), "wb") as f:
@@ -120,30 +118,25 @@ with tempfile.TemporaryDirectory() as d:
     im.start = numpy.empty(len(files16), "|O")
     im.stop = numpy.empty(len(files16), "|O")
 
-    def run(path):
-        # the host arm reads each file with read_wav, as extract_embeddings did before the device predecode
-        xsets._predecode = predecode if path == "device" else (lambda dataset, device: setattr(dataset, "_read", xsets.read_wav))
+    def run():
         torch.cuda.synchronize()
         t0 = time.perf_counter()
         ss = sk.nnet.extract_embeddings(im, m, d, torch.device("cuda"))
         torch.cuda.synchronize()
         return time.perf_counter() - t0, ss.stat1
 
-    run("host"), run("device")                                       # warm-up: every batch geometry, the page cache
-    res = {"host": [], "device": []}
-    emb = {}
+    run()                                                            # warm-up: every batch geometry, the page cache
+    res, emb = [], None
     for _ in range(args.rounds):
-        for path in ("host", "device"):
-            ts = []
-            for _ in range(3):
-                t, emb[path] = run(path)
-                ts.append(t)
-            res[path].append(sorted(ts)[1])
-    xsets._predecode = predecode
-    assert numpy.array_equal(emb["host"], emb["device"]), "host and device embeddings differ"
-    emit("(c) extract_embeddings wall time over %.1f audio-s of 16-bit WAV (median of 3 per round, %d alternating rounds): "
-         "host read_wav %s s, device predecode %s s; embeddings bit-identical"
-         % (total / 16000, args.rounds, " / ".join("%.3f" % t for t in res["host"]), " / ".join("%.3f" % t for t in res["device"])))
+        ts = []
+        for _ in range(3):
+            t, emb = run()
+            ts.append(t)
+        res.append(sorted(ts)[1])
+    ref = m.extract_varlen([xsets.read_wav(os.path.join(d, "u%d.wav" % i))[0].cuda() for i in range(len(files16))]).cpu().numpy()
+    assert numpy.array_equal(emb, ref), "extract_embeddings differs from read_wav + extract_varlen"
+    emit("(c) extract_embeddings wall time over %.1f audio-s of 16-bit WAV (median of 3 per round, %d rounds): %s s; "
+         "embeddings bit-identical to read_wav + extract_varlen" % (total / 16000, args.rounds, " / ".join("%.3f" % t for t in res)))
     paths = [os.path.join(d, "u%d.wav" % i) for i in range(len(files16))]
     tr, td = [], []
     for _ in range(5):
@@ -157,7 +150,7 @@ with tempfile.TemporaryDirectory() as d:
         audio.decode(paths, torch.device("cuda"))
         torch.cuda.synchronize()
         td.append(time.perf_counter() - t0)
-    t_read, t_dec, t_all = sorted(tr)[2], sorted(td)[2], sorted(res["device"])[len(res["device"]) // 2]
+    t_read, t_dec, t_all = sorted(tr)[2], sorted(td)[2], sorted(res)[len(res) // 2]
     emit("    device path breakdown (medians): reading the 130 files %.1f ms (%.0f %%), the whole decode call incl. that "
          "read, parse, staging and copy %.1f ms (%.0f %%), Python and extraction %.1f ms (%.0f %%) of %.1f ms"
          % (t_read * 1e3, 100 * t_read / t_all, t_dec * 1e3, 100 * t_dec / t_all, (t_all - t_dec) * 1e3,
